@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the geodesic-guidance hot path (BASELINE.json metric: geodesic maps/s).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -11,8 +11,8 @@ reference's own (cal_geodesic_vectorize takes a batch of scenes): --batch B scen
 calls, replayed as CUDA graphs on two alternating streams (the FPS / graph construction of one batch runs under
 the propagation of the previous one).
   value     whole-job maps/s with the scenes already resident in HBM: EXACTLY K steps between two CUDA events,
-            barrier + synchronize on both sides, max over ranks; the K-step region is repeated (--repeats) and the
-            MEDIAN region is reported, all regions listed in `repeats_ms`
+            barrier + synchronize on both sides, max over ranks; --repeats R times the K-step region R times and
+            reports the MEDIAN region, all regions listed in `repeats_ms`
   e2e       the same through the host-buffer C-ABI call gf_guidance_host: pinned host points in,
             seeds + maps back in pinned host memory, copies inside the timed region
   roofline  the propagation kernel (geo_bfs_batch_kernel, one launch per batch): algorithmic bytes of SURVEY 8(d)
@@ -22,6 +22,9 @@ the propagation of the previous one).
   cpu_baseline  the CPU oracle port (oracle/) on this box's host cores, bounded sample (N=1 only)
 --impl reference times that CPU port as the reference arm on all host cores (the reference's own torch code
 cannot travel to the GPU box and its kNN is faiss-gpu, absent everywhere; see DESIGN.md).
+--dump-outputs DIR writes what the last timed step returned (the seeds and the maps of one scene) as .npy files, so
+that two builds can be compared output for output: the scenes are generated from fixed seeds, so the same arguments
+give the same inputs on every run.
 """
 import argparse
 import ctypes
@@ -50,7 +53,8 @@ def parse_args():
     ap.add_argument("--workload", default="c2", choices=["c1", "c2", "c4"])
     ap.add_argument("--max-step", type=int, default=None, help="override the workload's level bound")
     ap.add_argument("--batch", type=int, default=20, help="scenes per library call (reduced to a divisor of --steps)")
-    ap.add_argument("--repeats", type=int, default=0, help="repetitions of the K-step timed region (0 = automatic)")
+    ap.add_argument("--repeats", type=int, default=1,
+                    help="repetitions of the K-step timed region, median reported (0 = automatic, 5 to 21)")
     ap.add_argument("--runners", type=int, default=2, help="batches in flight (alternating CUDA streams)")
     ap.add_argument("--no-graph", action="store_true", help="plain launches instead of CUDA-graph replay")
     ap.add_argument("--seed-sharded", default=None, choices=["shard", "nccl", "fused"],
@@ -61,7 +65,12 @@ def parse_args():
     ap.add_argument("--e2e-batch", type=int, default=4, help="scenes per host-buffer call")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip epilogues / eval setting / model setting records")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the seeds and geodesic maps of the last timed step to DIR/*.npy (default arm only)")
+    args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.seed_sharded):
+        ap.error("--dump-outputs needs the default arm (--impl ours, no --seed-sharded)")
+    return args
 
 
 def workload(args):
@@ -361,7 +370,7 @@ def run_seed_sharded(args):
     os.environ.setdefault("MASTER_PORT", "29511")
     dist.init_process_group("nccl", rank=rank, world_size=world, device_id=dev)
     cfg = workload(args)
-    K = min(args.steps, 32)
+    K = args.steps
     sampler = ClockSampler(local)
     sampler.start()
     rec = seed_sharded_record(cfg, args.seed_sharded, K, dist, dev, rank, world)
@@ -385,6 +394,25 @@ def pick_batch(K, want):
         if K % b == 0:
             return b
     return 1
+
+
+DUMP_MAX_VALUES = 8 << 20  # 32 MB of f32 maps per dump
+
+
+def dump_outputs(out_dir, seeds, geo):
+    """seeds.npy (Q,) f64 and geo.npy (Q, M) f32: all N columns of the (Q, N) maps when Q*N <= DUMP_MAX_VALUES, else
+    M = DUMP_MAX_VALUES // Q columns drawn with a fixed seed; geo_columns.npy (M,) f64 lists which."""
+    import numpy as np
+    import torch
+
+    Q, N = geo.shape
+    cols = np.arange(N)
+    if Q * N > DUMP_MAX_VALUES:
+        cols = np.sort(np.random.default_rng(0).choice(N, DUMP_MAX_VALUES // Q, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "seeds.npy"), seeds.cpu().numpy().astype(np.float64))
+    np.save(os.path.join(out_dir, "geo.npy"), geo[:, torch.from_numpy(cols).to(geo.device)].cpu().numpy())
+    np.save(os.path.join(out_dir, "geo_columns.npy"), cols.astype(np.float64))
 
 
 def run_ours(args):
@@ -498,6 +526,9 @@ def run_ours(args):
         host_reps.append(host_ms)
         prop_in_region += prop
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:  # the last step: the last scene of the last call
+        last = runners[(calls - 1) % n_run]
+        dump_outputs(args.dump_outputs, *((last.seeds[-1], last.geo[-1]) if batched else (last.seeds, last.geo)))
     if dist is not None:
         t = torch.tensor(reps, device=dev)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)  # per repetition: the slowest rank

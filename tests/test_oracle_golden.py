@@ -218,27 +218,6 @@ def test_bias_oracle_matches_reference_lines_fixture():
         assert np.array_equal(out.numpy(), g["d%d_out" % i], equal_nan=True), i
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/model/geoformer/geoformer_fs.py"),
-                    reason="the reference tree only exists in the build container")
-def test_bias_fixture_is_what_the_reference_lines_produce_today():
-    """regenerates the fixture's outputs from the reference source in this container (guards against a stale file)"""
-    import torch
-
-    from oracle import ref_bias
-
-    g, T = _bias_golden()
-    mask_fn, _ = ref_bias.load_mask_heads_forward()
-    dec_fn, _ = ref_bias.load_decoder_relative_pos()
-    for i in range(int(g["n_mask"])):
-        out = mask_fn(T(g["m%d_geo" % i]), T(g["m%d_coords" % i]), T(g["m%d_seed_xyz" % i]))
-        assert np.array_equal(out.numpy(), g["m%d_out" % i], equal_nan=True)
-    for i in range(int(g["n_dec"])):
-        B = int(g["d%d_B" % i])
-        out = dec_fn([T(g["d%d_geo%d" % (i, b)]) for b in range(B)], T(g["d%d_inds" % i]), T(g["d%d_qry" % i]),
-                     T(g["d%d_ctx" % i]))
-        assert np.array_equal(out.numpy(), g["d%d_out" % i], equal_nan=True)
-
-
 def test_attention_oracle_matches_reference_layer_fixture():
     """oracle/attention.py against tests/golden/attention_golden.npz = what the reference's OWN
     TransformerDecoderLayer.forward_pre_rel computes in its cross-attention block (transformer_detr.py:443-454),
