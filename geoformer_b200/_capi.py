@@ -53,6 +53,13 @@ SIGNATURES = {
     "gf_rel_cross_attention": (c_int, [_P, _P, _P, c_int, c_int, c_int, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, c_size_t, _P]),
     "gf_rel_cross_attention_fused": (c_int, [_P, _P, _P, _P, _P, _P, _P, _P, c_int, _P, _P, c_int, c_int, c_int,
                                              _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, c_size_t, _P]),
+    "gf_rel_cross_attention_save": (c_int, [_P, _P, _P, c_int, c_int, c_int] + [_P] * 12 + [c_size_t, _P]),
+    "gf_rel_cross_attention_fused_save": (c_int, [_P] * 8 + [c_int, _P, _P, c_int, c_int, c_int] + [_P] * 12
+                                          + [c_size_t, _P]),
+    "gf_rel_cross_attention_backward_workspace_bytes": (c_size_t, [c_int, c_int, c_int]),
+    "gf_rel_cross_attention_backward": (c_int, [_P, _P, _P, c_int, c_int, c_int] + [_P] * 24 + [c_size_t, _P]),
+    "gf_rel_cross_attention_fused_backward": (c_int, [_P] * 8 + [c_int, _P, _P, c_int, c_int, c_int] + [_P] * 23
+                                              + [c_size_t, _P]),
     "gf_group_mlp_pool": (c_int, [_P, _P, _P, _P, c_int, c_int, c_int, c_int, c_int, c_float, c_int, c_int, c_int, _P, _P,
                                   _P, _P, c_int, _P, _P]),
     "gf_guidance_workspace_bytes": (c_size_t, [c_int, c_int, c_int]),

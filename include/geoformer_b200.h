@@ -158,6 +158,45 @@ int gf_rel_cross_attention_fused(const float *tgt2, const float *memory, const f
                                  const float *wv, const float *bv, const float *wo, const float *bo, float *out,
                                  void *workspace, size_t workspace_bytes, void *stream);
 
+/* Training.  The _save variants are the forwards above that also write what the backward needs: o (Q,B,64), the
+ * softmax-weighted sum before out_mlp, and lse (Q,B,64) = max + log(sum) of the scores sim / 8; `out` is bitwise the
+ * same as without saving.  The _backward entries take the forward's inputs, out, o, lse and the upstream gradient
+ * dy (Q,B,64) and write the gradients of tgt2, memory, the eight weights and (unfused, when drel is not NULL)
+ * relative_pos, all f32 device, same shapes as the inputs.  They recompute the scores tile by tile on the tensor
+ * cores (TF32, like the forward) and reduce in a fixed order without atomics: two calls give bitwise-equal
+ * gradients.  db2 is exactly zero (the softmax is shift invariant per channel).  The fused backward takes the
+ * embedding ingredients as data: no gradient for the maps, locations or gauss_B.  The workspace holds a
+ * (Q,B,C,128) buffer: gf_rel_cross_attention_backward_workspace_bytes.                                        */
+int gf_rel_cross_attention_save(const float *tgt2, const float *memory, const float *relative_pos, int Q, int C,
+                                int B, const float *w1, const float *b1, const float *w2, const float *b2,
+                                const float *wv, const float *bv, const float *wo, const float *bo, float *out,
+                                float *o, float *lse, void *workspace, size_t workspace_bytes, void *stream);
+int gf_rel_cross_attention_fused_save(const float *tgt2, const float *memory, const float *const *geo_ptrs,
+                                      const int *geo_ld, const int *ctx_idx, const float *query_xyz,
+                                      const float *ctx_xyz, const float *gauss_B, int gauss_ld, const float *pc_min,
+                                      const float *pc_max, int Q, int C, int B, const float *w1, const float *b1,
+                                      const float *w2, const float *b2, const float *wv, const float *bv,
+                                      const float *wo, const float *bo, float *out, float *o, float *lse,
+                                      void *workspace, size_t workspace_bytes, void *stream);
+size_t gf_rel_cross_attention_backward_workspace_bytes(int Q, int C, int B);
+int gf_rel_cross_attention_backward(const float *tgt2, const float *memory, const float *relative_pos, int Q, int C,
+                                    int B, const float *w1, const float *b1, const float *w2, const float *b2,
+                                    const float *wv, const float *bv, const float *wo, const float *bo,
+                                    const float *out, const float *o, const float *lse, const float *dy, float *dtgt2,
+                                    float *dmemory, float *drel, float *dw1, float *db1, float *dw2, float *db2,
+                                    float *dwv, float *dbv, float *dwo, float *dbo, void *workspace,
+                                    size_t workspace_bytes, void *stream);
+int gf_rel_cross_attention_fused_backward(const float *tgt2, const float *memory, const float *const *geo_ptrs,
+                                          const int *geo_ld, const int *ctx_idx, const float *query_xyz,
+                                          const float *ctx_xyz, const float *gauss_B, int gauss_ld,
+                                          const float *pc_min, const float *pc_max, int Q, int C, int B,
+                                          const float *w1, const float *b1, const float *w2, const float *b2,
+                                          const float *wv, const float *bv, const float *wo, const float *bo,
+                                          const float *out, const float *o, const float *lse, const float *dy,
+                                          float *dtgt2, float *dmemory, float *dw1, float *db1, float *dw2,
+                                          float *db2, float *dwv, float *dbv, float *dwo, float *dbo,
+                                          void *workspace, size_t workspace_bytes, void *stream);
+
 /* ---- set_aggregator.mlp fused with its grouping (SURVEY 8(f) rank 3) --------------------------------------------
  * lib/pointnet2/pointnet2_modules.py:200-249 + QueryAndGroup.forward (pointnet2_utils.py:303-356) + SharedMLP
  * (pytorch_utils.py:9-32): per centre j and ball-query neighbour s the input [(xyz[idx] - new_xyz[j]) / radius |
