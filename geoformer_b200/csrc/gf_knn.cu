@@ -269,16 +269,6 @@ struct TopK {
   __device__ __forceinline__ void offer(float d2, int index) {
     unsigned long long kk = ((unsigned long long)__float_as_uint(d2) << 32) | (unsigned)index;
     if (kk < key[KT - 1]) {
-#ifdef KNN_SERIAL_INSERT
-      key[KT - 1] = kk;
-#pragma unroll
-      for (int i = KT - 1; i > 0; --i) {
-        unsigned long long a = key[i - 1], b = key[i];
-        bool sw = b < a;
-        key[i - 1] = sw ? b : a;
-        key[i] = sw ? a : b;
-      }
-#else
       // every slot decides for itself (no compare-exchange chain through the moving key): slot i takes its lower
       // neighbour if the new key sorts below that one, the new key if it sorts below the slot's own key, else it
       // keeps what it has; top down, so a slot's lower neighbour is still the old one when it is read
@@ -290,7 +280,6 @@ struct TopK {
         below = below_prev;
       }
       if (below) key[0] = kk;
-#endif
     }
   }
   __device__ __forceinline__ void offer_key(unsigned long long kk) {
@@ -372,8 +361,24 @@ struct TopK {
 };
 
 // ---- grid query ---------------------------------------------------------------------------------
+// Thread per query, count then collect.  Offering every candidate to the sorted list as it is scanned makes the
+// warp run the insertion at almost every candidate: a lane inserts at ~k (1 + ln(n/k)) of its n candidates, and the
+// 32 lanes insert at different ones.  Here the first shell (R <= 1: the 27 cells around the query's cell, nine
+// contiguous runs of `sorted`) is walked twice instead:
+//   count    each candidate's d2 goes to one of KNN_NB bins (a function of d2 that never decreases) in a per-lane
+//            histogram in shared memory; nothing is inserted;
+//   collect  the second walk recomputes d2 with the same expression and lists the positions of the candidates whose
+//            bin is at most b, the smallest bin with at least k candidates at or below it (every bin if the shell
+//            has fewer than k);
+//   insert   the listed candidates go through the unchanged TopK, ~k + 2 per lane, so most lanes insert together.
+// At least k keys have bin <= b and a key of a higher bin is larger than all of them, so the k smallest (d2, index)
+// keys of the shell are among the listed ones (keys tied at the threshold are all listed) and TopK orders them as
+// before: the result is bit-identical to offering every candidate.  A lane whose list overflows (duplicates,
+// lattices) offers every candidate of the shell instead.  Shells R >= 2 (after the unchanged termination test) offer
+// every candidate to a top-k that is already exact for the first shell, so few of them insert.
+constexpr int KNN_NB = 32;  // bins of d2 over [0, 4 h^2); the last one also takes everything beyond and NaN
 #ifndef KNN_MIN_BLOCKS
-#define KNN_MIN_BLOCKS 7  // 72 registers for k <= 16 (a few spilled words): measured 1 % ahead of 80 registers / 6 blocks per SM
+#define KNN_MIN_BLOCKS 7  // 72 registers for k <= 16, 24 KB of shared memory per block
 #endif
 template <int KT>
 __global__ void __launch_bounds__(128, KT <= 16 ? KNN_MIN_BLOCKS : 1)
@@ -381,8 +386,13 @@ __global__ void __launch_bounds__(128, KT <= 16 ? KNN_MIN_BLOCKS : 1)
                           const int *__restrict__ start, const float *__restrict__ queries, int nq, int k,
                           int do_sqrt, float *__restrict__ dist, long long *__restrict__ idx64,
                           int *__restrict__ idx32, const KnnEdgeOut eo) {
+  // counted on the c2 scene: a lane lists ~k + 2 candidates, at most k + 10 (k = 8, 16, 32)
+  constexpr int LIST = KT + 16;
+  __shared__ unsigned short hist[KNN_NB][128];  // per-lane counts (a shell of more than 65535 points is not binned)
+  __shared__ int list[LIST][128];               // per-lane positions in `sorted` of the collected candidates
   const KnnGrid g = *gp;
-  const int s = blockIdx.x * blockDim.x + threadIdx.x;
+  const int tid = threadIdx.x;
+  const int s = blockIdx.x * blockDim.x + tid;
   if (s >= nq) return;
   if (eo.tgt && s == 0) {  // the sentinel row N: only edges to N
     const int none = eo.rank ? (int)((((unsigned)nq >> 5) << 7) | ((unsigned)nq & 31u)) : nq;
@@ -403,73 +413,38 @@ __global__ void __launch_bounds__(128, KT <= 16 ? KNN_MIN_BLOCKS : 1)
             cz = cell_coord(qz, g.oz, g.inv_h, g.dz);
   TopK<KT> top;
   top.init(k);
-  const int rmax = max(g.dx, max(g.dy, g.dz));
-#ifndef KNN_PLAIN_ROW_ORDER
-  // distances from the query to the faces of its own cell: lower bounds for everything beyond them
-  const float gzl = qz - (g.oz + (float)cz * g.h), gzh = (g.oz + (float)(cz + 1) * g.h) - qz;
-  const float gyl = qy - (g.oy + (float)cy * g.h), gyh = (g.oy + (float)(cy + 1) * g.h) - qy;
-#endif
-  for (int R = 0; R <= rmax; ++R) {
-    const int xl = cx - R, xr = cx + R;
-    const int side = 2 * R + 1, nrows = side * side;
-    for (int ri = 0; ri < nrows; ++ri) {
-      // rows (dz, dy) of the shell.  R = 1 (where nearly all the work is): nearest rows first -- the row of the
-      // query's own cells, the four rows sharing a face with it, the four diagonal ones -- so that the k-th key is
-      // tight before the far cells are scanned, and a row whose slab lies beyond the current k-th distance is skipped.
-      int dz, dy;
-#ifndef KNN_PLAIN_ROW_ORDER
-      if (R == 1) {
-        // ri: 0 -> (0,0); 1..4 -> (0,-1) (0,1) (-1,0) (1,0); 5..8 -> (-1,-1) (-1,1) (1,-1) (1,1)
-        dz = (int)((0x28215u >> (2 * ri)) & 3u) - 1;  // 2-bit codes of dz + 1, ri = 0 in the low bits
-        dy = (int)((0x22161u >> (2 * ri)) & 3u) - 1;
-      } else
-#endif
-      {
-        dz = ri / side - R, dy = ri % side - R;
-      }
-      const int z = cz + dz, y = cy + dy;
-      if (z < 0 || z >= g.dz || y < 0 || y >= g.dy) continue;
-#ifndef KNN_PLAIN_ROW_ORDER
-      if (R == 1) {  // every point of the row is at least (gap_z, gap_y) away from the query
-        const float gz = dz < 0 ? gzl : (dz > 0 ? gzh : 0.f), gy = dy < 0 ? gyl : (dy > 0 ? gyh : 0.f);
-        const float bz = fmaxf(gz - g.slack, 0.f), by = fmaxf(gy - g.slack, 0.f);
-        if (bz * bz + by * by > top.kth_d2()) continue;  // (trimming the row's end cells as well: no further gain)
-      }
-#endif
-      const bool face = dz == -R || dz == R || dy == -R || dy == R;
-      const int rowbase = (z * g.dy + y) * g.dx;
-      // on a face of the shell the whole x-run belongs to it; otherwise only its two end cells
-      const int nseg = (face || R == 0) ? 1 : 2;
-      for (int sgi = 0; sgi < nseg; ++sgi) {
-        int xa, xb;
-        if (nseg == 1) {
-          xa = max(xl, 0), xb = min(xr, g.dx - 1);
-        } else {
-          xa = xb = sgi == 0 ? xl : xr;
-          if (xa < 0 || xa >= g.dx) continue;
-        }
-        if (xa > xb) continue;
-        const int p0 = __ldg(start + rowbase + xa), p1 = __ldg(start + rowbase + xb + 1);
-        int p = p0;
-        for (; p + 4 <= p1; p += 4) {  // four candidates in flight: the loads and distances overlap the offers
-          const float4 c0 = __ldg(sorted + p), c1 = __ldg(sorted + p + 1), c2 = __ldg(sorted + p + 2),
-                       c3 = __ldg(sorted + p + 3);
-          const float e0 = sq3(c0.x - qx, c0.y - qy, c0.z - qz), e1 = sq3(c1.x - qx, c1.y - qy, c1.z - qz),
-                      e2 = sq3(c2.x - qx, c2.y - qy, c2.z - qz), e3 = sq3(c3.x - qx, c3.y - qy, c3.z - qz);
-          top.offer(e0, __float_as_int(c0.w));
-          top.offer(e1, __float_as_int(c1.w));
-          top.offer(e2, __float_as_int(c2.w));
-          top.offer(e3, __float_as_int(c3.w));
-        }
-        for (; p < p1; ++p) {
-          float4 c = __ldg(sorted + p);
-          float d2 = sq3(c.x - qx, c.y - qy, c.z - qz);
-          top.offer(d2, __float_as_int(c.w));
-        }
-      }
+  auto offer_run = [&](int p, int p1) {
+    for (; p + 4 <= p1; p += 4) {  // four candidates in flight: the loads and distances overlap the offers
+      const float4 c0 = __ldg(sorted + p), c1 = __ldg(sorted + p + 1), c2 = __ldg(sorted + p + 2),
+                   c3 = __ldg(sorted + p + 3);
+      const float e0 = sq3(c0.x - qx, c0.y - qy, c0.z - qz), e1 = sq3(c1.x - qx, c1.y - qy, c1.z - qz),
+                  e2 = sq3(c2.x - qx, c2.y - qy, c2.z - qz), e3 = sq3(c3.x - qx, c3.y - qy, c3.z - qz);
+      top.offer(e0, __float_as_int(c0.w));
+      top.offer(e1, __float_as_int(c1.w));
+      top.offer(e2, __float_as_int(c2.w));
+      top.offer(e3, __float_as_int(c3.w));
     }
-    // distance from the query to the nearest face of the visited block that still has cells
-    // behind it; every unvisited point is at least that far away (minus the fp32 slack)
+    for (; p < p1; ++p) {
+      const float4 c = __ldg(sorted + p);
+      top.offer(sq3(c.x - qx, c.y - qy, c.z - qz), __float_as_int(c.w));
+    }
+  };
+  // run r (0..8) of the first shell: row (dz, dy) = (r / 3 - 1, r % 3 - 1), cells cx - 1 .. cx + 1 of the row
+  auto first_run = [&](int r, int &p0, int &p1) {
+    const int z = cz + r / 3 - 1, y = cy + r % 3 - 1;
+    p0 = p1 = 0;
+    if (z < 0 || z >= g.dz || y < 0 || y >= g.dy) return;
+    const int rowbase = (z * g.dy + y) * g.dx;
+    p0 = __ldg(start + rowbase + max(cx - 1, 0)), p1 = __ldg(start + rowbase + min(cx + 1, g.dx - 1) + 1);
+  };
+  const float bin_scale = (float)KNN_NB * 0.25f * g.inv_h * g.inv_h;
+  auto bin_of = [&](float d2) {
+    const float t = d2 * bin_scale;
+    return t < (float)(KNN_NB - 1) ? (int)t : KNN_NB - 1;  // NaN -> the last bin (NaN keys sort above +inf)
+  };
+  // distance from the query to the nearest face of the visited block that still has cells behind it; every
+  // unvisited point is at least that far away (minus the fp32 slack)
+  auto shells_done = [&](int R) {
     float mfd = __int_as_float(0x7f800000);
     if (cx - R > 0) mfd = fminf(mfd, qx - (g.ox + (float)(cx - R) * g.h));
     if (cx + R + 1 < g.dx) mfd = fminf(mfd, (g.ox + (float)(cx + R + 1) * g.h) - qx);
@@ -477,9 +452,98 @@ __global__ void __launch_bounds__(128, KT <= 16 ? KNN_MIN_BLOCKS : 1)
     if (cy + R + 1 < g.dy) mfd = fminf(mfd, (g.oy + (float)(cy + R + 1) * g.h) - qy);
     if (cz - R > 0) mfd = fminf(mfd, qz - (g.oz + (float)(cz - R) * g.h));
     if (cz + R + 1 < g.dz) mfd = fminf(mfd, (g.oz + (float)(cz + R + 1) * g.h) - qz);
-    if (mfd == __int_as_float(0x7f800000)) break;  // the whole grid has been visited
-    float ms = mfd - g.slack;
-    if (ms > 0.f && top.kth_d2() < ms * ms) break;
+    if (mfd == __int_as_float(0x7f800000)) return true;  // the whole grid has been visited
+    const float ms = mfd - g.slack;
+    return ms > 0.f && top.kth_d2() < ms * ms;
+  };
+
+  // first shell, count
+#pragma unroll
+  for (int j = 0; j < KNN_NB; ++j) hist[j][tid] = 0;
+  int ntot = 0;
+  for (int r = 0; r < 9; ++r) {
+    int p, p1;
+    first_run(r, p, p1);
+    ntot += p1 - p;
+    for (; p + 4 <= p1; p += 4) {
+      const float4 c0 = __ldg(sorted + p), c1 = __ldg(sorted + p + 1), c2 = __ldg(sorted + p + 2),
+                   c3 = __ldg(sorted + p + 3);
+      const int b0 = bin_of(sq3(c0.x - qx, c0.y - qy, c0.z - qz)), b1 = bin_of(sq3(c1.x - qx, c1.y - qy, c1.z - qz)),
+                b2 = bin_of(sq3(c2.x - qx, c2.y - qy, c2.z - qz)), b3 = bin_of(sq3(c3.x - qx, c3.y - qy, c3.z - qz));
+      ++hist[b0][tid], ++hist[b1][tid], ++hist[b2][tid], ++hist[b3][tid];
+    }
+    for (; p < p1; ++p) {
+      const float4 c = __ldg(sorted + p);
+      ++hist[bin_of(sq3(c.x - qx, c.y - qy, c.z - qz))][tid];
+    }
+  }
+  bool listed = false;
+  if (ntot <= 0xffff) {
+    // threshold: b = the number of bins below KNN_NB - 1 whose cumulative count is still short of k
+    int b = 0, cum = 0;
+#pragma unroll
+    for (int j = 0; j < KNN_NB - 1; ++j) {
+      cum += hist[j][tid];
+      b += cum < k;
+    }
+    // collect
+    int n = 0;
+    for (int r = 0; r < 9; ++r) {
+      int p, p1;
+      first_run(r, p, p1);
+      for (; p < p1; ++p) {
+        const float4 c = __ldg(sorted + p);
+        if (bin_of(sq3(c.x - qx, c.y - qy, c.z - qz)) <= b) {
+          if (n < LIST) list[n][tid] = p;
+          ++n;
+        }
+      }
+    }
+    // insert
+    if (n <= LIST) {
+      listed = true;
+      for (int i = 0; i < n; ++i) {
+        const float4 c = __ldg(sorted + list[i][tid]);
+        top.offer(sq3(c.x - qx, c.y - qy, c.z - qz), __float_as_int(c.w));
+      }
+    }
+  }
+  if (!listed) {
+    for (int r = 0; r < 9; ++r) {
+      int p, p1;
+      first_run(r, p, p1);
+      offer_run(p, p1);
+    }
+  }
+
+  // shells R >= 2: every candidate is offered
+  const int rmax = max(g.dx, max(g.dy, g.dz));
+  if (!shells_done(1)) {
+    for (int R = 2; R <= rmax; ++R) {
+      const int xl = cx - R, xr = cx + R;
+      const int side = 2 * R + 1, nrows = side * side;
+      for (int ri = 0; ri < nrows; ++ri) {
+        const int dz = ri / side - R, dy = ri % side - R;
+        const int z = cz + dz, y = cy + dy;
+        if (z < 0 || z >= g.dz || y < 0 || y >= g.dy) continue;
+        const bool face = dz == -R || dz == R || dy == -R || dy == R;
+        const int rowbase = (z * g.dy + y) * g.dx;
+        // on a face of the shell the whole x-run belongs to it; otherwise only its two end cells
+        const int nseg = face ? 1 : 2;
+        for (int sgi = 0; sgi < nseg; ++sgi) {
+          int xa, xb;
+          if (nseg == 1) {
+            xa = max(xl, 0), xb = min(xr, g.dx - 1);
+          } else {
+            xa = xb = sgi == 0 ? xl : xr;
+            if (xa < 0 || xa >= g.dx) continue;
+          }
+          if (xa > xb) continue;
+          offer_run(__ldg(start + rowbase + xa), __ldg(start + rowbase + xb + 1));
+        }
+      }
+      if (shells_done(R)) break;
+    }
   }
   if (dist || idx64 || idx32)
     top.store(k, do_sqrt != 0, dist ? dist + (size_t)row * k : nullptr, idx64 ? idx64 + (size_t)row * k : nullptr,
@@ -490,22 +554,17 @@ __global__ void __launch_bounds__(128, KT <= 16 ? KNN_MIN_BLOCKS : 1)
   }
 }
 
-// ---- grid query, warp-synchronous insertion --------------------------------------------------------
-// The kernel above spends its instructions on DIVERGENT insertions: a lane inserts at ~56 of its ~195 candidates
-// (k (1 + ln(n/k))), but the 32 lanes of a warp insert at different candidates, so the warp executes the
-// insertion network at nearly every candidate (12 of 32 lanes active on average).  Here a candidate that beats the
-// lane's current k-th key is only PUSHED onto a small per-lane stack in shared memory; the warp runs the
-// insertion network when some lane's stack is nearly full, and then every lane with a pending key inserts one
-// (LIFO: the order of insertions does not change the final set, keys are distinct; a key that no longer beats
-// the k-th is dropped at the pop).  ~85 executions of the network per warp instead of ~200, each at ~25 lanes.
+// ---- grid query, warp-synchronous insertion (k = 64) ------------------------------------------------
+// Offering every candidate as it is scanned, the 32 lanes of a warp insert at different candidates, so the warp
+// executes the insertion network at nearly every candidate.  Here a candidate that beats the lane's current k-th key
+// is only PUSHED onto a small per-lane stack in shared memory; the warp runs the insertion network when some lane's
+// stack is nearly full, and then every lane with a pending key inserts one (LIFO: the order of insertions does not
+// change the final set, keys are distinct; a key that no longer beats the k-th is dropped at the pop).
 // Control flow is warp-uniform (votes), every lane walks its own sequence of candidate ranges and never idles
 // before its shell is exhausted; the per-shell termination test is unchanged (after draining the stacks).
 constexpr int KNN_PEND = 8;  // stack depth; a step pushes at most 4, the network runs while a stack holds > 4
-#ifndef KNN_SYNC_MIN_BLOCKS
-#define KNN_SYNC_MIN_BLOCKS 1
-#endif
 template <int KT>
-__global__ void __launch_bounds__(128, KT <= 16 ? KNN_SYNC_MIN_BLOCKS : 1)
+__global__ void __launch_bounds__(128, 1)
     knn_grid_query_sync_kernel(const KnnGrid *__restrict__ gp, const float4 *__restrict__ sorted,
                                const int *__restrict__ start, const float *__restrict__ queries, int nq, int k,
                                int do_sqrt, float *__restrict__ dist, long long *__restrict__ idx64,
@@ -684,16 +743,9 @@ template <int KT>
 static void launch_grid_query(const KnnGrid *g, const float4 *sorted, const int *start, const float *queries, int nq,
                               int k, int do_sqrt, float *dist, long long *i64, int *i32, const KnnEdgeOut &eo,
                               cudaStream_t st) {
-  // GF_KNN_SYNC=0|1 forces one kernel for every k.  Measured (c2, B200): the two execute the same number of warp
-  // instructions at k = 16 (the saved insertions are spent on votes and the divergent range walk) and the
-  // synchronous one is 10 % slower alone, 1 % slower in the batched pipeline; at k = 64, where an insertion is 64
-  // compare-exchanges, it is 10-16 % faster.
-  static const int force = [] {
-    const char *e = getenv("GF_KNN_SYNC");
-    return e ? (e[0] == '0' ? 0 : 1) : -1;
-  }();
-  const bool sync = force >= 0 ? force == 1 : KT > 32;
-  if (sync)
+  // Measured (c2, B200): at k <= 32 the count-then-collect kernel; at k = 64, where an insertion is 64
+  // compare-exchanges, the warp-synchronous one (10-16 % faster than offering every candidate).
+  if constexpr (KT > 32)
     knn_grid_query_sync_kernel<KT><<<(nq + 127) / 128, 128, 0, st>>>(g, sorted, start, queries, nq, k, do_sqrt, dist, i64,
                                                                      i32, eo);
   else
