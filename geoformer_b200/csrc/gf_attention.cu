@@ -21,7 +21,7 @@
 //     either loaded from the (Q,C,B,64) tensor or -- fused with the decoder epilogue a10 -- computed on the fly
 //     from the geodesic maps, so that it never exists in memory).
 // tcgen05.mma is issued by one thread; completion is signalled through an mbarrier by tcgen05.commit.
-#include "gf_common.cuh"
+#include "gf_umma.cuh"
 
 namespace gf {
 
@@ -58,31 +58,8 @@ struct AttArgs {
   float *o_save, *lse_save;          // SAVE: (Q, B, 64) weighted sum before out_mlp and max + log(sum) of the scores
 };
 
-__device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-// K-major tile with 128-byte swizzle, `rows` rows: row r, fp32 column k (0..63) -> byte offset inside the tile
-template <int ROWS>
-__device__ __forceinline__ uint32_t sw128_off(int r, int k) {
-  const int half = k >> 5, kk = k & 31;
-  return (uint32_t)(half * (ROWS * 128) + r * 128 + ((((kk >> 2) ^ (r & 7)) << 4) | ((kk & 3) << 2)));
-}
-
-// shared-memory matrix descriptor: K-major, SWIZZLE_128B, 8-row groups 1024 bytes apart (cute::UMMA::SmemDescriptor)
-__device__ __forceinline__ uint64_t umma_desc(uint32_t saddr) {
-  return (uint64_t)((saddr & 0x3FFFFu) >> 4) | (1ull << 16) | (64ull << 32) | (1ull << 46) | (2ull << 61);
-}
-
-// instruction descriptor (cute::UMMA::InstrDescriptor): D = F32, A = B = TF32, both K-major, M = 128, N = 64
-constexpr uint32_t ATT_IDESC = (1u << 4) | (2u << 7) | (2u << 10) | ((ATT_TILE >> 3) << 17) | ((128u >> 4) << 24);
-
-__device__ __forceinline__ void umma_tf32(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}"
-      :
-      : "r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(ATT_IDESC), "r"(accumulate)
-      : "memory");
-}
+// instruction descriptor: M = 128, N = 64
+constexpr uint32_t ATT_IDESC = umma_idesc_tf32(128, ATT_TILE);
 
 // D (128 x 64, TMEM) (+)= A (128 x 64) * B^T (64 x 64): eight K = 8 steps, 32 bytes apart inside a swizzled row, the
 // second half of K in the second half-tile (A_HALF bytes further for A: the A tile may be 128 rows of a taller region)
@@ -91,44 +68,13 @@ __device__ __forceinline__ void umma_k64(uint32_t d_tmem, uint32_t a_saddr, uint
 #pragma unroll
   for (int kk = 0; kk < 8; ++kk) {
     const uint32_t ka = (uint32_t)((kk >> 2) * A_HALF + (kk & 3) * 32), kb = (uint32_t)((kk >> 2) * ATT_T_HALF + (kk & 3) * 32);
-    umma_tf32(d_tmem, umma_desc(a_saddr + ka), umma_desc(b_saddr + kb), accumulate || kk > 0);
+    umma_tf32<ATT_IDESC>(d_tmem, umma_desc(a_saddr + ka), umma_desc(b_saddr + kb), accumulate || kk > 0);
   }
-}
-
-// the completion of every tcgen05.mma this thread issued so far arrives on `mbar`
-__device__ __forceinline__ void umma_commit(uint32_t mbar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(mbar) : "memory");
 }
 
 __device__ __forceinline__ void umma_tile(uint32_t d_tmem, uint32_t a_saddr, uint32_t b_saddr, uint32_t mbar) {
   umma_k64<ATT_W_HALF>(d_tmem, a_saddr, b_saddr, false);
   umma_commit(mbar);
-}
-
-__device__ __forceinline__ void mbar_wait(uint32_t mbar, uint32_t parity) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "W: mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-      "@!p bra W;\n\t}"
-      :
-      : "r"(mbar), "r"(parity)
-      : "memory");
-}
-
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, float (&v)[32]) {
-  uint32_t r[32];
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-      "{%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]),
-        "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]),
-        "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-      : "r"(taddr)
-      : "memory");
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-  for (int i = 0; i < 32; ++i) v[i] = __uint_as_float(r[i]);
 }
 
 // The embedding tile of one (query, batch element), row = context, column = channel, in two steps, so that its global

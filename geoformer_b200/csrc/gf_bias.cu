@@ -5,7 +5,7 @@
 // so each is two kernels: a row-max reduction (with an ordered-int atomicMax for the global
 // maximum) and a fused element-wise pass that writes the reference's output layout directly
 // (no (Q,N,3) boolean-mask temporaries as in the reference).
-#include "gf_common.cuh"
+#include "gf_bias.cuh"
 
 namespace gf {
 
@@ -160,13 +160,6 @@ __global__ void __launch_bounds__(256)
   }
 }
 
-__device__ __forceinline__ float mask_push(float d, float s, bool unreached) {
-  // d + sqrt(rowmax) * sign(d) where the point is unreachable (:284-286); torch.sign: 0 -> 0, NaN -> NaN
-  if (!unreached) return d;
-  const float sg = d > 0.f ? 1.f : (d < 0.f ? -1.f : d);
-  return __fadd_rn(d, __fmul_rn(s, sg));
-}
-
 // row maxima handed over by the producer of the maps (gf_geodesic / gf_guidance `row_max`): no pass over geo.
 // One block: it also initialises the global maximum, so nothing has to be zeroed beforehand.
 __global__ void __launch_bounds__(1024)
@@ -245,6 +238,30 @@ int bias_ctx_rowmax(const float *const *geo_ptrs, const int *geo_ld, const int *
                                                            rowmax + (size_t)b * Q, gmax);
     GF_LAUNCHED();
   }
+  return GF_OK;
+}
+
+// ordered-uint row maxima of the (Q,N) maps and their global maximum (geoformer_fs.py:274-276), or the producer's
+// row_max imported; nothing has to be zeroed beforehand.  Shared with the fused mask head (gf_mask_head.cu).
+int bias_mask_rowmax(const float *geo, int Q, int N, const float *row_max, bool vec, uint32_t *rowmax, uint32_t *gmax,
+                     cudaStream_t st) {
+  if (!row_max) {
+    GF_CUDA(cudaMemsetAsync(rowmax, 0, sizeof(uint32_t) * (size_t)Q, st));
+    bias_init_kernel<<<1, 1, 0, st>>>(gmax);
+    GF_LAUNCHED();
+  }
+  const int work = vec ? N / 4 : N;
+  int chunks = (num_sms() * 8 + Q - 1) / Q;
+  if (chunks < 1) chunks = 1;
+  if (chunks > (work + 1023) / 1024) chunks = (work + 1023) / 1024;
+  if (chunks < 1) chunks = 1;
+  if (row_max)
+    bias_rowmax_import_kernel<<<1, 1024, 0, st>>>(row_max, Q, rowmax, gmax);
+  else if (vec)
+    bias_mask_rowmax_kernel<true><<<Q * chunks, 256, 0, st>>>(geo, N, chunks, rowmax, gmax);
+  else
+    bias_mask_rowmax_kernel<false><<<Q * chunks, 256, 0, st>>>(geo, N, chunks, rowmax, gmax);
+  GF_LAUNCHED();
   return GF_OK;
 }
 
@@ -342,25 +359,11 @@ extern "C" int gf_bias_mask_head(const float *geo, const float *coords, const fl
     return GF_ERR_WORKSPACE;
   }
   cudaStream_t st = (cudaStream_t)stream;
-  if (!row_max) {
-    GF_CUDA(cudaMemsetAsync(rowmax, 0, sizeof(uint32_t) * (size_t)Q, st));
-    bias_init_kernel<<<1, 1, 0, st>>>(gmax);
-    GF_LAUNCHED();
-  }
   // 16-byte path: N a multiple of 4 and all bases 16-byte aligned (torch allocations are)
   const bool vec = (N % 4 == 0) && ((((uintptr_t)geo | (uintptr_t)coords | (uintptr_t)out) & 15) == 0);
   const int work = vec ? N / 4 : N;
-  int chunks = (num_sms() * 8 + Q - 1) / Q;
-  if (chunks < 1) chunks = 1;
-  if (chunks > (work + 1023) / 1024) chunks = (work + 1023) / 1024;
-  if (chunks < 1) chunks = 1;
-  if (row_max)
-    bias_rowmax_import_kernel<<<1, 1024, 0, st>>>(row_max, Q, rowmax, gmax);
-  else if (vec)
-    bias_mask_rowmax_kernel<true><<<Q * chunks, 256, 0, st>>>(geo, N, chunks, rowmax, gmax);
-  else
-    bias_mask_rowmax_kernel<false><<<Q * chunks, 256, 0, st>>>(geo, N, chunks, rowmax, gmax);
-  GF_LAUNCHED();
+  const int rc = bias_mask_rowmax(geo, Q, N, row_max, vec, rowmax, gmax, st);
+  if (rc != GF_OK) return rc;
   int gx = (work + 255) / 256;
   int cap = (num_sms() * 16 + Q - 1) / Q;
   if (cap < 1) cap = 1;

@@ -10,7 +10,7 @@ exist in this image).  What runs is the real chain
 
 Every piece of the hot path has two implementations selected by `impl`:
     "b200"   the library: fused aggregator, batched geodesic guidance, fused cross-attention (embedding never
-             materialised), mask-head epilogue kernel
+             materialised), fused mask head (relative coordinates + both dynamic convolutions in one kernel)
     "torch"  the reference's formulation with plain torch ops on the same device (group -> conv/bn/relu -> pool; the
              level loop of cal_geodesic_vectorize is NOT rerun in torch: the maps are shared, they are bit-exact
              anyway; relative_pos materialised; three (Q,C,B,64) temporaries; boolean-mask indexing in the mask head)
@@ -27,7 +27,7 @@ import torch.nn.functional as F
 
 from . import aggregate as agg
 from . import attention as att
-from . import bias as gbias
+from . import mask_head as mh
 from .geodesic_utils import cal_geodesic_vectorize
 from .pointnet2 import _ext
 
@@ -162,11 +162,12 @@ class FewShotForward(nn.Module):
             weights = [w0.reshape(Qn * m, -1, 1), w1.reshape(Qn, -1, 1)]
             biases = [b0.reshape(Qn * m), b1.reshape(Qn)]
             feats_b = mask_features[b]  # (N, m)
-            if impl == "b200":
-                rel = gbias.mask_head_relative_coords(geo_dists[b], locs[b].contiguous(), query_locs[b].contiguous(),
-                                                      row_max=row_max[b] if row_max is not None else None)  # (Q,3,N)
-            else:
-                rel = torch_mask_head_relative_coords(geo_dists[b], locs[b], query_locs[b])
+            if impl == "b200":  # :263-300 in one kernel: no (Q, >1, N) temporary
+                out.append(mh.mask_heads_forward(geo_dists[b], feats_b, weights, biases, Qn, locs[b].contiguous(),
+                                                 query_locs[b].contiguous(),
+                                                 row_max=row_max[b] if row_max is not None else None))
+                continue
+            rel = torch_mask_head_relative_coords(geo_dists[b], locs[b], query_locs[b])
             x = feats_b.t()[None].repeat(Qn, 1, 1)  # :269
             x = torch.cat([rel, x], dim=1).reshape(1, -1, feats_b.shape[0])  # :291-293
             for i, (w, bb) in enumerate(zip(weights, biases)):

@@ -197,6 +197,30 @@ int gf_rel_cross_attention_fused_backward(const float *tgt2, const float *memory
                                           float *db2, float *dwv, float *dbv, float *dwo, float *dbo,
                                           void *workspace, size_t workspace_bytes, void *stream);
 
+/* ---- mask head fused (geoformer_fs.py:263-300, mask_heads_forward) ---------------------------------------------
+ * One scene: geo (Q,N) maps, feats (N,m) mask features, the dynamic weights w0 (Q*m, m+3), b0 (Q*m), w1 (Q, m),
+ * b1 (Q) as the controller's parameter split gives them, coords (N,3), seed_xyz (Q,3) and optionally row_max (Q)
+ * (the producer's row maxima, as gf_bias_mask_head takes them; NULL: computed from geo) -> out (Q,N) logits
+ *     rel = gf_bias_mask_head's (Q,3,N) output, x = [rel | feats^T] (the order of the reference's cat),
+ *     h = relu(w0 x + b0) per query, out = w1 h + b1.
+ * Only m = 16.  The feature part of w0 x runs on the tensor cores (TF32, fp32 accumulation); the coordinate part,
+ * the unreachable decisions and the second layer are fp32 on the CUDA cores.  Nothing of size (Q, >1, N) is
+ * written.  Workspace: gf_mask_head_workspace_bytes.
+ * The backward takes the same inputs and dlogit (Q,N) and writes the gradients of feats (N,m), w0 (Q*m, m+3),
+ * b0 (Q*m), w1 (Q,m) and b1 (Q).  It recomputes h with the forward's products (bit-identical ReLU masks) and sums
+ * in a fixed order without atomics: two calls give bitwise-equal gradients.  The maps and coordinates are data (no
+ * gradient).  Workspace: gf_mask_head_backward_workspace_bytes.                                                  */
+size_t gf_mask_head_workspace_bytes(int Q, int N);
+int gf_mask_head_logits(const float *geo, const float *feats, const float *w0, const float *b0, const float *w1,
+                        const float *b1, const float *coords, const float *seed_xyz, const float *row_max, int Q, int N,
+                        int m, float *out, void *workspace, size_t workspace_bytes, void *stream);
+size_t gf_mask_head_backward_workspace_bytes(int Q, int N);
+int gf_mask_head_logits_backward(const float *geo, const float *feats, const float *w0, const float *b0,
+                                 const float *w1, const float *b1, const float *coords, const float *seed_xyz,
+                                 const float *row_max, int Q, int N, int m, const float *dlogit, float *dfeats,
+                                 float *dw0, float *db0, float *dw1, float *db1, void *workspace,
+                                 size_t workspace_bytes, void *stream);
+
 /* ---- set_aggregator.mlp fused with its grouping (SURVEY 8(f) rank 3) --------------------------------------------
  * lib/pointnet2/pointnet2_modules.py:200-249 + QueryAndGroup.forward (pointnet2_utils.py:303-356) + SharedMLP
  * (pytorch_utils.py:9-32): per centre j and ball-query neighbour s the input [(xyz[idx] - new_xyz[j]) / radius |
