@@ -66,6 +66,12 @@ SIGNATURES = {
     "gf_mask_head_logits_backward": (c_int, [_P] * 9 + [c_int, c_int, c_int] + [_P] * 7 + [c_size_t, _P]),
     "gf_group_mlp_pool": (c_int, [_P, _P, _P, _P, c_int, c_int, c_int, c_int, c_int, c_float, c_int, c_int, c_int, _P, _P,
                                   _P, _P, c_int, _P, _P]),
+    "gf_group_mlp_pool_train_workspace_bytes": (c_size_t, [c_int, c_int]),
+    "gf_group_mlp_pool_train": (c_int, [_P, _P, _P, _P, c_int, c_int, c_int, c_int, c_int, c_float, c_int, c_int, c_int,
+                                        _P, _P, _P, _P, _P, _P, _P, c_int, _P, _P, c_size_t, _P]),
+    "gf_group_mlp_pool_backward_workspace_bytes": (c_size_t, [c_int, c_int, c_int, c_int, c_int]),
+    "gf_group_mlp_pool_backward": (c_int, [_P, _P, _P, _P, c_int, c_int, c_int, c_int, c_int, c_float, c_int, c_int,
+                                           c_int, _P, _P, _P, _P, c_int, _P, _P, _P, _P, _P, c_size_t, _P]),
     "gf_guidance_workspace_bytes": (c_size_t, [c_int, c_int, c_int]),
     "gf_guidance": (c_int, [_P, c_int, c_int, c_int, c_float, c_int, _P, _P, _P, _P, _P, _P, _P, c_size_t, _P]),
     "gf_guidance_seeded": (c_int, [_P, c_int, _P, c_int, c_int, c_float, c_int, _P, _P, _P, _P, _P, _P, c_size_t, _P]),

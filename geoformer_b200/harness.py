@@ -181,6 +181,17 @@ class FewShotForward(nn.Module):
     def forward(self, locs, output_feats, support_embedding, impl="b200", max_step=256, neighbor=64, geo_radius=0.05):
         """locs (B,N,3) foreground points of B equally sized scenes, output_feats (B,N,m) the stub backbone's point
         features, support_embedding (B, 2m).  Returns (list of (Q,N) mask logits, geo_dists, pre_enc_inds)."""
+        return self._chain(locs, output_feats, support_embedding, impl, max_step, neighbor, geo_radius)
+
+    def forward_train(self, locs, output_feats, support_embedding, impl="b200", max_step=128, neighbor=64,
+                      geo_radius=0.05):
+        """forward with autograd: one training step of the post-backbone path (the training setting of SURVEY 3.1 is a
+        model built with n_query_points=128 and max_step=128).  Call model.train() first for batch-statistics batch
+        norm.  Gradients reach every parameter through the aggregator, decoder and mask head of either impl; the
+        geodesic maps are data."""
+        return self._chain(locs, output_feats, support_embedding, impl, max_step, neighbor, geo_radius)
+
+    def _chain(self, locs, output_feats, support_embedding, impl, max_step, neighbor, geo_radius):
         B, N, _ = locs.shape
         pc_dims = [locs.min(dim=1)[0], locs.max(dim=1)[0]]
         mask_features = self.mask_tower(output_feats.transpose(1, 2)).transpose(1, 2)  # :477-483

@@ -235,6 +235,33 @@ int gf_group_mlp_pool(const float *xyz, const float *new_xyz, const float *featu
                       const float *const *weights, const float *const *scales, const float *const *shifts, int pool_avg,
                       float *out, void *stream);
 
+/* ---- set_aggregator in training form: batch statistics and the backward of gf_group_mlp_pool -------------------
+ * Same inputs as gf_group_mlp_pool.  consts (n_layers, 5, 32) device floats per layer: scale, shift, mean of W h,
+ * invstd, biased variance.  A layer with batch_stats[l] = 0 is FIXED: the caller fills its scale and shift (and, for
+ * the backward, mean and invstd of its batch norm) with zeros past its width.  A layer with batch_stats[l] = 1 uses
+ * the statistics of this call's input (torch's BatchNorm2d in training mode over all B * m * nsample elements): the
+ * forward computes its five rows on the device from gammas[l], betas[l], eps[l] (host arrays of device pointers and
+ * host floats), then runs gf_group_mlp_pool with them.  No host synchronisation.  Workspace:
+ * gf_group_mlp_pool_train_workspace_bytes.
+ * The backward takes the forward's consts and dout (B, widths[n_layers], m) and writes dweights[l] (widths[l+1],
+ * widths[l]), dvec (n_layers, 3, 32): gradients of the conv bias, gamma and beta, and dfeatures (B, C, N) (NULL: not
+ * computed).  It recomputes the forward with the forward's expressions (bit-identical ReLU masks and max-pool
+ * argmax, first maximal sample) and sums in a fixed order without float atomics: two calls give bitwise-equal
+ * gradients.  Workspace: gf_group_mlp_pool_backward_workspace_bytes.                                              */
+size_t gf_group_mlp_pool_train_workspace_bytes(int B, int m);
+int gf_group_mlp_pool_train(const float *xyz, const float *new_xyz, const float *features, const int *idx, int B,
+                            int N, int m, int nsample, int C, float radius, int normalize_xyz, int use_xyz,
+                            int n_layers, const int *widths, const float *const *weights, const float *const *gammas,
+                            const float *const *betas, const float *eps, const int *batch_stats, float *consts,
+                            int pool_avg, float *out, void *workspace, size_t workspace_bytes, void *stream);
+size_t gf_group_mlp_pool_backward_workspace_bytes(int B, int N, int m, int nsample, int C);
+int gf_group_mlp_pool_backward(const float *xyz, const float *new_xyz, const float *features, const int *idx, int B,
+                               int N, int m, int nsample, int C, float radius, int normalize_xyz, int use_xyz,
+                               int n_layers, const int *widths, const float *const *weights, const int *batch_stats,
+                               const float *consts, int pool_avg, const float *dout, float *dfeatures,
+                               float *const *dweights, float *dvec, void *workspace, size_t workspace_bytes,
+                               void *stream);
+
 /* ---- fused hot path: FPS -> kNN -> geodesic -------------------------------------------------- */
 
 /* Device-resident scene: xyz (N,3) -> seeds (Q) i32, geo (Q,N) f32.  knn_dist / knn_idx32 (N,k)
