@@ -17,7 +17,8 @@ w1 go through Hsum_q = sum_c dh, a sum over the contexts of terms that largely c
 so their relative error is that of the terms times the cancellation.  rel is per pair: a pair whose hidden
 pre-activation lies within TF32 rounding of ReLU's kink flips its mask, a few isolated entries (hence the small
 Frobenius error).  A missing term gives errors of order 1; the rel = 0 and memory = 0 cases make each term of dW1 /
-dWv dominant in turn."""
+dWv dominant in turn.  These tolerances tie the backward to the reference model; its arithmetic is pinned by elementwise
+bounds against the TF32-exact float64 emulation oracle/tf32.py (tests/test_tf32_reference.py)."""
 import ctypes
 import os
 import subprocess

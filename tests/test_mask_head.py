@@ -22,7 +22,9 @@ Frobenius error <= 3e-3, with the upstream gradient zeroed at the (q, n) where s
 forward's bound of ReLU's kink: there the mask may be set differently from the float64 one, and with random dlogit
 the sums over the points cancel enough for those few flips to reach 1.5e-2 of the result.  Measured on a B200 with
 that exclusion: dfeats, dw0, db0, db1 <= 4.3e-7 (max) and dw1 <= 2.6e-4 (max), 4.3e-4 (Frobenius): dw1 sums
-g relu(h), which carries the TF32 error of h itself, the others only its ReLU mask."""
+g relu(h), which carries the TF32 error of h itself, the others only its ReLU mask.  The kernel's arithmetic is
+pinned tighter against the TF32-exact float64 emulation oracle/tf32.py (truncated operands, as the B200 rounds them):
+tests/test_tf32_reference.py."""
 import ctypes
 import os
 import subprocess
