@@ -34,7 +34,6 @@
 // keeps only the visited bitmap on chip).  Optional by-products: the maximum of every row (for the
 // epilogues) and, for seed-sharded scenes, the finished row pushed into the peers' matrices over NVLink.
 // History of the formulations that were measured and replaced: DESIGN.md section 4.3.
-#include <stdlib.h>
 #include <string.h>
 
 #include "gf_geodesic.cuh"
@@ -42,6 +41,7 @@
 namespace gf {
 
 constexpr int GEO_QCAP = 4096;  // frontier entries kept in shared memory (per buffer)
+constexpr int GEO_THREADS = 1024;  // threads of the per-scene kernel: one CTA per seed, two per SM
 constexpr int GEO_UNROLL = 2;  // frontier points in flight per lane group (x 4 edges per lane)
 constexpr int GEO_MAX_PEERS = 15;
 constexpr uint32_t GEO_UNVISITED = 0xBF800000u;  // bits of -1.0f
@@ -166,7 +166,7 @@ __device__ __forceinline__ void geo_claim4(uint32_t key, const int4 t, int N, in
   geo_claim<MODE>(key + 3, t.w, N, level, vis, clm, rowu, nq, ovf, s_next_n);
 }
 
-template <int MODE, int GEO_THREADS>
+template <int MODE>
 __global__ void __launch_bounds__(GEO_THREADS, 2048 / GEO_THREADS) geo_seed_bfs_kernel(const GeoArgs a) {
   constexpr bool BITMAP = MODE >= 1;  // a visited bitmap lives in shared memory
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -422,7 +422,7 @@ __global__ void __launch_bounds__(GEO_THREADS, 2048 / GEO_THREADS) geo_seed_bfs_
 }
 
 // ---- the batched kernel (scenes whose two bitmaps fit on chip: N <~ 860k) -------------------------------------
-// Same algorithm as geo_seed_bfs_kernel<2, .> (level-synchronous first-visit BFS per seed, RED.MIN claim keys that
+// Same algorithm as geo_seed_bfs_kernel<2> (level-synchronous first-visit BFS per seed, RED.MIN claim keys that
 // reproduce the reference's tie rule, frontier read off a claimed bitmap), restated around what the round-2
 // profiles showed: a per-seed run is a CHAIN OF DEPENDENT MEMORY LATENCIES (per level: queue -> edge row ->
 // visited words -> barrier -> bitmap scan -> queue, plus the loads that turn a winning key into a distance), the
@@ -496,7 +496,7 @@ __device__ __forceinline__ void geo_claim4_enc(uint32_t key, const int4 t, uint3
   }
 }
 
-template <int THREADS, int U>
+template <int THREADS>
 __global__ void __launch_bounds__(THREADS, 2048 / THREADS) geo_bfs_batch_kernel(const GeoBatchArgs a) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   int *fq = reinterpret_cast<int *>(smem_raw);  // the frontier queue (rebuilt by every commit), a.qcap entries
@@ -611,26 +611,13 @@ __global__ void __launch_bounds__(THREADS, 2048 / THREADS) geo_bfs_batch_kernel(
           }
         }
       }
-      // ---- claims: KP/4 lanes per frontier point; lanes past the end expand the sentinel point N -------------
+      // ---- claims: KP/4 lanes per frontier point ------------------------------------------------------------
       const int Fs = F < QC ? F : QC;
-      for (int n0 = (int)group; n0 < Fs; n0 += (int)ngroups * U) {
-        unsigned pl[U], key[U];
-        int4 t[U];
-#pragma unroll
-        for (int u = 0; u < U; ++u) {
-          const int at = n0 + u * (int)ngroups;
-          const int p = at < Fs ? fq_at(at) : N;
-          pl[u] = (unsigned)p << lsb;
-          key[u] = (unsigned)p;
-          if (order) key[u] = at < Fs ? (unsigned)__ldg(order + p) : 0u;
-        }
-#pragma unroll
-        for (int u = 0; u < U; ++u) t[u] = __ldg(trow + pl[u]);
-#pragma unroll
-        for (int u = 0; u < U; ++u) {
-          if (u > 0 && n0 + u * (int)ngroups >= Fs) continue;  // whole groups of sentinel lanes
-          geo_claim4_enc((key[u] << sb) | keysub, t[u], vis_s, clm_s, claimb);
-        }
+      for (int n0 = (int)group; n0 < Fs; n0 += (int)ngroups) {
+        const int p = fq_at(n0);
+        const unsigned po = order ? (unsigned)__ldg(order + p) : (unsigned)p;
+        const int4 t = __ldg(trow + ((unsigned)p << lsb));
+        geo_claim4_enc((po << sb) | keysub, t, vis_s, clm_s, claimb);
       }
       for (int node = QC + (int)group; node < F; node += (int)ngroups) {  // spilled tail (rare)
         const int p = ovf[ovf_at(node, (level - 1) & 1)];
@@ -798,58 +785,41 @@ static int geo_slot_bits(int k) {
 }
 
 // ---- planning ---------------------------------------------------------------------------------------------
-static int env_int(const char *name, int dflt) {
-  const char *e = getenv(name);
-  return e ? atoi(e) : dflt;
-}
-
 static int geo_bitmap_words(int N) { return ((N + 1 + 127) / 128) * 4; }  // + the sentinel point N; whole 16-byte pieces
 
-// plan of the template kernel (big scenes, seed-sharded scenes, or GF_GEO_ENC=0)
+// plan of the per-scene kernel (big scenes, seed-sharded scenes)
 struct GeoPlan {
-  int grid, bitmap_words, mode, threads;
+  int grid, bitmap_words, mode;
   size_t smem;
 };
 
-// shared-memory plan, identical for sizing and launching: 227 KB usable per SM on sm_100 (1 KB reserved per CTA)
-static void geo_smem_plan(int N, int Q, GeoPlan *p, int *ctas_per_sm) {
+// identical for sizing and launching: 227 KB of shared memory usable per SM on sm_100 (1 KB reserved per CTA)
+static void plan_geo(int N, int Q, GeoPlan *p) {
   const int words = geo_bitmap_words(N);
-  static const int nobitmap = env_int("GF_GEO_NOBITMAP", 0);  // test knob: 1 = no on-chip state, 2 = visited bitmap only
-  static const int force_threads = env_int("GF_GEO_THREADS", 0);
-  int m = nobitmap == 1 ? 0 : (nobitmap == 2 ? 1 : 2);
   auto bytes_of = [&](int mode) {
     return sizeof(int) * (size_t)(mode == 2 ? 1 : 2) * GEO_QCAP + sizeof(uint32_t) * (size_t)mode * words;
   };
   // both bitmaps must fit for mode 2; otherwise mode 0 (two CTAs per SM) measured slightly faster at 1 M
   // points and 512 seeds than mode 1 (157 KB of shared memory: one CTA per SM).  With no more seeds than SMs (a
   // rank's block of a seed-sharded scene) one CTA per SM loses nothing and the visited test stays on chip: mode 1.
-  if (m == 2 && bytes_of(2) > (size_t)226 * 1024) m = (Q <= num_sms() && nobitmap == 0) ? 1 : 0;
+  int m = 2;
+  if (bytes_of(2) > (size_t)226 * 1024) m = Q <= num_sms() ? 1 : 0;
   if (m == 1 && bytes_of(1) > (size_t)226 * 1024) m = 0;
   const size_t bytes = bytes_of(m);
   int fit = (int)((size_t)(227 * 1024) / (bytes + 1024));
   if (fit < 1) fit = 1;
-  const int threads = force_threads == 512 ? 512 : 1024;
-  const int cap = 2048 / threads;
+  const int cap = 2048 / GEO_THREADS;
   p->bitmap_words = m > 0 ? words : 0;
   p->smem = bytes;
   p->mode = m;
-  p->threads = threads;
-  *ctas_per_sm = fit < cap ? fit : cap;
-}
-
-static void plan_geo(int N, int Q, GeoPlan *p) {
-  int per_sm = 1;
-  geo_smem_plan(N, Q, p, &per_sm);
-  static const int bps_cap = env_int("GF_GEO_BPS", 0);  // experiment knob
-  if (bps_cap > 0 && per_sm > bps_cap) per_sm = bps_cap;
-  int grid = num_sms() * per_sm;
+  int grid = num_sms() * (fit < cap ? fit : cap);
   if (grid > Q) grid = Q;
   p->grid = grid < 1 ? 1 : grid;
 }
 
 // plan of the batched kernel
 struct GeoBatchPlan {
-  int threads, unroll, per_sm, grid, qcap, words;
+  int threads, per_sm, grid, qcap, words;
   size_t smem, ovf_stride, arr_stride;
 };
 // bytes of per-CTA scratch (frontier overflow + claim keys + distances: 12 bytes per point and CTA) a launch may
@@ -858,21 +828,15 @@ constexpr size_t GEO_SCRATCH_BUDGET = (size_t)768 << 20;
 
 // true when the scene can run in the batched kernel (both bitmaps + a queue fit one CTA's shared memory)
 static bool geo_batchable(int maxN) {
-  static const int nobitmap = env_int("GF_GEO_NOBITMAP", 0), enc = env_int("GF_GEO_ENC", 2);
-  if (nobitmap != 0 || enc == 0) return false;
   return sizeof(int) * 1024 + 2 * sizeof(uint32_t) * (size_t)geo_bitmap_words(maxN) <= (size_t)226 * 1024;
 }
 
 static void plan_batch(int maxN, long long items, GeoBatchPlan *p) {
-  static const int force_threads = env_int("GF_GEO_THREADS", 0), unroll = env_int("GF_GEO_UNROLL", 1),
-                   bps_cap = env_int("GF_GEO_BPS", 0), many_threads = env_int("GF_GEO_BATCH_THREADS", 512);
   const int sms = num_sms();
   p->words = geo_bitmap_words(maxN);
   // One scene's worth of seeds cannot fill the thread slots anyway and a launch lasts as long as its slowest
   // seed: 1024 threads per seed.  A batch is throughput work: more, smaller CTAs per SM (see the kernel's header).
-  int threads = items <= 2ll * sms ? 1024 : many_threads;
-  if (force_threads == 256 || force_threads == 512 || force_threads == 1024) threads = force_threads;
-  if (threads != 256 && threads != 512 && threads != 1024) threads = 512;
+  const int threads = items <= 2ll * sms ? 1024 : 512;
   const int cap = 2048 / threads;
   int best_fit = 0, best_q = 0;
   for (int qcap = 4096; qcap >= 1024 && qcap >= threads; qcap >>= 1) {
@@ -883,9 +847,7 @@ static void plan_batch(int maxN, long long items, GeoBatchPlan *p) {
     if (fit > best_fit) best_fit = fit, best_q = qcap;  // the largest queue that reaches the most CTAs per SM
   }
   if (best_fit < 1) best_fit = 1, best_q = 1024;
-  if (bps_cap > 0 && best_fit > bps_cap) best_fit = bps_cap;
   p->threads = threads;
-  p->unroll = unroll == 1 ? 1 : 2;
   p->per_sm = best_fit;
   p->qcap = best_q;
   p->smem = sizeof(int) * (size_t)best_q + 2 * sizeof(uint32_t) * (size_t)p->words;
@@ -1068,25 +1030,17 @@ int geodesic_batch_launch(const GeoSceneDesc *scenes, int B, int k, int max_step
 #endif
   stage_mark(ST_GEO_READY, st);
   int rc = GF_OK;
-#define GF_GEO_BATCH(T, U)                                            \
-  do {                                                                \
-    static int done[64] = {0};                                        \
-    rc = geo_kernel_ready(geo_bfs_batch_kernel<T, U>, done);          \
-    if (rc) return rc;                                                \
-    geo_bfs_batch_kernel<T, U><<<p.grid, T, p.smem, st>>>(ga);        \
+#define GF_GEO_BATCH(T)                                            \
+  do {                                                             \
+    static int done[64] = {0};                                     \
+    rc = geo_kernel_ready(geo_bfs_batch_kernel<T>, done);          \
+    if (rc) return rc;                                             \
+    geo_bfs_batch_kernel<T><<<p.grid, T, p.smem, st>>>(ga);        \
   } while (0)
-  if (p.threads == 256 && p.unroll == 1)
-    GF_GEO_BATCH(256, 1);
-  else if (p.threads == 256)
-    GF_GEO_BATCH(256, 2);
-  else if (p.threads == 512 && p.unroll == 1)
-    GF_GEO_BATCH(512, 1);
-  else if (p.threads == 512)
-    GF_GEO_BATCH(512, 2);
-  else if (p.unroll == 1)
-    GF_GEO_BATCH(1024, 1);
+  if (p.threads == 512)
+    GF_GEO_BATCH(512);
   else
-    GF_GEO_BATCH(1024, 2);
+    GF_GEO_BATCH(1024);
 #undef GF_GEO_BATCH
   GF_LAUNCHED();
 #ifdef GF_TRACE
@@ -1179,25 +1133,19 @@ int geodesic_run(const float *D, const void *I, int is64, int N, int k, const in
   ga.trace = nullptr, ga.trace2 = nullptr;
 #endif
   int rc = GF_OK;
-#define GF_GEO_LAUNCH(M, T)                                        \
-  do {                                                             \
-    static int done[64] = {0};                                     \
-    rc = geo_kernel_ready(geo_seed_bfs_kernel<M, T>, done);        \
-    if (rc) return rc;                                             \
-    geo_seed_bfs_kernel<M, T><<<p.grid, T, p.smem, st>>>(ga);      \
+#define GF_GEO_LAUNCH(M)                                                  \
+  do {                                                                    \
+    static int done[64] = {0};                                            \
+    rc = geo_kernel_ready(geo_seed_bfs_kernel<M>, done);                  \
+    if (rc) return rc;                                                    \
+    geo_seed_bfs_kernel<M><<<p.grid, GEO_THREADS, p.smem, st>>>(ga);      \
   } while (0)
-  if (p.mode == 2 && p.threads == 512)
-    GF_GEO_LAUNCH(2, 512);
-  else if (p.mode == 2)
-    GF_GEO_LAUNCH(2, 1024);
-  else if (p.mode == 1 && p.threads == 512)
-    GF_GEO_LAUNCH(1, 512);
+  if (p.mode == 2)
+    GF_GEO_LAUNCH(2);
   else if (p.mode == 1)
-    GF_GEO_LAUNCH(1, 1024);
-  else if (p.threads == 512)
-    GF_GEO_LAUNCH(0, 512);
+    GF_GEO_LAUNCH(1);
   else
-    GF_GEO_LAUNCH(0, 1024);
+    GF_GEO_LAUNCH(0);
 #undef GF_GEO_LAUNCH
   GF_LAUNCHED();
   stage_mark(ST_GEO_DONE, st);

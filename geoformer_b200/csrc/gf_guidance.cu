@@ -15,10 +15,7 @@ namespace gf {
 // lanes.  Callers that keep several calls in flight on several streams get one set per stream, so their kernels
 // do not queue on a single hidden stream.  FPS lanes have the highest priority: FPS is the longest dependency
 // chain of a scene, its cluster should be placed as soon as SMs free up.
-#ifndef GF_LANES
-#define GF_LANES 4
-#endif
-constexpr int LANES = GF_LANES;
+constexpr int LANES = 4;  // 6 lanes measured the same, 8 slower (DESIGN section 8)
 struct ForkJoin {
   cudaStream_t fps[LANES] = {}, knn[LANES] = {};  // knn[0] stays null: lane 0 builds its graph on the caller's stream
   cudaEvent_t fork = nullptr, join_fps[LANES] = {}, join_knn[LANES] = {};

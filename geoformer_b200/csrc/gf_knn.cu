@@ -14,8 +14,6 @@
 //   algo 1  brute-force tiled scan (shared-memory tiles, register-resident sorted top-k).  This
 //           is the formulation named in BASELINE.json; kept as an independent cross-check.
 // 3-D coordinates make this a compare/select problem, not a contraction: no tensor cores.
-#include <stdlib.h>
-
 #include "gf_knn.cuh"
 
 namespace gf {
@@ -377,9 +375,7 @@ struct TopK {
 // lattices) offers every candidate of the shell instead.  Shells R >= 2 (after the unchanged termination test) offer
 // every candidate to a top-k that is already exact for the first shell, so few of them insert.
 constexpr int KNN_NB = 32;  // bins of d2 over [0, 4 h^2); the last one also takes everything beyond and NaN
-#ifndef KNN_MIN_BLOCKS
-#define KNN_MIN_BLOCKS 7  // 72 registers for k <= 16, 24 KB of shared memory per block
-#endif
+constexpr int KNN_MIN_BLOCKS = 7;  // 72 registers for k <= 16, 24 KB of shared memory per block
 template <int KT>
 __global__ void __launch_bounds__(128, KT <= 16 ? KNN_MIN_BLOCKS : 1)
     knn_grid_query_kernel(const KnnGrid *__restrict__ gp, const float4 *__restrict__ sorted,
@@ -780,13 +776,8 @@ int knn_grid_build(const float *xyz, int N, int k, void *workspace, size_t works
   }
   const int nb = num_sms() * 8;
   // target cell occupancy = tau_mul x k.  Measured (c2 / c1, B200): flat between 0.12 and 0.7 for k <= 32 (0.45 kept);
-  // at k = 64 smaller cells win (0.2: 0.88 ms vs 1.03 ms per graph).  GF_KNN_TAU overrides (experiments).
-  static const float tau_env = [] {
-    const char *e = getenv("GF_KNN_TAU");
-    const float v = e ? (float)atof(e) : 0.f;
-    return v > 0.f ? v : 0.f;
-  }();
-  const float tau_mul = tau_env > 0.f ? tau_env : (k > 32 ? 0.2f : 0.45f);
+  // at k = 64 smaller cells win (0.2: 0.88 ms vs 1.03 ms per graph).
+  const float tau_mul = k > 32 ? 0.2f : 0.45f;
   const float tau = fmaxf(2.f, tau_mul * (float)k);
   const int npt = min(nb, (N + 255) / 256);
   GF_CUDA(cudaMemsetAsync(ctl, 0, sizeof(KnnCtl), st));

@@ -1,62 +1,133 @@
-"""The propagation kernel has three state layouts (both bitmaps on chip / visited bitmap only / no on-chip
-state, chosen by scene size) and a global overflow area for frontiers beyond the on-chip queue.  The size
-rule would exercise the last two only at ~1M points, so they are forced here through the kernel's test knob
-(GF_GEO_NOBITMAP, read once per process => one subprocess per mode) on scenes the oracle finishes in
-seconds, including frontiers of tens of thousands of points (k = 64, no radius filter)."""
-import os
-import subprocess
-import sys
+"""Every propagation kernel the library can launch, reached through the rules that choose it from N, Q and the SM
+count, bit for bit against the oracle, with a check of which kernel ran:
 
+    geo_bfs_batch_kernel<1024>   scenes whose two bitmaps fit on chip, at most two seeds per SM
+    geo_bfs_batch_kernel<512>    the same with more seeds
+    geo_seed_bfs_kernel<2>       both bitmaps on chip: seed-sharded scenes (peers given: always the per-scene kernel)
+    geo_seed_bfs_kernel<1>       visited bitmap only: scenes too large for both bitmaps (N > ~860k), Q <= SM count
+    geo_seed_bfs_kernel<0>       no on-chip state: the same with more seeds (test_full_size_config_c4: k = 16)
+
+Each kernel also runs a case whose frontiers spill beyond the on-chip queue into the global overflow area.  The
+oracle's statistics show it: R reached pairs over Q seeds and levels + 1 levels (the seed's included) average more
+than the queue holds, so some level's frontier was larger."""
+import ctypes
+import functools
+import re
+
+import numpy as np
 import pytest
+import torch
 
 pytestmark = pytest.mark.gpu
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+QUEUE = 4096  # frontier entries of the on-chip queue (the batched kernel's queue is at most this long)
 
-CHILD = r"""
-import sys
-import numpy as np
-import torch
-sys.path.insert(0, %r)
-import oracle
-from geoformer_b200.geodesic_utils import geodesic_from_graph, knn_graph
-from geoformer_b200.scenes import scene
-dev = torch.device("cuda:0")
-cases = [
-    # N, room, Q, k, radius, max_step
-    (30000, dict(), 8, 16, 0.5, 40),
-    (50000, dict(L=(1.0, 1.0, 0.5), nbox=2), 6, 64, 10.0, 6),    # frontiers >> 4096: overflow area
-    (20000, dict(L=(2.0, 1.5, 1.0), nbox=4), 300, 8, 0.2, 300),  # more seeds than CTAs: persistent loop, deep
-    (4097, dict(L=(1.0, 1.0, 0.5), nbox=2), 5, 33, 10.0, 4),     # K = 32 exactly (KP = 32), N just over a queue
-]
-for N, room, Q, k, r, ms in cases:
-    x = scene(N, 17, **room)
+SCENES = {  # N, points
+    "n30k": (30000, "scene"),
+    # on the surfaces of `scene` a frontier grows linearly with the level and stays below the queue in any scene the
+    # batched kernel takes; in a filled volume it grows with the square of the level
+    "volume400k": (400_000, "volume"),
+    "n4097": (4097, "small_room"),  # N just over a queue
+    "n20k": (20000, "room_2x1.5"),
+    "room1m": (1_000_000, "room_1m"),
+}
+# scene, Q (a number or a function of the SM count), k, radius, max_step, entry point, kernel, spills beyond the queue.
+# The batched and one-peer runs of a case are adjacent: they share one graph and one oracle result.
+CASES = {}
+for name, q, k, r, ms, spills in [
+        ("n30k", 8, 16, 0.5, 40, False),
+        ("volume400k", 6, 64, 10.0, 24, True),
+        ("n4097", 5, 33, 10.0, 4, False),  # K = 32 exactly (KP = 32)
+        ("n20k", lambda sms: 2 * sms + 4, 8, 0.2, 300, False)]:  # a persistent loop over the seeds, deep
+    many = callable(q)
+    CASES["batched_%s" % name] = (name, q, k, r, ms, "geodesic", ("bfs_batch", 512 if many else 1024), spills)
+    CASES["one_peer_%s" % name] = (name, q, k, r, ms, "one_peer", ("seed_bfs", 2), spills)
+CASES["visited_only_k16"] = ("room1m", 8, 16, 0.5, 32, "geodesic", ("seed_bfs", 1), False)
+CASES["visited_only_k64"] = ("room1m", 8, 64, 10.0, 96, "geodesic", ("seed_bfs", 1), True)
+CASES["no_on_chip_state_k64"] = ("room1m", lambda sms: sms + 1, 64, 10.0, 80, "geodesic", ("seed_bfs", 0), True)
+
+
+def _sms():
+    return torch.cuda.get_device_properties(0).multi_processor_count
+
+
+def _points(n, gen):
+    from geoformer_b200.scenes import room, scene
+
+    if gen == "volume":
+        return torch.rand(n, 3, generator=torch.Generator().manual_seed(17))  # the unit cube, filled
+    if gen == "room_1m":
+        return room(n, 4321)
+    shape = {"scene": {}, "small_room": dict(L=(1.0, 1.0, 0.5), nbox=2), "room_2x1.5": dict(L=(2.0, 1.5, 1.0), nbox=4)}
+    return scene(n, 17, **shape[gen])
+
+
+@functools.lru_cache(maxsize=1)
+def _inputs(scene_name, Q, k, r, ms, oracle):
+    """the kNN graph on the device, FPS seeds, and the oracle's maps and statistics"""
+    from geoformer_b200.geodesic_utils import knn_graph
+
+    x = _points(*SCENES[scene_name])
     seeds = oracle.furthest_point_sampling(x[None].numpy(), Q)[0]
-    D, I = knn_graph(x.to(dev), k)
-    want = oracle.geodesic(D.cpu().numpy(), I.cpu().numpy(), seeds, r, ms)
-    rm = torch.zeros(Q, device=dev)
-    got = geodesic_from_graph(D, I, torch.from_numpy(seeds).to(dev), r, ms, row_max=rm).cpu().numpy()
-    assert np.array_equal(got, want), (N, Q, k, r, ms, int((got != want).sum()))
-    assert np.array_equal(rm.cpu().numpy(), want.max(axis=1)), "row_max by-product"
-    print("ok", N, Q, k, r, ms, "reached", int((want >= 0).sum()))
-"""
+    D, I = knn_graph(x.to("cuda:0"), k)
+    want, R, lev = oracle.geodesic(D.cpu().numpy(), I.cpu().numpy(), seeds, r, ms, return_stats=True)
+    return D, I, torch.from_numpy(seeds).to("cuda:0"), want, R, lev
 
 
-# (GF_GEO_NOBITMAP, GF_GEO_ENC, GF_GEO_UNROLL, GF_GEO_THREADS): every kernel the size rule or a knob can select
-VARIANTS = [("0", "2", "2", "0"),     # the default: batched two-bitmap kernel, thread count by the number of seeds
-            ("0", "2", "1", "1024"), ("0", "2", "2", "512"), ("0", "2", "1", "256"), ("0", "2", "2", "256"),
-            ("0", "0", "2", "1024"),  # the per-scene template kernel with plain edge targets (round 1)
-            ("0", "0", "2", "512"),
-            ("1", "2", "2", "1024"),  # no on-chip state (the layout of scenes beyond ~860k points)
-            ("2", "2", "2", "1024")]  # visited bitmap only
+def _launched(fn):
+    """fn() under the profiler -> its result and the propagation kernels it launched, as (kernel, template argument)"""
+    with torch.profiler.profile(activities=[torch.profiler.ProfilerActivity.CUDA]) as prof:
+        out = fn()
+        torch.cuda.synchronize()
+    found = (re.search(r"geo_(bfs_batch|seed_bfs)_kernel(?:<|ILi)(\d+)", e.name) for e in prof.events())
+    return out, [(m.group(1), int(m.group(2))) for m in found if m]
 
 
-@pytest.mark.parametrize("mode,enc,unroll,threads", VARIANTS)
-def test_geodesic_state_layouts_and_overflow(cuda_lib, oracle_lib, mode, enc, unroll, threads):
-    env = dict(os.environ)
-    env["GF_GEO_NOBITMAP"] = mode  # 0 = size rule (both bitmaps here), 1 = no on-chip state, 2 = visited bitmap only
-    env["GF_GEO_ENC"], env["GF_GEO_UNROLL"], env["GF_GEO_THREADS"] = enc, unroll, threads
-    out = subprocess.run([sys.executable, "-c", CHILD % ROOT], env=env, cwd=ROOT, capture_output=True, text=True,
-                         timeout=600)
-    assert out.returncode == 0, out.stdout[-2000:] + out.stderr[-4000:]
-    assert out.stdout.count("ok ") == 4
+def _geodesic(D, I, seeds, r, ms):
+    from geoformer_b200.geodesic_utils import geodesic_from_graph
+
+    rm = torch.zeros(seeds.numel(), device=D.device)
+    geo, stats = geodesic_from_graph(D, I, seeds, r, ms, return_stats=True, row_max=rm)
+    return geo, stats, rm
+
+
+def _geodesic_one_peer(D, I, seeds, r, ms):
+    """gf_geodesic_scatter with one peer matrix on the same device: the finished rows are also stored there"""
+    from geoformer_b200 import _capi as C
+
+    N, k = D.shape
+    Q = seeds.numel()
+    seeds = seeds.to(torch.int32).contiguous()
+    geo = torch.empty((Q, N), dtype=torch.float32, device=D.device)
+    peer = torch.full_like(geo, float("nan"))
+    stats = torch.zeros(2, dtype=torch.int64, device=D.device)
+    peers = (ctypes.c_void_p * 1)(peer.data_ptr())
+    L = C.lib()
+    with torch.cuda.device(D.device):
+        nbytes = L.gf_geodesic_workspace_bytes(N, k, Q)
+        ws = C.workspace.get(D.device, "geodesic", nbytes)
+        C.check(L.gf_geodesic_scatter(C.ptr(D), C.ptr(I), 1 if I.dtype == torch.int64 else 0, N, k, C.ptr(seeds), Q,
+                                      ctypes.c_float(r), ms, C.ptr(geo), ctypes.cast(peers, ctypes.c_void_p), 1,
+                                      C.ptr(stats), C.ptr(ws), nbytes, C.stream_of(D.device)), "geodesic_scatter")
+    return geo, peer, stats
+
+
+@pytest.mark.parametrize("case", list(CASES))
+def test_geodesic_state_layouts_and_overflow(cuda_lib, oracle_lib, case):
+    scene_name, Q, k, r, ms, entry, kernel, spills = CASES[case]
+    Q = Q(_sms()) if callable(Q) else Q
+    D, I, seeds, want, R, lev = _inputs(scene_name, Q, k, r, ms, oracle_lib)
+    if entry == "geodesic":
+        (geo, stats, rm), kernels = _launched(lambda: _geodesic(D, I, seeds, r, ms))
+    else:
+        (geo, peer, stats), kernels = _launched(lambda: _geodesic_one_peer(D, I, seeds, r, ms))
+    assert kernels == [kernel]
+    got = geo.cpu().numpy()
+    assert np.array_equal(got, want), int((got != want).sum())
+    if entry == "geodesic":
+        assert np.array_equal(rm.cpu().numpy(), want.max(axis=1)), "row_max by-product"
+    else:  # the seed-sharded entry point has no row-maximum output
+        assert torch.equal(peer, geo)
+    assert (int(stats[0]), int(stats[1])) == (R, lev)
+    if spills:
+        assert R / (Q * (lev + 1)) > QUEUE, (R, Q, lev)

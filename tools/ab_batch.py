@@ -1,7 +1,7 @@
 """A/B of the batched hot path: ms per scene for batches of B scenes of a workload, one batch in flight, per
-environment-knob combination (one subprocess each).
+combination of batch size and library (one subprocess each).
 
-    python tools/ab_batch.py c2 "B=1" "B=4" "B=8 GF_GEO_THREADS=256" ...
+    python tools/ab_batch.py c2 "B=1" "B=8" "B=8 GF_LIB=geoformer_b200/libgeoformer_b200_x.so" ...
 """
 import os
 import subprocess

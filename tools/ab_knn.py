@@ -1,7 +1,7 @@
-"""A/B of kNN query kernel variants (one subprocess per environment-knob combination): ms per kNN graph and a
-checksum of the index / distance tables, so that two variants can be compared for equality at a glance.
+"""A/B of kNN query kernel variants, each built into its own library (one subprocess per library): ms per kNN graph
+and a checksum of the index / distance tables, so that two variants can be compared for equality at a glance.
 
-    python tools/ab_knn.py "" "GF_KNN_TAU=0.3" "GF_LIB=geoformer_b200/libgeoformer_b200_x.so"
+    python tools/ab_knn.py "" "GF_LIB=geoformer_b200/libgeoformer_b200_x.so"
 """
 import os
 import subprocess

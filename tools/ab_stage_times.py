@@ -1,7 +1,7 @@
-"""A/B of kernel variants selected by environment knobs (read once per process => one subprocess per combination).
+"""A/B of libraries (GF_LIB, read once per process => one subprocess per combination).
 Prints per-stage CUDA-event times of the fused hot path, one scene in flight, for a workload.
 
-    python tools/ab_stage_times.py c2 "GF_GEO_ENC=0" "GF_GEO_ENC=1" "GF_GEO_ENC=2 GF_GEO_UNROLL=1" ...
+    python tools/ab_stage_times.py c2 "" "GF_LIB=geoformer_b200/libgeoformer_b200_x.so"
 """
 import json
 import os
