@@ -310,7 +310,11 @@ __global__ void __launch_bounds__(FPS_GRID_T, 1)
     if (u == 0) idx[0] = 0;
 
     for (int j = 1; j < m; ++j) {
-      const uint32_t tag = (uint32_t)b * (uint32_t)m + (uint32_t)j;  // >= 1, strictly increasing over the launch
+      // The rounds of the whole launch are numbered 1, 2, 3, ... without a gap, also from the last round of one
+      // scene to the first of the next, so consecutive rounds use different buffers: a CTA writes buffer X again
+      // only after every CTA has published the round in between, i.e. after every CTA has finished reading X.
+      // Tag 0 (the zeroed slots) means "never written".
+      const uint32_t tag = (uint32_t)b * (uint32_t)(m - 1) + (uint32_t)j;
       const int buf = tag & 1;
       float best = -1.f;
       uint32_t besti = 0;
@@ -592,7 +596,6 @@ extern "C" int gf_furthest_point_sampling(const float *xyz, int B, int N, int m,
   GF_FPS_CASE(256, 25);
   GF_FPS_CASE(256, 32);
   GF_FPS_CASE(512, 24);
-  GF_FPS_CASE(1024, 0);
 #undef GF_FPS_CASE
   set_error("furthest_point_sampling: no kernel variant for N=%d", N);
   return GF_ERR_INVALID;

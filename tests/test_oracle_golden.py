@@ -24,13 +24,11 @@ def test_golden_fixtures_exist():
     assert len(glob.glob(os.path.join(GOLD, "geodesic_*.npz"))) >= 4
 
 
-def _bitrev(v, bits):
-    return int(format(v, "0%db" % bits)[::-1], 2) if bits else 0
-
-
-def _fps_by_key_rule(xyz, m):
+def _fps_by_key_rule(xyz, m, rank=None):
     """Independent restatement of FPS through the closed-form tie rule of SURVEY F6(b): among equal maxima
-    the winner is the k with the smallest (bitrev_L(k mod bs), k div bs)."""
+    the winner is the k with the smallest (bitrev_L(k mod bs), k div bs).  `rank` (n,) replaces that order
+    with another one (smallest rank wins), e.g. np.arange(n) for the lowest index.  Exact wherever the float64
+    emulation of sq3 is, which includes every input on a coarse lattice."""
     n = xyz.shape[0]
     L = 0
     while (2 << L) <= n and L < 9:
@@ -46,7 +44,11 @@ def _fps_by_key_rule(xyz, m):
 
     elig = ~(sq3(x, y, z).astype(np.float64) <= 1e-3)
     temp = np.full(n, 1e10, dtype=f32)
-    rank = np.array([(_bitrev(k % bs, L) << 23) | (k // bs) for k in range(n)], dtype=np.int64)
+    if rank is None:
+        k = np.arange(n, dtype=np.int64)
+        rev = sum(((k % bs >> b) & 1) << (L - 1 - b) for b in range(L)) if L else np.zeros(n, dtype=np.int64)
+        rank = (rev << 23) | (k // bs)
+    rank = np.asarray(rank, dtype=np.int64)
     idx = np.zeros(m, dtype=np.int32)
     old = 0
     for j in range(1, m):
