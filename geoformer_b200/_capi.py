@@ -42,6 +42,8 @@ SIGNATURES = {
     "gf_three_interpolate_grad": (c_int, [_P, _P, _P, c_int, c_int, c_int, c_int, _P, _P]),
     "gf_knn_workspace_bytes": (c_size_t, [c_int, c_int, c_int, c_int]),
     "gf_knn": (c_int, [_P, c_int, _P, c_int, c_int, c_int, _P, _P, _P, c_int, _P, c_size_t, _P]),
+    "gf_knn_batch_workspace_bytes": (c_size_t, [_P, c_int]),
+    "gf_knn_batch": (c_int, [_P, _P, c_int, c_int, c_int, _P, _P, _P, c_size_t, _P]),
     "gf_geodesic_workspace_bytes": (c_size_t, [c_int, c_int, c_int]),
     "gf_geodesic": (c_int, [_P, _P, c_int, c_int, c_int, _P, c_int, c_float, c_int, _P, _P, _P, _P, c_size_t, _P]),
     "gf_bias_workspace_bytes": (c_size_t, [c_int, c_int]),

@@ -15,7 +15,11 @@ namespace gf {
 // lanes.  Callers that keep several calls in flight on several streams get one set per stream, so their kernels
 // do not queue on a single hidden stream.  FPS lanes have the highest priority: FPS is the longest dependency
 // chain of a scene, its cluster should be placed as soon as SMs free up.
-constexpr int LANES = 4;  // 6 lanes measured the same, 8 slower (DESIGN section 8)
+// Measured with the graphs of a 20-scene call built and queried in one launch each (c2 bench, B200 at 1000 W, two
+// runs each): 4 lanes 1.090 / 1.091 M maps/s, 6 lanes 1.094 / 1.095, 8 lanes 1.053 / 1.053.  6 lanes are 0.4 %
+// ahead, which does not pay for two more high-priority streams per caller stream; 8 lanes lose 3.5 % (DESIGN
+// section 8).
+constexpr int LANES = 4;
 struct ForkJoin {
   cudaStream_t fps[LANES] = {}, knn[LANES] = {};  // knn[0] stays null: lane 0 builds its graph on the caller's stream
   cudaEvent_t fork = nullptr, join_fps[LANES] = {}, join_knn[LANES] = {};
@@ -191,9 +195,10 @@ extern "C" int gf_guidance_seeded_scatter(const float *xyz, int N, const int *se
 
 // ---- a batch of scenes (the reference's call is batched: geodesic_utils.py:98 loops over the scenes) -------------
 namespace gf {
+static_assert(KNN_BATCH_MAX == GEO_BATCH_MAX, "one batched call builds and queries all its scenes' graphs at once");
 struct BatchPlan {
   size_t per_scene[GEO_BATCH_MAX * 4];  // offsets of (fps, knn, edges) per scene
-  size_t scratch, scratch_bytes, stats, total;
+  size_t knn_ctl, scratch, scratch_bytes, stats, total;
 };
 static int plan_batch_guidance(const int *Ns, int B, int Q, int k, BatchPlan *p, size_t *fps_b, size_t *knn_b,
                                size_t *edge_b) {
@@ -210,6 +215,8 @@ static int plan_batch_guidance(const int *Ns, int B, int Q, int k, BatchPlan *p,
     p->per_scene[b * 3 + 2] = off, off += edge_b[b];
     maxN = N > maxN ? N : maxN;
   }
+  p->knn_ctl = off;
+  off += align256(knn_ctl_block_bytes(B));
   p->scratch = off;
   p->scratch_bytes = align256(geodesic_batch_scratch_bytes(maxN, (long long)Q * B));
   off += p->scratch_bytes;
@@ -258,10 +265,15 @@ extern "C" int gf_guidance_batch(const float *const *xyz, const int *Ns, int B, 
   int rc = get_fork_join(st, &fj, lanes);
   if (rc) return rc;
   stage_mark(ST_BEGIN, st);
+  // The graphs.  Up to LANES scenes, every scene has a lane of its own (lane 0: the caller's stream) and its graph
+  // is one short chain next to its FPS.  With more scenes a lane would run several graphs one after another, each a
+  // chain of six launches ending in a single-wave tail; there the graphs of all scenes are built with one launch of
+  // each build kernel and queried with one launch, on the caller's stream (DESIGN section 4.2).
+  const bool batched = B > LANES;
   GF_CUDA(cudaEventRecord(fj->fork, st));
   for (int l = 0; l < lanes; ++l) {
     if (!seeds_given) GF_CUDA(cudaStreamWaitEvent(fj->fps[l], fj->fork, 0));
-    if (l > 0) GF_CUDA(cudaStreamWaitEvent(fj->knn[l], fj->fork, 0));
+    if (l > 0 && !batched) GF_CUDA(cudaStreamWaitEvent(fj->knn[l], fj->fork, 0));
   }
   GeoSceneDesc desc[GEO_BATCH_MAX];
   int64_t *d_stats = stats ? (int64_t *)(w + p.stats) : nullptr;
@@ -273,33 +285,49 @@ extern "C" int gf_guidance_batch(const float *const *xyz, const int *Ns, int B, 
                                       fj->fps[b % lanes]);
       if (rc) return rc;
     }
+  KnnBuildScene ks[GEO_BATCH_MAX];
+  KnnGridBuffers gb[GEO_BATCH_MAX];
+  KnnEdgeOut eo[GEO_BATCH_MAX];
+  KnnQueryJob jobs[GEO_BATCH_MAX];
+  for (int b = 0; b < B; ++b) ks[b] = {xyz[b], Ns[b], w + p.per_scene[b * 3 + 1], knn_b[b]};
+  if (batched) {
+    rc = knn_grid_build_batch(ks, B, k, w + p.knn_ctl, st, gb);
+    if (rc) return rc;
+  }
   for (int b = 0; b < B; ++b) {
     const int l = b % lanes;
-    cudaStream_t ks = l == 0 ? st : fj->knn[l];
-    KnnGridBuffers gb;
-    rc = knn_grid_build(xyz[b], Ns[b], k, w + p.per_scene[b * 3 + 1], knn_b[b], ks, &gb);
-    if (rc) return rc;
-    KnnEdgeOut eo;
-    eo.radius = radius;
+    cudaStream_t kst = l == 0 ? st : fj->knn[l];
+    if (!batched) {
+      rc = knn_grid_build_batch(&ks[b], 1, k, nullptr, kst, &gb[b]);
+      if (rc) return rc;
+    }
+    eo[b].radius = radius;
     int enc = 0;
-    rc = geodesic_edge_buffers(w + p.per_scene[b * 3 + 2], edge_b[b], Ns[b], k, 1, &eo.tgt, &eo.len, &eo.slot_bits,
-                               &enc);
+    rc = geodesic_edge_buffers(w + p.per_scene[b * 3 + 2], edge_b[b], Ns[b], k, 1, &eo[b].tgt, &eo[b].len,
+                               &eo[b].slot_bits, &enc);
     if (rc) return rc;
-    eo.rank = gb.rank;  // cell-order table (every scene of a batched call is batchable: checked above)
-    rc = knn_grid_query(gb, nullptr, Ns[b], k, /*sqrt=*/1, nullptr, nullptr, nullptr, ks, &eo);
-    if (rc) return rc;
-    desc[b].tgt = eo.tgt, desc[b].len = eo.len, desc[b].seeds = seeds[b], desc[b].geo = geo[b];
-    desc[b].rank = gb.rank, desc[b].order = gb.order;
+    eo[b].rank = gb[b].rank;  // cell-order table (every scene of a batched call is batchable: checked above)
+    jobs[b] = {gb[b], nullptr, Ns[b], nullptr, nullptr, nullptr, &eo[b]};
+    if (!batched) {
+      rc = knn_grid_query_batch(&jobs[b], 1, k, /*sqrt=*/1, kst);
+      if (rc) return rc;
+    }
+    desc[b].tgt = eo[b].tgt, desc[b].len = eo[b].len, desc[b].seeds = seeds[b], desc[b].geo = geo[b];
+    desc[b].rank = gb[b].rank, desc[b].order = gb[b].order;
     desc[b].row_max = row_max ? row_max[b] : nullptr;
     desc[b].stats = d_stats ? d_stats + 2 * b : nullptr;
     desc[b].N = Ns[b], desc[b].Q = Q;
+  }
+  if (batched) {
+    rc = knn_grid_query_batch(jobs, B, k, /*sqrt=*/1, st);
+    if (rc) return rc;
   }
   for (int l = 0; l < lanes; ++l) {
     if (!seeds_given) {
       GF_CUDA(cudaEventRecord(fj->join_fps[l], fj->fps[l]));
       GF_CUDA(cudaStreamWaitEvent(st, fj->join_fps[l], 0));
     }
-    if (l > 0) {
+    if (l > 0 && !batched) {
       GF_CUDA(cudaEventRecord(fj->join_knn[l], fj->knn[l]));
       GF_CUDA(cudaStreamWaitEvent(st, fj->join_knn[l], 0));
     }

@@ -117,10 +117,29 @@ __device__ __forceinline__ int cell_of(const KnnGrid &g, float x, float y, float
   return (cz * g.dy + cy) * g.dx + cx;
 }
 
+// ---- batched build: blockIdx.y = scene, blockIdx.x = block of that scene ------------------------------------------
+// Every kernel below reads its scene's descriptor from the parameter struct; gridDim.x blocks work on each scene, so the
+// per-scene planning tails ("last block done") and the scan's chaining stay within one scene.
+struct KnnBuildDesc {
+  const float *xyz;
+  KnnCtl *ctl;
+  int *coarse_count, *cell_count, *cell_start, *cell_id, *slot, *order, *rank;
+  float4 *sorted;
+  int N, cap_coarse, cap_fine;
+};
+struct KnnBuildArgs {
+  KnnBuildDesc s[KNN_BATCH_MAX];
+  float tau;
+};
+
 // build kernel 1 of 5: bounding box (+ tail: coarse grid plan) and the zero fill of both cell tables
-__global__ void __launch_bounds__(256) knn_bbox_kernel(const float *__restrict__ xyz, int N, KnnGrid *g, float tau,
-                                                       int cap_coarse, int4 *__restrict__ zero_a, int n4_a,
-                                                       int4 *__restrict__ zero_b, int n4_b) {
+__global__ void __launch_bounds__(256) knn_bbox_kernel(const __grid_constant__ KnnBuildArgs ba) {
+  const KnnBuildDesc &d = ba.s[blockIdx.y];
+  const float *__restrict__ xyz = d.xyz;
+  const int N = d.N;
+  KnnGrid *g = &d.ctl->g;
+  int4 *__restrict__ zero_a = (int4 *)d.coarse_count, *__restrict__ zero_b = (int4 *)d.cell_count;
+  const int n4_a = (d.cap_coarse + 3) / 4, n4_b = (d.cap_fine + 4) / 4;
   const int gtid = blockIdx.x * blockDim.x + threadIdx.x, gsz = gridDim.x * blockDim.x;
   const int4 z4 = make_int4(0, 0, 0, 0);
   for (int i = gtid; i < n4_a; i += gsz) zero_a[i] = z4;
@@ -146,15 +165,20 @@ __global__ void __launch_bounds__(256) knn_bbox_kernel(const float *__restrict__
       if (h) atomicMax(&g->mm[3 + a], h);
     }
   }
-  if (last_block_done(&g->done[0]) && threadIdx.x == 0) knn_plan(g, N, 0, tau, cap_coarse);
+  if (last_block_done(&g->done[0]) && threadIdx.x == 0) knn_plan(g, N, 0, ba.tau, d.cap_coarse);
 }
 
-// build kernels 2 and 3: population of every cell.  The coarse pass (cell_id == nullptr) also accumulates
-// sum c^2 = sum over the points of (2 * slot + 1) from the slots its atomics return, and ends with the plan of
-// the final grid; the final pass records every point's cell and slot for the scatter.
-__global__ void __launch_bounds__(256) knn_count_kernel(const float *__restrict__ xyz, int N, KnnGrid *gp,
-                                                        int *__restrict__ cell_count, int *__restrict__ cell_id,
-                                                        int *__restrict__ slot_in_cell, float tau, int cap_fine) {
+// build kernels 2 and 3: population of every cell.  The coarse pass (fine == 0) counts into the coarse table and also
+// accumulates sum c^2 = sum over the points of (2 * slot + 1) from the slots its atomics return, and ends with the plan
+// of the final grid; the final pass records every point's cell and slot for the scatter.
+__global__ void __launch_bounds__(256) knn_count_kernel(const __grid_constant__ KnnBuildArgs ba, int fine) {
+  const KnnBuildDesc &d = ba.s[blockIdx.y];
+  const float *__restrict__ xyz = d.xyz;
+  const int N = d.N;
+  KnnGrid *gp = &d.ctl->g;
+  int *__restrict__ cell_count = fine ? d.cell_count : d.coarse_count;
+  int *__restrict__ cell_id = fine ? d.cell_id : nullptr;
+  int *__restrict__ slot_in_cell = d.slot;
   const KnnGrid g = *gp;
   unsigned long long acc = 0;
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < N; i += gridDim.x * blockDim.x) {
@@ -171,16 +195,21 @@ __global__ void __launch_bounds__(256) knn_count_kernel(const float *__restrict_
   if (cell_id) return;
   for (int o = 16; o; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
   if ((threadIdx.x & 31) == 0 && acc) atomicAdd(&gp->sum_sq, acc);
-  if (last_block_done(&gp->done[1]) && threadIdx.x == 0) knn_plan(gp, N, 1, tau, cap_fine);
+  if (last_block_done(&gp->done[1]) && threadIdx.x == 0) knn_plan(gp, N, 1, ba.tau, d.cap_fine);
 }
 
-// build kernel 4: exclusive scan of the cell populations in one launch.  Block b sums its chunk and publishes
-// the sum; its carry-in is the sum of the published sums of the blocks before it (they were scheduled earlier,
-// so waiting for them cannot deadlock); then it rescans its chunk and writes the cell starts.
-__global__ void __launch_bounds__(256) knn_scan_kernel(KnnCtl *ctl, const int *__restrict__ cnt,
-                                                       int *__restrict__ start, int N) {
+// build kernel 4: exclusive scan of the cell populations in one launch.  Block b of a scene sums its chunk and
+// publishes the sum; its carry-in is the sum of the published sums of the scene's blocks before it (blocks are issued
+// x-fastest, so they were scheduled earlier and waiting for them cannot deadlock); then it rescans its chunk and
+// writes the cell starts.  gridDim.x <= KNN_SCAN_BLOCKS.
+__global__ void __launch_bounds__(256) knn_scan_kernel(const __grid_constant__ KnnBuildArgs ba) {
+  const KnnBuildDesc &d = ba.s[blockIdx.y];
+  KnnCtl *ctl = d.ctl;
+  const int *__restrict__ cnt = d.cell_count;
+  int *__restrict__ start = d.cell_start;
+  const int N = d.N;
   const int n = ctl->g.ncells;
-  const int chunk = (((n + KNN_SCAN_BLOCKS - 1) / KNN_SCAN_BLOCKS) + 3) & ~3;
+  const int chunk = (((n + (int)gridDim.x - 1) / (int)gridDim.x) + 3) & ~3;
   const int b0 = min(n, (int)blockIdx.x * chunk), b1 = min(n, b0 + chunk);
   __shared__ int ws[8];
   __shared__ int carry;
@@ -241,10 +270,13 @@ __global__ void __launch_bounds__(256) knn_scan_kernel(KnnCtl *ctl, const int *_
 }
 
 // build kernel 5: the points in cell order, each with its original index
-__global__ void knn_scatter_kernel(const float *__restrict__ xyz, int N, const int *__restrict__ cell_id,
-                                   const int *__restrict__ slot_in_cell, const int *__restrict__ start,
-                                   float4 *__restrict__ sorted, int *__restrict__ order, int *__restrict__ rank) {
-  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < N; i += gridDim.x * blockDim.x) {
+__global__ void __launch_bounds__(256) knn_scatter_kernel(const __grid_constant__ KnnBuildArgs ba) {
+  const KnnBuildDesc &d = ba.s[blockIdx.y];
+  const float *__restrict__ xyz = d.xyz;
+  const int *__restrict__ cell_id = d.cell_id, *__restrict__ slot_in_cell = d.slot, *__restrict__ start = d.cell_start;
+  float4 *__restrict__ sorted = d.sorted;
+  int *__restrict__ order = d.order, *__restrict__ rank = d.rank;
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < d.N; i += gridDim.x * blockDim.x) {
     int pos = start[cell_id[i]] + slot_in_cell[i];
     float x = __ldg(xyz + (size_t)i * 3), y = __ldg(xyz + (size_t)i * 3 + 1), z = __ldg(xyz + (size_t)i * 3 + 2);
     sorted[pos] = make_float4(x, y, z, __int_as_float(i));
@@ -359,6 +391,42 @@ struct TopK {
 };
 
 // ---- grid query ---------------------------------------------------------------------------------
+// One launch covers the queries of up to KNN_BATCH_MAX scenes: scene i owns the 128-query blocks
+// [block0, block0 + ceil(nq / 128)) of the grid, so a block belongs to exactly one scene.
+struct KnnQueryDesc {
+  const KnnGrid *grid;
+  const float4 *sorted;
+  const int *start;
+  const float *queries;  // nullptr: the scene's own points, in cell order
+  float *dist;
+  long long *idx64;
+  int *idx32;
+  KnnEdgeOut eo;
+  int nq, block0;
+};
+struct KnnQueryArgs {
+  KnnQueryDesc s[KNN_BATCH_MAX];
+  int B, k, do_sqrt;
+};
+// the block's scene (the last one whose first block is at or before this block) and its arguments under the names
+// the query code uses.  PTR is how the pointers are held: `const &` reads them from the parameter space where they are
+// used (copies held in registers from the start cost the k <= 16 kernels more spills than plain kernel parameters
+// do); `__restrict__` copies them (the k = 64 kernel, 1 block per SM, is faster that way: 0.88 vs 0.91 ms per c2
+// graph on a B200).
+#define KNN_QUERY_SCENE(a, PTR)                                                                       \
+  int sc_ = 0;                                                                                        \
+  while (sc_ + 1 < (a).B && (int)blockIdx.x >= (a).s[sc_ + 1].block0) ++sc_;                          \
+  const KnnQueryDesc &d = (a).s[sc_];                                                                 \
+  const KnnGrid *PTR gp = d.grid;                                                                     \
+  const float4 *PTR sorted = d.sorted;                                                                \
+  const int *PTR start = d.start;                                                                     \
+  const float *PTR queries = d.queries;                                                               \
+  float *PTR dist = d.dist;                                                                           \
+  long long *PTR idx64 = d.idx64;                                                                     \
+  int *PTR idx32 = d.idx32;                                                                           \
+  const KnnEdgeOut &eo = d.eo;                                                                        \
+  const int nq = d.nq, k = (a).k, do_sqrt = (a).do_sqrt
+
 // Thread per query, count then collect.  Offering every candidate to the sorted list as it is scanned makes the
 // warp run the insertion at almost every candidate: a lane inserts at ~k (1 + ln(n/k)) of its n candidates, and the
 // 32 lanes insert at different ones.  Here the first shell (R <= 1: the 27 cells around the query's cell, nine
@@ -378,17 +446,15 @@ constexpr int KNN_NB = 32;  // bins of d2 over [0, 4 h^2); the last one also tak
 constexpr int KNN_MIN_BLOCKS = 7;  // 72 registers for k <= 16, 24 KB of shared memory per block
 template <int KT>
 __global__ void __launch_bounds__(128, KT <= 16 ? KNN_MIN_BLOCKS : 1)
-    knn_grid_query_kernel(const KnnGrid *__restrict__ gp, const float4 *__restrict__ sorted,
-                          const int *__restrict__ start, const float *__restrict__ queries, int nq, int k,
-                          int do_sqrt, float *__restrict__ dist, long long *__restrict__ idx64,
-                          int *__restrict__ idx32, const KnnEdgeOut eo) {
+    knn_grid_query_kernel(const __grid_constant__ KnnQueryArgs a) {
   // counted on the c2 scene: a lane lists ~k + 2 candidates, at most k + 10 (k = 8, 16, 32)
   constexpr int LIST = KT + 16;
   __shared__ unsigned short hist[KNN_NB][128];  // per-lane counts (a shell of more than 65535 points is not binned)
   __shared__ int list[LIST][128];               // per-lane positions in `sorted` of the collected candidates
+  KNN_QUERY_SCENE(a, const &);
   const KnnGrid g = *gp;
   const int tid = threadIdx.x;
-  const int s = blockIdx.x * blockDim.x + tid;
+  const int s = (blockIdx.x - d.block0) * blockDim.x + tid;
   if (s >= nq) return;
   if (eo.tgt && s == 0) {  // the sentinel row N: only edges to N
     const int none = eo.rank ? (int)((((unsigned)nq >> 5) << 7) | ((unsigned)nq & 31u)) : nq;
@@ -560,16 +626,13 @@ __global__ void __launch_bounds__(128, KT <= 16 ? KNN_MIN_BLOCKS : 1)
 // before its shell is exhausted; the per-shell termination test is unchanged (after draining the stacks).
 constexpr int KNN_PEND = 8;  // stack depth; a step pushes at most 4, the network runs while a stack holds > 4
 template <int KT>
-__global__ void __launch_bounds__(128, 1)
-    knn_grid_query_sync_kernel(const KnnGrid *__restrict__ gp, const float4 *__restrict__ sorted,
-                               const int *__restrict__ start, const float *__restrict__ queries, int nq, int k,
-                               int do_sqrt, float *__restrict__ dist, long long *__restrict__ idx64,
-                               int *__restrict__ idx32, const KnnEdgeOut eo) {
+__global__ void __launch_bounds__(128, 1) knn_grid_query_sync_kernel(const __grid_constant__ KnnQueryArgs a) {
   __shared__ unsigned long long pend[KNN_PEND][128];
   constexpr unsigned FULL = 0xffffffffu;
+  KNN_QUERY_SCENE(a, __restrict__);
   const KnnGrid g = *gp;
   const int tid = threadIdx.x;
-  const int s = blockIdx.x * blockDim.x + tid;
+  const int s = (blockIdx.x - d.block0) * blockDim.x + tid;
   const bool live = s < nq;
   if (eo.tgt && s == 0) {  // the sentinel row N: only edges to N
     const int none = eo.rank ? (int)((((unsigned)nq >> 5) << 7) | ((unsigned)nq & 31u)) : nq;
@@ -736,17 +799,13 @@ size_t knn_grid_workspace_bytes(int N) {
 }
 
 template <int KT>
-static void launch_grid_query(const KnnGrid *g, const float4 *sorted, const int *start, const float *queries, int nq,
-                              int k, int do_sqrt, float *dist, long long *i64, int *i32, const KnnEdgeOut &eo,
-                              cudaStream_t st) {
+static void launch_grid_query(const KnnQueryArgs &a, int blocks, cudaStream_t st) {
   // Measured (c2, B200): at k <= 32 the count-then-collect kernel; at k = 64, where an insertion is 64
   // compare-exchanges, the warp-synchronous one (10-16 % faster than offering every candidate).
   if constexpr (KT > 32)
-    knn_grid_query_sync_kernel<KT><<<(nq + 127) / 128, 128, 0, st>>>(g, sorted, start, queries, nq, k, do_sqrt, dist, i64,
-                                                                     i32, eo);
+    knn_grid_query_sync_kernel<KT><<<blocks, 128, 0, st>>>(a);
   else
-    knn_grid_query_kernel<KT><<<(nq + 127) / 128, 128, 0, st>>>(g, sorted, start, queries, nq, k, do_sqrt, dist, i64, i32,
-                                                                eo);
+    knn_grid_query_kernel<KT><<<blocks, 128, 0, st>>>(a);
 }
 template <int KT>
 static void launch_brute(const float *xyz, int N, const float *queries, int nq, int k, int do_sqrt, float *dist,
@@ -754,70 +813,121 @@ static void launch_brute(const float *xyz, int N, const float *queries, int nq, 
   knn_brute_kernel<KT><<<(nq + 127) / 128, 128, 0, st>>>(xyz, N, queries, nq, k, do_sqrt, dist, i64, i32);
 }
 
-// Five launches and one memset (round 1: thirteen launches): bbox + coarse plan | coarse count + final plan |
-// final count | scan | scatter.  Nothing returns to the host; grid dimensions are read from the device.
-int knn_grid_build(const float *xyz, int N, int k, void *workspace, size_t workspace_bytes, cudaStream_t st,
-                   KnnGridBuffers *out) {
-  const int cap_fine = knn_cap_fine(N), cap_coarse = knn_cap_coarse(N);
-  Arena a(workspace, workspace_bytes);
-  KnnCtl *ctl = a.take<KnnCtl>(1);
-  KnnGrid *g = &ctl->g;
-  int *coarse_count = a.take<int>(cap_coarse);
-  int *cell_count = a.take<int>(cap_fine + 4);
-  int *cell_start = a.take<int>(cap_fine + 4);
-  int *cell_id = a.take<int>(N);
-  int *slot = a.take<int>(N);
-  int *order = a.take<int>(N);
-  int *rank = a.take<int>(N);
-  float4 *sorted = a.take<float4>(N);
-  if (!a.ok) {
-    set_error("knn: workspace too small (%zu bytes given, %zu needed)", workspace_bytes, knn_grid_workspace_bytes(N));
-    return GF_ERR_WORKSPACE;
+size_t knn_ctl_block_bytes(int B) { return align256(sizeof(KnnCtl)) * (size_t)(B > 0 ? B : 0); }
+
+// Five launches and one memset for the whole batch (round 1: thirteen launches per scene): bbox + coarse plan |
+// coarse count + final plan | final count | scan | scatter.  Nothing returns to the host; grid dimensions are read
+// from the device.  A scene gets nb / B blocks of each kernel (at least one, and for the count and scatter kernels no
+// more than its points need): one scene keeps the single-scene grids, a batch stays about one wave wide.  How many
+// blocks share a scene changes no result: the box and the occupancy are integer reductions, the scan is exact.
+int knn_grid_build_batch(const KnnBuildScene *scenes, int B, int k, void *ctl_block, cudaStream_t st,
+                         KnnGridBuffers *out) {
+  if (B < 1 || B > KNN_BATCH_MAX || (ctl_block == nullptr && B != 1)) {
+    set_error("knn: batched build of %d scenes (1..%d, control blocks %s)", B, KNN_BATCH_MAX,
+              ctl_block ? "given" : "missing");
+    return GF_ERR_INVALID;
+  }
+  KnnBuildArgs a;
+  int maxN = 1;
+  for (int b = 0; b < B; ++b) {
+    const int N = scenes[b].N;
+    KnnBuildDesc &d = a.s[b];
+    d.xyz = scenes[b].xyz;
+    d.N = N;
+    d.cap_fine = knn_cap_fine(N), d.cap_coarse = knn_cap_coarse(N);
+    Arena ar(scenes[b].workspace, scenes[b].workspace_bytes);
+    KnnCtl *own = ar.take<KnnCtl>(1);  // the head of a single-scene workspace; a batch uses ctl_block instead
+    d.ctl = ctl_block ? (KnnCtl *)((char *)ctl_block + align256(sizeof(KnnCtl)) * b) : own;
+    d.coarse_count = ar.take<int>(d.cap_coarse);
+    d.cell_count = ar.take<int>(d.cap_fine + 4);
+    d.cell_start = ar.take<int>(d.cap_fine + 4);
+    d.cell_id = ar.take<int>(N);
+    d.slot = ar.take<int>(N);
+    d.order = ar.take<int>(N);
+    d.rank = ar.take<int>(N);
+    d.sorted = ar.take<float4>(N);
+    if (!ar.ok) {
+      set_error("knn: workspace of scene %d too small (%zu bytes given, %zu needed)", b, scenes[b].workspace_bytes,
+                knn_grid_workspace_bytes(N));
+      return GF_ERR_WORKSPACE;
+    }
+    maxN = N > maxN ? N : maxN;
+    out[b].grid = &d.ctl->g;
+    out[b].cell_start = d.cell_start;
+    out[b].sorted = d.sorted;
+    out[b].order = d.order;
+    out[b].rank = d.rank;
   }
   const int nb = num_sms() * 8;
+  const int per_scene = nb / B > 1 ? nb / B : 1;
+  const int npt = min(per_scene, (maxN + 255) / 256);
+  const int nscan = min(per_scene, KNN_SCAN_BLOCKS);
   // target cell occupancy = tau_mul x k.  Measured (c2 / c1, B200): flat between 0.12 and 0.7 for k <= 32 (0.45 kept);
   // at k = 64 smaller cells win (0.2: 0.88 ms vs 1.03 ms per graph).
   const float tau_mul = k > 32 ? 0.2f : 0.45f;
-  const float tau = fmaxf(2.f, tau_mul * (float)k);
-  const int npt = min(nb, (N + 255) / 256);
-  GF_CUDA(cudaMemsetAsync(ctl, 0, sizeof(KnnCtl), st));
-  knn_bbox_kernel<<<nb, 256, 0, st>>>(xyz, N, g, tau, cap_coarse, (int4 *)coarse_count, (cap_coarse + 3) / 4,
-                                      (int4 *)cell_count, (cap_fine + 4) / 4);
+  a.tau = fmaxf(2.f, tau_mul * (float)k);
+  GF_CUDA(cudaMemsetAsync(a.s[0].ctl, 0, ctl_block ? knn_ctl_block_bytes(B) : sizeof(KnnCtl), st));
+  knn_bbox_kernel<<<dim3(per_scene, B), 256, 0, st>>>(a);
   GF_LAUNCHED();
-  knn_count_kernel<<<npt, 256, 0, st>>>(xyz, N, g, coarse_count, nullptr, nullptr, tau, cap_fine);
+  knn_count_kernel<<<dim3(npt, B), 256, 0, st>>>(a, 0);
   GF_LAUNCHED();
-  knn_count_kernel<<<npt, 256, 0, st>>>(xyz, N, g, cell_count, cell_id, slot, tau, cap_fine);
+  knn_count_kernel<<<dim3(npt, B), 256, 0, st>>>(a, 1);
   GF_LAUNCHED();
-  knn_scan_kernel<<<KNN_SCAN_BLOCKS, 256, 0, st>>>(ctl, cell_count, cell_start, N);
+  knn_scan_kernel<<<dim3(nscan, B), 256, 0, st>>>(a);
   GF_LAUNCHED();
-  knn_scatter_kernel<<<npt, 256, 0, st>>>(xyz, N, cell_id, slot, cell_start, sorted, order, rank);
+  knn_scatter_kernel<<<dim3(npt, B), 256, 0, st>>>(a);
   GF_LAUNCHED();
-  out->grid = g;
-  out->cell_start = cell_start;
-  out->sorted = sorted;
-  out->order = order;
-  out->rank = rank;
+  return GF_OK;
+}
+
+int knn_grid_build(const float *xyz, int N, int k, void *workspace, size_t workspace_bytes, cudaStream_t st,
+                   KnnGridBuffers *out) {
+  const KnnBuildScene sc = {xyz, N, workspace, workspace_bytes};
+  return knn_grid_build_batch(&sc, 1, k, nullptr, st, out);
+}
+
+int knn_grid_query_batch(const KnnQueryJob *jobs, int B, int k, int do_sqrt, cudaStream_t st) {
+  if (B < 1 || B > KNN_BATCH_MAX) {
+    set_error("knn: batched query of %d scenes (1..%d)", B, KNN_BATCH_MAX);
+    return GF_ERR_INVALID;
+  }
+  KnnQueryArgs a;
+  a.B = B, a.k = k, a.do_sqrt = do_sqrt;
+  int blocks = 0;
+  for (int b = 0; b < B; ++b) {
+    const KnnQueryJob &j = jobs[b];
+    KnnQueryDesc &d = a.s[b];
+    d.grid = (const KnnGrid *)j.grid.grid;
+    d.sorted = j.grid.sorted;
+    d.start = j.grid.cell_start;
+    d.queries = j.queries;
+    d.dist = j.dist, d.idx64 = j.idx64, d.idx32 = j.idx32;
+    d.eo = {nullptr, nullptr, 0.f, 0, nullptr};
+    if (j.edges && j.queries == nullptr) {
+      d.eo = *j.edges;
+      if (d.eo.rank) d.eo.rank = j.grid.rank;  // any non-null value asks for the cell-order format
+    }
+    d.nq = j.nq;
+    d.block0 = blocks;
+    blocks += (j.nq + 127) / 128;
+  }
+  if (blocks == 0) return GF_OK;
+  if (k <= 8)
+    launch_grid_query<8>(a, blocks, st);
+  else if (k <= 16)
+    launch_grid_query<16>(a, blocks, st);
+  else if (k <= 32)
+    launch_grid_query<32>(a, blocks, st);
+  else
+    launch_grid_query<64>(a, blocks, st);
+  GF_LAUNCHED();
   return GF_OK;
 }
 
 int knn_grid_query(const KnnGridBuffers &b, const float *queries, int nq, int k, int do_sqrt, float *dist,
                    long long *idx64, int *idx32, cudaStream_t st, const KnnEdgeOut *edges) {
-  const KnnGrid *g = (const KnnGrid *)b.grid;
-  KnnEdgeOut eo = {nullptr, nullptr, 0.f, 0, nullptr};
-  if (edges && queries == nullptr) {
-    eo = *edges;
-    if (eo.rank) eo.rank = b.rank;  // any non-null value asks for the cell-order format
-  }
-  if (k <= 8)
-    launch_grid_query<8>(g, b.sorted, b.cell_start, queries, nq, k, do_sqrt, dist, idx64, idx32, eo, st);
-  else if (k <= 16)
-    launch_grid_query<16>(g, b.sorted, b.cell_start, queries, nq, k, do_sqrt, dist, idx64, idx32, eo, st);
-  else if (k <= 32)
-    launch_grid_query<32>(g, b.sorted, b.cell_start, queries, nq, k, do_sqrt, dist, idx64, idx32, eo, st);
-  else
-    launch_grid_query<64>(g, b.sorted, b.cell_start, queries, nq, k, do_sqrt, dist, idx64, idx32, eo, st);
-  GF_LAUNCHED();
-  return GF_OK;
+  const KnnQueryJob j = {b, queries, nq, dist, idx64, idx32, edges};
+  return knn_grid_query_batch(&j, 1, k, do_sqrt, st);
 }
 
 }  // namespace gf
@@ -858,4 +968,46 @@ extern "C" int gf_knn(const float *xyz, int N, const float *queries, int nq, int
   int rc = knn_grid_build(xyz, N, k, workspace, workspace_bytes, st, &b);
   if (rc) return rc;
   return knn_grid_query(b, queries, nq, k, sqrt_out, dist, (long long *)idx64, idx32, st);
+}
+
+// ---- a batch of scenes, each against itself: one build and one query launch for all of them -------------------------
+static size_t knn_batch_layout(const int *Ns, int B, size_t *off) {
+  size_t o = align256(knn_ctl_block_bytes(B));
+  for (int b = 0; b < B; ++b) {
+    off[b] = o;
+    o += align256(knn_grid_workspace_bytes(Ns[b]));
+  }
+  return o + 1024;
+}
+
+extern "C" size_t gf_knn_batch_workspace_bytes(const int *Ns, int B) {
+  if (!Ns || B < 1 || B > KNN_BATCH_MAX) return 0;
+  for (int b = 0; b < B; ++b)
+    if (Ns[b] < 1) return 0;
+  size_t off[KNN_BATCH_MAX];
+  return knn_batch_layout(Ns, B, off);
+}
+
+extern "C" int gf_knn_batch(const float *const *xyz, const int *Ns, int B, int k, int sqrt_out, float *const *dist,
+                            int32_t *const *idx32, void *workspace, size_t workspace_bytes, void *stream) {
+  GF_CHECK_ARG(xyz && Ns && dist && idx32, "knn_batch: null pointer array");
+  GF_CHECK_ARG(B >= 1 && B <= KNN_BATCH_MAX, "knn_batch: B=%d outside [1,%d]", B, KNN_BATCH_MAX);
+  GF_CHECK_ARG(k >= 1 && k <= KNN_MAX_K, "knn_batch: k=%d outside [1,%d]", k, KNN_MAX_K);
+  for (int b = 0; b < B; ++b) GF_CHECK_ARG(Ns[b] >= 1 && xyz[b], "knn_batch: scene %d: empty or null", b);
+  size_t off[KNN_BATCH_MAX];
+  const size_t need = knn_batch_layout(Ns, B, off);
+  if (workspace == nullptr || workspace_bytes < need) {
+    set_error("knn_batch: workspace too small (%zu bytes given, %zu needed)", workspace_bytes, need);
+    return GF_ERR_WORKSPACE;
+  }
+  cudaStream_t st = (cudaStream_t)stream;
+  char *w = (char *)workspace;
+  KnnBuildScene sc[KNN_BATCH_MAX];
+  KnnGridBuffers gb[KNN_BATCH_MAX];
+  KnnQueryJob jobs[KNN_BATCH_MAX];
+  for (int b = 0; b < B; ++b) sc[b] = {xyz[b], Ns[b], w + off[b], align256(knn_grid_workspace_bytes(Ns[b]))};
+  int rc = knn_grid_build_batch(sc, B, k, w, st, gb);
+  if (rc) return rc;
+  for (int b = 0; b < B; ++b) jobs[b] = {gb[b], nullptr, Ns[b], dist[b], nullptr, idx32[b], nullptr};
+  return knn_grid_query_batch(jobs, B, k, sqrt_out, st);
 }

@@ -98,6 +98,13 @@ size_t gf_knn_workspace_bytes(int N, int nq, int k, int algo);
 int gf_knn(const float *xyz, int N, const float *queries, int nq, int k, int sqrt_out, float *dist, int64_t *idx64,
            int32_t *idx32, int algo, void *workspace, size_t workspace_bytes, void *stream);
 
+/* B <= 32 scenes, each against itself, through one launch of each grid-build kernel and one query launch:
+ * scene b's dist[b] (Ns[b],k) f32 and idx32[b] (Ns[b],k) i32 (either may be NULL) equal what gf_knn with
+ * queries == NULL and algo 0 writes for that scene alone.                                          */
+size_t gf_knn_batch_workspace_bytes(const int *Ns, int B);
+int gf_knn_batch(const float *const *xyz, const int *Ns, int B, int k, int sqrt_out, float *const *dist,
+                 int32_t *const *idx32, void *workspace, size_t workspace_bytes, void *stream);
+
 /* ---- geodesic propagation (cal_geodesic_vectorize, geodesic_utils.py:91-164) ---------------- */
 
 /* One scene.  knn_dist (N,k) f32 (sqrt'ed), knn_idx (N,k) i64 or i32 (idx_is_i64), column 0 is
