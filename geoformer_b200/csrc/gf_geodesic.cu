@@ -97,24 +97,47 @@ __global__ void geo_pack_edges_kernel(const float *__restrict__ D, const void *_
       const float w = __ldg(D + at);
       if (w <= radius && t >= 0 && t < N) to = (int)t, wo = w;
     }
-    tgt[e] = enc ? (int)(((unsigned)to >> 5) << 7 | ((unsigned)to & 31u)) : to;
+    tgt[e] = enc ? geo_edge_code((unsigned)to) : to;
     len[e] = wo;
   }
 }
 
 // ---- frontier storage -------------------------------------------------------------------------------
-// Entry i of a frontier: the first GEO_QCAP live in shared memory, the rest in the CTA's global
-// overflow area.  Consecutive levels hold disjoint point sets (F_L + F_{L+1} <= N + 1), so ONE buffer
+// Entry i of a frontier: the first qcap live in shared memory, the rest in the CTA's global overflow area
+// (both propagation kernels).  Consecutive levels hold disjoint point sets (F_L + F_{L+1} <= N + 1), so ONE buffer
 // of N + 2 entries serves both: odd levels grow up from index 0, even levels grow down from the top.
-__device__ __forceinline__ size_t ovf_index(int i, int level_parity, int N) {
-  const size_t j = (size_t)(i - GEO_QCAP);
+__device__ __forceinline__ size_t ovf_index(int i, int level_parity, int N, int qcap) {
+  const size_t j = (size_t)(i - qcap);
   return level_parity ? j : (size_t)N + 1 - j;
 }
 __device__ __forceinline__ void frontier_put(int *sq, int *ovf, int i, int level_parity, int N, int t) {
   if (i < GEO_QCAP)
     sq[i] = t;
   else
-    ovf[ovf_index(i, level_parity, N)] = t;
+    ovf[ovf_index(i, level_parity, N, GEO_QCAP)] = t;
+}
+
+// A row of N floats as 16-byte pieces: `head` floats before the first aligned address, `nvec` float4, then the
+// floats from `tail0` on
+struct RowSplit {
+  size_t head, nvec;
+  __device__ __forceinline__ size_t tail0() const { return head + nvec * 4; }
+};
+__device__ __forceinline__ RowSplit row_split(const float *row, int N) {
+  const size_t head = ((16 - ((uintptr_t)row & 15)) & 15) / 4;
+  const size_t h = head < (size_t)N ? head : (size_t)N;
+  return {h, ((size_t)N - h) / 4};
+}
+
+// The maximum over the block of v (unsigned), valid in thread 0.  s_max: THREADS / 32 words of shared memory.
+template <int THREADS>
+__device__ __forceinline__ uint32_t block_max_u32(uint32_t v, uint32_t *s_max, unsigned tid) {
+  const uint32_t wm = __reduce_max_sync(0xffffffffu, v);
+  if ((tid & 31u) == 0) s_max[tid >> 5] = wm;
+  __syncthreads();
+  uint32_t m = 0u;
+  if (tid < 32) m = __reduce_max_sync(0xffffffffu, tid < THREADS / 32 ? s_max[tid] : 0u);
+  return m;
 }
 
 // one candidate edge p --(slot)--> t of the current level (t == N for padding / unusable edges)
@@ -203,15 +226,12 @@ __global__ void __launch_bounds__(GEO_THREADS, 2048 / GEO_THREADS) geo_seed_bfs_
     if (tid == 0) asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(tr_t0));
 #endif
     {  // init: row = -1 (geodesic_utils.py:113), visited = claimed = {} (:114), sentinel bit N set
-      const size_t head = ((16 - ((uintptr_t)row & 15)) & 15) / 4;
-      const size_t h = head < (size_t)N ? head : (size_t)N;
-      const size_t nvec = ((size_t)N - h) / 4;
-      float4 *r4 = reinterpret_cast<float4 *>(row + h);
+      const RowSplit rs = row_split(row, N);
+      float4 *r4 = reinterpret_cast<float4 *>(row + rs.head);
       const float4 m1 = make_float4(-1.f, -1.f, -1.f, -1.f);
-      for (size_t i = tid; i < nvec; i += GEO_THREADS) r4[i] = m1;
-      if ((size_t)tid < h) row[tid] = -1.f;
-      const size_t tail0 = h + nvec * 4;
-      if ((size_t)tid < (size_t)N - tail0) row[tail0 + tid] = -1.f;
+      for (size_t i = tid; i < rs.nvec; i += GEO_THREADS) r4[i] = m1;
+      if ((size_t)tid < rs.head) row[tid] = -1.f;
+      if ((size_t)tid < (size_t)N - rs.tail0()) row[rs.tail0() + tid] = -1.f;
       if (BITMAP)
         for (int i = tid; i < (MODE == 2 ? 2 : 1) * a.bitmap_words; i += GEO_THREADS) vis[i] = 0u;  // vis, clm contiguous
     }
@@ -239,7 +259,9 @@ __global__ void __launch_bounds__(GEO_THREADS, 2048 / GEO_THREADS) geo_seed_bfs_
       row[t] = d;
       rmax = fmaxf(rmax, d);
     };
-    auto frontier_at = [&](const int *q, int i, int won) { return i < GEO_QCAP ? q[i] : ovf[ovf_index(i, won & 1, N)]; };
+    auto frontier_at = [&](const int *q, int i, int won) {
+      return i < GEO_QCAP ? q[i] : ovf[ovf_index(i, won & 1, N, GEO_QCAP)];
+    };
     while (F > 0 && level < a.max_step) {
       ++level;
       // The points of this frontier were won at level-1 and still hold their keys.  Their distances are
@@ -295,7 +317,7 @@ __global__ void __launch_bounds__(GEO_THREADS, 2048 / GEO_THREADS) geo_seed_bfs_
         }
       }
       for (int node = GEO_QCAP + (int)group; node < F; node += (int)ngroups) {  // spilled tail (rare)
-        const unsigned pl = (unsigned)ovf[ovf_index(node, (level - 1) & 1, N)] << lsb;
+        const unsigned pl = (unsigned)ovf[ovf_index(node, (level - 1) & 1, N, GEO_QCAP)] << lsb;
         const int4 t = __ldg(trow + pl);
         const uint32_t key = keybase | (pl << 2);
         geo_claim4<MODE>(key, t, N, level, vis, clm, rowu, nq, ovf, &s_next_n[level & 1]);
@@ -378,33 +400,25 @@ __global__ void __launch_bounds__(GEO_THREADS, 2048 / GEO_THREADS) geo_seed_bfs_
     if (a.row_max) {
       // max over the row = max over what was written (the seed's 0 included), or -1 for a row that stayed empty;
       // distances are non-negative, so their bit patterns order like unsigned integers
-      const uint32_t wm = __reduce_max_sync(0xffffffffu, __float_as_uint(rmax));
-      if ((tid & 31u) == 0) s_rmax[tid >> 5] = wm;
-      __syncthreads();
-      if (tid < 32) {
-        const uint32_t v = tid < GEO_THREADS / 32 ? s_rmax[tid] : 0u;
-        const uint32_t m = __reduce_max_sync(0xffffffffu, v);
-        if (tid == 0) a.row_max[q] = seed_ok ? __uint_as_float(m) : -1.f;
-      }
+      const uint32_t m = block_max_u32<GEO_THREADS>(__float_as_uint(rmax), s_rmax, tid);
+      if (tid == 0) a.row_max[q] = seed_ok ? __uint_as_float(m) : -1.f;
     }
     if (a.n_peers > 0) {
       // The row is final: push it into every peer's matrix now, while other CTAs are still propagating --
       // the exchange of a seed-sharded scene rides under the compute instead of following it as a
       // collective.  Same row index on every rank => same 16-byte alignment; stores over NVLink are posted.
       __syncthreads();
-      const size_t head = ((16 - ((uintptr_t)row & 15)) & 15) / 4;
-      const size_t h = head < (size_t)N ? head : (size_t)N;
-      const size_t nvec = ((size_t)N - h) / 4, tail0 = h + nvec * 4;
-      const float4 *s4 = reinterpret_cast<const float4 *>(row + h);
-      for (size_t i = tid; i < nvec; i += GEO_THREADS) {
+      const RowSplit rs = row_split(row, N);
+      const float4 *s4 = reinterpret_cast<const float4 *>(row + rs.head);
+      for (size_t i = tid; i < rs.nvec; i += GEO_THREADS) {
         const float4 v = __ldcg(s4 + i);
         for (int r = 0; r < a.n_peers; ++r)
-          __stcs(reinterpret_cast<float4 *>(a.peer_geo[r] + (size_t)q * N + h) + i, v);
+          __stcs(reinterpret_cast<float4 *>(a.peer_geo[r] + (size_t)q * N + rs.head) + i, v);
       }
-      if ((size_t)tid < h)
+      if ((size_t)tid < rs.head)
         for (int r = 0; r < a.n_peers; ++r) a.peer_geo[r][(size_t)q * N + tid] = __ldcg(row + tid);
-      if ((size_t)tid < (size_t)N - tail0)
-        for (int r = 0; r < a.n_peers; ++r) a.peer_geo[r][(size_t)q * N + tail0 + tid] = __ldcg(row + tail0 + tid);
+      if ((size_t)tid < (size_t)N - rs.tail0())
+        for (int r = 0; r < a.n_peers; ++r) a.peer_geo[r][(size_t)q * N + rs.tail0() + tid] = __ldcg(row + rs.tail0() + tid);
     }
 #ifdef GF_TRACE
     __syncthreads();
@@ -446,7 +460,7 @@ __global__ void __launch_bounds__(GEO_THREADS, 2048 / GEO_THREADS) geo_seed_bfs_
 //  * Work items are the (scene, seed) pairs of a whole BATCH of scenes (the reference's call is batched:
 //    cal_geodesic_vectorize loops over the scenes of a batch, geodesic_utils.py:98), pulled from one counter by
 //    persistent CTAs: one launch, one tail per batch instead of one per scene.
-//  * Edge targets are stored ENCODED (see geo_claim4_enc) so that the visited test is four instructions.
+//  * Edge targets are stored ENCODED (geo_edge_code, gf_geodesic.cuh) so that the visited test is four instructions.
 constexpr int GEO_MAXB = 32;  // scenes per launch (descriptors travel in the kernel parameters)
 constexpr uint32_t GEO_UNCLAIMED = 0xFFFFFFFFu;
 constexpr uint32_t GEO_DISTANCE = 0x80000000u;  // entries >= this are distances (or never touched), below: claim keys
@@ -473,25 +487,22 @@ struct GeoBatchArgs {
 #endif
 };
 
-// ENCODED edge targets: the edge table stores a target t as (t >> 5) << 7 | (t & 31), i.e. the byte offset of its
-// bitmap word shifted left by 5 with the bit number in the low five bits.  The visited test of an edge -- 93 % of
-// the edges of a kNN graph fail it -- is then four instructions (shift, LDS, funnel shift for the bit, LOP3 into a
-// predicate) instead of eight; the byte offset into the claim array (4 * t) is only rebuilt on the rare hit.
-// The four visited words are fetched first (independent loads), then tested.
+// The claims of four ENCODED edge targets (geo_edge_code, gf_geodesic.cuh).  The four visited words are fetched first
+// (independent loads), then tested.
 __device__ __forceinline__ void geo_claim4_enc(uint32_t key, const int4 t, uint32_t vis_s, uint32_t clm_s,
                                                unsigned char *claimb) {
   const unsigned tt[4] = {(unsigned)t.x, (unsigned)t.y, (unsigned)t.z, (unsigned)t.w};
   uint32_t w[4];
 #pragma unroll
-  for (int e = 0; e < 4; ++e) asm("ld.shared.u32 %0, [%1];" : "=r"(w[e]) : "r"(vis_s + (tt[e] >> 5)));
+  for (int e = 0; e < 4; ++e) asm("ld.shared.u32 %0, [%1];" : "=r"(w[e]) : "r"(vis_s + geo_edge_word_offset(tt[e])));
 #pragma unroll
   for (int e = 0; e < 4; ++e) {
     const uint32_t bit = __funnelshift_l(0u, 1u, tt[e]);  // 1 << (t & 31)
     if (!(w[e] & bit)) {
-      const uint32_t boff = (tt[e] & ~127u) | ((tt[e] & 31u) << 2);  // 4 * t
       // both fire and forget (RED.MIN, ATOMS.OR without a destination)
-      asm volatile("red.relaxed.gpu.global.min.u32 [%0], %1;" ::"l"(claimb + boff), "r"(key + e) : "memory");
-      asm volatile("red.shared.or.b32 [%0], %1;" ::"r"(clm_s + (tt[e] >> 5)), "r"(bit) : "memory");
+      asm volatile("red.relaxed.gpu.global.min.u32 [%0], %1;" ::"l"(claimb + geo_edge_entry_offset(tt[e])), "r"(key + e)
+                   : "memory");
+      asm volatile("red.shared.or.b32 [%0], %1;" ::"r"(clm_s + geo_edge_word_offset(tt[e])), "r"(bit) : "memory");
     }
   }
 }
@@ -542,10 +553,7 @@ __global__ void __launch_bounds__(THREADS, 2048 / THREADS) geo_bfs_batch_kernel(
     const GeoScene &S = a.sc[b];
     const int q = item - S.item0, N = S.N, words = S.bitmap_words;
     const int *__restrict__ rank = S.rank, *__restrict__ order = S.order;
-    // frontier entry i >= QC lives in the CTA's overflow area: consecutive levels hold disjoint point sets
-    // (F_L + F_{L+1} <= N + 1), so one buffer of N + 2 entries serves both, odd levels from the bottom, even from the top
-    auto ovf_at = [&](int i, int parity) { return parity ? (size_t)(i - QC) : (size_t)N + 1 - (size_t)(i - QC); };
-    auto frontier = [&](int i, int parity) { return i < QC ? fq_at(i) : ovf[ovf_at(i, parity)]; };
+    auto frontier = [&](int i, int parity) { return i < QC ? fq_at(i) : ovf[ovf_index(i, parity, N, QC)]; };
     uint32_t clm_s = vis_s + 4u * (uint32_t)words;
     asm volatile("mov.u32 %0, %0;" : "+r"(clm_s));
     const int4 *__restrict__ trow = reinterpret_cast<const int4 *>(S.tgt) + sub;  // + (p << lsb)
@@ -620,7 +628,7 @@ __global__ void __launch_bounds__(THREADS, 2048 / THREADS) geo_bfs_batch_kernel(
         geo_claim4_enc((po << sb) | keysub, t, vis_s, clm_s, claimb);
       }
       for (int node = QC + (int)group; node < F; node += (int)ngroups) {  // spilled tail (rare)
-        const int p = ovf[ovf_at(node, (level - 1) & 1)];
+        const int p = ovf[ovf_index(node, (level - 1) & 1, N, QC)];
         const unsigned po = order ? (unsigned)__ldg(order + p) : (unsigned)p;
         geo_claim4_enc((po << sb) | keysub, __ldg(trow + ((unsigned)p << lsb)), vis_s, clm_s, claimb);
       }
@@ -700,7 +708,7 @@ __global__ void __launch_bounds__(THREADS, 2048 / THREADS) geo_bfs_batch_kernel(
               if (at < QC)
                 fq[at] = t;
               else
-                ovf[ovf_at(at, par)] = t;
+                ovf[ovf_index(at, par, N, QC)] = t;
               ++at;
             }
           }
@@ -729,7 +737,7 @@ __global__ void __launch_bounds__(THREADS, 2048 / THREADS) geo_bfs_batch_kernel(
       float *row = S.geo + (size_t)q * N;
       auto value = [&](int r) {
         uint32_t w;
-        asm("ld.shared.u32 %0, [%1];" : "=r"(w) : "r"(vis_s + (((unsigned)r >> 3) & ~3u)));
+        asm("ld.shared.u32 %0, [%1];" : "=r"(w) : "r"(vis_s + geo_word_offset((unsigned)r)));
         return (w >> (r & 31)) & 1u ? __uint_as_float(__ldcg(claim + r) & 0x7FFFFFFFu) : -1.f;
       };
       if ((((uintptr_t)row) & 15) == 0) {
@@ -745,16 +753,10 @@ __global__ void __launch_bounds__(THREADS, 2048 / THREADS) geo_bfs_batch_kernel(
       }
     }
     if (S.row_max) {
-      // max over the row = max over the distances written (the seed's 0 included), or -1 for a row that stayed
-      // empty; distances are non-negative, so their bit patterns order like unsigned integers
-      const uint32_t wm = __reduce_max_sync(0xffffffffu, __float_as_uint(rmax));
-      if ((tid & 31u) == 0) s_rmax[tid >> 5] = wm;
-      __syncthreads();
-      if (tid < 32) {
-        const uint32_t v = tid < THREADS / 32 ? s_rmax[tid] : 0u;
-        const uint32_t m = __reduce_max_sync(0xffffffffu, v);
-        if (tid == 0) S.row_max[q] = seed_ok ? __uint_as_float(m) : -1.f;
-      }
+      // max over the row = max over what was written (the seed's 0 included), or -1 for a row that stayed empty;
+      // distances are non-negative, so their bit patterns order like unsigned integers
+      const uint32_t m = block_max_u32<THREADS>(__float_as_uint(rmax), s_rmax, tid);
+      if (tid == 0) S.row_max[q] = seed_ok ? __uint_as_float(m) : -1.f;
     }
     if (tid == 0 && S.stats) {
       if (reached) atomicAdd(S.stats, reached);
@@ -860,53 +862,72 @@ static void plan_batch(int maxN, long long items, GeoBatchPlan *p) {
   p->grid = (int)(grid < 1 ? 1 : grid);
 }
 
-static size_t geo_edge_bytes(int N, int k) {
-  return 2 * align256(sizeof(int) * (((size_t)N + 1) << geo_slot_bits(k)));
-}
+// ---- workspace layouts, each stated once in a carve function that sizes it (over a null workspace) and hands it out
+// Control block of a launch, cleared by one memset: the counter the CTAs pull seeds from, and the statistics
+// (accumulated with atomics, a line apart from the counter)
+struct GeoCtl {
+  unsigned counter;
+  alignas(128) unsigned long long stats[2];  // reached pairs, deepest level
+};
 
-// scratch of one batched launch: frontier overflow + the item counter
+// scratch of one batched launch: per CTA the frontier overflow and the claim array, then the control block
+struct GeoBatchScratch {
+  int *overflow;
+  uint32_t *claim;
+  GeoCtl *ctl;
+};
+static Arena geo_batch_carve(void *scratch, size_t scratch_bytes, const GeoBatchPlan &p, GeoBatchScratch *s) {
+  Arena a(scratch, scratch_bytes);
+  s->overflow = a.take<int>(p.ovf_stride * (size_t)p.grid);
+  s->claim = a.take<uint32_t>(p.arr_stride * (size_t)p.grid);
+  s->ctl = a.take<GeoCtl>(1);
+  return a;
+}
 size_t geodesic_batch_scratch_bytes(int maxN, long long items) {
   GeoBatchPlan p;
   plan_batch(maxN, items, &p);
-  return align256(sizeof(int) * p.ovf_stride * (size_t)p.grid) + align256(sizeof(int) * p.arr_stride * (size_t)p.grid) +
-         align256(256) + 1024;
+  GeoBatchScratch s;
+  return geo_batch_carve(nullptr, 0, p, &s).off + 1024;
 }
 
-size_t geodesic_workspace_bytes(int N, int k, int Q) {
-  const size_t edges = geo_edge_bytes(N, k);  // packed edge targets + lengths (+ sentinel row)
-  GeoPlan pl;
-  plan_geo(N, Q, &pl);
-  // the per-scene kernel (big scenes; seed-sharded scenes of any size): frontier overflow, seed counter + stats
-  size_t rest = align256(sizeof(int) * ((size_t)N + 2) * (size_t)pl.grid) + align256(256);
-  if (geo_batchable(N)) {
-    const size_t r2 = geodesic_batch_scratch_bytes(N, Q);
-    rest = r2 > rest ? r2 : rest;
-  }
-  return edges + rest + 1024;
-}
-
-// workspace carve-up of the single-scene entry points, identical for sizing, packing and launching
+// workspace of the single-scene entry points: the packed edge table (+ sentinel row), then the scratch of the kernel
+// that runs, sized for either: the per-scene kernel's (big scenes; seed-sharded scenes of any size) frontier overflow
+// and control block, or for a batchable scene the scratch of a batched launch, if that is larger
 struct GeoBuffers {
   int *tgt;
   float *len;
-  void *rest;  // overflow + control block (layout depends on the kernel)
+  int *overflow;  // the per-scene kernel's scratch ...
+  GeoCtl *ctl;
+  void *rest;  // ... or a batched launch's, at the same address
   size_t rest_bytes;
 };
-static bool geo_carve(void *workspace, size_t workspace_bytes, int N, int slot_bits, GeoBuffers *b) {
+static Arena geo_carve(void *workspace, size_t workspace_bytes, int N, int k, int Q, GeoBuffers *b) {
   Arena a(workspace, workspace_bytes);
+  const int slot_bits = geo_slot_bits(k);
   b->tgt = a.take<int>(((size_t)N + 1) << slot_bits);
   b->len = a.take<float>(((size_t)N + 1) << slot_bits);
   b->rest = a.ok ? (void *)(a.base + a.off) : nullptr;
   b->rest_bytes = a.ok ? a.size - a.off : 0;
-  return a.ok;
+  GeoPlan pl;
+  plan_geo(N, Q, &pl);
+  Arena r(b->rest, b->rest_bytes);
+  b->overflow = r.take<int>(((size_t)N + 2) * (size_t)pl.grid);
+  b->ctl = r.take<GeoCtl>(1);
+  const size_t batch = geo_batchable(N) ? geodesic_batch_scratch_bytes(N, Q) : 0;
+  (void)a.take<char>(batch > r.off ? batch : r.off);
+  return a;
+}
+
+size_t geodesic_workspace_bytes(int N, int k, int Q) {
+  GeoBuffers b;
+  return geo_carve(nullptr, 0, N, k, Q, &b).off + 1024;
 }
 
 int geodesic_edge_buffers(void *workspace, size_t workspace_bytes, int N, int k, int Q, int **tgt, float **len,
                           int *slot_bits, int *enc) {
-  (void)Q;
   GeoBuffers b;
   *slot_bits = geo_slot_bits(k);
-  if (!geo_carve(workspace, workspace_bytes, N, *slot_bits, &b)) {
+  if (!geo_carve(workspace, workspace_bytes, N, k, Q, &b).ok) {
     set_error("geodesic: workspace too small (%zu bytes given, %zu needed)", workspace_bytes,
               geodesic_workspace_bytes(N, k, Q));
     return GF_ERR_WORKSPACE;
@@ -1010,18 +1031,16 @@ int geodesic_batch_launch(const GeoSceneDesc *scenes, int B, int k, int max_step
   }
   GeoBatchPlan p;
   plan_batch(maxN, items, &p);
-  Arena a(scratch, scratch_bytes);
-  ga.overflow = a.take<int>(p.ovf_stride * (size_t)p.grid);
-  ga.claim = a.take<uint32_t>(p.arr_stride * (size_t)p.grid);
-  ga.item_counter = a.take<unsigned>(64);
-  if (!a.ok) {
+  GeoBatchScratch sc;
+  if (!geo_batch_carve(scratch, scratch_bytes, p, &sc).ok) {
     set_error("geodesic: scratch too small (%zu bytes given, %zu needed)", scratch_bytes,
               geodesic_batch_scratch_bytes(maxN, items));
     return GF_ERR_WORKSPACE;
   }
+  ga.overflow = sc.overflow, ga.claim = sc.claim, ga.item_counter = &sc.ctl->counter;
   ga.ovf_stride = p.ovf_stride, ga.arr_stride = p.arr_stride;
   ga.B = B, ga.total_items = (int)items, ga.max_step = max_step, ga.slot_bits = slot_bits, ga.qcap = p.qcap;
-  GF_CUDA(cudaMemsetAsync(ga.item_counter, 0, 256, st));
+  GF_CUDA(cudaMemsetAsync(sc.ctl, 0, sizeof(GeoCtl), st));
 #ifdef GF_TRACE
   if (!g_trace) cudaMalloc(&g_trace, 8 * 4 * 1024), cudaMalloc(&g_trace2, kTrace2N * 8);
   cudaMemsetAsync(g_trace, 0, 8 * 4 * 1024, st);
@@ -1066,8 +1085,7 @@ int geodesic_run(const float *D, const void *I, int is64, int N, int k, const in
     return GF_ERR_INVALID;
   }
   GeoBuffers b;
-  if (!geo_carve(workspace, workspace_bytes, N, slot_bits, &b) ||
-      workspace_bytes < geodesic_workspace_bytes(N, k, Q) - 1024) {
+  if (!geo_carve(workspace, workspace_bytes, N, k, Q, &b).ok) {
     set_error("geodesic: workspace too small (%zu bytes given, %zu needed)", workspace_bytes,
               geodesic_workspace_bytes(N, k, Q));
     return GF_ERR_WORKSPACE;
@@ -1086,40 +1104,30 @@ int geodesic_run(const float *D, const void *I, int is64, int N, int k, const in
     GF_LAUNCHED();
   }
   if (batched) {
-    // stats of the batched kernel are accumulated with atomics: clear them here (16 bytes of the control block)
-    Arena a(b.rest, b.rest_bytes);
+    // the stats slot of the launch's control block (cleared by the launch's memset)
     GeoBatchPlan p;
     plan_batch(N, Q, &p);
-    (void)a.take<int>(p.ovf_stride * (size_t)p.grid);
-    (void)a.take<uint32_t>(p.arr_stride * (size_t)p.grid);
-    unsigned *ctl = a.take<unsigned>(64);
-    unsigned long long *stats = (unsigned long long *)(ctl + 32);  // second half of the 256-byte control block
+    GeoBatchScratch sc;
+    geo_batch_carve(b.rest, b.rest_bytes, p, &sc);
+    unsigned long long *stats = sc.ctl->stats;
     GeoSceneDesc d;
     d.tgt = b.tgt, d.len = b.len, d.seeds = seeds, d.geo = geo, d.row_max = row_max;
     d.rank = D == nullptr ? rank : nullptr, d.order = D == nullptr ? order : nullptr;  // a packed foreign graph: identity
     d.stats = stats_out ? (int64_t *)stats : nullptr;
     d.N = N, d.Q = Q;
-    int rc = geodesic_batch_launch(&d, 1, k, max_step, b.rest, b.rest_bytes, st);  // its memset clears the stats too
+    int rc = geodesic_batch_launch(&d, 1, k, max_step, b.rest, b.rest_bytes, st);
     if (rc) return rc;
     if (stats_out) GF_CUDA(cudaMemcpyAsync(stats_out, stats, 16, cudaMemcpyDeviceToDevice, st));
     return GF_OK;
   }
   GeoPlan p;
   plan_geo(N, Q, &p);
-  Arena a(b.rest, b.rest_bytes);
-  int *overflow = a.take<int>(((size_t)N + 2) * (size_t)p.grid);
-  unsigned *counter = a.take<unsigned>(64);
-  unsigned long long *stats = (unsigned long long *)(counter + 32);
-  if (!a.ok) {
-    set_error("geodesic: workspace too small (%zu bytes given, %zu needed)", workspace_bytes,
-              geodesic_workspace_bytes(N, k, Q));
-    return GF_ERR_WORKSPACE;
-  }
-  GF_CUDA(cudaMemsetAsync(counter, 0, 256, st));  // seed counter + stats
+  unsigned long long *stats = b.ctl->stats;
+  GF_CUDA(cudaMemsetAsync(b.ctl, 0, sizeof(GeoCtl), st));
   stage_mark(ST_GEO_READY, st);
   GeoArgs ga;
   ga.tgt = b.tgt, ga.len = b.len, ga.N = N, ga.Q = Q, ga.max_step = max_step, ga.slot_bits = slot_bits;
-  ga.seeds = seeds, ga.geo = geo, ga.overflow = overflow, ga.seed_counter = counter, ga.stats = stats;
+  ga.seeds = seeds, ga.geo = geo, ga.overflow = b.overflow, ga.seed_counter = &b.ctl->counter, ga.stats = stats;
   ga.bitmap_words = p.bitmap_words;
   ga.row_max = row_max;
   ga.n_peers = n_peers;

@@ -23,8 +23,6 @@ constexpr int LANES = 4;
 struct ForkJoin {
   cudaStream_t fps[LANES] = {}, knn[LANES] = {};  // knn[0] stays null: lane 0 builds its graph on the caller's stream
   cudaEvent_t fork = nullptr, join_fps[LANES] = {}, join_knn[LANES] = {};
-  cudaStream_t aux = nullptr;  // = fps[0] (single-scene entry points)
-  cudaEvent_t join = nullptr;  // = join_fps[0]
 };
 
 static int get_fork_join(cudaStream_t user, ForkJoin **out, int lanes_needed = 1) {
@@ -75,8 +73,6 @@ static int get_fork_join(cudaStream_t user, ForkJoin **out, int lanes_needed = 1
     if (l > 0) GF_CUDA(cudaStreamCreateWithPriority(&f.knn[l], cudaStreamNonBlocking, lo));
     GF_CUDA(cudaEventCreateWithFlags(&f.join_knn[l], cudaEventDisableTiming));
   }
-  f.aux = f.fps[0];
-  f.join = f.join_fps[0];
   *out = &e->fj;
   return GF_OK;
 }
@@ -135,10 +131,10 @@ static int guidance_impl(const float *xyz, int N, int Q, int k, float radius, in
     if (rc) return rc;
     // fork: FPS on the auxiliary stream
     GF_CUDA(cudaEventRecord(fj->fork, st));
-    GF_CUDA(cudaStreamWaitEvent(fj->aux, fj->fork, 0));
-    rc = gf_furthest_point_sampling(xyz, 1, N, Q, seeds, ws_fps, p.fps, fj->aux);
+    GF_CUDA(cudaStreamWaitEvent(fj->fps[0], fj->fork, 0));
+    rc = gf_furthest_point_sampling(xyz, 1, N, Q, seeds, ws_fps, p.fps, fj->fps[0]);
     if (rc) return rc;
-    GF_CUDA(cudaEventRecord(fj->join, fj->aux));
+    GF_CUDA(cudaEventRecord(fj->join_fps[0], fj->fps[0]));
   }
   // main stream: kNN graph
   KnnGridBuffers gb;
@@ -158,7 +154,7 @@ static int guidance_impl(const float *xyz, int N, int Q, int k, float radius, in
   rc = knn_grid_query(gb, nullptr, N, k, /*sqrt=*/1, knn_dist, nullptr, knn_idx32, st, &eo);
   if (rc) return rc;
   // join, then propagate
-  if (!seeds_given) GF_CUDA(cudaStreamWaitEvent(st, fj->join, 0));
+  if (!seeds_given) GF_CUDA(cudaStreamWaitEvent(st, fj->join_fps[0], 0));
   stage_mark(ST_KNN_DONE, st);
   if (Qb == 0) return GF_OK;
   return geodesic_run(nullptr, nullptr, /*is64=*/0, N, k, seeds + q0, Qb, radius, max_step, geo, stats, ws_geo, p.geo,

@@ -14,6 +14,9 @@
 //   algo 1  brute-force tiled scan (shared-memory tiles, register-resident sorted top-k).  This
 //           is the formulation named in BASELINE.json; kept as an independent cross-check.
 // 3-D coordinates make this a compare/select problem, not a contraction: no tensor cores.
+#include <type_traits>
+
+#include "gf_geodesic.cuh"
 #include "gf_knn.cuh"
 
 namespace gf {
@@ -289,6 +292,9 @@ __global__ void __launch_bounds__(256) knn_scatter_kernel(const __grid_constant_
 // 64-bit keys (d2 bits << 32 | index): lexicographic (d2, index) order, all keys distinct.
 // The list is kept ascending; slots [0, KT-k) are pinned to 0 so that the live part is always the
 // last k entries and list[KT-1] is the current k-th best.
+__device__ __forceinline__ unsigned long long knn_key(float d2, int index) {
+  return ((unsigned long long)__float_as_uint(d2) << 32) | (unsigned)index;
+}
 template <int KT>
 struct TopK {
   unsigned long long key[KT];
@@ -296,8 +302,8 @@ struct TopK {
 #pragma unroll
     for (int i = 0; i < KT; ++i) key[i] = (i < KT - k) ? 0ull : ~0ull;
   }
-  __device__ __forceinline__ void offer(float d2, int index) {
-    unsigned long long kk = ((unsigned long long)__float_as_uint(d2) << 32) | (unsigned)index;
+  __device__ __forceinline__ void offer(float d2, int index) { offer_key(knn_key(d2, index)); }
+  __device__ __forceinline__ void offer_key(unsigned long long kk) {
     if (kk < key[KT - 1]) {
       // every slot decides for itself (no compare-exchange chain through the moving key): slot i takes its lower
       // neighbour if the new key sorts below that one, the new key if it sorts below the slot's own key, else it
@@ -312,33 +318,17 @@ struct TopK {
       if (below) key[0] = kk;
     }
   }
-  __device__ __forceinline__ void offer_key(unsigned long long kk) {
-    if (kk < key[KT - 1]) {
-      bool below = true;
-#pragma unroll
-      for (int i = KT - 1; i > 0; --i) {
-        const bool below_prev = kk < key[i - 1];
-        key[i] = below_prev ? key[i - 1] : (below ? kk : key[i]);
-        below = below_prev;
-      }
-      if (below) key[0] = kk;
-    }
-  }
   __device__ __forceinline__ float kth_d2() const { return __uint_as_float((unsigned)(key[KT - 1] >> 32)); }
   // The row of the propagation's edge table (gf_geodesic.cu: geo_pack_edges_kernel, same rule): neighbour
   // 1 + e of the result as edge e if it may ever be used (sqrt(d2) <= radius, geodesic_utils.py:123,151),
   // else an edge to the sentinel point N; padded with such edges to KP = 1 << slot_bits entries.
   // rank != nullptr: the table lives in CELL ORDER (the caller passes the row of the query's cell-order position and
-  // targets are translated through rank[]) with encoded targets; else original indices, plain.
+  // targets are translated through rank[]) with encoded targets (geo_edge_code); else original indices, plain.
   __device__ __forceinline__ void store_edges(int k, float radius, int N, int slot_bits, const int *__restrict__ rank,
                                               int *__restrict__ tgt, float *__restrict__ len) const {
     const int KP = 1 << slot_bits;
-    auto code = [&](int t) {
-      if (!rank) return t;
-      const unsigned r = (unsigned)__ldg(rank + t);
-      return (int)(((r >> 5) << 7) | (r & 31u));
-    };
-    const int none = rank ? (int)((((unsigned)N >> 5) << 7) | ((unsigned)N & 31u)) : N;
+    auto code = [&](int t) { return rank ? geo_edge_code((unsigned)__ldg(rank + t)) : t; };
+    const int none = geo_edge_none(N, rank != nullptr);
     if (k == KT && KP == KT) {  // the usual case (k a power of two): whole 16-byte stores
 #pragma unroll
       for (int e0 = 0; e0 < KT; e0 += 4) {
@@ -427,6 +417,57 @@ struct KnnQueryArgs {
   const KnnEdgeOut &eo = d.eo;                                                                        \
   const int nq = d.nq, k = (a).k, do_sqrt = (a).do_sqrt
 
+// the sentinel row N of the edge table (written by the thread of query 0): only edges to N
+__device__ __forceinline__ void knn_sentinel_row(const KnnEdgeOut &eo, int nq) {
+  const int none = geo_edge_none(nq, eo.rank != nullptr);
+  for (int e = 0; e < (1 << eo.slot_bits); ++e)
+    eo.tgt[((size_t)nq << eo.slot_bits) + e] = none, eo.len[((size_t)nq << eo.slot_bits) + e] = 0.f;
+}
+
+// The bound of the termination test after shell R: the distance from the query to the nearest face of the visited
+// block that still has cells behind it (+inf once the whole grid has been visited).  Every unvisited point is at
+// least that far away, minus the fp32 slack g.slack.
+__device__ __forceinline__ float knn_unvisited_bound(const KnnGrid &g, int cx, int cy, int cz, float qx, float qy,
+                                                     float qz, int R) {
+  float mfd = __int_as_float(0x7f800000);
+  if (cx - R > 0) mfd = fminf(mfd, qx - (g.ox + (float)(cx - R) * g.h));
+  if (cx + R + 1 < g.dx) mfd = fminf(mfd, (g.ox + (float)(cx + R + 1) * g.h) - qx);
+  if (cy - R > 0) mfd = fminf(mfd, qy - (g.oy + (float)(cy - R) * g.h));
+  if (cy + R + 1 < g.dy) mfd = fminf(mfd, (g.oy + (float)(cy + R + 1) * g.h) - qy);
+  if (cz - R > 0) mfd = fminf(mfd, qz - (g.oz + (float)(cz - R) * g.h));
+  if (cz + R + 1 < g.dz) mfd = fminf(mfd, (g.oz + (float)(cz + R + 1) * g.h) - qz);
+  return mfd;
+}
+
+// The two macros below are the parts of both query kernels that read the pointers of KNN_QUERY_SCENE: macros, so
+// that each kernel keeps holding them as it declares them (a function taking them changes the count-then-collect
+// kernels' register allocation).
+// query s and the row its results go to: a point of the scene in cell order (queries == nullptr), or queries[s]
+#define KNN_QUERY_POINT()                                                                                        \
+  do {                                                                                                           \
+    if (queries == nullptr) {                                                                                    \
+      float4 me = sorted[s];                                                                                     \
+      qx = me.x, qy = me.y, qz = me.z;                                                                           \
+      row = __float_as_int(me.w);                                                                                \
+    } else {                                                                                                     \
+      qx = __ldg(queries + (size_t)s * 3), qy = __ldg(queries + (size_t)s * 3 + 1);                              \
+      qz = __ldg(queries + (size_t)s * 3 + 2);                                                                   \
+      row = s;                                                                                                   \
+    }                                                                                                            \
+  } while (0)
+// the epilogue: the (row, k) results that were asked for; for a self query (nq == N) the propagation's edge rows,
+// written straight from the registers, in the cell-order row (= this thread's s) or the original row
+#define KNN_QUERY_EPILOGUE(top)                                                                                  \
+  do {                                                                                                           \
+    if (dist || idx64 || idx32)                                                                                  \
+      (top).store(k, do_sqrt != 0, dist ? dist + (size_t)row * k : nullptr,                                      \
+                  idx64 ? idx64 + (size_t)row * k : nullptr, idx32 ? idx32 + (size_t)row * k : nullptr);         \
+    if (eo.tgt) {                                                                                                \
+      const size_t er = (size_t)(eo.rank ? s : row) << eo.slot_bits;                                             \
+      (top).store_edges(k, eo.radius, nq, eo.slot_bits, eo.rank, eo.tgt + er, eo.len + er);                      \
+    }                                                                                                            \
+  } while (0)
+
 // Thread per query, count then collect.  Offering every candidate to the sorted list as it is scanned makes the
 // warp run the insertion at almost every candidate: a lane inserts at ~k (1 + ln(n/k)) of its n candidates, and the
 // 32 lanes insert at different ones.  Here the first shell (R <= 1: the 27 cells around the query's cell, nine
@@ -456,21 +497,10 @@ __global__ void __launch_bounds__(128, KT <= 16 ? KNN_MIN_BLOCKS : 1)
   const int tid = threadIdx.x;
   const int s = (blockIdx.x - d.block0) * blockDim.x + tid;
   if (s >= nq) return;
-  if (eo.tgt && s == 0) {  // the sentinel row N: only edges to N
-    const int none = eo.rank ? (int)((((unsigned)nq >> 5) << 7) | ((unsigned)nq & 31u)) : nq;
-    for (int e = 0; e < (1 << eo.slot_bits); ++e)
-      eo.tgt[((size_t)nq << eo.slot_bits) + e] = none, eo.len[((size_t)nq << eo.slot_bits) + e] = 0.f;
-  }
+  if (eo.tgt && s == 0) knn_sentinel_row(eo, nq);
   float qx, qy, qz;
   int row;
-  if (queries == nullptr) {
-    float4 me = sorted[s];
-    qx = me.x, qy = me.y, qz = me.z;
-    row = __float_as_int(me.w);
-  } else {
-    qx = __ldg(queries + (size_t)s * 3), qy = __ldg(queries + (size_t)s * 3 + 1), qz = __ldg(queries + (size_t)s * 3 + 2);
-    row = s;
-  }
+  KNN_QUERY_POINT();
   const int cx = cell_coord(qx, g.ox, g.inv_h, g.dx), cy = cell_coord(qy, g.oy, g.inv_h, g.dy),
             cz = cell_coord(qz, g.oz, g.inv_h, g.dz);
   TopK<KT> top;
@@ -504,16 +534,8 @@ __global__ void __launch_bounds__(128, KT <= 16 ? KNN_MIN_BLOCKS : 1)
     const float t = d2 * bin_scale;
     return t < (float)(KNN_NB - 1) ? (int)t : KNN_NB - 1;  // NaN -> the last bin (NaN keys sort above +inf)
   };
-  // distance from the query to the nearest face of the visited block that still has cells behind it; every
-  // unvisited point is at least that far away (minus the fp32 slack)
   auto shells_done = [&](int R) {
-    float mfd = __int_as_float(0x7f800000);
-    if (cx - R > 0) mfd = fminf(mfd, qx - (g.ox + (float)(cx - R) * g.h));
-    if (cx + R + 1 < g.dx) mfd = fminf(mfd, (g.ox + (float)(cx + R + 1) * g.h) - qx);
-    if (cy - R > 0) mfd = fminf(mfd, qy - (g.oy + (float)(cy - R) * g.h));
-    if (cy + R + 1 < g.dy) mfd = fminf(mfd, (g.oy + (float)(cy + R + 1) * g.h) - qy);
-    if (cz - R > 0) mfd = fminf(mfd, qz - (g.oz + (float)(cz - R) * g.h));
-    if (cz + R + 1 < g.dz) mfd = fminf(mfd, (g.oz + (float)(cz + R + 1) * g.h) - qz);
+    const float mfd = knn_unvisited_bound(g, cx, cy, cz, qx, qy, qz, R);
     if (mfd == __int_as_float(0x7f800000)) return true;  // the whole grid has been visited
     const float ms = mfd - g.slack;
     return ms > 0.f && top.kth_d2() < ms * ms;
@@ -607,13 +629,7 @@ __global__ void __launch_bounds__(128, KT <= 16 ? KNN_MIN_BLOCKS : 1)
       if (shells_done(R)) break;
     }
   }
-  if (dist || idx64 || idx32)
-    top.store(k, do_sqrt != 0, dist ? dist + (size_t)row * k : nullptr, idx64 ? idx64 + (size_t)row * k : nullptr,
-              idx32 ? idx32 + (size_t)row * k : nullptr);
-  if (eo.tgt) {  // self query only (nq == N): the propagation's edge rows, written straight from the registers
-    const size_t er = (size_t)(eo.rank ? s : row) << eo.slot_bits;  // cell-order row (= this thread) or original row
-    top.store_edges(k, eo.radius, nq, eo.slot_bits, eo.rank, eo.tgt + er, eo.len + er);
-  }
+  KNN_QUERY_EPILOGUE(top);
 }
 
 // ---- grid query, warp-synchronous insertion (k = 64) ------------------------------------------------
@@ -634,23 +650,10 @@ __global__ void __launch_bounds__(128, 1) knn_grid_query_sync_kernel(const __gri
   const int tid = threadIdx.x;
   const int s = (blockIdx.x - d.block0) * blockDim.x + tid;
   const bool live = s < nq;
-  if (eo.tgt && s == 0) {  // the sentinel row N: only edges to N
-    const int none = eo.rank ? (int)((((unsigned)nq >> 5) << 7) | ((unsigned)nq & 31u)) : nq;
-    for (int e = 0; e < (1 << eo.slot_bits); ++e)
-      eo.tgt[((size_t)nq << eo.slot_bits) + e] = none, eo.len[((size_t)nq << eo.slot_bits) + e] = 0.f;
-  }
+  if (eo.tgt && s == 0) knn_sentinel_row(eo, nq);
   float qx = 0.f, qy = 0.f, qz = 0.f;
   int row = 0;
-  if (live) {
-    if (queries == nullptr) {
-      float4 me = sorted[s];
-      qx = me.x, qy = me.y, qz = me.z;
-      row = __float_as_int(me.w);
-    } else {
-      qx = __ldg(queries + (size_t)s * 3), qy = __ldg(queries + (size_t)s * 3 + 1), qz = __ldg(queries + (size_t)s * 3 + 2);
-      row = s;
-    }
-  }
+  if (live) KNN_QUERY_POINT();
   const int cx = cell_coord(qx, g.ox, g.inv_h, g.dx), cy = cell_coord(qy, g.oy, g.inv_h, g.dy),
             cz = cell_coord(qz, g.oz, g.inv_h, g.dz);
   TopK<KT> top;
@@ -707,7 +710,7 @@ __global__ void __launch_bounds__(128, 1) knn_grid_query_sync_kernel(const __gri
         for (int u = 0; u < 4; ++u)
           if (u < n) {
             const float d2 = sq3(c[u].x - qx, c[u].y - qy, c[u].z - qz);
-            const unsigned long long kk = ((unsigned long long)__float_as_uint(d2) << 32) | (unsigned)__float_as_int(c[u].w);
+            const unsigned long long kk = knn_key(d2, __float_as_int(c[u].w));
             if (kk < top.key[KT - 1]) pend[npend++][tid] = kk;
           }
         p += 4;
@@ -716,28 +719,14 @@ __global__ void __launch_bounds__(128, 1) knn_grid_query_sync_kernel(const __gri
     }
     while (__any_sync(FULL, npend > 0)) insert_round();
     if (active) {
-      // distance from the query to the nearest face of the visited block that still has cells
-      // behind it; every unvisited point is at least that far away (minus the fp32 slack)
-      float mfd = __int_as_float(0x7f800000);
-      if (cx - R > 0) mfd = fminf(mfd, qx - (g.ox + (float)(cx - R) * g.h));
-      if (cx + R + 1 < g.dx) mfd = fminf(mfd, (g.ox + (float)(cx + R + 1) * g.h) - qx);
-      if (cy - R > 0) mfd = fminf(mfd, qy - (g.oy + (float)(cy - R) * g.h));
-      if (cy + R + 1 < g.dy) mfd = fminf(mfd, (g.oy + (float)(cy + R + 1) * g.h) - qy);
-      if (cz - R > 0) mfd = fminf(mfd, qz - (g.oz + (float)(cz - R) * g.h));
-      if (cz + R + 1 < g.dz) mfd = fminf(mfd, (g.oz + (float)(cz + R + 1) * g.h) - qz);
+      const float mfd = knn_unvisited_bound(g, cx, cy, cz, qx, qy, qz, R);
       if (mfd == __int_as_float(0x7f800000)) active = false;  // the whole grid has been visited
       const float ms = mfd - g.slack;
       if (ms > 0.f && top.kth_d2() < ms * ms) active = false;
     }
   }
   if (!live) return;
-  if (dist || idx64 || idx32)
-    top.store(k, do_sqrt != 0, dist ? dist + (size_t)row * k : nullptr, idx64 ? idx64 + (size_t)row * k : nullptr,
-              idx32 ? idx32 + (size_t)row * k : nullptr);
-  if (eo.tgt) {  // self query only (nq == N): the propagation's edge rows, written straight from the registers
-    const size_t er = (size_t)(eo.rank ? s : row) << eo.slot_bits;  // cell-order row (= this thread) or original row
-    top.store_edges(k, eo.radius, nq, eo.slot_bits, eo.rank, eo.tgt + er, eo.len + er);
-  }
+  KNN_QUERY_EPILOGUE(top);
 }
 
 // ---- brute force (algo 1) -----------------------------------------------------------------------
@@ -788,29 +777,41 @@ static int knn_cap_coarse(int N) {
   return c > KNN_PASS0_CELLS ? KNN_PASS0_CELLS : c;
 }
 
-size_t knn_grid_workspace_bytes(int N) {
-  size_t b = 0;
-  b += align256(sizeof(KnnCtl));
-  b += align256(sizeof(int) * (size_t)knn_cap_coarse(N));
-  b += align256(sizeof(int) * (size_t)(knn_cap_fine(N) + 4)) * 2;  // cell_count, cell_start
-  b += align256(sizeof(int) * (size_t)N) * 4;                        // cell_id, slot_in_cell, order, rank
-  b += align256(sizeof(float4) * (size_t)N);
-  return b + 1024;
+// The layout of one scene's grid workspace, for sizing (over a null workspace the Arena only measures) and for the
+// build: the control block (a batch uses its ctl_block instead), both cell tables, the per-point arrays.
+static Arena knn_carve(void *workspace, size_t workspace_bytes, int N, KnnBuildDesc *d) {
+  Arena ar(workspace, workspace_bytes);
+  d->N = N;
+  d->cap_fine = knn_cap_fine(N), d->cap_coarse = knn_cap_coarse(N);
+  d->ctl = ar.take<KnnCtl>(1);
+  d->coarse_count = ar.take<int>(d->cap_coarse);
+  d->cell_count = ar.take<int>(d->cap_fine + 4);
+  d->cell_start = ar.take<int>(d->cap_fine + 4);
+  d->cell_id = ar.take<int>(N);
+  d->slot = ar.take<int>(N);
+  d->order = ar.take<int>(N);
+  d->rank = ar.take<int>(N);
+  d->sorted = ar.take<float4>(N);
+  return ar;
 }
 
-template <int KT>
-static void launch_grid_query(const KnnQueryArgs &a, int blocks, cudaStream_t st) {
-  // Measured (c2, B200): at k <= 32 the count-then-collect kernel; at k = 64, where an insertion is 64
-  // compare-exchanges, the warp-synchronous one (10-16 % faster than offering every candidate).
-  if constexpr (KT > 32)
-    knn_grid_query_sync_kernel<KT><<<blocks, 128, 0, st>>>(a);
-  else
-    knn_grid_query_kernel<KT><<<blocks, 128, 0, st>>>(a);
+size_t knn_grid_workspace_bytes(int N) {
+  KnnBuildDesc d;
+  return knn_carve(nullptr, 0, N, &d).off + 1024;
 }
-template <int KT>
-static void launch_brute(const float *xyz, int N, const float *queries, int nq, int k, int do_sqrt, float *dist,
-                         long long *i64, int *i32, cudaStream_t st) {
-  knn_brute_kernel<KT><<<(nq + 127) / 128, 128, 0, st>>>(xyz, N, queries, nq, k, do_sqrt, dist, i64, i32);
+
+// the register-resident top-k is sized KT = the power of two >= k (8 .. 64); launch(KT) is called with it as a
+// compile-time constant (std::integral_constant)
+template <typename F>
+static void with_kt(int k, F &&launch) {
+  if (k <= 8)
+    launch(std::integral_constant<int, 8>());
+  else if (k <= 16)
+    launch(std::integral_constant<int, 16>());
+  else if (k <= 32)
+    launch(std::integral_constant<int, 32>());
+  else
+    launch(std::integral_constant<int, 64>());
 }
 
 size_t knn_ctl_block_bytes(int B) { return align256(sizeof(KnnCtl)) * (size_t)(B > 0 ? B : 0); }
@@ -833,20 +834,9 @@ int knn_grid_build_batch(const KnnBuildScene *scenes, int B, int k, void *ctl_bl
     const int N = scenes[b].N;
     KnnBuildDesc &d = a.s[b];
     d.xyz = scenes[b].xyz;
-    d.N = N;
-    d.cap_fine = knn_cap_fine(N), d.cap_coarse = knn_cap_coarse(N);
-    Arena ar(scenes[b].workspace, scenes[b].workspace_bytes);
-    KnnCtl *own = ar.take<KnnCtl>(1);  // the head of a single-scene workspace; a batch uses ctl_block instead
-    d.ctl = ctl_block ? (KnnCtl *)((char *)ctl_block + align256(sizeof(KnnCtl)) * b) : own;
-    d.coarse_count = ar.take<int>(d.cap_coarse);
-    d.cell_count = ar.take<int>(d.cap_fine + 4);
-    d.cell_start = ar.take<int>(d.cap_fine + 4);
-    d.cell_id = ar.take<int>(N);
-    d.slot = ar.take<int>(N);
-    d.order = ar.take<int>(N);
-    d.rank = ar.take<int>(N);
-    d.sorted = ar.take<float4>(N);
-    if (!ar.ok) {
+    const bool ok = knn_carve(scenes[b].workspace, scenes[b].workspace_bytes, N, &d).ok;
+    if (ctl_block) d.ctl = (KnnCtl *)((char *)ctl_block + align256(sizeof(KnnCtl)) * b);
+    if (!ok) {
       set_error("knn: workspace of scene %d too small (%zu bytes given, %zu needed)", b, scenes[b].workspace_bytes,
                 knn_grid_workspace_bytes(N));
       return GF_ERR_WORKSPACE;
@@ -912,14 +902,15 @@ int knn_grid_query_batch(const KnnQueryJob *jobs, int B, int k, int do_sqrt, cud
     blocks += (j.nq + 127) / 128;
   }
   if (blocks == 0) return GF_OK;
-  if (k <= 8)
-    launch_grid_query<8>(a, blocks, st);
-  else if (k <= 16)
-    launch_grid_query<16>(a, blocks, st);
-  else if (k <= 32)
-    launch_grid_query<32>(a, blocks, st);
-  else
-    launch_grid_query<64>(a, blocks, st);
+  with_kt(k, [&](auto kt) {
+    // Measured (c2, B200): at k <= 32 the count-then-collect kernel; at k = 64, where an insertion is 64
+    // compare-exchanges, the warp-synchronous one (10-16 % faster than offering every candidate).
+    constexpr int KT = decltype(kt)::value;
+    if constexpr (KT > 32)
+      knn_grid_query_sync_kernel<KT><<<blocks, 128, 0, st>>>(a);
+    else
+      knn_grid_query_kernel<KT><<<blocks, 128, 0, st>>>(a);
+  });
   GF_LAUNCHED();
   return GF_OK;
 }
@@ -953,14 +944,10 @@ extern "C" int gf_knn(const float *xyz, int N, const float *queries, int nq, int
   GF_CHECK_ARG(xyz || N == 0, "knn: null xyz");
   if (algo == 1 || N == 0) {
     const float *q = queries ? queries : xyz;
-    if (k <= 8)
-      launch_brute<8>(xyz, N, q, nq, k, sqrt_out, dist, (long long *)idx64, idx32, st);
-    else if (k <= 16)
-      launch_brute<16>(xyz, N, q, nq, k, sqrt_out, dist, (long long *)idx64, idx32, st);
-    else if (k <= 32)
-      launch_brute<32>(xyz, N, q, nq, k, sqrt_out, dist, (long long *)idx64, idx32, st);
-    else
-      launch_brute<64>(xyz, N, q, nq, k, sqrt_out, dist, (long long *)idx64, idx32, st);
+    with_kt(k, [&](auto kt) {
+      knn_brute_kernel<decltype(kt)::value>
+          <<<(nq + 127) / 128, 128, 0, st>>>(xyz, N, q, nq, k, sqrt_out, dist, (long long *)idx64, idx32);
+    });
     GF_LAUNCHED();
     return GF_OK;
   }

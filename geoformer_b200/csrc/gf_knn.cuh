@@ -21,7 +21,7 @@ struct KnnEdgeOut {
   float radius;
   int slot_bits;
   const int *rank;  // != nullptr: table in CELL ORDER (rows and targets are cell-order positions), targets stored
-                    // encoded as (t >> 5) << 7 | (t & 31) (gf_geodesic.cu); nullptr: original indices, plain
+                    // encoded (geo_edge_code, gf_geodesic.cuh); nullptr: original indices, plain
 };
 
 // Scenes per batched build / query launch (the batched propagation's GEO_BATCH_MAX).  The kernels take one
