@@ -10,6 +10,8 @@ import torch
 pytestmark = pytest.mark.gpu
 
 from geoformer_b200.scenes import scene  # noqa: E402
+from test_gpu_ops_launch_shapes import (assert_atomic_sum, gather_grad_terms, group_grad_terms,  # noqa: E402
+                                        interpolate_grad_terms)
 
 
 @pytest.fixture(scope="module")
@@ -112,7 +114,7 @@ def test_gather_and_grad(oracle_lib, dev):
     assert np.array_equal(out, oracle_lib.gather_points(feats.numpy(), idx.numpy()))
     go = torch.randn(2, 5, 300, generator=g)
     gr = _ext.gather_points_grad(go.to(dev), idx.to(dev), 700).cpu().numpy()
-    np.testing.assert_allclose(gr, oracle_lib.gather_points_grad(go.numpy(), idx.numpy(), 700), rtol=1e-5, atol=1e-5)
+    assert_atomic_sum(gr, *gather_grad_terms(go.numpy(), idx.numpy(), 700))
 
 
 def test_group_and_grad(oracle_lib, dev):
@@ -125,7 +127,7 @@ def test_group_and_grad(oracle_lib, dev):
     assert np.array_equal(out, oracle_lib.group_points(feats.numpy(), idx.numpy()))
     go = torch.randn(2, 19, 128, 16, generator=g)
     gr = _ext.group_points_grad(go.to(dev), idx.to(dev), 900).cpu().numpy()
-    np.testing.assert_allclose(gr, oracle_lib.group_points_grad(go.numpy(), idx.numpy(), 900), rtol=1e-4, atol=1e-4)
+    assert_atomic_sum(gr, *group_grad_terms(go.numpy(), idx.numpy(), 900))
 
 
 @pytest.mark.parametrize("N,m,r,ns", [(3000, 200, 0.2, 64), (20000, 512, 0.2, 64), (20000, 300, 0.05, 16),
@@ -156,8 +158,7 @@ def test_three_nn_and_interpolate(oracle_lib, dev):
     assert np.array_equal(out, oracle_lib.three_interpolate(feats.numpy(), ridx, w.numpy()))
     go = torch.randn(1, 6, 3000, generator=g)
     gr = _ext.three_interpolate_grad(go.to(dev), idx, w.to(dev), 1500).cpu().numpy()
-    np.testing.assert_allclose(gr, oracle_lib.three_interpolate_grad(go.numpy(), ridx, w.numpy(), 1500), rtol=1e-4,
-                               atol=1e-4)
+    assert_atomic_sum(gr, *interpolate_grad_terms(go.numpy(), ridx, w.numpy(), 1500))
     # fewer than three known points: +inf / index 0 (interpolate_gpu.cu:31-32,56-61)
     d2s, idxs = _ext.three_nn(unknown[:, :10].contiguous().to(dev), known[:, :2].contiguous().to(dev))
     rd2s, ridxs = oracle_lib.three_nn(unknown[:, :10].numpy(), known[:, :2].numpy())
@@ -181,7 +182,8 @@ def test_operator_preconditions(dev):
 # ------------------------------------------------------------------------------------------ kNN
 @pytest.mark.parametrize("N,k,algo", [(5, 8, "grid"), (17, 16, "brute"), (1000, 8, "grid"), (1000, 8, "brute"),
                                       (20000, 16, "grid"), (20000, 16, "brute"), (20000, 64, "grid"),
-                                      (20000, 33, "grid"), (50000, 8, "grid")])
+                                      (20000, 33, "grid"), (50000, 8, "grid"), (5000, 33, "brute"),
+                                      (5000, 64, "brute"), (40, 64, "brute"), (20, 33, "brute")])
 def test_knn_matches_oracle(oracle_lib, dev, N, k, algo):
     from geoformer_b200.geodesic_utils import knn_graph
 

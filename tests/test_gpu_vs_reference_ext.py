@@ -13,6 +13,8 @@ import torch
 pytestmark = pytest.mark.gpu
 
 from geoformer_b200.scenes import scene  # noqa: E402
+from test_gpu_ops_launch_shapes import (assert_atomic_sum, gather_grad_terms, group_grad_terms,  # noqa: E402
+                                        interpolate_grad_terms)
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
@@ -81,12 +83,14 @@ def test_ball_query_group_gather_three_way(oracle_lib, dev):
     assert np.array_equal(_ext.gather_points(feats.to(dev), sel).cpu().numpy(),
                           oracle_lib.gather_points(feats.numpy(), sel.cpu().numpy()))
     go = torch.randn(1, 16, 2048, 8, generator=torch.Generator().manual_seed(3))
-    np.testing.assert_allclose(_ext.group_points_grad(go.to(dev), ours, 30000).cpu().numpy(),
-                               oracle_lib.group_points_grad(go.numpy(), ref, 30000),
-                               rtol=1e-4, atol=1e-4)  # fp32 atomic order differs run to run on the GPU
+    # fp32 atomic order differs run to run on the GPU: the float64 sum with a bound per number of contributors.  It is
+    # exact for single contributors but, at r = 1.5, wider than a 1e-4 tolerance for the heavily padded low-index points
+    # (around 10^3 contributors); test_gpu_ops_launch_shapes.py checks these gradients where single terms are resolved
+    assert_atomic_sum(_ext.group_points_grad(go.to(dev), ours, 30000).cpu().numpy(),
+                      *group_grad_terms(go.numpy(), ref, 30000))
     go2 = torch.randn(1, 16, 2048, generator=torch.Generator().manual_seed(4))
-    np.testing.assert_allclose(_ext.gather_points_grad(go2.to(dev), sel, 30000).cpu().numpy(),
-                               oracle_lib.gather_points_grad(go2.numpy(), sel.cpu().numpy(), 30000), rtol=1e-4, atol=1e-4)
+    assert_atomic_sum(_ext.gather_points_grad(go2.to(dev), sel, 30000).cpu().numpy(),
+                      *gather_grad_terms(go2.numpy(), sel.cpu().numpy(), 30000))
 
 
 def test_three_nn_interpolate_three_way(oracle_lib, dev):
@@ -102,9 +106,8 @@ def test_three_nn_interpolate_three_way(oracle_lib, dev):
     assert np.array_equal(_ext.three_interpolate(feats, idx, w).cpu().numpy(),
                           oracle_lib.three_interpolate(feats.cpu().numpy(), oidx, w.cpu().numpy()))
     go = torch.randn(1, 8, 5000, generator=g).to(dev)
-    np.testing.assert_allclose(_ext.three_interpolate_grad(go, idx, w, 2000).cpu().numpy(),
-                               oracle_lib.three_interpolate_grad(go.cpu().numpy(), oidx, w.cpu().numpy(), 2000),
-                               rtol=1e-4, atol=1e-4)
+    assert_atomic_sum(_ext.three_interpolate_grad(go, idx, w, 2000).cpu().numpy(),
+                      *interpolate_grad_terms(go.cpu().numpy(), oidx, w.cpu().numpy(), 2000))
 
 
 def test_reference_python_surface_runs_on_our_ext(oracle_lib, dev):
