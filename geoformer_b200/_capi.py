@@ -32,9 +32,12 @@ SIGNATURES = {
     "gf_event_elapsed_ms": (c_float, [_P, _P]),
     "gf_fps_workspace_bytes": (c_size_t, [c_int, c_int, c_int]),
     "gf_furthest_point_sampling": (c_int, [_P, c_int, c_int, c_int, _P, _P, c_size_t, _P]),
+    "gf_fps_batch_workspace_bytes": (c_size_t, [_P, c_int, c_int]),
+    "gf_furthest_point_sampling_batch": (c_int, [_P, _P, c_int, c_int, _P, _P, c_size_t, _P]),
     "gf_gather_points": (c_int, [_P, _P, c_int, c_int, c_int, c_int, _P, _P]),
     "gf_gather_points_grad": (c_int, [_P, _P, c_int, c_int, c_int, c_int, _P, _P]),
     "gf_ball_query": (c_int, [_P, _P, c_int, c_int, c_int, c_float, c_int, _P, _P]),
+    "gf_ball_query_batch": (c_int, [_P, _P, _P, c_int, c_int, c_float, c_int, _P, _P]),
     "gf_group_points": (c_int, [_P, _P, c_int, c_int, c_int, c_int, c_int, _P, _P]),
     "gf_group_points_grad": (c_int, [_P, _P, c_int, c_int, c_int, c_int, c_int, _P, _P]),
     "gf_three_nn": (c_int, [_P, _P, c_int, c_int, c_int, _P, _P, _P]),

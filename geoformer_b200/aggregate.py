@@ -7,6 +7,10 @@ differentiate.  group_mlp_pool_train takes the unfolded parameters and is an aut
 statistics where torch's would use them (training mode, or no running statistics), the running statistics updated as
 nn.BatchNorm2d updates them, and a deterministic backward to the conv weights and biases, gamma, beta and the
 features (gf_aggregate_train.cu).  aggregate() picks the form from the module's mode and whether a gradient is wanted.
+
+aggregate_batch() takes a ragged batch (flat points + offsets, scenes of different sizes) the way forward_aggregator
+holds it: ragged FPS and ball query (gf_furthest_point_sampling_batch, gf_ball_query_batch), then one MLP call over
+the whole batch.
 """
 import ctypes
 
@@ -257,6 +261,13 @@ def aggregate(module, xyz, features, inds=None, npoint_new=None, pooling=None):
     new_xyz = _ext.gather_points(xyz.transpose(1, 2).contiguous(), inds).transpose(1, 2).contiguous()
     g = module.grouper
     idx = _ext.ball_query(new_xyz, xyz.contiguous(), float(g.radius), int(g.nsample))
+    return new_xyz, _mlp(module, xyz, new_xyz, features, idx, pooling), inds
+
+
+def _mlp(module, xyz, new_xyz, features, idx, pooling):
+    """module.mlp on the groups of idx, in the form the module's mode and the gradient wanted choose: the folded
+    inference kernel, or group_mlp_pool_train"""
+    g = module.grouper
     pooling = pooling if pooling is not None else module.pooling
     features = features.contiguous() if features is not None else None
     layers = _shared_mlp_layers(module.mlp_module)
@@ -266,14 +277,13 @@ def aggregate(module, xyz, features, inds=None, npoint_new=None, pooling=None):
     wants_grad = torch.is_grad_enabled() and any(t.requires_grad for t in params + [xyz, features] if t is not None)
     if not any(batch) and not wants_grad:
         widths, Ws, scs, shs = fold_shared_mlp(module.mlp_module)
-        out = group_mlp_pool(xyz.contiguous(), new_xyz, features, idx, g.radius, g.normalize_xyz, g.use_xyz, widths,
-                             Ws, scs, shs, pooling=pooling)
-        return new_xyz, out, inds
+        return group_mlp_pool(xyz.contiguous(), new_xyz, features, idx, g.radius, g.normalize_xyz, g.use_xyz, widths,
+                              Ws, scs, shs, pooling=pooling)
 
     def ones_if_none(t, bn, value):  # BatchNorm2d(affine=False)
         return t if t is not None else torch.full((bn.num_features,), value, device=xyz.device)
 
-    out = group_mlp_pool_train(
+    return group_mlp_pool_train(
         xyz.contiguous(), new_xyz, features, idx, g.radius, g.normalize_xyz, g.use_xyz,
         [conv.weight for conv, _ in layers], [conv.bias for conv, _ in layers],
         [ones_if_none(bn.weight, bn, 1.0) if bn else None for _, bn in layers],
@@ -283,4 +293,79 @@ def aggregate(module, xyz, features, inds=None, npoint_new=None, pooling=None):
         pooling=pooling,
         num_batches_tracked=[bn.num_batches_tracked if bn is not None and bn.training and bn.track_running_stats
                              else None for _, bn in layers])
-    return new_xyz, out, inds
+
+
+def batch_offsets_list(batch_offsets, n_points):
+    """batch_offsets (B+1) tensor or sequence -> list of ints, checked: starts at 0, rises strictly (no empty scene)
+    and ends at n_points"""
+    off = [int(v) for v in (batch_offsets.tolist() if isinstance(batch_offsets, torch.Tensor) else batch_offsets)]
+    C.require(len(off) >= 2 and off[0] == 0, "batch_offsets must start at 0 and describe at least one scene")
+    C.require(all(b > a for a, b in zip(off, off[1:])), "batch_offsets must rise strictly (a scene is empty)")
+    C.require(off[-1] == n_points, "batch_offsets end at %d, the batch has %d points" % (off[-1], n_points))
+    return off
+
+
+def furthest_point_sampling_batch(xyz, offsets, m):
+    """xyz (sum N, 3) f32 flat, offsets (B+1) host ints -> (B, m) i32 scene-local seeds; row b equals
+    _ext.furthest_point_sampling of scene b alone"""
+    C.check_cuda_f32(xyz, "xyz")
+    B = len(offsets) - 1
+    out = torch.empty((B, int(m)), dtype=torch.int32, device=xyz.device)
+    offs = (ctypes.c_int * (B + 1))(*offsets)
+    lib = C.lib()
+    with torch.cuda.device(xyz.device):
+        nbytes = lib.gf_fps_batch_workspace_bytes(offs, B, int(m))
+        ws = C.workspace.get(xyz.device, "fps", nbytes) if nbytes else None
+        C.check(lib.gf_furthest_point_sampling_batch(C.ptr(xyz), offs, B, int(m), C.ptr(out), C.ptr(ws), nbytes,
+                                                     C.stream_of(xyz.device)), "furthest_point_sampling_batch")
+    return out
+
+
+def ball_query_batch(new_xyz, xyz, offsets, radius, nsample):
+    """new_xyz (B, m, 3), xyz (sum N, 3) flat, offsets (B+1) host ints -> (B, m, nsample) i32 scene-local; row b
+    equals _ext.ball_query of scene b alone"""
+    C.check_cuda_f32(new_xyz, "new_xyz")
+    C.check_cuda_f32(xyz, "xyz")
+    B, m = new_xyz.shape[0], new_xyz.shape[1]
+    C.require(B == len(offsets) - 1, "new_xyz has %d scenes, offsets %d" % (B, len(offsets) - 1))
+    out = torch.empty((B, m, int(nsample)), dtype=torch.int32, device=new_xyz.device)
+    with torch.cuda.device(new_xyz.device):
+        C.check(C.lib().gf_ball_query_batch(C.ptr(new_xyz), C.ptr(xyz), (ctypes.c_int * (B + 1))(*offsets), B, m,
+                                            float(radius), int(nsample), C.ptr(out), C.stream_of(new_xyz.device)),
+                "ball_query_batch")
+    return out
+
+
+def aggregate_batch(module, locs_float_, features_, batch_offsets_, inds=None, npoint_new=None, pooling=None):
+    """aggregate() over a RAGGED batch, as forward_aggregator (geoformer_fs.py:619-660) holds it: locs_float_ (sum N, 3),
+    features_ (sum N, C) point-major or None, batch_offsets_ (B+1) tensor or list.  One FPS launch and one ball-query
+    launch (per 32 scenes) for all scenes, then ONE group_mlp_pool[_train] call over the whole batch as a single scene
+    of sum N points and B * m centres: batch statistics cover all B * m * nsample samples, as the reference's one
+    module.mlp call over the concatenated groups.  inds (B, m) i32 scene-local seeds skip the FPS.
+    Returns (context_locs (B, m, 3), context_feats (B, C_out, m), pre_enc_inds (B, m) i32)."""
+    npoint = int(npoint_new if npoint_new is not None else module.npoint)
+    C.check_cuda_f32(locs_float_, "locs_float_")
+    C.require(locs_float_.dim() == 2 and locs_float_.shape[1] == 3, "locs_float_ must be (sum N, 3)")
+    n_points = locs_float_.shape[0]
+    off = batch_offsets_list(batch_offsets_, n_points)
+    B = len(off) - 1
+    dev = locs_float_.device
+    if features_ is not None:
+        C.require(isinstance(features_, torch.Tensor) and features_.is_cuda, "features_: CPU not supported")
+        C.require(features_.dtype == torch.float32, "features_ must be a float tensor")
+        C.require(features_.dim() == 2 and features_.shape[0] == n_points,
+                  "features_ must be (sum N, C) with sum N = %d rows" % n_points)
+    if inds is None:
+        inds = furthest_point_sampling_batch(locs_float_, off, npoint)
+    else:
+        C.check_cuda_i32(inds, "inds")
+        C.require(tuple(inds.shape) == (B, npoint), "inds must be (B, npoint)")
+    start = torch.tensor(off[:-1], dtype=torch.int32, device=dev)
+    new_xyz = locs_float_.detach()[(inds + start[:, None]).long()]
+    g = module.grouper
+    idx = ball_query_batch(new_xyz, locs_float_, off, g.radius, g.nsample)
+    # the whole batch as one scene: global indices, features channel-major once
+    idx1 = (idx + start[:, None, None]).reshape(1, B * npoint, -1)
+    feats1 = features_.t().unsqueeze(0).contiguous() if features_ is not None else None
+    out = _mlp(module, locs_float_.unsqueeze(0), new_xyz.reshape(1, B * npoint, 3), feats1, idx1, pooling)
+    return new_xyz, out[0].reshape(out.shape[1], B, npoint).transpose(0, 1).contiguous(), inds

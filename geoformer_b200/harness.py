@@ -95,27 +95,50 @@ class FewShotForward(nn.Module):
         self.eval()
 
     # ---- :619-660 ---------------------------------------------------------------------------------------
-    def forward_aggregator(self, locs, feats, impl):
-        """locs (B,N,3), feats (B,N,m) -> context_locs (B,C,3), context_feats (B,C,2m), pre_enc_inds (B,C) i32"""
-        xyz = locs.contiguous()
-        f = feats.transpose(1, 2).contiguous()
-        if impl == "b200":
-            class _G:
-                radius, nsample, normalize_xyz, use_xyz = self.radius, self.nsample, True, True
+    def _aggregator_module(self):
+        """the set aggregator's attributes aggregate() / aggregate_batch() read"""
+        class _G:
+            radius, nsample, normalize_xyz, use_xyz = self.radius, self.nsample, True, True
 
-            class _M:
-                npoint, pooling, grouper, mlp_module = self.C, "max", _G, self.mlp_module
+        class _M:
+            npoint, pooling, grouper, mlp_module = self.C, "max", _G, self.mlp_module
 
-            new_xyz, out, inds = agg.aggregate(_M, xyz, f)
-            return new_xyz, out.transpose(1, 2), inds
+        return _M
+
+    def _group_torch(self, xyz, f):
+        """group_points of the reference (pointnet2_modules.py:200-232): xyz (B,N,3), f (B,m,N) -> centres (B,C,3),
+        grouped input (B, 3+m, C, nsample), seeds (B,C) i32"""
         inds = _ext.furthest_point_sampling(xyz, self.C)
         new_xyz = _ext.gather_points(xyz.transpose(1, 2).contiguous(), inds).transpose(1, 2).contiguous()
         idx = _ext.ball_query(new_xyz, xyz, self.radius, self.nsample)
         g_xyz = _ext.group_points(xyz.transpose(1, 2).contiguous(), idx)  # pointnet2_utils.py:330-341
         g_xyz = (g_xyz - new_xyz.transpose(1, 2).unsqueeze(-1)) / self.radius
-        x = torch.cat([g_xyz, _ext.group_points(f, idx)], dim=1)
+        return new_xyz, torch.cat([g_xyz, _ext.group_points(f, idx)], dim=1), inds
+
+    def _mlp_pool_torch(self, x):
         x = self.mlp_module(x)
-        return new_xyz, F.max_pool2d(x, kernel_size=[1, x.size(3)]).squeeze(-1).transpose(1, 2), inds
+        return F.max_pool2d(x, kernel_size=[1, x.size(3)]).squeeze(-1).transpose(1, 2)
+
+    def forward_aggregator(self, locs, feats, impl):
+        """locs (B,N,3), feats (B,N,m) -> context_locs (B,C,3), context_feats (B,C,2m), pre_enc_inds (B,C) i32"""
+        xyz = locs.contiguous()
+        f = feats.transpose(1, 2).contiguous()
+        if impl == "b200":
+            new_xyz, out, inds = agg.aggregate(self._aggregator_module(), xyz, f)
+            return new_xyz, out.transpose(1, 2), inds
+        new_xyz, x, inds = self._group_torch(xyz, f)
+        return new_xyz, self._mlp_pool_torch(x), inds
+
+    def forward_aggregator_batch(self, locs, feats, offsets, impl):
+        """the ragged form of :619-660: locs (sum N,3), feats (sum N,m), offsets (B+1) ints -> as forward_aggregator.
+        "torch" groups every scene on its own, concatenates the groups and runs ONE mlp over them (:643-657)."""
+        if impl == "b200":
+            new_xyz, out, inds = agg.aggregate_batch(self._aggregator_module(), locs, feats, offsets)
+            return new_xyz, out.transpose(1, 2), inds
+        groups = [self._group_torch(locs[a:b][None].contiguous(), feats[a:b].t()[None].contiguous())
+                  for a, b in zip(offsets, offsets[1:])]
+        new_xyz, x, inds = (torch.cat(t, dim=0) for t in zip(*groups))
+        return new_xyz, self._mlp_pool_torch(x), inds
 
     # ---- :662-723 ---------------------------------------------------------------------------------------
     def forward_decoder(self, context_locs, aggregation, query_locs, pc_dims, geo_dists, pre_enc_inds, impl):
@@ -178,20 +201,26 @@ class FewShotForward(nn.Module):
         return out
 
     @torch.no_grad()
-    def forward(self, locs, output_feats, support_embedding, impl="b200", max_step=256, neighbor=64, geo_radius=0.05):
+    def forward(self, locs, output_feats, support_embedding, impl="b200", max_step=256, neighbor=64, geo_radius=0.05,
+                batch_offsets=None):
         """locs (B,N,3) foreground points of B equally sized scenes, output_feats (B,N,m) the stub backbone's point
-        features, support_embedding (B, 2m).  Returns (list of (Q,N) mask logits, geo_dists, pre_enc_inds)."""
-        return self._chain(locs, output_feats, support_embedding, impl, max_step, neighbor, geo_radius)
+        features, support_embedding (B, 2m).  Returns (list of (Q,N) mask logits, geo_dists, pre_enc_inds).
+        batch_offsets (B+1), tensor or list: a ragged batch as the model holds it, locs (sum N,3) and output_feats
+        (sum N,m) flat; the logits are then (Q, N_b) per scene."""
+        return self._chain(locs, output_feats, support_embedding, impl, max_step, neighbor, geo_radius, batch_offsets)
 
     def forward_train(self, locs, output_feats, support_embedding, impl="b200", max_step=128, neighbor=64,
-                      geo_radius=0.05):
+                      geo_radius=0.05, batch_offsets=None):
         """forward with autograd: one training step of the post-backbone path (the training setting of SURVEY 3.1 is a
         model built with n_query_points=128 and max_step=128).  Call model.train() first for batch-statistics batch
         norm.  Gradients reach every parameter through the aggregator, decoder and mask head of either impl; the
-        geodesic maps are data."""
-        return self._chain(locs, output_feats, support_embedding, impl, max_step, neighbor, geo_radius)
+        geodesic maps are data.  batch_offsets: as in forward."""
+        return self._chain(locs, output_feats, support_embedding, impl, max_step, neighbor, geo_radius, batch_offsets)
 
-    def _chain(self, locs, output_feats, support_embedding, impl, max_step, neighbor, geo_radius):
+    def _chain(self, locs, output_feats, support_embedding, impl, max_step, neighbor, geo_radius, batch_offsets=None):
+        if batch_offsets is not None:
+            return self._chain_ragged(locs, output_feats, support_embedding, impl, max_step, neighbor, geo_radius,
+                                      agg.batch_offsets_list(batch_offsets, locs.shape[0]))
         B, N, _ = locs.shape
         pc_dims = [locs.min(dim=1)[0], locs.max(dim=1)[0]]
         mask_features = self.mask_tower(output_feats.transpose(1, 2)).transpose(1, 2)  # :477-483
@@ -204,6 +233,22 @@ class FewShotForward(nn.Module):
         aggregation = torch.cat([context_feats * se, context_feats - se, context_feats], dim=2)  # :543-548
         dec = self.forward_decoder(context_locs, aggregation, query_locs, pc_dims, geo_dists, pre_enc_inds, impl)
         logits = self.mask_logits(geo_dists, dec[-1], mask_features, locs, query_locs, None, impl)
+        return logits, geo_dists, pre_enc_inds
+
+    def _chain_ragged(self, locs, output_feats, support_embedding, impl, max_step, neighbor, geo_radius, offsets):
+        """_chain on the flat (sum N, .) arrays of a ragged batch: per-scene extents, mask features and mask heads"""
+        scenes = [slice(a, b) for a, b in zip(offsets, offsets[1:])]
+        pc_dims = [torch.stack([locs[s].min(dim=0)[0] for s in scenes]), torch.stack([locs[s].max(dim=0)[0] for s in scenes])]
+        mask_features = self.mask_tower(output_feats.t()[None])[0].t()  # a 1x1 conv: per point
+        context_locs, context_feats, pre_enc_inds = self.forward_aggregator_batch(locs, output_feats, offsets, impl)
+        query_locs = context_locs[:, : self.Q, :].contiguous()
+        geo_dists = cal_geodesic_vectorize(None, pre_enc_inds, locs.contiguous(), offsets, max_step=max_step,
+                                           neighbor=neighbor, radius=geo_radius, n_queries=self.Q)
+        se = support_embedding.unsqueeze(1)
+        aggregation = torch.cat([context_feats * se, context_feats - se, context_feats], dim=2)
+        dec = self.forward_decoder(context_locs, aggregation, query_locs, pc_dims, geo_dists, pre_enc_inds, impl)
+        logits = self.mask_logits(geo_dists, dec[-1], [mask_features[s] for s in scenes], [locs[s] for s in scenes],
+                                  query_locs, None, impl)
         return logits, geo_dists, pre_enc_inds
 
 

@@ -59,6 +59,15 @@ size_t gf_fps_workspace_bytes(int B, int N, int m);
 int gf_furthest_point_sampling(const float *xyz, int B, int N, int m, int *idx, void *workspace,
                                size_t workspace_bytes, void *stream);
 
+/* The same over a RAGGED batch: xyz the flat (offsets[B],3) array, scene b its rows [offsets[b], offsets[b+1]);
+ * offsets (B+1) is a HOST array, non-decreasing from 0.  idx (B,m) i32 with scene-local indices: row b is bit-identical
+ * to gf_furthest_point_sampling on scene b alone.  The scenes that fit one thread-block cluster (N <= 196,608 with
+ * 16-CTA clusters) run side by side, one launch per 32 of them, planned for the largest; each larger scene then runs
+ * the single-scene whole-GPU kernel.  Workspace: gf_fps_batch_workspace_bytes (0 when every scene fits a cluster). */
+size_t gf_fps_batch_workspace_bytes(const int *offsets, int B, int m);
+int gf_furthest_point_sampling_batch(const float *xyz, const int *offsets, int B, int m, int *idx, void *workspace,
+                                     size_t workspace_bytes, void *stream);
+
 /* gather_points / gather_points_grad  (sampling.cpp:17-65, sampling_gpu.cu:11-60)
  * points (B,C,N), idx (B,m) -> out (B,C,m);   grad_out (B,C,m), idx -> grad_points (B,C,N)      */
 int gf_gather_points(const float *points, const int *idx, int B, int C, int N, int m, float *out, void *stream);
@@ -70,6 +79,13 @@ int gf_gather_points_grad(const float *grad_out, const int *idx, int B, int C, i
  * d2 < radius^2, padded with the first hit, all zero when there is none.                        */
 int gf_ball_query(const float *new_xyz, const float *xyz, int B, int N, int m, float radius, int nsample, int *idx,
                   void *stream);
+
+/* The same over a RAGGED batch: new_xyz (B,m,3), xyz the flat (offsets[B],3) array with offsets (B+1) a HOST array
+ * as in gf_furthest_point_sampling_batch -> idx (B,m,nsample) i32, scene-local.  A centre of scene b searches only
+ * the rows [offsets[b], offsets[b+1]); its row is bit-identical to gf_ball_query on scene b alone.  One launch per
+ * 32 scenes.                                                                                                      */
+int gf_ball_query_batch(const float *new_xyz, const float *xyz, const int *offsets, int B, int m, float radius,
+                        int nsample, int *idx, void *stream);
 
 /* group_points / group_points_grad  (group_points.cpp:15-62, group_points_gpu.cu:11-78)
  * points (B,C,N), idx (B,np,ns) -> out (B,C,np,ns);  grad_out (B,C,np,ns) -> grad_points (B,C,N) */
