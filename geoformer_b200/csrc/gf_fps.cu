@@ -19,6 +19,7 @@
 #include <cooperative_groups.h>
 
 #include "gf_common.cuh"
+#include "gf_fps.cuh"
 
 namespace cg = cooperative_groups;
 
@@ -366,6 +367,20 @@ static int launch_fps_grid(const float *xyz, int B, int N, int m, int L, float *
   return GF_OK;
 }
 
+// FPS is the longest dependency chain of the hot path (m - 1 dependent rounds on a few SMs): its CTAs should be
+// placed ahead of queued bulk work.  As a launch attribute the priority also survives stream capture (a graph's
+// kernel nodes do not inherit the priority of the stream they were captured on).
+static cudaLaunchAttribute fps_priority() {
+  static const int prio_hi = [] {
+    int lo = 0, hi = 0;
+    return cudaDeviceGetStreamPriorityRange(&lo, &hi) == cudaSuccess ? hi : 0;
+  }();
+  cudaLaunchAttribute a;
+  a.id = cudaLaunchAttributePriority;
+  a.val.priority = prio_hi;
+  return a;
+}
+
 // B clusters of CS CTAs x T threads, one per scene
 template <class... KArgs, class... Args>
 static int launch_clusters(void (*kern)(KArgs...), int T, int B, int CS, cudaStream_t st, Args... args) {
@@ -380,15 +395,7 @@ static int launch_clusters(void (*kern)(KArgs...), int T, int B, int CS, cudaStr
   attr[0].val.clusterDim.x = CS;
   attr[0].val.clusterDim.y = 1;
   attr[0].val.clusterDim.z = 1;
-  // FPS is the longest dependency chain of the hot path (m - 1 dependent rounds on <= 16 SMs): its cluster should be
-  // placed ahead of queued bulk work.  As a launch attribute the priority also survives stream capture (a graph's
-  // kernel nodes do not inherit the priority of the stream they were captured on).
-  static const int prio_hi = [] {
-    int lo = 0, hi = 0;
-    return cudaDeviceGetStreamPriorityRange(&lo, &hi) == cudaSuccess ? hi : 0;
-  }();
-  attr[1].id = cudaLaunchAttributePriority;
-  attr[1].val.priority = prio_hi;
+  attr[1] = fps_priority();
   cfg.attrs = attr;
   cfg.numAttrs = 2;
   GF_CUDA(cudaLaunchKernelEx(&cfg, kern, args...));
@@ -429,6 +436,264 @@ static int max_cluster_size() {
   (void)cudaGetLastError();
   cached = ok16 ? 16 : 8;
   return cached;
+}
+
+// ---------------------------------------------------------------------------------------------------
+// Culled FPS on the cell order of the kNN grid: the seeds of a batched guidance call, one 1024-thread CTA per scene.
+// A new seed c can only lower the running minimum t of a point closer to c than t, a neighbourhood of c that shrinks
+// as seeds accumulate.  The points are taken in blocks of S consecutive cell-order positions (KnnGridBuffers::sorted),
+// each with the tight box of its eligible points and the largest key of its points kept on chip; a round updates a
+// block only if a lower bound of sq3(p - c) over its box is below the block's largest t, which skips 87-94 % of the
+// point updates at c2 (tools/fps_cells_mirror.py).  Keys, tie order and the no-eligible-point rule are those of the
+// cluster body, so the seeds are the reference's bit for bit.
+//
+// Exactness of a skip: every point of a skipped block keeps t, because its computed d = sq3(px - cx, ...) >= lb >= t.
+// Per axis fl(px - cx) is at least the box gap fl(lo - cx) (or fl(cx - hi)) in magnitude, since rounding is monotonic,
+// and sq3 is monotonic in the magnitudes of its arguments: sq3 of the gaps never exceeds the computed d.  The bound is
+// shrunk by 2^-20 all the same, which can only make a block update that did not need it.
+//
+// A round: every warp tests its own blocks (block b: warp b % NW, lane (b / NW) % 32, state at warp-major index so
+// that a warp's lanes read consecutive words) and appends the ones to update to one list; after a barrier all warps
+// take the list U blocks at a time (a warp per block, the U blocks' loads in flight together), so the round's
+// dependent L2 round trips are shared by the whole CTA however the updated blocks are spread; after a second barrier
+// every warp reduces its blocks' keys, and a third closes the round (candidates double-buffered by round parity).
+constexpr int FPS_CELLS_T = 1024;
+constexpr int FPS_CELLS_NW = FPS_CELLS_T / 32;
+constexpr int FPS_CELLS_WORDS = 12;               // per block: box lo xyz, hi xyz, key (v, lo), key's point xyz, list
+constexpr size_t FPS_CELLS_SMEM_MAX = 96 * 1024;  // the largest S (512 points) keeps every batchable scene under it
+constexpr float FPS_CELLS_SHRINK = 1.f - 1.f / 1048576.f;
+
+struct FpsCellsSlot {
+  uint32_t v, lo;
+  float x, y, z;
+};
+
+template <int SPL>  // S = 32 * SPL points per block, SPL per lane
+__global__ void __launch_bounds__(FPS_CELLS_T, 1)
+    fps_cells_kernel(const float4 *__restrict__ sorted, const float *__restrict__ xyz, int N, int m, int L,
+                     float *__restrict__ tmin, int *__restrict__ idx) {
+  // U blocks of a warp are updated together, QC points per lane and block loaded at a time: 4 loads in flight
+  constexpr int S = 32 * SPL, U = SPL >= 4 ? 1 : 4 / SPL, QC = SPL > 4 ? 4 : SPL, NW = FPS_CELLS_NW;
+  extern __shared__ uint32_t fc_smem[];
+  __shared__ FpsCellsSlot slot[2][NW];
+  __shared__ int list_n[2];
+  const unsigned lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int nb = (N + S - 1) / S;
+  const int nper = (nb + NW - 1) / NW;  // state of block warp + NW * n at [warp * nper + n]
+  const int nown = (int)warp < nb ? (nb - 1 - (int)warp) / NW + 1 : 0;
+  // FPS_CELLS_WORDS arrays of NW * nper words: box lo x y z, hi x y z, key v lo, key's point x y z, update list
+  const int stride = NW * nper;
+  float *const sf = (float *)fc_smem;
+  uint32_t *const su = fc_smem;
+  int *const list = (int *)fc_smem + 11 * stride;
+  const uint32_t low = (1u << L) - 1u;
+
+  float cx = __ldg(xyz + 0), cy = __ldg(xyz + 1), cz = __ldg(xyz + 2);
+  if (threadIdx.x == 0) idx[0] = 0, list_n[0] = list_n[1] = 0;
+
+  // Updates blocks b[u] (b[u] < 0: none; warp-uniform) for the seed at c; lane 0 stores their states.  init: the
+  // first round, which also sets the running minima (1e10 if eligible, else -1: gf_fps_cluster_body.cuh) and boxes.
+  auto update = [&](const int (&b)[U], bool init) {
+    uint32_t bv[U] = {}, bl[U] = {};
+    float bx[U], by[U], bz[U];
+    float lx[U], ly[U], lz[U], hx[U], hy[U], hz[U];
+#pragma unroll
+    for (int u = 0; u < U; ++u) {
+      bx[u] = by[u] = bz[u] = 0.f;
+      lx[u] = ly[u] = lz[u] = __int_as_float(0x7f800000), hx[u] = hy[u] = hz[u] = -lx[u];
+    }
+#pragma unroll 1
+    for (int q0 = 0; q0 < SPL; q0 += QC) {
+      float4 p[U][QC];
+      float t[U][QC];
+#pragma unroll
+      for (int u = 0; u < U; ++u)
+#pragma unroll
+        for (int q = 0; q < QC; ++q) {
+          const int pos = b[u] * S + (q0 + q) * 32 + (int)lane;
+          p[u][q] = make_float4(0.f, 0.f, 0.f, 0.f);
+          t[u][q] = -1.f;
+          if (b[u] >= 0 && pos < N) {
+            p[u][q] = __ldg(sorted + pos);
+            if (!init) t[u][q] = tmin[pos];
+          }
+        }
+#pragma unroll
+      for (int u = 0; u < U; ++u)
+#pragma unroll
+        for (int q = 0; q < QC; ++q) {
+          const int pos = b[u] * S + (q0 + q) * 32 + (int)lane;
+          const bool real = b[u] >= 0 && pos < N;  // b[u] < 0 gives a negative pos: no point, nothing stored
+          const float4 a = p[u][q];
+          float told = t[u][q];
+          if (init && real && !((double)sq3(a.x, a.y, a.z) <= 1e-3)) {
+            told = 1e10f;
+            lx[u] = fminf(lx[u], a.x), ly[u] = fminf(ly[u], a.y), lz[u] = fminf(lz[u], a.z);
+            hx[u] = fmaxf(hx[u], a.x), hy[u] = fmaxf(hy[u], a.y), hz[u] = fmaxf(hz[u], a.z);
+          }
+          const float nt = fminf(sq3(a.x - cx, a.y - cy, a.z - cz), told);
+          if (real && (init || nt != told)) tmin[pos] = nt;
+          if (nt >= 0.f) {
+            const uint32_t i = (uint32_t)__float_as_int(a.w);
+            const uint32_t v = __float_as_uint(nt), lo = ~(__brev(i & low) | (i >> L));
+            if (v > bv[u] || (v == bv[u] && lo > bl[u])) bv[u] = v, bl[u] = lo, bx[u] = a.x, by[u] = a.y, bz[u] = a.z;
+          }
+        }
+    }
+#pragma unroll
+    for (int u = 0; u < U; ++u) {
+      if (b[u] < 0) continue;
+      const uint32_t wv = __reduce_max_sync(0xffffffffu, bv[u]);
+      const uint32_t wl = __reduce_max_sync(0xffffffffu, bv[u] == wv ? bl[u] : 0u);
+      const int src = __ffs(__ballot_sync(0xffffffffu, bv[u] == wv && bl[u] == wl)) - 1;
+      const float x = __shfl_sync(0xffffffffu, bx[u], src), y = __shfl_sync(0xffffffffu, by[u], src),
+                  z = __shfl_sync(0xffffffffu, bz[u], src);
+      float box[6];
+      if (init) {  // the box as order-preserving integers: six REDUX instead of thirty shuffles
+        box[0] = ord2f(__reduce_min_sync(0xffffffffu, f2ord(lx[u])));
+        box[1] = ord2f(__reduce_min_sync(0xffffffffu, f2ord(ly[u])));
+        box[2] = ord2f(__reduce_min_sync(0xffffffffu, f2ord(lz[u])));
+        box[3] = ord2f(__reduce_max_sync(0xffffffffu, f2ord(hx[u])));
+        box[4] = ord2f(__reduce_max_sync(0xffffffffu, f2ord(hy[u])));
+        box[5] = ord2f(__reduce_max_sync(0xffffffffu, f2ord(hz[u])));
+      }
+      if (lane == 0) {
+        const int e = (b[u] % NW) * nper + b[u] / NW;
+        su[6 * stride + e] = wv, su[7 * stride + e] = wl;
+        sf[8 * stride + e] = x, sf[9 * stride + e] = y, sf[10 * stride + e] = z;
+        if (init)
+#pragma unroll
+          for (int a = 0; a < 6; ++a) sf[a * stride + e] = box[a];
+      }
+    }
+  };
+
+  for (int n0 = 0; n0 < nown; n0 += U) {  // the first round: every block, each warp its own
+    int b[U];
+#pragma unroll
+    for (int u = 0; u < U; ++u) b[u] = n0 + u < nown ? (int)warp + NW * (n0 + u) : -1;
+    update(b, true);
+  }
+  __syncthreads();  // the states written by lane 0 of a warp, read by the block's lane below
+
+  for (int j = 1; j < m; ++j) {
+    const int buf = j & 1;
+    if (j > 1) {
+      // the blocks of this warp the seed at c can change, appended to the round's list
+      for (int n0 = 0; n0 < nown; n0 += 32) {
+        const int n = n0 + (int)lane;
+        bool up = false;
+        if (n < nown) {
+          const int e = (int)warp * nper + n;
+          const float gx = fmaxf(fmaxf(sf[e] - cx, cx - sf[3 * stride + e]), 0.f);
+          const float gy = fmaxf(fmaxf(sf[stride + e] - cy, cy - sf[4 * stride + e]), 0.f);
+          const float gz = fmaxf(fmaxf(sf[2 * stride + e] - cz, cz - sf[5 * stride + e]), 0.f);
+          // a block without an eligible point has key v = 0 and is never updated
+          up = __fmul_rn(sq3(gx, gy, gz), FPS_CELLS_SHRINK) < __uint_as_float(su[6 * stride + e]);
+        }
+        const unsigned mask = __ballot_sync(0xffffffffu, up);
+        int base = 0;
+        if (lane == 0 && mask) base = atomicAdd(&list_n[buf], __popc(mask));
+        base = __shfl_sync(0xffffffffu, base, 0);
+        if (up) list[base + __popc(mask & ((1u << lane) - 1u))] = (int)warp + NW * n;
+      }
+      __syncthreads();
+      const int cnt = list_n[buf];
+      for (int i0 = (int)warp * U; i0 < cnt; i0 += NW * U) {
+        int b[U];
+#pragma unroll
+        for (int u = 0; u < U; ++u) b[u] = i0 + u < cnt ? list[i0 + u] : -1;
+        update(b, false);
+      }
+      __syncthreads();  // every updated state is visible to its owner
+    }
+    // this warp's largest block key, then the CTA's
+    uint32_t bv = 0, bl = 0;
+    int be = 0;
+    for (int n = (int)lane; n < nown; n += 32) {
+      const int e = (int)warp * nper + n;
+      const uint32_t v = su[6 * stride + e], lo = su[7 * stride + e];
+      if (v > bv || (v == bv && lo > bl)) bv = v, bl = lo, be = e;
+    }
+    const uint32_t wv = __reduce_max_sync(0xffffffffu, bv);
+    const uint32_t wl = __reduce_max_sync(0xffffffffu, bv == wv ? bl : 0u);
+    if ((unsigned)(__ffs(__ballot_sync(0xffffffffu, bv == wv && bl == wl)) - 1) == lane)
+      slot[buf][warp] = (wv | wl) ? FpsCellsSlot{wv, wl, sf[8 * stride + be], sf[9 * stride + be], sf[10 * stride + be]}
+                                  : FpsCellsSlot{0u, 0u, 0.f, 0.f, 0.f};
+    if (threadIdx.x == 0) list_n[buf ^ 1] = 0;  // the next round's list (its last reader finished before this round)
+    __syncthreads();
+    const uint32_t sv = slot[buf][lane].v, sl = slot[buf][lane].lo;  // NW == 32: one candidate per lane
+    const uint32_t gv = __reduce_max_sync(0xffffffffu, sv);
+    const uint32_t gl = __reduce_max_sync(0xffffffffu, sv == gv ? sl : 0u);
+    int old;
+    if ((gv | gl) == 0u) {  // no eligible point anywhere: the reference's tree yields index 0
+      old = 0;
+      cx = __ldg(xyz + 0), cy = __ldg(xyz + 1), cz = __ldg(xyz + 2);
+    } else {
+      const int ws = __ffs(__ballot_sync(0xffffffffu, sv == gv && sl == gl)) - 1;
+      const uint32_t rk = ~gl;
+      old = L ? (int)(((rk & ((1u << (32 - L)) - 1u)) << L) | brev_bits(rk >> (32 - L), L)) : (int)rk;
+      cx = slot[buf][ws].x, cy = slot[buf][ws].y, cz = slot[buf][ws].z;
+    }
+    if (threadIdx.x == 0) idx[j] = old;
+  }
+}
+static_assert(FPS_CELLS_NW == 32, "the final reduction takes one warp candidate per lane");
+
+// points per lane of a block: the smallest whose block states fit FPS_CELLS_SMEM_MAX
+static int fps_cells_spl(int N, size_t *smem) {
+  for (int spl = 2; spl <= 16; spl *= 2) {
+    const long long nb = ((long long)N + 32 * spl - 1) / (32 * spl);
+    const size_t bytes = sizeof(uint32_t) * FPS_CELLS_WORDS * FPS_CELLS_NW * (size_t)((nb + FPS_CELLS_NW - 1) / FPS_CELLS_NW);
+    if (bytes <= FPS_CELLS_SMEM_MAX) {
+      *smem = bytes;
+      return spl;
+    }
+  }
+  return 0;
+}
+
+template <int SPL>
+static int launch_fps_cells(const float4 *sorted, const float *xyz, int N, int m, float *tmin, int *idx, size_t smem,
+                            cudaStream_t st) {
+  static int ready[64];  // the opt-in to more than 48 KB of dynamic shared memory: once per device
+  int dev = 0;
+  GF_CUDA(cudaGetDevice(&dev));
+  if (dev < 0 || dev >= 64) dev = 0;
+  if (!__atomic_load_n(&ready[dev], __ATOMIC_ACQUIRE)) {
+    GF_CUDA(cudaFuncSetAttribute(fps_cells_kernel<SPL>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                 (int)FPS_CELLS_SMEM_MAX));
+    __atomic_store_n(&ready[dev], 1, __ATOMIC_RELEASE);
+  }
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = dim3(1, 1, 1);
+  cfg.blockDim = dim3(FPS_CELLS_T, 1, 1);
+  cfg.dynamicSmemBytes = smem;
+  cfg.stream = st;
+  cudaLaunchAttribute attr[1] = {fps_priority()};
+  cfg.attrs = attr;
+  cfg.numAttrs = 1;
+  GF_CUDA(cudaLaunchKernelEx(&cfg, fps_cells_kernel<SPL>, sorted, xyz, N, m, ref_log2_block(N), tmin, idx));
+  count_launch();
+  return GF_OK;
+}
+
+size_t fps_cells_workspace_bytes(int N) { return align256(sizeof(float) * (size_t)N); }
+
+int fps_cells(const float4 *sorted, const float *xyz, int N, int m, void *workspace, size_t workspace_bytes, int *idx,
+              cudaStream_t st) {
+  GF_CHECK_ARG(N >= 1 && m >= 1, "fps_cells: need N >= 1 and m >= 1 (N=%d m=%d)", N, m);
+  GF_CHECK_ARG(workspace && workspace_bytes >= fps_cells_workspace_bytes(N), "fps_cells: workspace too small");
+  size_t smem = 0;
+  float *tmin = (float *)workspace;
+  switch (fps_cells_spl(N, &smem)) {
+    case 2: return launch_fps_cells<2>(sorted, xyz, N, m, tmin, idx, smem, st);
+    case 4: return launch_fps_cells<4>(sorted, xyz, N, m, tmin, idx, smem, st);
+    case 8: return launch_fps_cells<8>(sorted, xyz, N, m, tmin, idx, smem, st);
+    case 16: return launch_fps_cells<16>(sorted, xyz, N, m, tmin, idx, smem, st);
+  }
+  set_error("fps_cells: N=%d does not fit the on-chip block states", N);
+  return GF_ERR_INVALID;
 }
 
 }  // namespace gf

@@ -5,6 +5,7 @@
 // waits for both.
 #include <stdlib.h>
 
+#include "gf_fps.cuh"
 #include "gf_geodesic.cuh"
 #include "gf_knn.cuh"
 
@@ -14,18 +15,23 @@ namespace gf {
 // cluster, latency bound) runs next to the kNN kernels, and the scenes of a batch run side by side on LANES
 // lanes.  Callers that keep several calls in flight on several streams get one set per stream, so their kernels
 // do not queue on a single hidden stream.  FPS lanes have the highest priority: FPS is the longest dependency
-// chain of a scene, its cluster should be placed as soon as SMs free up.
-// Measured with the graphs of a 20-scene call built and queried in one launch each (c2 bench, B200 at 1000 W, two
-// runs each): 4 lanes 1.090 / 1.091 M maps/s, 6 lanes 1.094 / 1.095, 8 lanes 1.053 / 1.053.  6 lanes are 0.4 %
-// ahead, which does not pay for two more high-priority streams per caller stream; 8 lanes lose 3.5 % (DESIGN
-// section 8).
+// chain of a scene, its CTAs should be placed as soon as SMs free up.
+// LANES: calls of up to LANES scenes give every scene a lane of its own, where its graph is built next to its
+// cluster FPS.  Measured with 16-CTA cluster FPS on the lanes of a 20-scene call (c2 bench, B200 at 1000 W, two runs
+// each): 4 lanes 1.090 / 1.091 M maps/s, 6 lanes 1.094 / 1.095, 8 lanes 1.053 / 1.053 (DESIGN section 8).
+// CELL_LANES: calls of more scenes build and query all graphs with one launch each on the caller's stream and sample
+// the seeds with the culled one-CTA FPS on the grids (fps_cells), CELL_LANES scenes side by side (DESIGN section 4.2).
+// A c2 scene takes ~1.4 ms on its CTA, so a 20-scene call needs 20 lanes for its FPS to end before its query: one
+// 20-scene call alone, FPS / kNN stage 2.99 ms with 10 lanes, 1.67 ms with 20; bench.py (two calls in flight) 1.174 M
+// maps/s with either (B200 at 1000 W, profiles/r12/).
 constexpr int LANES = 4;
+constexpr int CELL_LANES = 20;
 struct ForkJoin {
-  cudaStream_t fps[LANES] = {}, knn[LANES] = {};  // knn[0] stays null: lane 0 builds its graph on the caller's stream
-  cudaEvent_t fork = nullptr, join_fps[LANES] = {}, join_knn[LANES] = {};
+  cudaStream_t fps[CELL_LANES] = {}, knn[LANES] = {};  // knn[0] stays null: lane 0 builds on the caller's stream
+  cudaEvent_t fork = nullptr, built = nullptr, join_fps[CELL_LANES] = {}, join_knn[LANES] = {};
 };
 
-static int get_fork_join(cudaStream_t user, ForkJoin **out, int lanes_needed = 1) {
+static int get_fork_join(cudaStream_t user, ForkJoin **out, int fps_lanes = 1, int knn_lanes = 1) {
   constexpr int SLOTS = 16;
   struct Entry {
     int dev;
@@ -51,6 +57,7 @@ static int get_fork_join(cudaStream_t user, ForkJoin **out, int lanes_needed = 1
     if (e && !e->used) {
       e->fj = ForkJoin();
       GF_CUDA(cudaEventCreateWithFlags(&e->fj.fork, cudaEventDisableTiming));
+      GF_CUDA(cudaEventCreateWithFlags(&e->fj.built, cudaEventDisableTiming));
       e->used = true;
       e->dev = dev;
     }
@@ -62,14 +69,18 @@ static int get_fork_join(cudaStream_t user, ForkJoin **out, int lanes_needed = 1
   }
   // Lanes are created on first use: every stream beyond the device's hardware queues (CUDA_DEVICE_MAX_CONNECTIONS,
   // 8 by default) shares a queue with another one and inherits false dependencies -- a single-scene call needs
-  // exactly one auxiliary stream, only a batch of four or more scenes all of them.
+  // exactly one auxiliary stream, a call of up to LANES scenes one FPS and one kNN lane per scene, a larger call
+  // CELL_LANES FPS lanes and no kNN lane.
   ForkJoin &f = e->fj;
-  for (int l = 0; l < lanes_needed && l < LANES; ++l) {
+  int lo = 0, hi = 0;
+  GF_CUDA(cudaDeviceGetStreamPriorityRange(&lo, &hi));  // hi = numerically lowest = greatest priority
+  for (int l = 0; l < fps_lanes && l < CELL_LANES; ++l) {
     if (f.fps[l]) continue;
-    int lo = 0, hi = 0;
-    GF_CUDA(cudaDeviceGetStreamPriorityRange(&lo, &hi));  // hi = numerically lowest = greatest priority
     GF_CUDA(cudaStreamCreateWithPriority(&f.fps[l], cudaStreamNonBlocking, hi));
     GF_CUDA(cudaEventCreateWithFlags(&f.join_fps[l], cudaEventDisableTiming));
+  }
+  for (int l = 0; l < knn_lanes && l < LANES; ++l) {
+    if (f.join_knn[l]) continue;
     if (l > 0) GF_CUDA(cudaStreamCreateWithPriority(&f.knn[l], cudaStreamNonBlocking, lo));
     GF_CUDA(cudaEventCreateWithFlags(&f.join_knn[l], cudaEventDisableTiming));
   }
@@ -192,6 +203,9 @@ extern "C" int gf_guidance_seeded_scatter(const float *xyz, int N, const int *se
 // ---- a batch of scenes (the reference's call is batched: geodesic_utils.py:98 loops over the scenes) -------------
 namespace gf {
 static_assert(KNN_BATCH_MAX == GEO_BATCH_MAX, "one batched call builds and queries all its scenes' graphs at once");
+// more scenes than LANES: the graphs of all scenes are built and queried with one launch each, the seeds sampled on
+// the grids (fps_cells)
+static bool batched_graphs(int B) { return B > LANES; }
 struct BatchPlan {
   size_t per_scene[GEO_BATCH_MAX * 4];  // offsets of (fps, knn, edges) per scene
   size_t knn_ctl, scratch, scratch_bytes, stats, total;
@@ -202,7 +216,7 @@ static int plan_batch_guidance(const int *Ns, int B, int Q, int k, BatchPlan *p,
   int maxN = 1;
   for (int b = 0; b < B; ++b) {
     const int N = Ns[b];
-    fps_b[b] = align256(gf_fps_workspace_bytes(1, N, Q));
+    fps_b[b] = batched_graphs(B) ? fps_cells_workspace_bytes(N) : align256(gf_fps_workspace_bytes(1, N, Q));
     knn_b[b] = align256(knn_grid_workspace_bytes(N));
     // the edge tables are the head of a single-scene geodesic workspace; only that head is used here
     edge_b[b] = align256(geodesic_workspace_bytes(N, k, 1));
@@ -257,25 +271,27 @@ extern "C" int gf_guidance_batch(const float *const *xyz, const int *Ns, int B, 
   cudaStream_t st = (cudaStream_t)stream;
   char *w = (char *)workspace;
   ForkJoin *fj = nullptr;
-  const int lanes = B < LANES ? B : LANES;
-  int rc = get_fork_join(st, &fj, lanes);
-  if (rc) return rc;
-  stage_mark(ST_BEGIN, st);
   // The graphs.  Up to LANES scenes, every scene has a lane of its own (lane 0: the caller's stream) and its graph
   // is one short chain next to its FPS.  With more scenes a lane would run several graphs one after another, each a
   // chain of six launches ending in a single-wave tail; there the graphs of all scenes are built with one launch of
-  // each build kernel and queried with one launch, on the caller's stream (DESIGN section 4.2).
-  const bool batched = B > LANES;
+  // each build kernel and queried with one launch, on the caller's stream (DESIGN section 4.2), and the FPS lanes
+  // wait for the build: they sample the seeds on its grids (fps_cells, DESIGN section 4.1).
+  const bool batched = batched_graphs(B);
+  const int lanes = batched ? (B < CELL_LANES ? B : CELL_LANES) : B;
+  int rc = get_fork_join(st, &fj, lanes, batched ? 1 : lanes);
+  if (rc) return rc;
+  stage_mark(ST_BEGIN, st);
   GF_CUDA(cudaEventRecord(fj->fork, st));
-  for (int l = 0; l < lanes; ++l) {
-    if (!seeds_given) GF_CUDA(cudaStreamWaitEvent(fj->fps[l], fj->fork, 0));
-    if (l > 0 && !batched) GF_CUDA(cudaStreamWaitEvent(fj->knn[l], fj->fork, 0));
-  }
+  if (!batched)
+    for (int l = 0; l < lanes; ++l) {
+      if (!seeds_given) GF_CUDA(cudaStreamWaitEvent(fj->fps[l], fj->fork, 0));
+      if (l > 0) GF_CUDA(cudaStreamWaitEvent(fj->knn[l], fj->fork, 0));
+    }
   GeoSceneDesc desc[GEO_BATCH_MAX];
   int64_t *d_stats = stats ? (int64_t *)(w + p.stats) : nullptr;
   if (d_stats) GF_CUDA(cudaMemsetAsync(d_stats, 0, 16 * (size_t)B, st));
   // FPS first on every lane (the longest chains start first), then the graphs
-  if (!seeds_given)
+  if (!seeds_given && !batched)
     for (int b = 0; b < B; ++b) {
       rc = gf_furthest_point_sampling(xyz[b], 1, Ns[b], Q, seeds[b], w + p.per_scene[b * 3 + 0], fps_b[b],
                                       fj->fps[b % lanes]);
@@ -289,10 +305,19 @@ extern "C" int gf_guidance_batch(const float *const *xyz, const int *Ns, int B, 
   if (batched) {
     rc = knn_grid_build_batch(ks, B, k, w + p.knn_ctl, st, gb);
     if (rc) return rc;
+    if (!seeds_given) {  // the FPS lanes start when the grids are built, next to the query on the caller's stream
+      GF_CUDA(cudaEventRecord(fj->built, st));
+      for (int l = 0; l < lanes; ++l) GF_CUDA(cudaStreamWaitEvent(fj->fps[l], fj->built, 0));
+      for (int b = 0; b < B; ++b) {
+        rc = fps_cells(gb[b].sorted, xyz[b], Ns[b], Q, w + p.per_scene[b * 3 + 0], fps_b[b], seeds[b],
+                       fj->fps[b % lanes]);
+        if (rc) return rc;
+      }
+    }
   }
   for (int b = 0; b < B; ++b) {
     const int l = b % lanes;
-    cudaStream_t kst = l == 0 ? st : fj->knn[l];
+    cudaStream_t kst = l == 0 || batched ? st : fj->knn[l];
     if (!batched) {
       rc = knn_grid_build_batch(&ks[b], 1, k, nullptr, kst, &gb[b]);
       if (rc) return rc;
