@@ -18,6 +18,10 @@
 // right point) and reducing the 64-bit key (d2 bits, ~rank) with max.
 #include <cooperative_groups.h>
 
+#include <algorithm>
+#include <iterator>
+#include <type_traits>
+
 #include "gf_common.cuh"
 #include "gf_fps.cuh"
 
@@ -25,8 +29,50 @@ namespace cg = cooperative_groups;
 
 namespace gf {
 
+// ---- the sampling rules of every FPS kernel ----------------------------------------------------------------------
+
+// |p|^2 > 1e-3, compared in double (sampling_gpu.cu:103-104; sampling.cpp:74-76): only such a point can be a seed
+__device__ __forceinline__ bool fps_eligible(float x, float y, float z) { return !((double)sq3(x, y, z) <= 1e-3); }
+
+// The rank of original index i, (bitrev_L(i mod 2^L), i div 2^L) as one word: ascending rank is the reference's order
+// among equal distances.  fps_rank_hi is the part of the residue c = i mod 2^L, bitrev_L(c) in the top L bits.
+__device__ __forceinline__ uint32_t fps_rank_hi(uint32_t c, int L) { return L ? (__brev(c) >> (32 - L)) << (32 - L) : 0u; }
+__device__ __forceinline__ uint32_t fps_rank(uint32_t i, int L) { return fps_rank_hi(i & ((1u << L) - 1u), L) | (i >> L); }
+// the original index of the key word lo = ~rank
+__device__ __forceinline__ int fps_index(uint32_t lo, int L) {
+  const uint32_t rk = ~lo;
+  return L ? (int)(((rk & ((1u << (32 - L)) - 1u)) << L) | (__brev(rk >> (32 - L)) >> (32 - L))) : (int)rk;
+}
+
+// A candidate's 64-bit key: the bits of its running minimum, then ~rank; the largest key wins a round, and {0, 0}
+// stands for no eligible point.
+struct FpsKey {
+  uint32_t v, lo;
+};
+__device__ __forceinline__ bool operator==(FpsKey a, FpsKey b) { return a.v == b.v && a.lo == b.lo; }
+__device__ __forceinline__ bool operator>(FpsKey a, FpsKey b) { return a.v > b.v || (a.v == b.v && a.lo > b.lo); }
+// the largest key of the warp, by two REDUX
+__device__ __forceinline__ FpsKey warp_max(FpsKey k) {
+  const uint32_t v = __reduce_max_sync(0xffffffffu, k.v);
+  return {v, __reduce_max_sync(0xffffffffu, k.v == v ? k.lo : 0u)};
+}
+
+// The end of a round won by key w at (x, y, z): returns the seed and moves the centre c there.  With no eligible
+// point anywhere (w = {0, 0}) the reference's tree yields index 0, and the centre is point 0.
+__device__ __forceinline__ int fps_round_end(FpsKey w, float x, float y, float z, const float *__restrict__ xyz, int L,
+                                             float &cx, float &cy, float &cz) {
+  if ((w.v | w.lo) == 0u) {
+    cx = __ldg(xyz + 0), cy = __ldg(xyz + 1), cz = __ldg(xyz + 2);
+    return 0;
+  }
+  cx = x, cy = y, cz = z;
+  return fps_index(w.lo, L);
+}
+
+// ---- the cluster kernels -----------------------------------------------------------------------------------------
+
 struct __align__(16) FpsSlot {
-  uint32_t v, lo;  // key: distance bits, ~rank (0,0 = no eligible point in that CTA)
+  uint32_t v, lo;  // key (0,0 = no eligible point in that CTA)
   float x, y;
   float z;
   float pad[3];
@@ -34,8 +80,6 @@ struct __align__(16) FpsSlot {
 static_assert(sizeof(FpsSlot) == 32, "slot is two 16-byte vectors");
 
 constexpr int FPS_MAX_CLUSTER = 16;
-
-__device__ __forceinline__ uint32_t brev_bits(uint32_t c, int L) { return L ? (__brev(c) >> (32 - L)) : 0u; }
 
 // ---- cluster-scope mbarrier signalling (replaces barrier.cluster in the round loop) -----------------
 __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -76,13 +120,11 @@ __device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity) {
   } while (!done);
 }
 
-// P > 0 : register-resident variant, thread owns points k = c + bs*(g*P + i), i < P
-// P == 0: streaming variant for scenes that do not fit on chip: thread walks k = c + bs*(g + G*i)
-//         and keeps the running min-distance in `temp` (global, L2 resident)
+// thread u = g * 2^L + c of the cluster owns points k = c + 2^L * (g*P + i), i < P, in registers
 template <int T, int P>
 __global__ void __launch_bounds__(T, 1)
-    fps_cluster_kernel(const float *__restrict__ xyz_all, int N, int m, int L, float *__restrict__ temp_all,
-                       int *__restrict__ idx_all) {
+    fps_cluster_kernel(const float *__restrict__ xyz_all, int N, int m, int L, int *__restrict__ idx_all) {
+  static_assert(P > 0, "a scene of the cluster kernel is held in registers");
   cg::cluster_group cluster = cg::this_cluster();
   const unsigned CS = cluster.num_blocks();
   const unsigned crank = cluster.block_rank();
@@ -116,7 +158,6 @@ __global__ void __launch_bounds__(T, 1) fps_cluster_batch_kernel(const __grid_co
   const float *__restrict__ xyz = a.s[scene].xyz;
   int *__restrict__ idx = a.s[scene].idx;
   const int N = a.s[scene].N, L = a.s[scene].L;
-  float *__restrict__ temp_all = nullptr;  // register-resident instances only
 
 #include "gf_fps_cluster_body.cuh"
 }
@@ -165,7 +206,7 @@ __global__ void __launch_bounds__(FPS_GRID_T, 1)
   const unsigned bs = 1u << L;
   const unsigned c = u & (bs - 1), g = u >> L;
   const unsigned G = (nctas * T) >> L;
-  const uint32_t rank_hi = L ? (brev_bits(c, L) << (32 - L)) : 0u;
+  const uint32_t rank_hi = fps_rank_hi(c, L);
   constexpr int PR = P > 0 ? P : 1;
 
   for (int b = 0; b < B; ++b) {
@@ -183,7 +224,7 @@ __global__ void __launch_bounds__(FPS_GRID_T, 1)
           px[i] = __ldg(xyz + (size_t)k * 3 + 0);
           py[i] = __ldg(xyz + (size_t)k * 3 + 1);
           pz[i] = __ldg(xyz + (size_t)k * 3 + 2);
-          if (!((double)sq3(px[i], py[i], pz[i]) <= 1e-3)) tmp[i] = 1e10f;
+          if (fps_eligible(px[i], py[i], pz[i])) tmp[i] = 1e10f;
         }
       }
     } else {
@@ -217,7 +258,7 @@ __global__ void __launch_bounds__(FPS_GRID_T, 1)
         uint32_t i = 0;
         for (unsigned k = c + bs * g; k < (unsigned)N; k += bs * G, ++i) {
           float x = __ldg(xyz + (size_t)k * 3 + 0), y = __ldg(xyz + (size_t)k * 3 + 1), z = __ldg(xyz + (size_t)k * 3 + 2);
-          if ((double)sq3(x, y, z) <= 1e-3) continue;
+          if (!fps_eligible(x, y, z)) continue;
           float t = fminf(sq3(x - cx, y - cy, z - cz), temp[k]);
           temp[k] = t;
           if (t > best) {
@@ -228,22 +269,17 @@ __global__ void __launch_bounds__(FPS_GRID_T, 1)
         }
       }
       const bool has = best >= 0.f;
-      const uint32_t vb = has ? __float_as_uint(best) : 0u;
-      const uint32_t rank = rank_hi | (P > 0 ? (g * PR + besti) : besti);
-      const uint32_t lo = has ? ~rank : 0u;
-      uint32_t wv = __reduce_max_sync(0xffffffffu, vb);
-      uint32_t wl = __reduce_max_sync(0xffffffffu, vb == wv ? lo : 0u);
+      const FpsKey key = {has ? __float_as_uint(best) : 0u, has ? ~(rank_hi | (P > 0 ? (g * PR + besti) : besti)) : 0u};
+      const FpsKey wk = warp_max(key);
       if (lane == 0) {
-        wkey_v[buf][warp] = wv;
-        wkey_lo[buf][warp] = wl;
+        wkey_v[buf][warp] = wk.v;
+        wkey_lo[buf][warp] = wk.lo;
       }
       __syncthreads();
-      uint32_t tv = lane < T / 32 ? wkey_v[buf][lane] : 0u;
-      uint32_t tl = lane < T / 32 ? wkey_lo[buf][lane] : 0u;
-      const uint32_t cv = __reduce_max_sync(0xffffffffu, tv);
-      const uint32_t cl = __reduce_max_sync(0xffffffffu, tv == cv ? tl : 0u);
-      const bool owner = has && vb == cv && lo == cl;
-      const bool nobody = (cv | cl) == 0u;
+      const FpsKey ck = warp_max({lane < T / 32 ? wkey_v[buf][lane] : 0u, lane < T / 32 ? wkey_lo[buf][lane] : 0u});
+      // field by field: `has && key == ck` allocates the kernel's registers differently
+      const bool owner = has && key.v == ck.v && key.lo == ck.lo;
+      const bool nobody = (ck.v | ck.lo) == 0u;
       if (owner || (nobody && tid == 0)) {
         if (P > 0 && owner) {
 #pragma unroll
@@ -251,8 +287,8 @@ __global__ void __launch_bounds__(FPS_GRID_T, 1)
             if (besti == (uint32_t)i) bx = px[i], by = py[i], bz = pz[i];
         }
         uint2 *dst = slots + ((size_t)buf * nctas + blockIdx.x) * FPS_SLOT_WORDS;
-        st_cg_v2(dst + 0, cv, tag);
-        st_cg_v2(dst + 1, cl, tag);
+        st_cg_v2(dst + 0, ck.v, tag);
+        st_cg_v2(dst + 1, ck.lo, tag);
         st_cg_v2(dst + 2, __float_as_uint(bx), tag);
         st_cg_v2(dst + 3, __float_as_uint(by), tag);
         st_cg_v2(dst + 4, __float_as_uint(bz), tag);
@@ -264,7 +300,8 @@ __global__ void __launch_bounds__(FPS_GRID_T, 1)
         // one L2 round trip per word, and polling all five words of every slot made the 148 x 32 pollers
         // congest the few L2 lines that hold the slots.
         constexpr int MAXS = (FPS_MAX_GRID_CTAS + 31) / 32;
-        uint32_t gv = 0, gl = 0, src = 0;
+        FpsKey gk = {0u, 0u};
+        uint32_t src = 0;
         unsigned pend = 0;
 #pragma unroll
         for (int sI = 0; sI < MAXS; ++sI)
@@ -285,14 +322,12 @@ __global__ void __launch_bounds__(FPS_GRID_T, 1)
           for (int sI = 0; sI < MAXS; ++sI)
             if (((pend >> sI) & 1u) && (uint32_t)(w[sI][0] >> 32) == tag && (uint32_t)(w[sI][1] >> 32) == tag) {
               pend &= ~(1u << sI);
-              const uint32_t sv = (uint32_t)w[sI][0], sl = (uint32_t)w[sI][1];
-              if (sv > gv || (sv == gv && sl > gl)) gv = sv, gl = sl, src = lane + 32u * sI;
+              const FpsKey sk = {(uint32_t)w[sI][0], (uint32_t)w[sI][1]};
+              if (sk > gk) gk = sk, src = lane + 32u * sI;
             }
         }
-        const uint32_t mv = __reduce_max_sync(0xffffffffu, gv);
-        const uint32_t ml = __reduce_max_sync(0xffffffffu, gv == mv ? gl : 0u);
-        const unsigned wm = __ballot_sync(0xffffffffu, gv == mv && gl == ml);
-        if (lane == (unsigned)(__ffs(wm) - 1)) {
+        const FpsKey mk = warp_max(gk);
+        if (lane == (unsigned)(__ffs(__ballot_sync(0xffffffffu, gk == mk)) - 1)) {
           const uint2 *sp = slots + ((size_t)buf * nctas + src) * FPS_SLOT_WORDS;
           unsigned long long x, y, z;
           do {  // the three coordinate words of the winner, requested together
@@ -301,21 +336,13 @@ __global__ void __launch_bounds__(FPS_GRID_T, 1)
           s_center[buf][0] = __uint_as_float((uint32_t)x);
           s_center[buf][1] = __uint_as_float((uint32_t)y);
           s_center[buf][2] = __uint_as_float((uint32_t)z);
-          s_win[buf][0] = mv;
-          s_win[buf][1] = ml;
+          s_win[buf][0] = mk.v;
+          s_win[buf][1] = mk.lo;
         }
       }
       __syncthreads();
-      const uint32_t gv = s_win[buf][0], gl = s_win[buf][1];
-      int old;
-      if ((gv | gl) == 0u) {  // no eligible point anywhere: the reference's tree yields index 0
-        old = 0;
-        cx = __ldg(xyz + 0), cy = __ldg(xyz + 1), cz = __ldg(xyz + 2);
-      } else {
-        const uint32_t rk = ~gl;
-        old = L ? (int)(((rk & ((1u << (32 - L)) - 1u)) << L) | brev_bits(rk >> (32 - L), L)) : (int)rk;
-        cx = s_center[buf][0], cy = s_center[buf][1], cz = s_center[buf][2];
-      }
+      const int old = fps_round_end({s_win[buf][0], s_win[buf][1]}, s_center[buf][0], s_center[buf][1],
+                                    s_center[buf][2], xyz, L, cx, cy, cz);
       if (u == 0) idx[j] = old;
     }
   }
@@ -328,43 +355,67 @@ static int ref_log2_block(int n) {
   return L;
 }
 
+// The cluster kernels' shapes, in the order plan_fps tries them; a cluster of CS CTAs holds CS * T * P points.  Few,
+// fat warps: a round costs (points per SM) x ~10 instructions of arithmetic plus ~150 instructions of reduction /
+// signalling PER WARP, so 8 warps with up to 32 register-resident points per thread beat 32 warps with 8 (measured:
+// 1.87 us -> see profiles/).
+struct FpsShape {
+  int T, P;
+};
+constexpr FpsShape kFpsClusterShapes[] = {{256, 1},  {256, 2},  {256, 4},  {256, 8},  {256, 12},
+                                          {256, 16}, {256, 20}, {256, 25}, {256, 32}, {512, 24}};
+constexpr FpsShape kFpsLargestShape = kFpsClusterShapes[std::size(kFpsClusterShapes) - 1];
+// the grid kernel's points per thread; the last, 0, streams them from L2 and takes any N
+constexpr int kFpsGridP[] = {8, 16, 24, 32, 0};
+
+static long long fps_cluster_capacity(int cs) { return (long long)cs * kFpsLargestShape.T * kFpsLargestShape.P; }
+
 struct FpsPlan {
-  int T, P, CS;  // CS == 0: whole-GPU (cooperative) variant, T = 256
+  bool grid;  // the whole-GPU cooperative kernel (T = FPS_GRID_T) instead of one cluster per scene
+  int T, P;   // threads per CTA, points per thread
+  int ctas;   // CTAs per cluster, or of the whole grid
 };
 
-// Few, fat warps: a round costs (points per SM) x ~10 instructions of arithmetic plus ~150 instructions
-// of reduction / signalling PER WARP, so 8 warps with up to 32 register-resident points per thread beat
-// 32 warps with 8 (measured: 1.87 us -> see profiles/).  Capacity = CS * T * P.
-static const int kFpsP256[] = {1, 2, 4, 8, 12, 16, 20, 25, 32};
-
 static FpsPlan plan_fps(int N, int max_cs) {
-  if (N < 512) return {256, N <= 256 ? 1 : 2, 1};  // reference block size bs <= 256 <= T
+  if (N < 512) return {false, 256, N <= 256 ? 1 : 2, 1};  // reference block size bs <= 256 <= T
   // smallest power-of-two cluster (>= 2 so that CS * 256 covers the 512 residue classes) whose
   // 256-thread CTAs hold the scene with P <= 32; prefer the largest cluster (least work per SM per round)
   int cs = max_cs;
   while (cs > 2 && (long long)(cs / 2) * 256 * 4 >= N) cs /= 2;  // tiny scenes: do not spread thinner than 4 pts/thread
-  for (int pi = 0; pi < (int)(sizeof(kFpsP256) / sizeof(int)); ++pi)
-    if ((long long)cs * 256 * kFpsP256[pi] >= N) return {256, kFpsP256[pi], cs};
-  if ((long long)max_cs * 512 * 24 >= N) return {512, 24, max_cs};
+  // a cluster smaller than max_cs holds the scene at P = 4, so the 512-thread shape only ever runs on max_cs CTAs
+  for (const FpsShape &s : kFpsClusterShapes)
+    if ((long long)cs * s.T * s.P >= N) return {false, s.T, s.P, cs};
   // beyond one cluster: one CTA per SM, registers if the scene fits (P <= 32), else streaming from L2
-  int ctas = num_sms() & ~1;  // even, so that CTAs * 256 covers whole sets of 512 residue classes
-  if (ctas > FPS_MAX_GRID_CTAS) ctas = FPS_MAX_GRID_CTAS;  // what launch_fps_grid launches
-  const int p_opts[4] = {8, 16, 24, 32};
-  for (int pi = 0; pi < 4; ++pi)
-    if ((long long)ctas * FPS_GRID_T * p_opts[pi] >= N) return {FPS_GRID_T, p_opts[pi], 0};
-  return {FPS_GRID_T, 0, 0};
+  const int ctas = std::min(num_sms() & ~1, FPS_MAX_GRID_CTAS);  // even: CTAs * 256 covers whole sets of 512 classes
+  int P = 0;  // the streaming instance, unless the scene fits in registers
+  for (int p : kFpsGridP)
+    if (P == 0 && p && (long long)ctas * FPS_GRID_T * p >= N) P = p;
+  return {true, FPS_GRID_T, P, ctas};
 }
 
-template <int P>
-static int launch_fps_grid(const float *xyz, int B, int N, int m, int L, float *temp, int *idx, uint2 *slots,
-                           cudaStream_t st) {
-  int ctas = num_sms() & ~1;
-  if (ctas > FPS_MAX_GRID_CTAS) ctas = FPS_MAX_GRID_CTAS;
-  GF_CUDA(cudaMemsetAsync(slots, 0, sizeof(uint2) * 2 * FPS_SLOT_WORDS * (size_t)ctas, st));  // tag 0 = never written
-  void *args[] = {(void *)&xyz, &B, &N, &m, &L, &temp, &idx, &slots};
-  GF_CUDA(cudaLaunchCooperativeKernel((const void *)fps_grid_kernel<P>, dim3(ctas), dim3(FPS_GRID_T), args, 0, st));
-  count_launch();
-  return GF_OK;
+// launch(T, P) with the cluster shape (T, P) as compile-time constants (std::integral_constant)
+template <int I = 0, typename F>
+static int with_cluster_shape(int T, int P, F &&launch) {
+  constexpr FpsShape s = kFpsClusterShapes[I];
+  if (T == s.T && P == s.P) return launch(std::integral_constant<int, s.T>(), std::integral_constant<int, s.P>());
+  if constexpr (I + 1 < (int)std::size(kFpsClusterShapes)) {
+    return with_cluster_shape<I + 1>(T, P, launch);
+  } else {
+    set_error("furthest_point_sampling: no cluster kernel for T=%d P=%d", T, P);
+    return GF_ERR_INVALID;
+  }
+}
+
+// launch(P) with the grid kernel's P as a compile-time constant
+template <int I = 0, typename F>
+static int with_grid_p(int P, F &&launch) {
+  if (P == kFpsGridP[I]) return launch(std::integral_constant<int, kFpsGridP[I]>());
+  if constexpr (I + 1 < (int)std::size(kFpsGridP)) {
+    return with_grid_p<I + 1>(P, launch);
+  } else {
+    set_error("furthest_point_sampling: no grid kernel for P=%d", P);
+    return GF_ERR_INVALID;
+  }
 }
 
 // FPS is the longest dependency chain of the hot path (m - 1 dependent rounds on a few SMs): its CTAs should be
@@ -403,26 +454,16 @@ static int launch_clusters(void (*kern)(KArgs...), int T, int B, int CS, cudaStr
   return GF_OK;
 }
 
-template <int T, int P>
-static int launch_fps(const float *xyz, int B, int N, int m, int L, int CS, float *temp, int *idx, cudaStream_t st) {
-  return launch_clusters(fps_cluster_kernel<T, P>, T, B, CS, st, xyz, N, m, L, temp, idx);
-}
-
-template <int T, int P>
-static int launch_fps_batch(const FpsBatchArgs &a, int B, int m, int CS, cudaStream_t st) {
-  return launch_clusters(fps_cluster_batch_kernel<T, P>, T, B, CS, st, a, m);
-}
-
 static int max_cluster_size() {
-  // 16 (non-portable) when the device can co-schedule a 16-CTA x 1024-thread cluster, else 8
+  // 16 (non-portable) when the device can co-schedule a 16-CTA cluster of the largest shape, else 8
   static int cached = 0;
   if (cached) return cached;
-  auto kern = fps_cluster_kernel<1024, 0>;
+  auto kern = fps_cluster_kernel<kFpsLargestShape.T, kFpsLargestShape.P>;
   int ok16 = 0;
   if (cudaFuncSetAttribute(kern, cudaFuncAttributeNonPortableClusterSizeAllowed, 1) == cudaSuccess) {
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(16, 1, 1);
-    cfg.blockDim = dim3(1024, 1, 1);
+    cfg.blockDim = dim3(kFpsLargestShape.T, 1, 1);
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeClusterDimension;
     attr[0].val.clusterDim.x = 16;
@@ -438,6 +479,15 @@ static int max_cluster_size() {
   return cached;
 }
 
+// The workspace of the whole-GPU kernel, for sizing (over a null workspace the Arena only measures) and for the
+// launch: exchange slots for up to 256 CTAs, then the (B, N) running minima of the streaming instance.
+static Arena fps_carve(void *workspace, size_t workspace_bytes, int B, int N, uint2 **slots, float **temp) {
+  Arena ar(workspace, workspace_bytes);
+  *slots = ar.take<uint2>(2 * FPS_SLOT_WORDS * 256);
+  *temp = ar.take<float>((size_t)B * N);
+  return ar;
+}
+
 // ---------------------------------------------------------------------------------------------------
 // Culled FPS on the cell order of the kNN grid: the seeds of a batched guidance call, one 1024-thread CTA per scene.
 // A new seed c can only lower the running minimum t of a point closer to c than t, a neighbourhood of c that shrinks
@@ -445,7 +495,9 @@ static int max_cluster_size() {
 // each with the tight box of its eligible points and the largest key of its points kept on chip; a round updates a
 // block only if a lower bound of sq3(p - c) over its box is below the block's largest t, which skips 87-94 % of the
 // point updates at c2 (tools/fps_cells_mirror.py).  Keys, tie order and the no-eligible-point rule are those of the
-// cluster body, so the seeds are the reference's bit for bit.
+// sampling rules above, so the seeds are the reference's bit for bit.  The key order (FpsKey's operator>), the rank
+// (fps_rank) and the end of a round (fps_round_end) are written out in place here: through those helpers the kernel
+// compiled to other code and bench.py ran 0.1-0.3 % slower on a B200 (profiles/r13).
 //
 // Exactness of a skip: every point of a skipped block keeps t, because its computed d = sq3(px - cx, ...) >= lb >= t.
 // Per axis fl(px - cx) is at least the box gap fl(lo - cx) (or fl(cx - hi)) in magnitude, since rounding is monotonic,
@@ -526,7 +578,7 @@ __global__ void __launch_bounds__(FPS_CELLS_T, 1)
           const bool real = b[u] >= 0 && pos < N;  // b[u] < 0 gives a negative pos: no point, nothing stored
           const float4 a = p[u][q];
           float told = t[u][q];
-          if (init && real && !((double)sq3(a.x, a.y, a.z) <= 1e-3)) {
+          if (init && real && fps_eligible(a.x, a.y, a.z)) {
             told = 1e10f;
             lx[u] = fminf(lx[u], a.x), ly[u] = fminf(ly[u], a.y), lz[u] = fminf(lz[u], a.z);
             hx[u] = fmaxf(hx[u], a.x), hy[u] = fmaxf(hy[u], a.y), hz[u] = fmaxf(hz[u], a.z);
@@ -543,8 +595,8 @@ __global__ void __launch_bounds__(FPS_CELLS_T, 1)
 #pragma unroll
     for (int u = 0; u < U; ++u) {
       if (b[u] < 0) continue;
-      const uint32_t wv = __reduce_max_sync(0xffffffffu, bv[u]);
-      const uint32_t wl = __reduce_max_sync(0xffffffffu, bv[u] == wv ? bl[u] : 0u);
+      const FpsKey wk = warp_max({bv[u], bl[u]});
+      const uint32_t wv = wk.v, wl = wk.lo;
       const int src = __ffs(__ballot_sync(0xffffffffu, bv[u] == wv && bl[u] == wl)) - 1;
       const float x = __shfl_sync(0xffffffffu, bx[u], src), y = __shfl_sync(0xffffffffu, by[u], src),
                   z = __shfl_sync(0xffffffffu, bz[u], src);
@@ -615,24 +667,23 @@ __global__ void __launch_bounds__(FPS_CELLS_T, 1)
       const uint32_t v = su[6 * stride + e], lo = su[7 * stride + e];
       if (v > bv || (v == bv && lo > bl)) bv = v, bl = lo, be = e;
     }
-    const uint32_t wv = __reduce_max_sync(0xffffffffu, bv);
-    const uint32_t wl = __reduce_max_sync(0xffffffffu, bv == wv ? bl : 0u);
+    const FpsKey wk = warp_max({bv, bl});
+    const uint32_t wv = wk.v, wl = wk.lo;
     if ((unsigned)(__ffs(__ballot_sync(0xffffffffu, bv == wv && bl == wl)) - 1) == lane)
       slot[buf][warp] = (wv | wl) ? FpsCellsSlot{wv, wl, sf[8 * stride + be], sf[9 * stride + be], sf[10 * stride + be]}
                                   : FpsCellsSlot{0u, 0u, 0.f, 0.f, 0.f};
     if (threadIdx.x == 0) list_n[buf ^ 1] = 0;  // the next round's list (its last reader finished before this round)
     __syncthreads();
     const uint32_t sv = slot[buf][lane].v, sl = slot[buf][lane].lo;  // NW == 32: one candidate per lane
-    const uint32_t gv = __reduce_max_sync(0xffffffffu, sv);
-    const uint32_t gl = __reduce_max_sync(0xffffffffu, sv == gv ? sl : 0u);
+    const FpsKey gk = warp_max({sv, sl});
+    const uint32_t gv = gk.v, gl = gk.lo;
     int old;
     if ((gv | gl) == 0u) {  // no eligible point anywhere: the reference's tree yields index 0
       old = 0;
       cx = __ldg(xyz + 0), cy = __ldg(xyz + 1), cz = __ldg(xyz + 2);
     } else {
       const int ws = __ffs(__ballot_sync(0xffffffffu, sv == gv && sl == gl)) - 1;
-      const uint32_t rk = ~gl;
-      old = L ? (int)(((rk & ((1u << (32 - L)) - 1u)) << L) | brev_bits(rk >> (32 - L), L)) : (int)rk;
+      old = fps_index(gl, L);
       cx = slot[buf][ws].x, cy = slot[buf][ws].y, cz = slot[buf][ws].z;
     }
     if (threadIdx.x == 0) idx[j] = old;
@@ -700,14 +751,13 @@ int fps_cells(const float4 *sorted, const float *xyz, int N, int m, void *worksp
 
 using namespace gf;
 
-// workspace layout (only for scenes beyond the smallest cluster capacity): [slots: 4 x 256 uint4][temp: (B,N) f32]
-static const size_t kFpsSlotBytes = sizeof(uint2) * 2 * FPS_SLOT_WORDS * 256;  // up to 256 CTAs
-
 extern "C" size_t gf_fps_workspace_bytes(int B, int N, int m) {
   (void)m;
   if (B <= 0 || N <= 0) return 0;
-  if ((long long)8 * 512 * 24 >= N) return 0;  // fits an 8-CTA cluster on every device: no scratch at all
-  return align256(kFpsSlotBytes) + align256(sizeof(float) * (size_t)B * N);
+  if (fps_cluster_capacity(8) >= N) return 0;  // fits an 8-CTA cluster on every device: no scratch at all
+  uint2 *slots;
+  float *temp;
+  return fps_carve(nullptr, 0, B, N, &slots, &temp).off;
 }
 
 extern "C" int gf_furthest_point_sampling(const float *xyz, int B, int N, int m, int *idx, void *workspace,
@@ -721,41 +771,26 @@ extern "C" int gf_furthest_point_sampling(const float *xyz, int B, int N, int m,
     return GF_OK;
   }
   GF_CHECK_ARG(xyz, "furthest_point_sampling: null xyz");
-  const int L = ref_log2_block(N);
-  FpsPlan p = plan_fps(N, max_cluster_size());
-  float *temp = nullptr;
-  uint2 *slots = nullptr;
-  if (p.P == 0 || p.CS == 0) {
-    size_t need = align256(kFpsSlotBytes) + align256(sizeof(float) * (size_t)B * N);
-    if (workspace == nullptr || workspace_bytes < need) {
-      set_error("furthest_point_sampling: N=%d needs a %zu-byte workspace (gf_fps_workspace_bytes)", N, need);
-      return GF_ERR_WORKSPACE;
-    }
-    slots = (uint2 *)workspace;
-    temp = (float *)((char *)workspace + align256(kFpsSlotBytes));
+  int L = ref_log2_block(N);
+  const FpsPlan p = plan_fps(N, max_cluster_size());
+  if (!p.grid)
+    return with_cluster_shape(p.T, p.P, [&](auto T, auto P) {
+      return launch_clusters(fps_cluster_kernel<T, P>, T, B, p.ctas, st, xyz, N, m, L, idx);
+    });
+  uint2 *slots;
+  float *temp;
+  const Arena ar = fps_carve(workspace, workspace_bytes, B, N, &slots, &temp);
+  if (!ar.ok) {
+    set_error("furthest_point_sampling: N=%d needs a %zu-byte workspace (gf_fps_workspace_bytes)", N, ar.off);
+    return GF_ERR_WORKSPACE;
   }
-  if (p.CS == 0) {
-    if (p.P == 8) return launch_fps_grid<8>(xyz, B, N, m, L, temp, idx, slots, st);
-    if (p.P == 16) return launch_fps_grid<16>(xyz, B, N, m, L, temp, idx, slots, st);
-    if (p.P == 24) return launch_fps_grid<24>(xyz, B, N, m, L, temp, idx, slots, st);
-    if (p.P == 32) return launch_fps_grid<32>(xyz, B, N, m, L, temp, idx, slots, st);
-    return launch_fps_grid<0>(xyz, B, N, m, L, temp, idx, slots, st);
-  }
-#define GF_FPS_CASE(TT, PP) \
-  if (p.T == TT && p.P == PP) return launch_fps<TT, PP>(xyz, B, N, m, L, p.CS, temp, idx, st)
-  GF_FPS_CASE(256, 1);
-  GF_FPS_CASE(256, 2);
-  GF_FPS_CASE(256, 4);
-  GF_FPS_CASE(256, 8);
-  GF_FPS_CASE(256, 12);
-  GF_FPS_CASE(256, 16);
-  GF_FPS_CASE(256, 20);
-  GF_FPS_CASE(256, 25);
-  GF_FPS_CASE(256, 32);
-  GF_FPS_CASE(512, 24);
-#undef GF_FPS_CASE
-  set_error("furthest_point_sampling: no kernel variant for N=%d", N);
-  return GF_ERR_INVALID;
+  return with_grid_p(p.P, [&](auto P) {
+    GF_CUDA(cudaMemsetAsync(slots, 0, sizeof(uint2) * 2 * FPS_SLOT_WORDS * (size_t)p.ctas, st));  // tag 0 = unwritten
+    void *args[] = {(void *)&xyz, &B, &N, &m, &L, &temp, &idx, &slots};
+    GF_CUDA(cudaLaunchCooperativeKernel((const void *)fps_grid_kernel<P>, dim3(p.ctas), dim3(FPS_GRID_T), args, 0, st));
+    count_launch();
+    return GF_OK;
+  });
 }
 
 // ---- a ragged batch: scenes b of the flat (offsets[B], 3) array --------------------------------------------------
@@ -763,26 +798,6 @@ extern "C" int gf_furthest_point_sampling(const float *xyz, int B, int N, int m,
 // a larger scene runs the whole-GPU kernel of the single-scene call, after the cluster launches.  The largest scene
 // sets the cluster size: at the model's sizes (60k-150k points) a smaller cluster cannot hold it (8 CTAs: 98,304
 // points), so a batch with more scenes than co-resident clusters runs them in waves rather than on thinner clusters.
-static int launch_fps_batch(const FpsPlan &p, const FpsBatchArgs &a, int B, int m, cudaStream_t st) {
-#define GF_FPS_CASE(TT, PP) \
-  if (p.T == TT && p.P == PP) return launch_fps_batch<TT, PP>(a, B, m, p.CS, st)
-  GF_FPS_CASE(256, 1);
-  GF_FPS_CASE(256, 2);
-  GF_FPS_CASE(256, 4);
-  GF_FPS_CASE(256, 8);
-  GF_FPS_CASE(256, 12);
-  GF_FPS_CASE(256, 16);
-  GF_FPS_CASE(256, 20);
-  GF_FPS_CASE(256, 25);
-  GF_FPS_CASE(256, 32);
-  GF_FPS_CASE(512, 24);
-#undef GF_FPS_CASE
-  set_error("furthest_point_sampling_batch: no cluster kernel variant for T=%d P=%d", p.T, p.P);
-  return GF_ERR_INVALID;
-}
-
-static int fps_cluster_capacity() { return max_cluster_size() * 512 * 24; }
-
 extern "C" size_t gf_fps_batch_workspace_bytes(const int *offsets, int B, int m) {
   if (!offsets || B <= 0) return 0;
   size_t need = 0;
@@ -803,7 +818,7 @@ extern "C" int gf_furthest_point_sampling_batch(const float *xyz, const int *off
     GF_CHECK_ARG(offsets[b + 1] >= offsets[b], "furthest_point_sampling_batch: offsets fall at scene %d", b);
   GF_CHECK_ARG(xyz || offsets[B] == 0, "furthest_point_sampling_batch: null xyz");
   cudaStream_t st = (cudaStream_t)stream;
-  const int cap = fps_cluster_capacity();
+  const long long cap = fps_cluster_capacity(max_cluster_size());
   int Nmax = 0;
   for (int b = 0; b < B; ++b) {
     const int N = offsets[b + 1] - offsets[b];
@@ -817,7 +832,9 @@ extern "C" int gf_furthest_point_sampling_batch(const float *xyz, const int *off
       const int N = b < B ? offsets[b + 1] - offsets[b] : 0;
       if (b < B && N >= 1 && N <= cap) a.s[n++] = {xyz + (size_t)offsets[b] * 3, idx + (size_t)b * m, N, ref_log2_block(N)};
       if (n == FPS_BATCH_MAX || (b == B && n > 0)) {
-        const int rc = launch_fps_batch(p, a, n, m, st);
+        const int rc = with_cluster_shape(p.T, p.P, [&](auto T, auto P) {
+          return launch_clusters(fps_cluster_batch_kernel<T, P>, T, n, p.ctas, st, a, m);
+        });
         if (rc) return rc;
         n = 0;
       }

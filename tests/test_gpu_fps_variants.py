@@ -23,8 +23,8 @@ import torch
 
 from test_oracle_golden import _fps_by_key_rule
 
-P256 = (1, 2, 4, 8, 12, 16, 20, 25, 32)  # kFpsP256
-GRID_P = (8, 16, 24, 32)
+P256 = (1, 2, 4, 8, 12, 16, 20, 25, 32)  # the 256-thread shapes of kFpsClusterShapes
+GRID_P = (8, 16, 24, 32)  # kFpsGridP without the streaming 0
 GRID_T = 256  # FPS_GRID_T
 MAX_GRID_CTAS = 160  # FPS_MAX_GRID_CTAS
 B200 = (16, 148)  # (largest cluster, SMs) of a B200: the shape the CPU checks are made for
@@ -41,7 +41,7 @@ def _grid_ctas(sms):
 
 
 def _plan(N, max_cs, sms):
-    """plan_fps (gf_fps.cu:453-469) restated -> (("cluster", T, P) or ("grid", P), CTAs per scene)"""
+    """plan_fps (gf_fps.cu) restated -> (("cluster", T, P) or ("grid", P), CTAs per scene)"""
     if N < 512:
         return ("cluster", 256, 1 if N <= 256 else 2), 1
     cs = max_cs
