@@ -439,9 +439,17 @@ static void agt_fill(AgtArgs &a, const float *xyz, const float *new_xyz, const f
 
 using namespace gf;
 
+// the training forward's workspace: the per-CTA partial batch statistics
+static Arena agt_train_carve(void *workspace, size_t workspace_bytes, int B, int m, double **spart) {
+  Arena a(workspace, workspace_bytes);
+  *spart = a.take<double>((size_t)agt_grid(B, m, AGT_STATS_PER_SM) * 2 * AGT_W);
+  return a;
+}
+
 extern "C" size_t gf_group_mlp_pool_train_workspace_bytes(int B, int m) {
   if (B <= 0 || m <= 0) return 0;
-  return align256(sizeof(double) * 2 * AGT_W * (size_t)agt_grid(B, m, AGT_STATS_PER_SM));
+  double *spart;
+  return agt_train_carve(nullptr, 0, B, m, &spart).off;
 }
 
 extern "C" int gf_group_mlp_pool_train(const float *xyz, const float *new_xyz, const float *features, const int *idx,
@@ -459,12 +467,9 @@ extern "C" int gf_group_mlp_pool_train(const float *xyz, const float *new_xyz, c
       GF_CHECK_ARG(gammas[l] && betas[l] && eps[l] > 0.f, "group_mlp_pool_train: layer %d needs gamma, beta, eps > 0", l);
   if (B == 0 || m == 0) return GF_OK;
   const int grid = agt_grid(B, m, AGT_STATS_PER_SM);
-  Arena ar(workspace, workspace_bytes);
-  double *spart = ar.take<double>((size_t)grid * 2 * AGT_W);
-  if (!ar.ok) {
-    set_error("group_mlp_pool_train: workspace too small");
-    return GF_ERR_WORKSPACE;
-  }
+  double *spart;
+  const Arena ar = agt_train_carve(workspace, workspace_bytes, B, m, &spart);
+  if (!ar.ok) return ar.fail("group_mlp_pool_train");
   AgtArgs a;
   agt_fill(a, xyz, new_xyz, features, idx, B, N, m, nsample, C, radius, normalize_xyz, use_xyz, n_layers, widths,
            weights, batch_stats, consts, pool_avg);
@@ -490,14 +495,38 @@ extern "C" int gf_group_mlp_pool_train(const float *xyz, const float *new_xyz, c
                            widths, weights, sc, sh, pool_avg, out, stream);
 }
 
+// The backward's workspace: the pooling winners, the statistics and per-CTA partial sums of the layers, the
+// gradient of every grouped sample, and the counting sort of the samples by source point that gathers dfeatures
+struct AgtBwdLayout {
+  int *arg;
+  double *S;
+  float *wpart;
+  double *Spart;
+  float *gx;
+  int *cnt, *off, *slot, *tsum;
+  int tiles;
+};
+static Arena agt_bwd_carve(void *workspace, size_t workspace_bytes, int B, int N, int m, int nsample, int C,
+                           AgtBwdLayout *l) {
+  Arena a(workspace, workspace_bytes);
+  const size_t grid = (size_t)agt_grid(B, m, AGT_BWD_PER_SM), ent = (size_t)B * m * nsample, nkeys = (size_t)B * N;
+  l->tiles = (int)((nkeys + AGT_SCAN_THREADS - 1) / AGT_SCAN_THREADS);
+  l->arg = a.take<int>((size_t)B * m * AGT_W);
+  l->S = a.take<double>(AGT_MAX_LAYERS * 2 * AGT_W);
+  l->wpart = a.take<float>(grid * AGT_WROW);
+  l->Spart = a.take<double>(grid * 2 * AGT_W);
+  l->gx = a.take<float>(ent * (size_t)C);
+  l->cnt = a.take<int>(nkeys);
+  l->off = a.take<int>(nkeys + 1);
+  l->slot = a.take<int>(ent);
+  l->tsum = a.take<int>((size_t)l->tiles);
+  return a;
+}
+
 extern "C" size_t gf_group_mlp_pool_backward_workspace_bytes(int B, int N, int m, int nsample, int C) {
   if (B <= 0 || m <= 0 || N <= 0 || nsample <= 0 || C < 0) return 0;
-  const size_t grid = (size_t)agt_grid(B, m, AGT_BWD_PER_SM), ent = (size_t)B * m * nsample;
-  return align256(sizeof(int) * (size_t)B * m * AGT_W) + align256(sizeof(double) * AGT_MAX_LAYERS * 2 * AGT_W) +
-         align256(sizeof(float) * grid * AGT_WROW) + align256(sizeof(double) * grid * 2 * AGT_W) +
-         align256(sizeof(float) * ent * (size_t)C) + align256(sizeof(int) * (size_t)B * N) +
-         align256(sizeof(int) * ((size_t)B * N + 1)) + align256(sizeof(int) * ent) +
-         align256(sizeof(int) * (((size_t)B * N + AGT_SCAN_THREADS - 1) / AGT_SCAN_THREADS));
+  AgtBwdLayout l;
+  return agt_bwd_carve(nullptr, 0, B, N, m, nsample, C, &l).off;
 }
 
 extern "C" int gf_group_mlp_pool_backward(const float *xyz, const float *new_xyz, const float *features,
@@ -520,29 +549,17 @@ extern "C" int gf_group_mlp_pool_backward(const float *xyz, const float *new_xyz
     if (dfeatures && C > 0) GF_CUDA(cudaMemsetAsync(dfeatures, 0, sizeof(float) * (size_t)B * C * N, st));
     return GF_OK;
   }
+  AgtBwdLayout l;
+  const Arena ar = agt_bwd_carve(workspace, workspace_bytes, B, N, m, nsample, C, &l);
+  if (!ar.ok) return ar.fail("group_mlp_pool_backward");
   const int grid = agt_grid(B, m, AGT_BWD_PER_SM);
   const size_t ent = (size_t)B * m * nsample;
-  Arena ar(workspace, workspace_bytes);
   AgtArgs a;
   agt_fill(a, xyz, new_xyz, features, idx, B, N, m, nsample, C, radius, normalize_xyz, use_xyz, n_layers, widths,
            weights, batch_stats, const_cast<float *>(consts), pool_avg);
   a.dout = dout;
-  a.arg = ar.take<int>((size_t)B * m * AGT_W);
-  double *S = ar.take<double>(AGT_MAX_LAYERS * 2 * AGT_W);
-  a.S = S;
-  a.wpart = ar.take<float>((size_t)grid * AGT_WROW);
-  a.Spart = ar.take<double>((size_t)grid * 2 * AGT_W);
-  a.gx = ar.take<float>(ent * (size_t)C);
-  int *cnt = ar.take<int>((size_t)B * N);
-  int *off = ar.take<int>((size_t)B * N + 1);
-  int *slot = ar.take<int>(ent);
+  a.arg = l.arg, a.S = l.S, a.wpart = l.wpart, a.Spart = l.Spart, a.gx = l.gx;
   const long long nkeys = (long long)B * N;
-  const int tiles = (int)((nkeys + AGT_SCAN_THREADS - 1) / AGT_SCAN_THREADS);
-  int *tsum = ar.take<int>((size_t)tiles);
-  if (!ar.ok) {
-    set_error("group_mlp_pool_backward: workspace too small");
-    return GF_ERR_WORKSPACE;
-  }
   const bool want_dfeat = dfeatures && C > 0;
   if (!want_dfeat) a.gx = nullptr;
   if (want_dfeat) GF_CUDA(cudaMemsetAsync(a.gx, 0, sizeof(float) * ent * C, st));  // samples without gradient
@@ -558,25 +575,25 @@ extern "C" int gf_group_mlp_pool_backward(const float *xyz, const float *new_xyz
     GF_LAUNCHED();
     agg_backward_finish_kernel<<<fin_blocks, 128, 0, st>>>(a.wpart, a.Spart, grid, p, n_layers,
                                                           p < n_layers ? widths[p + 1] : 0, p < n_layers ? widths[p] : 0,
-                                                          p < n_layers ? dweights[p] : nullptr, dvec, S,
+                                                          p < n_layers ? dweights[p] : nullptr, dvec, l.S,
                                                           p >= 1 ? widths[p] : 0);
     GF_LAUNCHED();
   }
   if (!want_dfeat) return GF_OK;
   const int mns = m * nsample;
   const int eb = (int)((ent + 255) / 256 < (size_t)num_sms() * 16 ? (ent + 255) / 256 : (size_t)num_sms() * 16);
-  GF_CUDA(cudaMemsetAsync(cnt, 0, sizeof(int) * (size_t)B * N, st));
-  agg_count_kernel<<<eb, 256, 0, st>>>(idx, (long long)ent, mns, N, cnt);
+  GF_CUDA(cudaMemsetAsync(l.cnt, 0, sizeof(int) * (size_t)B * N, st));
+  agg_count_kernel<<<eb, 256, 0, st>>>(idx, (long long)ent, mns, N, l.cnt);
   GF_LAUNCHED();
-  agg_scan_tiles_kernel<<<tiles, AGT_SCAN_THREADS, 0, st>>>(cnt, nkeys, off, tsum);
+  agg_scan_tiles_kernel<<<l.tiles, AGT_SCAN_THREADS, 0, st>>>(l.cnt, nkeys, l.off, l.tsum);
   GF_LAUNCHED();
-  agg_scan_totals_kernel<<<1, AGT_SCAN_THREADS, 0, st>>>(tsum, tiles, off + nkeys);
+  agg_scan_totals_kernel<<<1, AGT_SCAN_THREADS, 0, st>>>(l.tsum, l.tiles, l.off + nkeys);
   GF_LAUNCHED();
-  agg_scan_add_kernel<<<(unsigned)((nkeys + 255) / 256), 256, 0, st>>>(off, nkeys, tsum);
+  agg_scan_add_kernel<<<(unsigned)((nkeys + 255) / 256), 256, 0, st>>>(l.off, nkeys, l.tsum);
   GF_LAUNCHED();
-  agg_place_kernel<<<eb, 256, 0, st>>>(idx, (long long)ent, mns, N, off, cnt, slot);
+  agg_place_kernel<<<eb, 256, 0, st>>>(idx, (long long)ent, mns, N, l.off, l.cnt, l.slot);
   GF_LAUNCHED();
-  agg_segment_sum_kernel<<<(unsigned)(((long long)B * N + 255) / 256), 256, 0, st>>>(off, slot, a.gx, B, N, C,
+  agg_segment_sum_kernel<<<(unsigned)(((long long)B * N + 255) / 256), 256, 0, st>>>(l.off, l.slot, a.gx, B, N, C,
                                                                                       dfeatures);
   GF_LAUNCHED();
   return GF_OK;

@@ -21,6 +21,7 @@
 //     either loaded from the (Q,C,B,64) tensor or -- fused with the decoder epilogue a10 -- computed on the fly
 //     from the geodesic maps, so that it never exists in memory).
 // tcgen05.mma is issued by one thread; completion is signalled through an mbarrier by tcgen05.commit.
+#include "gf_bias.cuh"
 #include "gf_umma.cuh"
 
 namespace gf {
@@ -610,38 +611,55 @@ __global__ void att_tables_kernel(const float *__restrict__ tgt2, const float *_
   }
 }
 
-extern "C" size_t gf_rel_cross_attention_workspace_bytes(int Q, int C, int B) {
-  if (Q <= 0 || C <= 0 || B <= 0) return 0;
-  return align256(sizeof(float) * 64 * (size_t)B * Q) + 2 * align256(sizeof(float) * 64 * (size_t)B * C) +
-         align256(sizeof(uint32_t) * ((size_t)B * Q + 1)) + 1024;
+// The workspace: the projection tables and the row maxima of the gathered maps (taken by the unfused variant too),
+// then for the backward its per-row, per-CTA and per-pair buffers
+struct AttLayout {
+  float *aq, *p1, *pv;
+  RowMax rm;
+  float *dz, *dout_o, *hsum, *part, *pairs, *dhdv;
+};
+static Arena att_carve(void *workspace, size_t workspace_bytes, int Q, int C, int B, bool backward, AttLayout *l) {
+  Arena a(workspace, workspace_bytes);
+  const size_t QB = (size_t)Q * B, CB = (size_t)C * B;
+  l->aq = a.take<float>(64 * QB);
+  l->p1 = a.take<float>(64 * CB);
+  l->pv = a.take<float>(64 * CB);
+  l->rm = take_rowmax(a, QB);
+  if (backward) {
+    l->dz = a.take<float>(64 * QB);
+    l->dout_o = a.take<float>(64 * QB);
+    l->hsum = a.take<float>(64 * QB);
+    l->part = a.take<float>(3 * 4096 * QB);
+    l->pairs = a.take<float>(128 * QB * C);
+    l->dhdv = a.take<float>(128 * CB);
+  }
+  return a;
 }
 
-namespace gf {
-// row maxima of the gathered maps, gf_bias.cu
-int bias_ctx_rowmax(const float *const *geo_ptrs, const int *geo_ld, const int *ctx_idx, int B, int Q, int C,
-                    uint32_t *rowmax, uint32_t *gmax, cudaStream_t st);
-}  // namespace gf
+extern "C" size_t gf_rel_cross_attention_workspace_bytes(int Q, int C, int B) {
+  if (Q <= 0 || C <= 0 || B <= 0) return 0;
+  AttLayout l;
+  return att_carve(nullptr, 0, Q, C, B, false, &l).off;
+}
 
-// the tables (and for the fused variant the row maxima of the gathered maps) at the front of the workspace
+extern "C" size_t gf_rel_cross_attention_backward_workspace_bytes(int Q, int C, int B) {
+  if (Q <= 0 || C <= 0 || B <= 0) return 0;
+  AttLayout l;
+  return att_carve(nullptr, 0, Q, C, B, true, &l).off;
+}
+
+// the tables (and for the fused variant the row maxima of the gathered maps), into the carved workspace
 static int att_prepare(AttArgs &a, const float *tgt2, const float *memory, const float *b1, const float *bv,
-                       const float *const *geo_ptrs, const int *geo_ld, Arena &ar, const char *name, size_t needed,
-                       cudaStream_t st) {
-  float *aq = ar.take<float>(64 * (size_t)a.B * a.Q);
-  float *p1 = ar.take<float>(64 * (size_t)a.B * a.C);
-  float *pv = ar.take<float>(64 * (size_t)a.B * a.C);
-  uint32_t *rm = ar.take<uint32_t>((size_t)a.B * a.Q + 1);
-  if (!ar.ok) {
-    set_error("%s: workspace too small (%zu bytes given, %zu needed)", name, ar.size, needed);
-    return GF_ERR_WORKSPACE;
-  }
-  att_tables_kernel<<<dim3(a.Q + a.C, a.B), 64, 0, st>>>(tgt2, memory, a.Q, a.C, a.B, a.w1, b1, a.wv, bv, aq, p1, pv);
+                       const float *const *geo_ptrs, const int *geo_ld, const AttLayout &l, cudaStream_t st) {
+  att_tables_kernel<<<dim3(a.Q + a.C, a.B), 64, 0, st>>>(tgt2, memory, a.Q, a.C, a.B, a.w1, b1, a.wv, bv, l.aq, l.p1,
+                                                         l.pv);
   GF_LAUNCHED();
-  a.aq = aq, a.p1 = p1, a.pv = pv;
+  a.aq = l.aq, a.p1 = l.p1, a.pv = l.pv;
   if (geo_ptrs) {
     for (int b = 0; b < a.B; ++b) a.geo[b] = geo_ptrs[b], a.geo_ld[b] = geo_ld[b];
-    int rc = bias_ctx_rowmax(geo_ptrs, geo_ld, a.ctx_idx, a.B, a.Q, a.C, rm, rm + (size_t)a.B * a.Q, st);
+    int rc = bias_ctx_rowmax(geo_ptrs, geo_ld, a.ctx_idx, a.B, a.Q, a.C, l.rm, st);
     if (rc) return rc;
-    a.rowmax = rm, a.gmax = rm + (size_t)a.B * a.Q;
+    a.rowmax = l.rm.rowmax, a.gmax = l.rm.gmax;
   }
   return GF_OK;
 }
@@ -668,9 +686,10 @@ static int att_launch(AttArgs &a, const float *tgt2, const float *memory, const 
                       const float *const *geo_ptrs, const int *geo_ld, void *workspace, size_t workspace_bytes,
                       cudaStream_t st) {
   const bool fused = geo_ptrs != nullptr, save = a.o_save != nullptr;
-  Arena ar(workspace, workspace_bytes);
-  int rc = att_prepare(a, tgt2, memory, b1, bv, geo_ptrs, geo_ld, ar, "rel_cross_attention",
-                       gf_rel_cross_attention_workspace_bytes(a.Q, a.C, a.B), st);
+  AttLayout l;
+  const Arena ar = att_carve(workspace, workspace_bytes, a.Q, a.C, a.B, false, &l);
+  if (!ar.ok) return ar.fail("rel_cross_attention");
+  int rc = att_prepare(a, tgt2, memory, b1, bv, geo_ptrs, geo_ld, l, st);
   if (rc) return rc;
   if ((rc = att_set_smem())) return rc;
   const dim3 grid(a.Q, a.B);
@@ -882,14 +901,6 @@ __global__ void __launch_bounds__(256) att_bwd_drel_kernel(const float *__restri
   }
 }
 
-extern "C" size_t gf_rel_cross_attention_backward_workspace_bytes(int Q, int C, int B) {
-  if (Q <= 0 || C <= 0 || B <= 0) return 0;
-  const size_t QB = (size_t)Q * B, CB = (size_t)C * B;
-  return gf_rel_cross_attention_workspace_bytes(Q, C, B) + 3 * align256(sizeof(float) * 64 * QB) +
-         align256(sizeof(float) * 3 * 4096 * QB) + align256(sizeof(float) * 128 * QB * C) +
-         align256(sizeof(float) * 128 * CB);
-}
-
 static int att_bwd_launch(AttArgs &a, const float *tgt2, const float *memory, const float *b1, const float *bv,
                           const float *const *geo_ptrs, const int *geo_ld, const float *o, const float *lse,
                           const float *dy, float *dtgt2, float *dmemory, float *drel, float *dw1, float *db1,
@@ -897,20 +908,14 @@ static int att_bwd_launch(AttArgs &a, const float *tgt2, const float *memory, co
                           size_t workspace_bytes, cudaStream_t st) {
   const int Q = a.Q, C = a.C, B = a.B;
   const size_t QB = (size_t)Q * B;
-  const size_t needed = gf_rel_cross_attention_backward_workspace_bytes(Q, C, B);
-  Arena ar(workspace, workspace_bytes);
-  int rc = att_prepare(a, tgt2, memory, b1, bv, geo_ptrs, geo_ld, ar, "rel_cross_attention_backward", needed, st);
+  AttLayout l;
+  const Arena ar = att_carve(workspace, workspace_bytes, Q, C, B, true, &l);
+  if (!ar.ok) return ar.fail("rel_cross_attention_backward");
+  int rc = att_prepare(a, tgt2, memory, b1, bv, geo_ptrs, geo_ld, l, st);
   if (rc) return rc;
   AttBwdArgs g = {};
-  float *dz = ar.take<float>(64 * QB), *dout_o = ar.take<float>(64 * QB);
-  g.hsum = ar.take<float>(64 * QB);
-  g.part = ar.take<float>(3 * 4096 * QB);
-  g.pairs = ar.take<float>(128 * QB * C);
-  float *dhdv = ar.take<float>(128 * (size_t)C * B);
-  if (!ar.ok) {
-    set_error("rel_cross_attention_backward: workspace too small (%zu bytes given, %zu needed)", workspace_bytes, needed);
-    return GF_ERR_WORKSPACE;
-  }
+  float *dz = l.dz, *dout_o = l.dout_o, *dhdv = l.dhdv;
+  g.hsum = l.hsum, g.part = l.part, g.pairs = l.pairs;
   g.o = o, g.lse = lse, g.dout_o = dout_o;
   if ((rc = att_set_smem())) return rc;
   att_bwd_prologue_kernel<<<(unsigned)QB, 64, 0, st>>>(a.out, dy, a.wo, dz, dout_o);

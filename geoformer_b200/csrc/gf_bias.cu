@@ -225,17 +225,13 @@ __global__ void __launch_bounds__(256)
 // ordered-uint row maxima of the gathered maps and their global maximum (geoformer_fs.py:685-692); geo_ptrs / geo_ld
 // are HOST arrays of B device pointers / row strides.  Shared with the fused cross-attention (gf_attention.cu).
 int bias_ctx_rowmax(const float *const *geo_ptrs, const int *geo_ld, const int *ctx_idx, int B, int Q, int C,
-                    uint32_t *rowmax, uint32_t *gmax, cudaStream_t st) {
-  if (gmax != rowmax + (size_t)B * Q) {
-    set_error("bias: the global maximum must follow the row maxima (they are cleared together)");
-    return GF_ERR_INVALID;
-  }
-  bias_zero_kernel<<<(B * Q + 256) / 256, 256, 0, st>>>(rowmax, B * Q + 1);
+                    const RowMax &rm, cudaStream_t st) {
+  bias_zero_kernel<<<(B * Q + 256) / 256, 256, 0, st>>>(rm.rowmax, B * Q + 1);  // the row maxima and gmax after them
   GF_LAUNCHED();
   const int rchunks = C >= 1024 ? 4 : 1;
   for (int b = 0; b < B; ++b) {
     bias_ctx_rowmax_kernel<<<dim3(rchunks, Q), 256, 0, st>>>(geo_ptrs[b], geo_ld[b], ctx_idx + (size_t)b * C, C,
-                                                           rowmax + (size_t)b * Q, gmax);
+                                                           rm.rowmax + (size_t)b * Q, rm.gmax);
     GF_LAUNCHED();
   }
   return GF_OK;
@@ -243,8 +239,8 @@ int bias_ctx_rowmax(const float *const *geo_ptrs, const int *geo_ld, const int *
 
 // ordered-uint row maxima of the (Q,N) maps and their global maximum (geoformer_fs.py:274-276), or the producer's
 // row_max imported; nothing has to be zeroed beforehand.  Shared with the fused mask head (gf_mask_head.cu).
-int bias_mask_rowmax(const float *geo, int Q, int N, const float *row_max, bool vec, uint32_t *rowmax, uint32_t *gmax,
-                     cudaStream_t st) {
+int bias_mask_rowmax(const float *geo, int Q, int N, const float *row_max, bool vec, const RowMax &rm, cudaStream_t st) {
+  uint32_t *rowmax = rm.rowmax, *gmax = rm.gmax;
   if (!row_max) {
     GF_CUDA(cudaMemsetAsync(rowmax, 0, sizeof(uint32_t) * (size_t)Q, st));
     bias_init_kernel<<<1, 1, 0, st>>>(gmax);
@@ -269,9 +265,17 @@ int bias_mask_rowmax(const float *geo, int Q, int N, const float *row_max, bool 
 
 using namespace gf;
 
+// the workspace of the three epilogues: the row maxima of the `rows` maps
+static Arena bias_carve(void *workspace, size_t workspace_bytes, size_t rows, RowMax *rm) {
+  Arena a(workspace, workspace_bytes);
+  *rm = take_rowmax(a, rows);
+  return a;
+}
+
 extern "C" size_t gf_bias_workspace_bytes(int B, int Q) {
   if (B <= 0 || Q <= 0) return 0;
-  return align256(sizeof(float) * (size_t)B * Q) + 256 + 256;
+  RowMax rm;
+  return bias_carve(nullptr, 0, (size_t)B * Q, &rm).off;
 }
 
 extern "C" int gf_bias_decoder(const float *const *geo_ptrs, const int *geo_ld, const int *ctx_idx,
@@ -280,28 +284,18 @@ extern "C" int gf_bias_decoder(const float *const *geo_ptrs, const int *geo_ld, 
   GF_CHECK_ARG(B >= 0 && Q >= 0 && C >= 0, "bias_decoder: negative size");
   if ((long long)B * Q * C == 0) return GF_OK;
   GF_CHECK_ARG(geo_ptrs && geo_ld && ctx_idx && query_xyz && ctx_xyz && out, "bias_decoder: null pointer");
-  Arena a(workspace, workspace_bytes);
-  uint32_t *rowmax = a.take<uint32_t>((size_t)B * Q + 1);  // + the global maximum, zeroed together
-  uint32_t *gmax = rowmax + (size_t)B * Q;
-  if (!a.ok) {
-    set_error("bias_decoder: workspace too small");
-    return GF_ERR_WORKSPACE;
-  }
+  RowMax rm;
+  const Arena a = bias_carve(workspace, workspace_bytes, (size_t)B * Q, &rm);
+  if (!a.ok) return a.fail("bias_decoder");
   cudaStream_t st = (cudaStream_t)stream;
-  bias_zero_kernel<<<(B * Q + 256) / 256, 256, 0, st>>>(rowmax, B * Q + 1);
-  GF_LAUNCHED();
-  const int rchunks = C >= 1024 ? 4 : 1;
-  for (int b = 0; b < B; ++b) {
-    bias_ctx_rowmax_kernel<<<dim3(rchunks, Q), 256, 0, st>>>(geo_ptrs[b], geo_ld[b], ctx_idx + (size_t)b * C, C,
-                                                           rowmax + (size_t)b * Q, gmax);
-    GF_LAUNCHED();
-  }
+  const int rc = bias_ctx_rowmax(geo_ptrs, geo_ld, ctx_idx, B, Q, C, rm, st);
+  if (rc) return rc;
   for (int b = 0; b < B; ++b) {
     int grid = (Q * C + 255) / 256;
     if (grid > num_sms() * 8) grid = num_sms() * 8;
     bias_ctx_write_kernel<<<grid, 256, 0, st>>>(geo_ptrs[b], geo_ld[b], ctx_idx + (size_t)b * C,
                                                 query_xyz + (size_t)b * Q * 3, ctx_xyz + (size_t)b * C * 3, Q, C,
-                                                rowmax + (size_t)b * Q, gmax, out + (size_t)b * Q * C * 3);
+                                                rm.rowmax + (size_t)b * Q, rm.gmax, out + (size_t)b * Q * C * 3);
     GF_LAUNCHED();
   }
   return GF_OK;
@@ -317,28 +311,18 @@ extern "C" int gf_bias_decoder_fourier(const float *const *geo_ptrs, const int *
   if ((long long)B * Q * C == 0) return GF_OK;
   GF_CHECK_ARG(geo_ptrs && geo_ld && ctx_idx && query_xyz && ctx_xyz && gauss_B && pc_min && pc_max && out,
                "bias_decoder_fourier: null pointer");
-  Arena a(workspace, workspace_bytes);
-  uint32_t *rowmax = a.take<uint32_t>((size_t)B * Q + 1);  // + the global maximum, zeroed together
-  uint32_t *gmax = rowmax + (size_t)B * Q;
-  if (!a.ok) {
-    set_error("bias_decoder_fourier: workspace too small");
-    return GF_ERR_WORKSPACE;
-  }
+  RowMax rm;
+  const Arena a = bias_carve(workspace, workspace_bytes, (size_t)B * Q, &rm);
+  if (!a.ok) return a.fail("bias_decoder_fourier");
   cudaStream_t st = (cudaStream_t)stream;
-  bias_zero_kernel<<<(B * Q + 256) / 256, 256, 0, st>>>(rowmax, B * Q + 1);
-  GF_LAUNCHED();
-  const int rchunks = C >= 1024 ? 4 : 1;
-  for (int b = 0; b < B; ++b) {
-    bias_ctx_rowmax_kernel<<<dim3(rchunks, Q), 256, 0, st>>>(geo_ptrs[b], geo_ld[b], ctx_idx + (size_t)b * C, C,
-                                                           rowmax + (size_t)b * Q, gmax);
-    GF_LAUNCHED();
-  }
+  const int rc = bias_ctx_rowmax(geo_ptrs, geo_ld, ctx_idx, B, Q, C, rm, st);
+  if (rc) return rc;
   for (int b = 0; b < B; ++b) {
     int gx = (C + 255) / 256;  // 8 warps x 32 contexts per block: one pass per warp, no ragged second round
     if (gx > 4096) gx = 4096;
     bias_ctx_fourier_kernel<<<dim3(gx, Q), 256, 0, st>>>(
         geo_ptrs[b], geo_ld[b], ctx_idx + (size_t)b * C, query_xyz + (size_t)b * Q * 3, ctx_xyz + (size_t)b * C * 3, Q, C,
-        rowmax + (size_t)b * Q, gmax, gauss_B, d_out, gauss_ld, pc_min + (size_t)b * 3, pc_max + (size_t)b * 3,
+        rm.rowmax + (size_t)b * Q, rm.gmax, gauss_B, d_out, gauss_ld, pc_min + (size_t)b * 3, pc_max + (size_t)b * 3,
         out + (size_t)b * Q * C * 2 * d_out);
     GF_LAUNCHED();
   }
@@ -351,27 +335,23 @@ extern "C" int gf_bias_mask_head(const float *geo, const float *coords, const fl
   GF_CHECK_ARG(Q >= 0 && N >= 0, "bias_mask_head: negative size");
   if ((long long)Q * N == 0) return GF_OK;
   GF_CHECK_ARG(geo && coords && seed_xyz && out, "bias_mask_head: null pointer");
-  Arena a(workspace, workspace_bytes);
-  uint32_t *rowmax = a.take<uint32_t>((size_t)Q);
-  uint32_t *gmax = a.take<uint32_t>(1);
-  if (!a.ok) {
-    set_error("bias_mask_head: workspace too small");
-    return GF_ERR_WORKSPACE;
-  }
+  RowMax rm;
+  const Arena a = bias_carve(workspace, workspace_bytes, (size_t)Q, &rm);
+  if (!a.ok) return a.fail("bias_mask_head");
   cudaStream_t st = (cudaStream_t)stream;
   // 16-byte path: N a multiple of 4 and all bases 16-byte aligned (torch allocations are)
   const bool vec = (N % 4 == 0) && ((((uintptr_t)geo | (uintptr_t)coords | (uintptr_t)out) & 15) == 0);
   const int work = vec ? N / 4 : N;
-  const int rc = bias_mask_rowmax(geo, Q, N, row_max, vec, rowmax, gmax, st);
+  const int rc = bias_mask_rowmax(geo, Q, N, row_max, vec, rm, st);
   if (rc != GF_OK) return rc;
   int gx = (work + 255) / 256;
   int cap = (num_sms() * 16 + Q - 1) / Q;
   if (cap < 1) cap = 1;
   if (gx > cap) gx = cap;
   if (vec)
-    bias_mask_write_kernel<true><<<dim3(gx, Q), 256, 0, st>>>(geo, coords, seed_xyz, Q, N, rowmax, gmax, out);
+    bias_mask_write_kernel<true><<<dim3(gx, Q), 256, 0, st>>>(geo, coords, seed_xyz, Q, N, rm.rowmax, rm.gmax, out);
   else
-    bias_mask_write_kernel<false><<<dim3(gx, Q), 256, 0, st>>>(geo, coords, seed_xyz, Q, N, rowmax, gmax, out);
+    bias_mask_write_kernel<false><<<dim3(gx, Q), 256, 0, st>>>(geo, coords, seed_xyz, Q, N, rm.rowmax, rm.gmax, out);
   GF_LAUNCHED();
   return GF_OK;
 }

@@ -48,15 +48,24 @@ enum Stage { ST_BEGIN = 0, ST_KNN_BUILT = 1, ST_KNN_DONE = 2, ST_GEO_READY = 3, 
 void stage_mark(int stage, cudaStream_t st);
 
 // ---- bump allocator over a caller-provided workspace -------------------------------------------
+// A piece of a workspace handed down to a nested layout, which carves it in turn.
+struct Span {
+  void *ptr;
+  size_t bytes;
+};
+
+// Every layout is stated once, in a carve function: over a null workspace the Arena only measures (`off` ends as the
+// layout's size), over the caller's workspace it hands out the pieces.  Pieces start at multiples of 256 bytes from a
+// base that must itself be 256-byte aligned: the kernels read them with 16-byte loads.
 struct Arena {
   char *base;
   size_t size, off;
   bool ok;
-  Arena(void *p, size_t n) : base((char *)p), size(n), off(0), ok(true) {}
+  Arena(void *p, size_t n) : base((char *)p), size(n), off(0), ok(((uintptr_t)p & 255) == 0) {}
   template <typename T>
   T *take(size_t count) {
     size_t bytes = (count * sizeof(T) + 255) & ~size_t(255);
-    if (base == nullptr || off + bytes > size) {
+    if (!ok || base == nullptr || off + bytes > size) {
       ok = false;
       off += bytes;
       return nullptr;
@@ -65,8 +74,16 @@ struct Arena {
     off += bytes;
     return r;
   }
+  Span span(size_t bytes) { return {take<char>(bytes), bytes}; }
+  // the error of a carve that failed, once it has measured the whole layout
+  int fail(const char *who) const {
+    if ((uintptr_t)base & 255)
+      set_error("%s: workspace %p is not 256-byte aligned", who, (void *)base);
+    else
+      set_error("%s: workspace too small (%zu bytes given, %zu needed)", who, size, off);
+    return GF_ERR_WORKSPACE;
+  }
 };
-static inline size_t align256(size_t b) { return (b + 255) & ~size_t(255); }
 
 // ---- device helpers ---------------------------------------------------------------------------
 

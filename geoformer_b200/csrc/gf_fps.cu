@@ -729,14 +729,25 @@ static int launch_fps_cells(const float4 *sorted, const float *xyz, int N, int m
   return GF_OK;
 }
 
-size_t fps_cells_workspace_bytes(int N) { return align256(sizeof(float) * (size_t)N); }
+// the running minima, in cell order
+static Arena fps_cells_carve(void *workspace, size_t workspace_bytes, int N, float **tmin) {
+  Arena ar(workspace, workspace_bytes);
+  *tmin = ar.take<float>((size_t)N);
+  return ar;
+}
+
+size_t fps_cells_workspace_bytes(int N) {
+  float *tmin;
+  return fps_cells_carve(nullptr, 0, N, &tmin).off;
+}
 
 int fps_cells(const float4 *sorted, const float *xyz, int N, int m, void *workspace, size_t workspace_bytes, int *idx,
               cudaStream_t st) {
   GF_CHECK_ARG(N >= 1 && m >= 1, "fps_cells: need N >= 1 and m >= 1 (N=%d m=%d)", N, m);
-  GF_CHECK_ARG(workspace && workspace_bytes >= fps_cells_workspace_bytes(N), "fps_cells: workspace too small");
+  float *tmin;
+  const Arena ar = fps_cells_carve(workspace, workspace_bytes, N, &tmin);
+  if (!ar.ok) return ar.fail("fps_cells");
   size_t smem = 0;
-  float *tmin = (float *)workspace;
   switch (fps_cells_spl(N, &smem)) {
     case 2: return launch_fps_cells<2>(sorted, xyz, N, m, tmin, idx, smem, st);
     case 4: return launch_fps_cells<4>(sorted, xyz, N, m, tmin, idx, smem, st);
@@ -780,10 +791,7 @@ extern "C" int gf_furthest_point_sampling(const float *xyz, int B, int N, int m,
   uint2 *slots;
   float *temp;
   const Arena ar = fps_carve(workspace, workspace_bytes, B, N, &slots, &temp);
-  if (!ar.ok) {
-    set_error("furthest_point_sampling: N=%d needs a %zu-byte workspace (gf_fps_workspace_bytes)", N, ar.off);
-    return GF_ERR_WORKSPACE;
-  }
+  if (!ar.ok) return ar.fail("furthest_point_sampling");
   return with_grid_p(p.P, [&](auto P) {
     GF_CUDA(cudaMemsetAsync(slots, 0, sizeof(uint2) * 2 * FPS_SLOT_WORDS * (size_t)p.ctas, st));  // tag 0 = unwritten
     void *args[] = {(void *)&xyz, &B, &N, &m, &L, &temp, &idx, &slots};
@@ -819,10 +827,17 @@ extern "C" int gf_furthest_point_sampling_batch(const float *xyz, const int *off
   GF_CHECK_ARG(xyz || offsets[B] == 0, "furthest_point_sampling_batch: null xyz");
   cudaStream_t st = (cudaStream_t)stream;
   const long long cap = fps_cluster_capacity(max_cluster_size());
-  int Nmax = 0;
+  int Nmax = 0, Nbig = 0;
   for (int b = 0; b < B; ++b) {
     const int N = offsets[b + 1] - offsets[b];
     if (N <= cap && N > Nmax) Nmax = N;
+    if (N > cap && N > Nbig) Nbig = N;
+  }
+  if (Nbig > 0) {  // the scenes above the cluster capacity run the whole-GPU kernel, each on the whole workspace
+    uint2 *slots;
+    float *temp;
+    const Arena ar = fps_carve(workspace, workspace_bytes, 1, Nbig, &slots, &temp);
+    if (!ar.ok) return ar.fail("furthest_point_sampling_batch");
   }
   if (Nmax > 0) {
     const FpsPlan p = plan_fps(Nmax, max_cluster_size());

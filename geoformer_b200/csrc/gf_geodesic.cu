@@ -887,15 +887,20 @@ size_t geodesic_batch_scratch_bytes(int maxN, long long items) {
   GeoBatchPlan p;
   plan_batch(maxN, items, &p);
   GeoBatchScratch s;
-  return geo_batch_carve(nullptr, 0, p, &s).off + 1024;
+  return geo_batch_carve(nullptr, 0, p, &s).off;
+}
+
+void geo_edges_carve(Arena &a, int N, int k, GeoEdges *e) {
+  e->slot_bits = geo_slot_bits(k);
+  e->tgt = a.take<int>(((size_t)N + 1) << e->slot_bits);
+  e->len = a.take<float>(((size_t)N + 1) << e->slot_bits);
 }
 
 // workspace of the single-scene entry points: the packed edge table (+ sentinel row), then the scratch of the kernel
 // that runs, sized for either: the per-scene kernel's (big scenes; seed-sharded scenes of any size) frontier overflow
 // and control block, or for a batchable scene the scratch of a batched launch, if that is larger
 struct GeoBuffers {
-  int *tgt;
-  float *len;
+  GeoEdges e;
   int *overflow;  // the per-scene kernel's scratch ...
   GeoCtl *ctl;
   void *rest;  // ... or a batched launch's, at the same address
@@ -903,9 +908,7 @@ struct GeoBuffers {
 };
 static Arena geo_carve(void *workspace, size_t workspace_bytes, int N, int k, int Q, GeoBuffers *b) {
   Arena a(workspace, workspace_bytes);
-  const int slot_bits = geo_slot_bits(k);
-  b->tgt = a.take<int>(((size_t)N + 1) << slot_bits);
-  b->len = a.take<float>(((size_t)N + 1) << slot_bits);
+  geo_edges_carve(a, N, k, &b->e);
   b->rest = a.ok ? (void *)(a.base + a.off) : nullptr;
   b->rest_bytes = a.ok ? a.size - a.off : 0;
   GeoPlan pl;
@@ -920,19 +923,14 @@ static Arena geo_carve(void *workspace, size_t workspace_bytes, int N, int k, in
 
 size_t geodesic_workspace_bytes(int N, int k, int Q) {
   GeoBuffers b;
-  return geo_carve(nullptr, 0, N, k, Q, &b).off + 1024;
+  return geo_carve(nullptr, 0, N, k, Q, &b).off;
 }
 
-int geodesic_edge_buffers(void *workspace, size_t workspace_bytes, int N, int k, int Q, int **tgt, float **len,
-                          int *slot_bits, int *enc) {
+int geodesic_edge_buffers(void *workspace, size_t workspace_bytes, int N, int k, int Q, GeoEdges *e, int *enc) {
   GeoBuffers b;
-  *slot_bits = geo_slot_bits(k);
-  if (!geo_carve(workspace, workspace_bytes, N, k, Q, &b).ok) {
-    set_error("geodesic: workspace too small (%zu bytes given, %zu needed)", workspace_bytes,
-              geodesic_workspace_bytes(N, k, Q));
-    return GF_ERR_WORKSPACE;
-  }
-  *tgt = b.tgt, *len = b.len;
+  const Arena a = geo_carve(workspace, workspace_bytes, N, k, Q, &b);
+  if (!a.ok) return a.fail("geodesic");
+  *e = b.e;
   *enc = geo_batchable(N) ? 1 : 0;
   return GF_OK;
 }
@@ -1032,11 +1030,8 @@ int geodesic_batch_launch(const GeoSceneDesc *scenes, int B, int k, int max_step
   GeoBatchPlan p;
   plan_batch(maxN, items, &p);
   GeoBatchScratch sc;
-  if (!geo_batch_carve(scratch, scratch_bytes, p, &sc).ok) {
-    set_error("geodesic: scratch too small (%zu bytes given, %zu needed)", scratch_bytes,
-              geodesic_batch_scratch_bytes(maxN, items));
-    return GF_ERR_WORKSPACE;
-  }
+  const Arena a = geo_batch_carve(scratch, scratch_bytes, p, &sc);
+  if (!a.ok) return a.fail("geodesic: scratch");
   ga.overflow = sc.overflow, ga.claim = sc.claim, ga.item_counter = &sc.ctl->counter;
   ga.ovf_stride = p.ovf_stride, ga.arr_stride = p.arr_stride;
   ga.B = B, ga.total_items = (int)items, ga.max_step = max_step, ga.slot_bits = slot_bits, ga.qcap = p.qcap;
@@ -1085,11 +1080,8 @@ int geodesic_run(const float *D, const void *I, int is64, int N, int k, const in
     return GF_ERR_INVALID;
   }
   GeoBuffers b;
-  if (!geo_carve(workspace, workspace_bytes, N, k, Q, &b).ok) {
-    set_error("geodesic: workspace too small (%zu bytes given, %zu needed)", workspace_bytes,
-              geodesic_workspace_bytes(N, k, Q));
-    return GF_ERR_WORKSPACE;
-  }
+  const Arena a = geo_carve(workspace, workspace_bytes, N, k, Q, &b);
+  if (!a.ok) return a.fail("geodesic");
   // also the format of an already packed edge table (seed-sharded scenes always run the per-scene kernel)
   const bool batched = geo_batchable(N) && n_peers == 0;
   if (D != nullptr) {
@@ -1098,9 +1090,9 @@ int geodesic_run(const float *D, const void *I, int is64, int N, int k, const in
     const long long cap = (long long)num_sms() * 16;
     const int grid = (int)(blocks < cap ? (blocks > 0 ? blocks : 1) : cap);
     if (is64)
-      geo_pack_edges_kernel<true><<<grid, 256, 0, st>>>(D, I, N, k, radius, slot_bits, batched ? 1 : 0, b.tgt, b.len);
+      geo_pack_edges_kernel<true><<<grid, 256, 0, st>>>(D, I, N, k, radius, slot_bits, batched ? 1 : 0, b.e.tgt, b.e.len);
     else
-      geo_pack_edges_kernel<false><<<grid, 256, 0, st>>>(D, I, N, k, radius, slot_bits, batched ? 1 : 0, b.tgt, b.len);
+      geo_pack_edges_kernel<false><<<grid, 256, 0, st>>>(D, I, N, k, radius, slot_bits, batched ? 1 : 0, b.e.tgt, b.e.len);
     GF_LAUNCHED();
   }
   if (batched) {
@@ -1111,7 +1103,7 @@ int geodesic_run(const float *D, const void *I, int is64, int N, int k, const in
     geo_batch_carve(b.rest, b.rest_bytes, p, &sc);
     unsigned long long *stats = sc.ctl->stats;
     GeoSceneDesc d;
-    d.tgt = b.tgt, d.len = b.len, d.seeds = seeds, d.geo = geo, d.row_max = row_max;
+    d.tgt = b.e.tgt, d.len = b.e.len, d.seeds = seeds, d.geo = geo, d.row_max = row_max;
     d.rank = D == nullptr ? rank : nullptr, d.order = D == nullptr ? order : nullptr;  // a packed foreign graph: identity
     d.stats = stats_out ? (int64_t *)stats : nullptr;
     d.N = N, d.Q = Q;
@@ -1126,7 +1118,7 @@ int geodesic_run(const float *D, const void *I, int is64, int N, int k, const in
   GF_CUDA(cudaMemsetAsync(b.ctl, 0, sizeof(GeoCtl), st));
   stage_mark(ST_GEO_READY, st);
   GeoArgs ga;
-  ga.tgt = b.tgt, ga.len = b.len, ga.N = N, ga.Q = Q, ga.max_step = max_step, ga.slot_bits = slot_bits;
+  ga.tgt = b.e.tgt, ga.len = b.e.len, ga.N = N, ga.Q = Q, ga.max_step = max_step, ga.slot_bits = slot_bits;
   ga.seeds = seeds, ga.geo = geo, ga.overflow = b.overflow, ga.seed_counter = &b.ctl->counter, ga.stats = stats;
   ga.bitmap_words = p.bitmap_words;
   ga.row_max = row_max;

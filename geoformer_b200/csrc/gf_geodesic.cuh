@@ -26,10 +26,19 @@ int geodesic_batch_launch(const GeoSceneDesc *scenes, int B, int k, int max_step
                           cudaStream_t st);
 constexpr int GEO_BATCH_MAX = 32;
 
+// the packed edge table of one scene, with its sentinel row N: (N + 1) << slot_bits targets and lengths
+struct GeoEdges {
+  int *tgt;
+  float *len;
+  int slot_bits;
+};
+// takes the edge table of a scene of N points with k neighbours from `a` (the head of the single-scene workspace; a
+// batched call takes one per scene)
+void geo_edges_carve(Arena &a, int N, int k, GeoEdges *e);
+
 // where the packed edge table of a later geodesic_run(D = nullptr, ...) on the same workspace lives; the workspace
 // must hold the whole layout that run uses, geodesic_workspace_bytes(N, k, Q) bytes
-int geodesic_edge_buffers(void *workspace, size_t workspace_bytes, int N, int k, int Q, int **tgt, float **len,
-                          int *slot_bits, int *enc);
+int geodesic_edge_buffers(void *workspace, size_t workspace_bytes, int N, int k, int Q, GeoEdges *e, int *enc);
 
 int geodesic_edge_format(int N);  // 1 = encoded targets (the batched kernel takes the scene), 0 = plain
 

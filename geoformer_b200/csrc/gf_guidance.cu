@@ -88,17 +88,16 @@ static int get_fork_join(cudaStream_t user, ForkJoin **out, int fps_lanes = 1, i
   return GF_OK;
 }
 
-struct GuidancePlan {
-  size_t fps, knn, geo, total;
+// the workspace of one scene: the workspaces of its FPS, its kNN grid and its propagation (edge table first)
+struct GuidanceLayout {
+  Span fps, knn, geo;
 };
-
-static GuidancePlan plan_guidance(int N, int Q, int k) {
-  GuidancePlan p;
-  p.fps = align256(gf_fps_workspace_bytes(1, N, Q));
-  p.knn = align256(knn_grid_workspace_bytes(N));
-  p.geo = align256(geodesic_workspace_bytes(N, k, Q));
-  p.total = p.fps + p.knn + p.geo + 1024;
-  return p;
+static Arena guidance_carve(void *workspace, size_t workspace_bytes, int N, int Q, int k, GuidanceLayout *l) {
+  Arena a(workspace, workspace_bytes);
+  l->fps = a.span(gf_fps_workspace_bytes(1, N, Q));
+  l->knn = a.span(knn_grid_workspace_bytes(N));
+  l->geo = a.span(geodesic_workspace_bytes(N, k, Q));
+  return a;
 }
 
 }  // namespace gf
@@ -107,7 +106,8 @@ using namespace gf;
 
 extern "C" size_t gf_guidance_workspace_bytes(int N, int Q, int k) {
   if (N <= 0 || Q <= 0 || k <= 0) return 0;
-  return plan_guidance(N, Q, k).total;
+  GuidanceLayout l;
+  return guidance_carve(nullptr, 0, N, Q, k, &l).off;
 }
 
 // seeds_given == 0: run FPS (forked stream) and write `seeds`; != 0: `seeds` is an input
@@ -121,21 +121,17 @@ static int guidance_impl(const float *xyz, int N, int Q, int k, float radius, in
   GF_CHECK_ARG(q0 >= 0 && q0 <= q1 && q1 <= Q, "guidance: seed block [%d, %d) outside [0, %d)", q0, q1, Q);
   GF_CHECK_ARG(k >= 1 && k <= KNN_MAX_K, "guidance: k=%d outside [1,%d]", k, KNN_MAX_K);
   GF_CHECK_ARG(xyz && seeds && geo, "guidance: null pointer");
-  GuidancePlan p = plan_guidance(N, Q, k);
-  if (workspace == nullptr || workspace_bytes < p.total) {
-    set_error("guidance: workspace too small (%zu bytes given, %zu needed)", workspace_bytes, p.total);
-    return GF_ERR_WORKSPACE;
-  }
+  GuidanceLayout l;
+  const Arena ar = guidance_carve(workspace, workspace_bytes, N, Q, k, &l);
+  if (!ar.ok) return ar.fail("guidance");
+  // the query kernel writes the propagation's edge table straight from its registers; the (N,k) distance / index
+  // arrays are only written when the caller asked for them
+  GeoEdges edges;
+  int enc = 0;
+  int rc = geodesic_edge_buffers(l.geo.ptr, l.geo.bytes, N, k, Q, &edges, &enc);
+  if (rc) return rc;
   cudaStream_t st = (cudaStream_t)stream;
-  char *w = (char *)workspace;
-  void *ws_fps = w;
-  w += p.fps;
-  void *ws_knn = w;
-  w += p.knn;
-  void *ws_geo = w;
-
   ForkJoin *fj = nullptr;
-  int rc = GF_OK;
   stage_mark(ST_BEGIN, st);
   if (!seeds_given) {
     rc = get_fork_join(st, &fj);
@@ -143,23 +139,19 @@ static int guidance_impl(const float *xyz, int N, int Q, int k, float radius, in
     // fork: FPS on the auxiliary stream
     GF_CUDA(cudaEventRecord(fj->fork, st));
     GF_CUDA(cudaStreamWaitEvent(fj->fps[0], fj->fork, 0));
-    rc = gf_furthest_point_sampling(xyz, 1, N, Q, seeds, ws_fps, p.fps, fj->fps[0]);
+    rc = gf_furthest_point_sampling(xyz, 1, N, Q, seeds, l.fps.ptr, l.fps.bytes, fj->fps[0]);
     if (rc) return rc;
     GF_CUDA(cudaEventRecord(fj->join_fps[0], fj->fps[0]));
   }
   // main stream: kNN graph
   KnnGridBuffers gb;
-  rc = knn_grid_build(xyz, N, k, ws_knn, p.knn, st, &gb);
+  rc = knn_grid_build(xyz, N, k, l.knn.ptr, l.knn.bytes, st, &gb);
   if (rc) return rc;
   stage_mark(ST_KNN_BUILT, st);
-  // the query kernel writes the propagation's edge table straight from its registers; the (N,k) distance / index
-  // arrays are only written when the caller asked for them
   KnnEdgeOut eo;
+  eo.tgt = edges.tgt, eo.len = edges.len, eo.slot_bits = edges.slot_bits;
   eo.radius = radius;
-  int enc = 0;
   const int Qb = q1 - q0;  // the workspace was sized for Q >= Qb seeds: enough for any block
-  rc = geodesic_edge_buffers(ws_geo, p.geo, N, k, Q, &eo.tgt, &eo.len, &eo.slot_bits, &enc);
-  if (rc) return rc;
   if (n_peers > 0) enc = 0;  // seed-sharded scenes run the per-scene kernel: original numbering, plain targets
   eo.rank = enc ? gb.rank : nullptr;
   rc = knn_grid_query(gb, nullptr, N, k, /*sqrt=*/1, knn_dist, nullptr, knn_idx32, st, &eo);
@@ -168,8 +160,8 @@ static int guidance_impl(const float *xyz, int N, int Q, int k, float radius, in
   if (!seeds_given) GF_CUDA(cudaStreamWaitEvent(st, fj->join_fps[0], 0));
   stage_mark(ST_KNN_DONE, st);
   if (Qb == 0) return GF_OK;
-  return geodesic_run(nullptr, nullptr, /*is64=*/0, N, k, seeds + q0, Qb, radius, max_step, geo, stats, ws_geo, p.geo,
-                      st, peer_geo, n_peers, row_max, enc ? gb.rank : nullptr, enc ? gb.order : nullptr);
+  return geodesic_run(nullptr, nullptr, /*is64=*/0, N, k, seeds + q0, Qb, radius, max_step, geo, stats, l.geo.ptr,
+                      l.geo.bytes, st, peer_geo, n_peers, row_max, enc ? gb.rank : nullptr, enc ? gb.order : nullptr);
 }
 
 extern "C" int gf_guidance(const float *xyz, int N, int Q, int k, float radius, int max_step, int *seeds, float *geo,
@@ -206,34 +198,30 @@ static_assert(KNN_BATCH_MAX == GEO_BATCH_MAX, "one batched call builds and queri
 // more scenes than LANES: the graphs of all scenes are built and queried with one launch each, the seeds sampled on
 // the grids (fps_cells)
 static bool batched_graphs(int B) { return B > LANES; }
-struct BatchPlan {
-  size_t per_scene[GEO_BATCH_MAX * 4];  // offsets of (fps, knn, edges) per scene
-  size_t knn_ctl, scratch, scratch_bytes, stats, total;
+// The workspace of a batch: per scene the workspace of its FPS (the culled FPS's running minima when the graphs are
+// batched), of its kNN grid and its edge table; then the control blocks of a batched build, the scratch of the batched
+// propagation and the statistics of every scene
+struct BatchLayout {
+  Span fps[GEO_BATCH_MAX], knn[GEO_BATCH_MAX];
+  GeoEdges edges[GEO_BATCH_MAX];
+  void *knn_ctl;
+  Span scratch;
+  int64_t *stats;
 };
-static int plan_batch_guidance(const int *Ns, int B, int Q, int k, BatchPlan *p, size_t *fps_b, size_t *knn_b,
-                               size_t *edge_b) {
-  size_t off = 0;
+static Arena batch_carve(void *workspace, size_t workspace_bytes, const int *Ns, int B, int Q, int k, BatchLayout *l) {
+  Arena a(workspace, workspace_bytes);
   int maxN = 1;
   for (int b = 0; b < B; ++b) {
     const int N = Ns[b];
-    fps_b[b] = batched_graphs(B) ? fps_cells_workspace_bytes(N) : align256(gf_fps_workspace_bytes(1, N, Q));
-    knn_b[b] = align256(knn_grid_workspace_bytes(N));
-    // the edge tables are the head of a single-scene geodesic workspace; only that head is used here
-    edge_b[b] = align256(geodesic_workspace_bytes(N, k, 1));
-    p->per_scene[b * 3 + 0] = off, off += fps_b[b];
-    p->per_scene[b * 3 + 1] = off, off += knn_b[b];
-    p->per_scene[b * 3 + 2] = off, off += edge_b[b];
+    l->fps[b] = a.span(batched_graphs(B) ? fps_cells_workspace_bytes(N) : gf_fps_workspace_bytes(1, N, Q));
+    l->knn[b] = a.span(knn_grid_workspace_bytes(N));
+    geo_edges_carve(a, N, k, &l->edges[b]);
     maxN = N > maxN ? N : maxN;
   }
-  p->knn_ctl = off;
-  off += align256(knn_ctl_block_bytes(B));
-  p->scratch = off;
-  p->scratch_bytes = align256(geodesic_batch_scratch_bytes(maxN, (long long)Q * B));
-  off += p->scratch_bytes;
-  p->stats = off;
-  off += align256(16 * (size_t)B);
-  p->total = off + 1024;
-  return maxN;
+  l->knn_ctl = a.take<char>(knn_ctl_block_bytes(B));
+  l->scratch = a.span(geodesic_batch_scratch_bytes(maxN, (long long)Q * B));
+  l->stats = a.take<int64_t>(2 * (size_t)B);
+  return a;
 }
 }  // namespace gf
 
@@ -241,10 +229,8 @@ extern "C" size_t gf_guidance_batch_workspace_bytes(const int *Ns, int B, int Q,
   if (!Ns || B <= 0 || B > GEO_BATCH_MAX || Q <= 0 || k <= 0) return 0;
   for (int b = 0; b < B; ++b)
     if (Ns[b] <= 0) return 0;
-  BatchPlan p;
-  size_t f[GEO_BATCH_MAX], n[GEO_BATCH_MAX], e[GEO_BATCH_MAX];
-  plan_batch_guidance(Ns, B, Q, k, &p, f, n, e);
-  return p.total;
+  BatchLayout l;
+  return batch_carve(nullptr, 0, Ns, B, Q, k, &l).off;
 }
 
 extern "C" int gf_guidance_batch(const float *const *xyz, const int *Ns, int B, int Q, int k, float radius,
@@ -261,15 +247,10 @@ extern "C" int gf_guidance_batch(const float *const *xyz, const int *Ns, int B, 
                  "guidance_batch: scene %d has %d points, beyond the on-chip bitmaps of the batched kernel "
                  "(use gf_guidance per scene)", b, Ns[b]);
   }
-  BatchPlan p;
-  size_t fps_b[GEO_BATCH_MAX], knn_b[GEO_BATCH_MAX], edge_b[GEO_BATCH_MAX];
-  plan_batch_guidance(Ns, B, Q, k, &p, fps_b, knn_b, edge_b);
-  if (workspace == nullptr || workspace_bytes < p.total) {
-    set_error("guidance_batch: workspace too small (%zu bytes given, %zu needed)", workspace_bytes, p.total);
-    return GF_ERR_WORKSPACE;
-  }
+  BatchLayout w;
+  const Arena ar = batch_carve(workspace, workspace_bytes, Ns, B, Q, k, &w);
+  if (!ar.ok) return ar.fail("guidance_batch");
   cudaStream_t st = (cudaStream_t)stream;
-  char *w = (char *)workspace;
   ForkJoin *fj = nullptr;
   // The graphs.  Up to LANES scenes, every scene has a lane of its own (lane 0: the caller's stream) and its graph
   // is one short chain next to its FPS.  With more scenes a lane would run several graphs one after another, each a
@@ -288,12 +269,12 @@ extern "C" int gf_guidance_batch(const float *const *xyz, const int *Ns, int B, 
       if (l > 0) GF_CUDA(cudaStreamWaitEvent(fj->knn[l], fj->fork, 0));
     }
   GeoSceneDesc desc[GEO_BATCH_MAX];
-  int64_t *d_stats = stats ? (int64_t *)(w + p.stats) : nullptr;
+  int64_t *d_stats = stats ? w.stats : nullptr;
   if (d_stats) GF_CUDA(cudaMemsetAsync(d_stats, 0, 16 * (size_t)B, st));
   // FPS first on every lane (the longest chains start first), then the graphs
   if (!seeds_given && !batched)
     for (int b = 0; b < B; ++b) {
-      rc = gf_furthest_point_sampling(xyz[b], 1, Ns[b], Q, seeds[b], w + p.per_scene[b * 3 + 0], fps_b[b],
+      rc = gf_furthest_point_sampling(xyz[b], 1, Ns[b], Q, seeds[b], w.fps[b].ptr, w.fps[b].bytes,
                                       fj->fps[b % lanes]);
       if (rc) return rc;
     }
@@ -301,16 +282,15 @@ extern "C" int gf_guidance_batch(const float *const *xyz, const int *Ns, int B, 
   KnnGridBuffers gb[GEO_BATCH_MAX];
   KnnEdgeOut eo[GEO_BATCH_MAX];
   KnnQueryJob jobs[GEO_BATCH_MAX];
-  for (int b = 0; b < B; ++b) ks[b] = {xyz[b], Ns[b], w + p.per_scene[b * 3 + 1], knn_b[b]};
+  for (int b = 0; b < B; ++b) ks[b] = {xyz[b], Ns[b], w.knn[b].ptr, w.knn[b].bytes};
   if (batched) {
-    rc = knn_grid_build_batch(ks, B, k, w + p.knn_ctl, st, gb);
+    rc = knn_grid_build_batch(ks, B, k, w.knn_ctl, st, gb);
     if (rc) return rc;
     if (!seeds_given) {  // the FPS lanes start when the grids are built, next to the query on the caller's stream
       GF_CUDA(cudaEventRecord(fj->built, st));
       for (int l = 0; l < lanes; ++l) GF_CUDA(cudaStreamWaitEvent(fj->fps[l], fj->built, 0));
       for (int b = 0; b < B; ++b) {
-        rc = fps_cells(gb[b].sorted, xyz[b], Ns[b], Q, w + p.per_scene[b * 3 + 0], fps_b[b], seeds[b],
-                       fj->fps[b % lanes]);
+        rc = fps_cells(gb[b].sorted, xyz[b], Ns[b], Q, w.fps[b].ptr, w.fps[b].bytes, seeds[b], fj->fps[b % lanes]);
         if (rc) return rc;
       }
     }
@@ -322,11 +302,8 @@ extern "C" int gf_guidance_batch(const float *const *xyz, const int *Ns, int B, 
       rc = knn_grid_build_batch(&ks[b], 1, k, nullptr, kst, &gb[b]);
       if (rc) return rc;
     }
+    eo[b].tgt = w.edges[b].tgt, eo[b].len = w.edges[b].len, eo[b].slot_bits = w.edges[b].slot_bits;
     eo[b].radius = radius;
-    int enc = 0;
-    rc = geodesic_edge_buffers(w + p.per_scene[b * 3 + 2], edge_b[b], Ns[b], k, 1, &eo[b].tgt, &eo[b].len,
-                               &eo[b].slot_bits, &enc);
-    if (rc) return rc;
     eo[b].rank = gb[b].rank;  // cell-order table (every scene of a batched call is batchable: checked above)
     jobs[b] = {gb[b], nullptr, Ns[b], nullptr, nullptr, nullptr, &eo[b]};
     if (!batched) {
@@ -354,42 +331,52 @@ extern "C" int gf_guidance_batch(const float *const *xyz, const int *Ns, int B, 
     }
   }
   stage_mark(ST_KNN_DONE, st);
-  rc = geodesic_batch_launch(desc, B, k, max_step, w + p.scratch, p.scratch_bytes, st);
+  rc = geodesic_batch_launch(desc, B, k, max_step, w.scratch.ptr, w.scratch.bytes, st);
   if (rc) return rc;
   if (stats) GF_CUDA(cudaMemcpyAsync(stats, d_stats, 16 * (size_t)B, cudaMemcpyDeviceToDevice, st));
   return GF_OK;
 }
 
+// the workspace of a host-buffer scene: its points, seeds and maps on the device, then the device call's workspace
+namespace gf {
+struct HostLayout {
+  float *xyz;
+  int *seeds;
+  float *geo;
+  Span inner;
+};
+static Arena host_carve(void *workspace, size_t workspace_bytes, int N, int Q, int k, HostLayout *l) {
+  Arena a(workspace, workspace_bytes);
+  l->xyz = a.take<float>(3 * (size_t)N);
+  l->seeds = a.take<int>((size_t)Q);
+  l->geo = a.take<float>((size_t)Q * N);
+  l->inner = a.span(gf_guidance_workspace_bytes(N, Q, k));
+  return a;
+}
+}  // namespace gf
+
 extern "C" size_t gf_guidance_host_workspace_bytes(int N, int Q, int k) {
   if (N <= 0 || Q <= 0 || k <= 0) return 0;
-  return plan_guidance(N, Q, k).total + align256(sizeof(float) * (size_t)N * 3) + align256(sizeof(int) * (size_t)Q) +
-         align256(sizeof(float) * (size_t)Q * N) + 1024;
+  HostLayout l;
+  return host_carve(nullptr, 0, N, Q, k, &l).off;
 }
 
 extern "C" int gf_guidance_host(const float *xyz_host, int N, int Q, int k, float radius, int max_step,
                                 int *seeds_host, float *geo_host, void *workspace, size_t workspace_bytes,
                                 void *stream) {
   GF_CHECK_ARG(N >= 1 && Q >= 1, "guidance_host: need N >= 1 and Q >= 1");
+  GF_CHECK_ARG(k >= 1 && k <= KNN_MAX_K, "guidance_host: k=%d outside [1,%d]", k, KNN_MAX_K);
   GF_CHECK_ARG(xyz_host && seeds_host && geo_host, "guidance_host: null host pointer");
-  size_t need = gf_guidance_host_workspace_bytes(N, Q, k);
-  if (workspace == nullptr || workspace_bytes < need) {
-    set_error("guidance_host: workspace too small (%zu bytes given, %zu needed)", workspace_bytes, need);
-    return GF_ERR_WORKSPACE;
-  }
+  HostLayout l;
+  const Arena ar = host_carve(workspace, workspace_bytes, N, Q, k, &l);
+  if (!ar.ok) return ar.fail("guidance_host");
   cudaStream_t st = (cudaStream_t)stream;
-  char *w = (char *)workspace;
-  float *d_xyz = (float *)w;
-  w += align256(sizeof(float) * (size_t)N * 3);
-  int *d_seeds = (int *)w;
-  w += align256(sizeof(int) * (size_t)Q);
-  float *d_geo = (float *)w;
-  w += align256(sizeof(float) * (size_t)Q * N);
-  size_t inner = plan_guidance(N, Q, k).total;
-  GF_CUDA(cudaMemcpyAsync(d_xyz, xyz_host, sizeof(float) * (size_t)N * 3, cudaMemcpyHostToDevice, st));
-  int rc = gf_guidance(d_xyz, N, Q, k, radius, max_step, d_seeds, d_geo, nullptr, nullptr, nullptr, nullptr, w, inner, st);
+  GF_CUDA(cudaMemcpyAsync(l.xyz, xyz_host, sizeof(float) * (size_t)N * 3, cudaMemcpyHostToDevice, st));
+  int rc = gf_guidance(l.xyz, N, Q, k, radius, max_step, l.seeds, l.geo, nullptr, nullptr, nullptr, nullptr,
+                       l.inner.ptr, l.inner.bytes, st);
   if (rc) return rc;
-  GF_CUDA(cudaMemcpyAsync(seeds_host, d_seeds, sizeof(int) * (size_t)Q, cudaMemcpyDeviceToHost, st));
-  GF_CUDA(cudaMemcpyAsync(geo_host, d_geo, sizeof(float) * (size_t)Q * N, cudaMemcpyDeviceToHost, st));
+  GF_CUDA(cudaMemcpyAsync(seeds_host, l.seeds, sizeof(int) * (size_t)Q, cudaMemcpyDeviceToHost, st));
+  GF_CUDA(cudaMemcpyAsync(geo_host, l.geo, sizeof(float) * (size_t)Q * N, cudaMemcpyDeviceToHost, st));
   GF_CUDA(cudaStreamSynchronize(st));
   return GF_OK;
 }
@@ -424,21 +411,26 @@ static int get_host_lanes(HostLanes **out) {
   return GF_OK;
 }
 
-struct HostBatchPlan {
-  size_t xyz[GEO_BATCH_MAX], seeds[GEO_BATCH_MAX], geo[GEO_BATCH_MAX], lane_ws[HOST_LANES], lane_bytes, total;
+// the workspace: every scene's points, seeds and maps on the device, then one device-call workspace per lane, sized
+// for the largest scene
+struct HostBatchLayout {
+  float *xyz[GEO_BATCH_MAX];
+  int *seeds[GEO_BATCH_MAX];
+  float *geo[GEO_BATCH_MAX];
+  Span lane[HOST_LANES];
 };
-static void plan_host_batch(const int *Ns, int B, int Q, int k, HostBatchPlan *p) {
-  size_t off = 0;
+static Arena host_batch_carve(void *workspace, size_t workspace_bytes, const int *Ns, int B, int Q, int k,
+                              HostBatchLayout *l) {
+  Arena a(workspace, workspace_bytes);
   int maxN = 1;
   for (int b = 0; b < B; ++b) {
-    p->xyz[b] = off, off += align256(sizeof(float) * 3 * (size_t)Ns[b]);
-    p->seeds[b] = off, off += align256(sizeof(int) * (size_t)Q);
-    p->geo[b] = off, off += align256(sizeof(float) * (size_t)Q * Ns[b]);
+    l->xyz[b] = a.take<float>(3 * (size_t)Ns[b]);
+    l->seeds[b] = a.take<int>((size_t)Q);
+    l->geo[b] = a.take<float>((size_t)Q * Ns[b]);
     maxN = Ns[b] > maxN ? Ns[b] : maxN;
   }
-  p->lane_bytes = align256(plan_guidance(maxN, Q, k).total);
-  for (int l = 0; l < HOST_LANES; ++l) p->lane_ws[l] = off, off += p->lane_bytes;
-  p->total = off + 1024;
+  for (int i = 0; i < HOST_LANES; ++i) l->lane[i] = a.span(gf_guidance_workspace_bytes(maxN, Q, k));
+  return a;
 }
 }  // namespace gf
 
@@ -446,9 +438,8 @@ extern "C" size_t gf_guidance_batch_host_workspace_bytes(const int *Ns, int B, i
   if (!Ns || B <= 0 || B > GEO_BATCH_MAX || Q <= 0 || k <= 0) return 0;
   for (int b = 0; b < B; ++b)
     if (Ns[b] <= 0) return 0;
-  HostBatchPlan p;
-  plan_host_batch(Ns, B, Q, k, &p);
-  return p.total;
+  HostBatchLayout l;
+  return host_batch_carve(nullptr, 0, Ns, B, Q, k, &l).off;
 }
 
 extern "C" int gf_guidance_batch_host(const float *const *xyz_host, const int *Ns, int B, int Q, int k, float radius,
@@ -459,14 +450,10 @@ extern "C" int gf_guidance_batch_host(const float *const *xyz_host, const int *N
   GF_CHECK_ARG(k >= 1 && k <= KNN_MAX_K, "guidance_batch_host: k=%d outside [1,%d]", k, KNN_MAX_K);
   for (int b = 0; b < B; ++b)
     GF_CHECK_ARG(Ns[b] >= 1 && xyz_host[b] && seeds_host[b] && geo_host[b], "guidance_batch_host: scene %d: empty or null", b);
-  HostBatchPlan p;
-  plan_host_batch(Ns, B, Q, k, &p);
-  if (workspace == nullptr || workspace_bytes < p.total) {
-    set_error("guidance_batch_host: workspace too small (%zu bytes given, %zu needed)", workspace_bytes, p.total);
-    return GF_ERR_WORKSPACE;
-  }
+  HostBatchLayout w;
+  const Arena ar = host_batch_carve(workspace, workspace_bytes, Ns, B, Q, k, &w);
+  if (!ar.ok) return ar.fail("guidance_batch_host");
   cudaStream_t st = (cudaStream_t)stream;
-  char *w = (char *)workspace;
   HostLanes *hl = nullptr;
   int rc = get_host_lanes(&hl);
   if (rc) return rc;
@@ -476,15 +463,12 @@ extern "C" int gf_guidance_batch_host(const float *const *xyz_host, const int *N
   for (int b = 0; b < B; ++b) {
     const int l = b % lanes;
     cudaStream_t ls = hl->lane[l];
-    float *d_xyz = (float *)(w + p.xyz[b]);
-    int *d_seeds = (int *)(w + p.seeds[b]);
-    float *d_geo = (float *)(w + p.geo[b]);
-    GF_CUDA(cudaMemcpyAsync(d_xyz, xyz_host[b], sizeof(float) * 3 * (size_t)Ns[b], cudaMemcpyHostToDevice, ls));
-    rc = gf_guidance(d_xyz, Ns[b], Q, k, radius, max_step, d_seeds, d_geo, nullptr, nullptr, nullptr, nullptr,
-                     w + p.lane_ws[l], p.lane_bytes, ls);
+    GF_CUDA(cudaMemcpyAsync(w.xyz[b], xyz_host[b], sizeof(float) * 3 * (size_t)Ns[b], cudaMemcpyHostToDevice, ls));
+    rc = gf_guidance(w.xyz[b], Ns[b], Q, k, radius, max_step, w.seeds[b], w.geo[b], nullptr, nullptr, nullptr, nullptr,
+                     w.lane[l].ptr, w.lane[l].bytes, ls);
     if (rc) return rc;
-    GF_CUDA(cudaMemcpyAsync(seeds_host[b], d_seeds, sizeof(int) * (size_t)Q, cudaMemcpyDeviceToHost, ls));
-    GF_CUDA(cudaMemcpyAsync(geo_host[b], d_geo, sizeof(float) * (size_t)Q * Ns[b], cudaMemcpyDeviceToHost, ls));
+    GF_CUDA(cudaMemcpyAsync(seeds_host[b], w.seeds[b], sizeof(int) * (size_t)Q, cudaMemcpyDeviceToHost, ls));
+    GF_CUDA(cudaMemcpyAsync(geo_host[b], w.geo[b], sizeof(float) * (size_t)Q * Ns[b], cudaMemcpyDeviceToHost, ls));
   }
   for (int l = 0; l < lanes; ++l) {
     GF_CUDA(cudaEventRecord(hl->join[l], hl->lane[l]));

@@ -797,7 +797,19 @@ static Arena knn_carve(void *workspace, size_t workspace_bytes, int N, KnnBuildD
 
 size_t knn_grid_workspace_bytes(int N) {
   KnnBuildDesc d;
-  return knn_carve(nullptr, 0, N, &d).off + 1024;
+  return knn_carve(nullptr, 0, N, &d).off;
+}
+
+// the control blocks of a batched build, one per scene, cleared together by one memset
+static Arena knn_ctl_carve(void *ctl_block, size_t bytes, int B, KnnCtl **ctl) {
+  Arena ar(ctl_block, bytes);
+  for (int b = 0; b < B; ++b) ctl[b] = ar.take<KnnCtl>(1);
+  return ar;
+}
+
+size_t knn_ctl_block_bytes(int B) {
+  KnnCtl *ctl[KNN_BATCH_MAX];
+  return knn_ctl_carve(nullptr, 0, B, ctl).off;
 }
 
 // the register-resident top-k is sized KT = the power of two >= k (8 .. 64); launch(KT) is called with it as a
@@ -814,8 +826,6 @@ static void with_kt(int k, F &&launch) {
     launch(std::integral_constant<int, 64>());
 }
 
-size_t knn_ctl_block_bytes(int B) { return align256(sizeof(KnnCtl)) * (size_t)(B > 0 ? B : 0); }
-
 // Five launches and one memset for the whole batch (round 1: thirteen launches per scene): bbox + coarse plan |
 // coarse count + final plan | final count | scan | scatter.  Nothing returns to the host; grid dimensions are read
 // from the device.  A scene gets nb / B blocks of each kernel (at least one, and for the count and scatter kernels no
@@ -829,18 +839,19 @@ int knn_grid_build_batch(const KnnBuildScene *scenes, int B, int k, void *ctl_bl
     return GF_ERR_INVALID;
   }
   KnnBuildArgs a;
+  KnnCtl *ctl[KNN_BATCH_MAX];
+  if (ctl_block) {
+    const Arena ar = knn_ctl_carve(ctl_block, knn_ctl_block_bytes(B), B, ctl);
+    if (!ar.ok) return ar.fail("knn: control blocks");
+  }
   int maxN = 1;
   for (int b = 0; b < B; ++b) {
     const int N = scenes[b].N;
     KnnBuildDesc &d = a.s[b];
     d.xyz = scenes[b].xyz;
-    const bool ok = knn_carve(scenes[b].workspace, scenes[b].workspace_bytes, N, &d).ok;
-    if (ctl_block) d.ctl = (KnnCtl *)((char *)ctl_block + align256(sizeof(KnnCtl)) * b);
-    if (!ok) {
-      set_error("knn: workspace of scene %d too small (%zu bytes given, %zu needed)", b, scenes[b].workspace_bytes,
-                knn_grid_workspace_bytes(N));
-      return GF_ERR_WORKSPACE;
-    }
+    const Arena ar = knn_carve(scenes[b].workspace, scenes[b].workspace_bytes, N, &d);
+    if (!ar.ok) return ar.fail("knn");
+    if (ctl_block) d.ctl = ctl[b];
     maxN = N > maxN ? N : maxN;
     out[b].grid = &d.ctl->g;
     out[b].cell_start = d.cell_start;
@@ -958,21 +969,22 @@ extern "C" int gf_knn(const float *xyz, int N, const float *queries, int nq, int
 }
 
 // ---- a batch of scenes, each against itself: one build and one query launch for all of them -------------------------
-static size_t knn_batch_layout(const int *Ns, int B, size_t *off) {
-  size_t o = align256(knn_ctl_block_bytes(B));
-  for (int b = 0; b < B; ++b) {
-    off[b] = o;
-    o += align256(knn_grid_workspace_bytes(Ns[b]));
-  }
-  return o + 1024;
+// the workspace: the control blocks, then every scene's grid workspace
+static Arena knn_batch_carve(void *workspace, size_t workspace_bytes, const int *Ns, int B, void **ctl_block,
+                             Span *scene) {
+  Arena a(workspace, workspace_bytes);
+  *ctl_block = a.take<char>(knn_ctl_block_bytes(B));
+  for (int b = 0; b < B; ++b) scene[b] = a.span(knn_grid_workspace_bytes(Ns[b]));
+  return a;
 }
 
 extern "C" size_t gf_knn_batch_workspace_bytes(const int *Ns, int B) {
   if (!Ns || B < 1 || B > KNN_BATCH_MAX) return 0;
   for (int b = 0; b < B; ++b)
     if (Ns[b] < 1) return 0;
-  size_t off[KNN_BATCH_MAX];
-  return knn_batch_layout(Ns, B, off);
+  void *ctl_block;
+  Span scene[KNN_BATCH_MAX];
+  return knn_batch_carve(nullptr, 0, Ns, B, &ctl_block, scene).off;
 }
 
 extern "C" int gf_knn_batch(const float *const *xyz, const int *Ns, int B, int k, int sqrt_out, float *const *dist,
@@ -981,19 +993,16 @@ extern "C" int gf_knn_batch(const float *const *xyz, const int *Ns, int B, int k
   GF_CHECK_ARG(B >= 1 && B <= KNN_BATCH_MAX, "knn_batch: B=%d outside [1,%d]", B, KNN_BATCH_MAX);
   GF_CHECK_ARG(k >= 1 && k <= KNN_MAX_K, "knn_batch: k=%d outside [1,%d]", k, KNN_MAX_K);
   for (int b = 0; b < B; ++b) GF_CHECK_ARG(Ns[b] >= 1 && xyz[b], "knn_batch: scene %d: empty or null", b);
-  size_t off[KNN_BATCH_MAX];
-  const size_t need = knn_batch_layout(Ns, B, off);
-  if (workspace == nullptr || workspace_bytes < need) {
-    set_error("knn_batch: workspace too small (%zu bytes given, %zu needed)", workspace_bytes, need);
-    return GF_ERR_WORKSPACE;
-  }
+  void *ctl_block;
+  Span scene[KNN_BATCH_MAX];
+  const Arena ar = knn_batch_carve(workspace, workspace_bytes, Ns, B, &ctl_block, scene);
+  if (!ar.ok) return ar.fail("knn_batch");
   cudaStream_t st = (cudaStream_t)stream;
-  char *w = (char *)workspace;
   KnnBuildScene sc[KNN_BATCH_MAX];
   KnnGridBuffers gb[KNN_BATCH_MAX];
   KnnQueryJob jobs[KNN_BATCH_MAX];
-  for (int b = 0; b < B; ++b) sc[b] = {xyz[b], Ns[b], w + off[b], align256(knn_grid_workspace_bytes(Ns[b]))};
-  int rc = knn_grid_build_batch(sc, B, k, w, st, gb);
+  for (int b = 0; b < B; ++b) sc[b] = {xyz[b], Ns[b], scene[b].ptr, scene[b].bytes};
+  int rc = knn_grid_build_batch(sc, B, k, ctl_block, st, gb);
   if (rc) return rc;
   for (int b = 0; b < B; ++b) jobs[b] = {gb[b], nullptr, Ns[b], dist[b], nullptr, idx32[b], nullptr};
   return knn_grid_query_batch(jobs, B, k, sqrt_out, st);

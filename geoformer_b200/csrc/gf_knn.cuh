@@ -29,7 +29,7 @@ struct KnnEdgeOut {
 constexpr int KNN_BATCH_MAX = 32;
 
 size_t knn_grid_workspace_bytes(int N);
-// the B control blocks of a batched build: one contiguous area, cleared by a single memset
+// the B <= KNN_BATCH_MAX control blocks of a batched build: one contiguous area, cleared by a single memset
 size_t knn_ctl_block_bytes(int B);
 
 // one scene of a batched build: its points and its own workspace of knn_grid_workspace_bytes(N) bytes

@@ -371,32 +371,40 @@ static int mh_grid(int N) {
 
 using namespace gf;
 
+// the workspace: the row maxima of the maps, and for the backward the per-CTA partial sums of the weight gradients
+struct MhLayout {
+  RowMax rm;
+  float *part;
+};
+static Arena mh_carve(void *workspace, size_t workspace_bytes, int Q, int N, bool backward, MhLayout *l) {
+  Arena a(workspace, workspace_bytes);
+  l->rm = take_rowmax(a, (size_t)Q);
+  l->part = backward ? a.take<float>((size_t)mh_grid(N) * Q * MH_NPART) : nullptr;
+  return a;
+}
+
 extern "C" size_t gf_mask_head_workspace_bytes(int Q, int N) {
   if (Q <= 0 || N <= 0) return 0;
-  return align256(sizeof(uint32_t) * (size_t)Q) + 256;
+  MhLayout l;
+  return mh_carve(nullptr, 0, Q, N, false, &l).off;
 }
 
 extern "C" size_t gf_mask_head_backward_workspace_bytes(int Q, int N) {
   if (Q <= 0 || N <= 0) return 0;
-  return gf_mask_head_workspace_bytes(Q, N) + align256(sizeof(float) * (size_t)mh_grid(N) * Q * MH_NPART);
+  MhLayout l;
+  return mh_carve(nullptr, 0, Q, N, true, &l).off;
 }
 
-// arguments common to both entries; returns the workspace's row maxima
+// arguments common to both entries, and the row maxima into the carved workspace
 static int mh_prepare(MhArgs &a, const float *geo, const float *feats, const float *w0, const float *b0,
                       const float *w1, const float *b1, const float *coords, const float *seed_xyz,
-                      const float *row_max, int Q, int N, Arena &ar, cudaStream_t st) {
-  uint32_t *rowmax = ar.take<uint32_t>((size_t)Q);
-  uint32_t *gmax = ar.take<uint32_t>(1);
-  if (!ar.ok) {
-    set_error("mask_head: workspace too small");
-    return GF_ERR_WORKSPACE;
-  }
+                      const float *row_max, int Q, int N, const MhLayout &l, cudaStream_t st) {
   int rc = mh_set_smem();
   if (rc) return rc;
   const bool vec = (N % 4 == 0) && (((uintptr_t)geo & 15) == 0);
-  if ((rc = bias_mask_rowmax(geo, Q, N, row_max, vec, rowmax, gmax, st))) return rc;
+  if ((rc = bias_mask_rowmax(geo, Q, N, row_max, vec, l.rm, st))) return rc;
   a.geo = geo, a.feats = feats, a.w0 = w0, a.b0 = b0, a.w1 = w1, a.b1 = b1, a.coords = coords, a.seed_xyz = seed_xyz;
-  a.rowmax = rowmax, a.gmax = gmax, a.Q = Q, a.N = N;
+  a.rowmax = l.rm.rowmax, a.gmax = l.rm.gmax, a.Q = Q, a.N = N;
   a.out = nullptr, a.dlogit = nullptr, a.dfeats = nullptr;
   return GF_OK;
 }
@@ -410,9 +418,11 @@ extern "C" int gf_mask_head_logits(const float *geo, const float *feats, const f
   if ((long long)Q * N == 0) return GF_OK;
   GF_CHECK_ARG(geo && feats && w0 && b0 && w1 && b1 && coords && seed_xyz && out, "mask_head: null pointer");
   cudaStream_t st = (cudaStream_t)stream;
-  Arena ar(workspace, workspace_bytes);
+  MhLayout l;
+  const Arena ar = mh_carve(workspace, workspace_bytes, Q, N, false, &l);
+  if (!ar.ok) return ar.fail("mask_head");
   MhArgs a;
-  int rc = mh_prepare(a, geo, feats, w0, b0, w1, b1, coords, seed_xyz, row_max, Q, N, ar, st);
+  int rc = mh_prepare(a, geo, feats, w0, b0, w1, b1, coords, seed_xyz, row_max, Q, N, l, st);
   if (rc) return rc;
   a.out = out;
   mask_head_kernel<false><<<mh_grid(N), MH_THREADS, MH_SMEM, st>>>(a);
@@ -440,16 +450,14 @@ extern "C" int gf_mask_head_logits_backward(const float *geo, const float *feats
     if (Q > 0 && db1) GF_CUDA(cudaMemsetAsync(db1, 0, sizeof(float) * (size_t)Q, st));
     return GF_OK;
   }
-  Arena ar(workspace, workspace_bytes);
+  MhLayout l;
+  const Arena ar = mh_carve(workspace, workspace_bytes, Q, N, true, &l);
+  if (!ar.ok) return ar.fail("mask_head_backward");
   MhArgs a;
   const int grid = mh_grid(N);
-  int rc = mh_prepare(a, geo, feats, w0, b0, w1, b1, coords, seed_xyz, row_max, Q, N, ar, st);
+  int rc = mh_prepare(a, geo, feats, w0, b0, w1, b1, coords, seed_xyz, row_max, Q, N, l, st);
   if (rc) return rc;
-  a.part = ar.take<float>((size_t)grid * Q * MH_NPART);
-  if (!ar.ok) {
-    set_error("mask_head_backward: workspace too small");
-    return GF_ERR_WORKSPACE;
-  }
+  a.part = l.part;
   a.dlogit = dlogit, a.dfeats = dfeats;
   mask_head_kernel<true><<<grid, MH_THREADS, MH_BWD_SMEM, st>>>(a);
   GF_LAUNCHED();

@@ -17,7 +17,9 @@
  *     operators, batch-major (B,N,3) coordinates, channel-major (B,C,N) features, everything
  *     contiguous.  Outputs are fully written by the callee (the reference's zero-initialisation,
  *     e.g. ball_query rows without a hit, is reproduced by the callee, not assumed of the caller).
- *   - scratch memory is provided by the caller: gf_*_workspace_bytes() says how much.
+ *   - scratch memory is provided by the caller: gf_*_workspace_bytes() says how much.  Its base must
+ *     be 256-byte aligned (cudaMalloc and torch allocations are).  A call that returns
+ *     GF_ERR_WORKSPACE (too small or misaligned) has enqueued nothing on `stream`.
  *   - there is no CPU fallback: every entry point needs a CUDA device.
  */
 #ifndef GEOFORMER_B200_H
