@@ -69,6 +69,10 @@ SIGNATURES = {
     "gf_mask_head_logits": (c_int, [_P] * 9 + [c_int, c_int, c_int, _P, _P, c_size_t, _P]),
     "gf_mask_head_backward_workspace_bytes": (c_size_t, [c_int, c_int]),
     "gf_mask_head_logits_backward": (c_int, [_P] * 9 + [c_int, c_int, c_int] + [_P] * 7 + [c_size_t, _P]),
+    "gf_mask_head_batch_workspace_bytes": (c_size_t, [_P, c_int, c_int]),
+    "gf_mask_head_logits_batch": (c_int, [_P, _P, c_int, c_int, c_int] + [_P] * 9 + [_P, c_size_t, _P]),
+    "gf_mask_head_batch_backward_workspace_bytes": (c_size_t, [_P, c_int, c_int]),
+    "gf_mask_head_logits_batch_backward": (c_int, [_P, _P, c_int, c_int, c_int] + [_P] * 14 + [_P, c_size_t, _P]),
     "gf_group_mlp_pool": (c_int, [_P, _P, _P, _P, c_int, c_int, c_int, c_int, c_int, c_float, c_int, c_int, c_int, _P, _P,
                                   _P, _P, c_int, _P, _P]),
     "gf_group_mlp_pool_train_workspace_bytes": (c_size_t, [c_int, c_int]),

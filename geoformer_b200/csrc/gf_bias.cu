@@ -176,6 +176,51 @@ __global__ void __launch_bounds__(1024)
   if (threadIdx.x == 0) *gmax = r > -__int_as_float(0x7f800000) ? f2ord(r) : 0u;
 }
 
+// bias_mask_rowmax_kernel over the rows of a batch: block (row, chunk) with row = b*Q + q reduces its chunk of scene
+// b's row q into rowmax[row] and scene b's own maximum gmax[b] (:276 takes the maximum over one scene's rows only)
+__global__ void __launch_bounds__(256)
+    bias_mask_rowmax_batch_kernel(const __grid_constant__ MaskMaps maps, uint32_t *__restrict__ rowmax_ord,
+                                  uint32_t *__restrict__ gmax) {
+  __shared__ float sm[8];
+  const int row = blockIdx.x, b = row / maps.Q, q = row - b * maps.Q, N = maps.N[b], chunks = gridDim.y;
+  const float *rp = maps.geo[b] + (size_t)q * N;
+  float v = -__int_as_float(0x7f800000);
+  if (N % 4 == 0 && ((uintptr_t)maps.geo[b] & 15) == 0) {
+    const int n4 = N >> 2, per = (n4 + chunks - 1) / chunks;
+    const int p0 = blockIdx.y * per, p1 = min(n4, p0 + per);
+    const float4 *r4 = reinterpret_cast<const float4 *>(rp);
+    for (int p = p0 + threadIdx.x; p < p1; p += blockDim.x) {
+      const float4 g = __ldg(r4 + p);
+      v = fmaxf(fmaxf(v, fmaxf(g.x, g.y)), fmaxf(g.z, g.w));
+    }
+  } else {
+    const int per = (N + chunks - 1) / chunks;
+    const int p0 = blockIdx.y * per, p1 = min(N, p0 + per);
+    for (int p = p0 + threadIdx.x; p < p1; p += blockDim.x) v = fmaxf(v, __ldg(rp + p));
+  }
+  float r = block_max(v, sm);
+  if (threadIdx.x == 0 && r > -__int_as_float(0x7f800000)) {
+    atomicMax(rowmax_ord + row, f2ord(r));
+    atomicMax(gmax + b, f2ord(r));
+  }
+}
+
+// bias_rowmax_import_kernel per scene: block b imports row_max[b] (Q) and sets gmax[b]
+__global__ void __launch_bounds__(1024)
+    bias_rowmax_import_batch_kernel(const float *__restrict__ row_max, int Q, uint32_t *__restrict__ rowmax_ord,
+                                    uint32_t *__restrict__ gmax) {
+  __shared__ float sm[32];
+  const size_t base = (size_t)blockIdx.x * Q;
+  float v = -__int_as_float(0x7f800000);
+  for (int q = threadIdx.x; q < Q; q += blockDim.x) {
+    const float r = row_max[base + q];
+    rowmax_ord[base + q] = f2ord(r);
+    v = fmaxf(v, r);
+  }
+  const float r = block_max(v, sm);
+  if (threadIdx.x == 0) gmax[blockIdx.x] = r > -__int_as_float(0x7f800000) ? f2ord(r) : 0u;
+}
+
 // out[q,a,p] = d + (geo[q,p] < 0 ? sqrt(m_q) * sign(d) : 0),  d = seed_xyz[q,a] - coords[p,a]   (:271-289)
 template <bool VEC>
 __global__ void __launch_bounds__(256)
@@ -257,6 +302,28 @@ int bias_mask_rowmax(const float *geo, int Q, int N, const float *row_max, bool 
     bias_mask_rowmax_kernel<true><<<Q * chunks, 256, 0, st>>>(geo, N, chunks, rowmax, gmax);
   else
     bias_mask_rowmax_kernel<false><<<Q * chunks, 256, 0, st>>>(geo, N, chunks, rowmax, gmax);
+  GF_LAUNCHED();
+  return GF_OK;
+}
+
+// row maxima of a batch's maps, each scene's maximum its own; gmax must follow rowmax (B*Q) so that one fill clears both
+int bias_mask_rowmax_batch(const MaskMaps &maps, const float *row_max, uint32_t *rowmax, uint32_t *gmax,
+                           cudaStream_t st) {
+  const int rows = maps.B * maps.Q;
+  if (row_max) {
+    bias_rowmax_import_batch_kernel<<<maps.B, 1024, 0, st>>>(row_max, maps.Q, rowmax, gmax);
+    GF_LAUNCHED();
+    return GF_OK;
+  }
+  bias_zero_kernel<<<(rows + maps.B + 255) / 256, 256, 0, st>>>(rowmax, rows + maps.B);
+  GF_LAUNCHED();
+  int nmax = 0;
+  for (int b = 0; b < maps.B; ++b) nmax = maps.N[b] > nmax ? maps.N[b] : nmax;
+  // as bias_mask_rowmax: about 8 blocks per SM, no chunk of the largest scene under 1024 loads
+  int chunks = (num_sms() * 8 + rows - 1) / rows;
+  if (chunks > (nmax / 4 + 1023) / 1024) chunks = (nmax / 4 + 1023) / 1024;
+  if (chunks < 1) chunks = 1;
+  bias_mask_rowmax_batch_kernel<<<dim3(rows, chunks), 256, 0, st>>>(maps, rowmax, gmax);
   GF_LAUNCHED();
   return GF_OK;
 }

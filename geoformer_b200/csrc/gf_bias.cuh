@@ -31,4 +31,17 @@ int bias_ctx_rowmax(const float *const *geo_ptrs, const int *geo_ld, const int *
 // vec: N % 4 == 0 and geo 16-byte aligned
 int bias_mask_rowmax(const float *geo, int Q, int N, const float *row_max, bool vec, const RowMax &rm, cudaStream_t st);
 
+// the (Q, N_b) maps of a batched mask head, up to 32 scenes (gf_mask_head.cu)
+constexpr int MH_BATCH_MAX = 32;
+struct MaskMaps {
+  const float *geo[MH_BATCH_MAX];
+  int N[MH_BATCH_MAX];
+  int B, Q;
+};
+
+// ordered-uint row maxima (B, Q) of a batch's maps and each scene's own maximum of them, gmax (B), or row_max (B, Q)
+// imported: one launch (after one zero fill when computed) for the whole batch (gf_bias.cu)
+int bias_mask_rowmax_batch(const MaskMaps &maps, const float *row_max, uint32_t *rowmax, uint32_t *gmax,
+                           cudaStream_t st);
+
 }  // namespace gf

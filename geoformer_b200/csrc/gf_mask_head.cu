@@ -170,154 +170,7 @@ __global__ void __launch_bounds__(MH_THREADS, 1) mask_head_kernel(const MhArgs a
   uint32_t it = 0;
   bool first_tile = true;
   for (int tile = blockIdx.x; tile < T; tile += gridDim.x) {
-    const int p = (int)(lq * 32u + lane), n = tile * MH_TILE + p;
-    const bool valid = n < a.N;
-    {  // feats tile: row = point (zero past N), 16 channels of the 32-float swizzled row
-      const int r = (int)(tid >> 2), c0 = (int)(tid & 3u) * 4, nr = tile * MH_TILE + r;
-      float4 f = make_float4(0.f, 0.f, 0.f, 0.f);
-      if (nr < a.N) {
-        const float *src = a.feats + (size_t)nr * MH_M + c0;
-        f = make_float4(__ldg(src), __ldg(src + 1), __ldg(src + 2), __ldg(src + 3));
-      }
-      *reinterpret_cast<float4 *>(sA + sw128_off<MH_TILE>(r, c0)) = f;
-    }
-    const float px = valid ? __ldg(a.coords + (size_t)n * 3 + 0) : 0.f, py = valid ? __ldg(a.coords + (size_t)n * 3 + 1) : 0.f,
-                pz = valid ? __ldg(a.coords + (size_t)n * 3 + 2) : 0.f;
-    float fx[BWD ? MH_M : 1], dfa[BWD ? MH_M : 1];
-    if (BWD) {
-#pragma unroll
-      for (int c = 0; c < MH_M; ++c) {
-        fx[c] = valid ? __ldg(a.feats + (size_t)n * MH_M + c) : 0.f;
-        dfa[c] = 0.f;
-      }
-    }
-    mh_stage_group(a, 0, sB + (it & 1u) * MH_B_BYTES, reinterpret_cast<MhConst *>(sCraw + (it & 1u) * MH_C_BYTES), tid);
-    mh_sync_for_mma();
-    if (tid == 0) issue(it);
-
-    for (int g = 0; g < G; ++g) {
-      const uint32_t cur = it + (uint32_t)g, buf = cur & 1u;
-      // map entries (and upstream gradients) of this warp's 4 queries, in flight while the product runs
-      float gv[4], dl[4];
-#pragma unroll
-      for (int i = 0; i < 4; ++i) {
-        const int q = g * MH_QG + (int)qq * 4 + i;
-        const bool live = valid && q < a.Q;
-        gv[i] = live ? __ldg(a.geo + (size_t)q * a.N + n) : 0.f;
-        dl[i] = BWD && live ? __ldg(a.dlogit + (size_t)q * a.N + n) : 0.f;
-      }
-      if (g + 1 < G) {
-        mh_stage_group(a, g + 1, sB + (buf ^ 1u) * MH_B_BYTES, reinterpret_cast<MhConst *>(sCraw + (buf ^ 1u) * MH_C_BYTES), tid);
-        mh_sync_for_mma();
-        if (tid == 0) issue(cur + 1);
-      }
-      mbar_wait(buf ? mbar1 : mbar0, (cur >> 1) & 1u);
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-      const MhConst *sc = reinterpret_cast<const MhConst *>(sCraw + buf * MH_C_BYTES);
-#pragma unroll
-      for (int i = 0; i < 4; ++i) {
-        const int ql = (int)qq * 4 + i, q = g * MH_QG + ql;
-        float d[16];
-        tmem_ld16(t_lane + buf * MH_COLS + (uint32_t)i * 16u, d);  // every lane: .sync.aligned
-        if (q >= a.Q) continue;  // warp-uniform
-        const float4 sd = sc->seed[ql];
-        const bool un = gv[i] < 0.f;
-        const float r0 = mask_push(__fsub_rn(sd.x, px), sd.w, un), r1 = mask_push(__fsub_rn(sd.y, py), sd.w, un),
-                    r2 = mask_push(__fsub_rn(sd.z, pz), sd.w, un);
-        if (!BWD) {
-          float o = sc->b1[ql];
-#pragma unroll
-          for (int j = 0; j < MH_M; ++j) {
-            const int col = ql * MH_M + j;
-            o = __fmaf_rn(sc->w1[col], mh_relu(mh_hidden(d[j], sc->wr[col], r0, r1, r2)), o);
-          }
-          if (valid) __stcs(a.out + (size_t)q * a.N + n, o);
-        } else {
-          const float gl = dl[i];
-          float grh[MH_M], dh[MH_M];
-#pragma unroll
-          for (int j = 0; j < MH_M; ++j) {
-            const int col = ql * MH_M + j;
-            const float h = mh_hidden(d[j], sc->wr[col], r0, r1, r2);
-            grh[j] = __fmul_rn(gl, mh_relu(h));
-            dh[j] = h <= 0.f ? 0.f : __fmul_rn(gl, sc->w1[col]);  // torch's ReLU backward: a NaN h passes g
-          }
-          float *dst = sPart + ((size_t)lq * MH_QG + ql) * MH_NPART;
-          // dw1, db0, dw0 coordinate part (and db1): four channels j per 32-value chunk
-#pragma unroll
-          for (int j4 = 0; j4 < MH_M; j4 += 4) {
-            float v[32];
-#pragma unroll
-            for (int jj = 0; jj < 4; ++jj) {
-              const float x = dh[j4 + jj];
-              v[jj * 8 + 0] = grh[j4 + jj];
-              v[jj * 8 + 1] = x;
-              v[jj * 8 + 2] = __fmul_rn(x, r0);
-              v[jj * 8 + 3] = __fmul_rn(x, r1);
-              v[jj * 8 + 4] = __fmul_rn(x, r2);
-              v[jj * 8 + 5] = (j4 + jj == 0) ? gl : 0.f;
-              v[jj * 8 + 6] = 0.f;
-              v[jj * 8 + 7] = 0.f;
-            }
-            dst[256 + j4 * 8 + lane] = mh_warp_reduce32(v, lane);
-          }
-          // dw0 feature part: two channels j per chunk; dfeats += dh w0f in fixed (q, j) order
-#pragma unroll
-          for (int jp = 0; jp < MH_M; jp += 2) {
-            float v[32];
-#pragma unroll
-            for (int jj = 0; jj < 2; ++jj) {
-              const int row = ql * MH_M + jp + jj;
-#pragma unroll
-              for (int c4 = 0; c4 < MH_M; c4 += 4) {
-                const float4 w = *reinterpret_cast<const float4 *>(sB + buf * MH_B_BYTES + sw128_off<MH_COLS>(row, c4));
-                dfa[c4 + 0] = __fmaf_rn(dh[jp + jj], w.x, dfa[c4 + 0]);
-                dfa[c4 + 1] = __fmaf_rn(dh[jp + jj], w.y, dfa[c4 + 1]);
-                dfa[c4 + 2] = __fmaf_rn(dh[jp + jj], w.z, dfa[c4 + 2]);
-                dfa[c4 + 3] = __fmaf_rn(dh[jp + jj], w.w, dfa[c4 + 3]);
-              }
-#pragma unroll
-              for (int c = 0; c < MH_M; ++c) v[jj * 16 + c] = __fmul_rn(dh[jp + jj], fx[c]);
-            }
-            dst[jp * 16 + lane] = mh_warp_reduce32(v, lane);
-          }
-        }
-      }
-      // TMEM buffer, constants (and partial sums) of this group are free once every thread is past this point
-      asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-      __syncthreads();
-      if (BWD) {  // the tile's sums over its four lane quarters, added to this CTA's partials in tile order
-        for (int e = (int)tid; e < MH_QG * MH_NPART; e += MH_THREADS) {
-          const int ql = e / MH_NPART, q = g * MH_QG + ql;
-          if (q >= a.Q) continue;
-          float s = sPart[e];
-          s = __fadd_rn(s, sPart[MH_QG * MH_NPART + e]);
-          s = __fadd_rn(s, sPart[2 * MH_QG * MH_NPART + e]);
-          s = __fadd_rn(s, sPart[3 * MH_QG * MH_NPART + e]);
-          float *pp = part + (size_t)g * MH_QG * MH_NPART + e;
-          *pp = first_tile ? s : __fadd_rn(*pp, s);
-        }
-        __syncthreads();
-      }
-    }
-    it += (uint32_t)G;
-    if (BWD) {  // dfeats of the tile: the four query quarters summed in order
-      float *sD = sPart;
-#pragma unroll
-      for (int c = 0; c < MH_M; ++c) sD[((size_t)qq * MH_TILE + p) * MH_M + c] = dfa[c];
-      __syncthreads();
-      for (int e = (int)tid; e < MH_TILE * MH_M; e += MH_THREADS) {
-        const int pr = e / MH_M, nr = tile * MH_TILE + pr;
-        if (nr >= a.N) continue;
-        float s = sD[e];
-        s = __fadd_rn(s, sD[MH_TILE * MH_M + e]);
-        s = __fadd_rn(s, sD[2 * MH_TILE * MH_M + e]);
-        s = __fadd_rn(s, sD[3 * MH_TILE * MH_M + e]);
-        a.dfeats[(size_t)nr * MH_M + (e - pr * MH_M)] = s;
-      }
-      __syncthreads();
-    }
-    first_tile = false;
+#include "gf_mask_head_tile.cuh"
   }
   asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
   __syncthreads();
@@ -327,15 +180,9 @@ __global__ void __launch_bounds__(MH_THREADS, 1) mask_head_kernel(const MhArgs a
   }
 }
 
-// the weight gradients: per (query, partial) the CTAs' partial sums in CTA order, scattered to the callers' layouts
-__global__ void __launch_bounds__(256) mask_head_bwd_finish_kernel(const float *__restrict__ part, int nparts, int Q,
-                                                                   float *__restrict__ dw0, float *__restrict__ db0,
-                                                                   float *__restrict__ dw1, float *__restrict__ db1) {
-  const int e = blockIdx.x * blockDim.x + threadIdx.x;
-  if (e >= Q * MH_NPART) return;
-  float s = 0.f;
-  for (int b = 0; b < nparts; ++b) s = __fadd_rn(s, part[(size_t)b * Q * MH_NPART + e]);
-  const int q = e / MH_NPART, k = e - q * MH_NPART;
+// partial sum k of query q (the layout of mask_head_kernel<true>'s partials) to the callers' gradient layouts
+__device__ __forceinline__ void mh_scatter_grad(float s, int q, int k, float *__restrict__ dw0, float *__restrict__ db0,
+                                                float *__restrict__ dw1, float *__restrict__ db1) {
   if (k < 256) {
     const int j = k >> 4, c = k & 15;
     dw0[((size_t)q * MH_M + j) * MH_CIN + 3 + c] = s;
@@ -349,6 +196,126 @@ __global__ void __launch_bounds__(256) mask_head_bwd_finish_kernel(const float *
   else if (t == 5 && j == 0) db1[q] = s;
 }
 
+// the weight gradients: per (query, partial) the CTAs' partial sums in CTA order, scattered to the callers' layouts
+__global__ void __launch_bounds__(256) mask_head_bwd_finish_kernel(const float *__restrict__ part, int nparts, int Q,
+                                                                   float *__restrict__ dw0, float *__restrict__ db0,
+                                                                   float *__restrict__ dw1, float *__restrict__ db1) {
+  const int e = blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= Q * MH_NPART) return;
+  float s = 0.f;
+  for (int b = 0; b < nparts; ++b) s = __fadd_rn(s, part[(size_t)b * Q * MH_NPART + e]);
+  const int q = e / MH_NPART, k = e - q * MH_NPART;
+  mh_scatter_grad(s, q, k, dw0, db0, dw1, db1);
+}
+
+// ---- ragged batches: up to MH_BATCH_MAX scenes in one launch ------------------------------------------------------
+// The tiles of all scenes form one space: scene b owns the global tiles [tile0[b], tile0[b+1]), its tile i holding
+// points 128 i.. of the scene (a tile never straddles two scenes).  CTA c takes the contiguous tiles
+// [mh_range(c), mh_range(c + 1)).  The backward keeps one partial row per (CTA, scene) segment: the CTAs whose range
+// meets scene b are cfirst[b].. in order, and their segments are seg0[b].. in the same order, at most
+// grid + B - 1 segments in all.
+struct MhBatchArgs {
+  const float *geo[MH_BATCH_MAX];  // scene b's (Q, N_b) maps
+  int off[MH_BATCH_MAX + 1];       // offsets: scene b is points off[b] .. off[b+1] of the flat arrays
+  int tile0[MH_BATCH_MAX + 1];
+  int seg0[MH_BATCH_MAX + 1];
+  int cfirst[MH_BATCH_MAX];
+  int B, Q;
+  const float *feats, *coords;     // (sum N, 16), (sum N, 3)
+  const float *w0, *b0, *w1, *b1;  // stacked: scene b's queries are rows b*Q ..
+  const float *seed_xyz;           // (B, Q, 3)
+  const uint32_t *rowmax, *gmax;   // (B, Q), (B): each scene's own maximum
+  float *out;                      // scene b's (Q, N_b) block at Q * off[b]
+  const float *dlogit;             // as out
+  float *dfeats;                   // (sum N, 16)
+  float *part;                     // (segments, Q, 384)
+};
+
+__host__ __device__ __forceinline__ int mh_range(int c, int T, int grid) { return (int)((long long)c * T / grid); }
+
+// mask_head_kernel<BWD> over the tiles of a batch; each tile runs the single-scene kernel's tile body on its scene
+template <bool BWD>
+__global__ void __launch_bounds__(MH_THREADS, 1) mask_head_batch_kernel(const __grid_constant__ MhBatchArgs ba) {
+  extern __shared__ unsigned char mh_smem_raw[];
+  __shared__ __align__(8) unsigned long long s_mbar[2];
+  __shared__ uint32_t s_tmem;
+  const unsigned tid = threadIdx.x, warp = tid >> 5, lane = tid & 31u;
+  const unsigned lq = warp & 3u, qq = warp >> 2;
+  unsigned char *smem = reinterpret_cast<unsigned char *>((reinterpret_cast<uintptr_t>(mh_smem_raw) + 1023) & ~(uintptr_t)1023);
+  unsigned char *sA = smem, *sB = sA + MH_A_BYTES, *sCraw = sB + 2 * MH_B_BYTES;
+  float *sPart = reinterpret_cast<float *>(sCraw + 2 * MH_C_BYTES);  // BWD only
+  const uint32_t mbar0 = smem_u32(&s_mbar[0]), mbar1 = smem_u32(&s_mbar[1]);
+  if (warp == 0) {
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 512;" ::"r"(smem_u32(&s_tmem)) : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+  }
+  if (tid == 0) {
+    asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(mbar0) : "memory");
+    asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(mbar1) : "memory");
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+  }
+  mh_sync_for_mma();
+  const uint32_t tmem = s_tmem;
+  const uint32_t t_lane = tmem + ((lq * 32u) << 16) + qq * 64u;
+  const uint32_t sA_s = smem_u32(sA), sB_s = smem_u32(sB);
+  const int Q = ba.Q, G = (Q + MH_QG - 1) / MH_QG, T = ba.tile0[ba.B];
+
+  auto issue = [&](uint32_t k) {
+    const uint32_t buf = k & 1u;
+#pragma unroll
+    for (int kk = 0; kk < 2; ++kk)
+      umma_tf32<MH_IDESC>(tmem + buf * MH_COLS, umma_desc(sA_s + kk * 32), umma_desc(sB_s + buf * MH_B_BYTES + kk * 32),
+                          kk > 0);
+    umma_commit(buf ? mbar1 : mbar0);
+  };
+
+  uint32_t it = 0;
+  const int t0 = mh_range((int)blockIdx.x, T, (int)gridDim.x), t1 = mh_range((int)blockIdx.x + 1, T, (int)gridDim.x);
+  int b = 0;
+  for (int t = t0; t < t1; ++t) {
+    while (t >= ba.tile0[b + 1]) ++b;
+    const int tile = t - ba.tile0[b], n0 = ba.off[b];
+    bool first_tile = t == t0 || tile == 0;  // a new (CTA, scene) segment
+    const size_t qb = (size_t)b * Q;
+    MhArgs a;
+    a.geo = ba.geo[b], a.Q = Q, a.N = ba.off[b + 1] - n0;
+    a.feats = ba.feats + (size_t)n0 * MH_M, a.coords = ba.coords + (size_t)n0 * 3;
+    a.w0 = ba.w0 + qb * MH_M * MH_CIN, a.b0 = ba.b0 + qb * MH_M, a.w1 = ba.w1 + qb * MH_M, a.b1 = ba.b1 + qb;
+    a.seed_xyz = ba.seed_xyz + qb * 3, a.rowmax = ba.rowmax + qb, a.gmax = ba.gmax + b;
+    a.out = BWD ? nullptr : ba.out + (size_t)Q * n0;
+    a.dlogit = BWD ? ba.dlogit + (size_t)Q * n0 : nullptr;
+    a.dfeats = BWD ? ba.dfeats + (size_t)n0 * MH_M : nullptr;
+    a.part = nullptr;
+    float *part = BWD ? ba.part + (size_t)(ba.seg0[b] + (int)blockIdx.x - ba.cfirst[b]) * Q * MH_NPART : nullptr;
+#include "gf_mask_head_tile.cuh"
+  }
+  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  __syncthreads();
+  if (warp == 0) {
+    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" ::"r"(tmem) : "memory");
+  }
+}
+
+struct MhSegments {
+  int seg0[MH_BATCH_MAX + 1];
+};
+
+// the weight gradients of a batch: per (scene, query, partial) the scene's segments summed in CTA order
+__global__ void __launch_bounds__(256) mask_head_batch_bwd_finish_kernel(const float *__restrict__ part,
+                                                                         const __grid_constant__ MhSegments sg, int B,
+                                                                         int Q, float *__restrict__ dw0,
+                                                                         float *__restrict__ db0,
+                                                                         float *__restrict__ dw1,
+                                                                         float *__restrict__ db1) {
+  const int e = blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= B * Q * MH_NPART) return;
+  const int qg = e / MH_NPART, k = e - qg * MH_NPART, b = qg / Q, q = qg - b * Q;
+  float s = 0.f;
+  for (int seg = sg.seg0[b]; seg < sg.seg0[b + 1]; ++seg) s = __fadd_rn(s, part[((size_t)seg * Q + q) * MH_NPART + k]);
+  mh_scatter_grad(s, qg, k, dw0, db0, dw1, db1);
+}
+
 static int mh_set_smem() {
   static int done[64] = {0};
   int dev = 0;
@@ -357,6 +324,9 @@ static int mh_set_smem() {
   if (!__atomic_load_n(&done[dev], __ATOMIC_ACQUIRE)) {
     GF_CUDA(cudaFuncSetAttribute(mask_head_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, MH_SMEM));
     GF_CUDA(cudaFuncSetAttribute(mask_head_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, MH_BWD_SMEM));
+    GF_CUDA(cudaFuncSetAttribute(mask_head_batch_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, MH_SMEM));
+    GF_CUDA(cudaFuncSetAttribute(mask_head_batch_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                 MH_BWD_SMEM));
     __atomic_store_n(&done[dev], 1, __ATOMIC_RELEASE);
   }
   return GF_OK;
@@ -462,6 +432,151 @@ extern "C" int gf_mask_head_logits_backward(const float *geo, const float *feats
   mask_head_kernel<true><<<grid, MH_THREADS, MH_BWD_SMEM, st>>>(a);
   GF_LAUNCHED();
   mask_head_bwd_finish_kernel<<<(Q * MH_NPART + 255) / 256, 256, 0, st>>>(a.part, grid, Q, dw0, db0, dw1, db1);
+  GF_LAUNCHED();
+  return GF_OK;
+}
+
+// ---- ragged batches -------------------------------------------------------------------------------------------------
+// the sizes of a batched call: 1..32 scenes, offsets from 0 rising strictly (no empty scene), Q >= 1
+static int mh_batch_sizes(const int *offsets, int B, int Q, const char *who) {
+  GF_CHECK_ARG(B >= 1 && B <= MH_BATCH_MAX, "%s: B=%d (1 to %d scenes per call)", who, B, MH_BATCH_MAX);
+  GF_CHECK_ARG(Q >= 1, "%s: Q=%d (at least one query)", who, Q);
+  GF_CHECK_ARG((long long)B * Q * MH_NPART < (1LL << 31), "%s: B*Q=%lld queries is too many", who, (long long)B * Q);
+  GF_CHECK_ARG(offsets, "%s: null pointer (offsets)", who);
+  GF_CHECK_ARG(offsets[0] == 0, "%s: offsets[0]=%d (must start at 0)", who, offsets[0]);
+  for (int b = 0; b < B; ++b)
+    GF_CHECK_ARG(offsets[b + 1] > offsets[b], "%s: scene %d is empty (offsets must rise strictly)", who, b);
+  return GF_OK;
+}
+
+// the partition of a batched call's tiles over the CTAs (see MhBatchArgs) and its segment count
+static void mh_batch_plan(const int *offsets, int B, int Q, MhBatchArgs *a, int *grid, int *nseg) {
+  a->B = B, a->Q = Q;
+  a->tile0[0] = 0;
+  for (int b = 0; b <= B; ++b) a->off[b] = offsets[b];
+  for (int b = 0; b < B; ++b) a->tile0[b + 1] = a->tile0[b] + (offsets[b + 1] - offsets[b] + MH_TILE - 1) / MH_TILE;
+  const int T = a->tile0[B], g = T < num_sms() ? T : num_sms();
+  auto owner = [&](int t) { return (int)(((long long)(t + 1) * g - 1) / T); };  // the c with t in [mh_range(c), ..)
+  a->seg0[0] = 0;
+  for (int b = 0; b < B; ++b) {
+    a->cfirst[b] = owner(a->tile0[b]);
+    a->seg0[b + 1] = a->seg0[b] + owner(a->tile0[b + 1] - 1) - a->cfirst[b] + 1;
+  }
+  *grid = g;
+  *nseg = a->seg0[B];
+}
+
+// the workspace of a batched call: the row maxima (B, Q) with each scene's maximum (B) right after them (one zero
+// fill clears both), and for the backward one partial row per segment
+struct MhBatchLayout {
+  uint32_t *rowmax, *gmax;
+  float *part;
+};
+static Arena mh_batch_carve(void *workspace, size_t workspace_bytes, int B, int Q, int nseg, bool backward,
+                            MhBatchLayout *l) {
+  Arena a(workspace, workspace_bytes);
+  uint32_t *r = a.take<uint32_t>((size_t)B * Q + B);
+  l->rowmax = r, l->gmax = r ? r + (size_t)B * Q : nullptr;
+  l->part = backward ? a.take<float>((size_t)nseg * Q * MH_NPART) : nullptr;
+  return a;
+}
+
+static size_t mh_batch_workspace_bytes(const int *offsets, int B, int Q, bool backward) {
+  if (mh_batch_sizes(offsets, B, Q, "mask_head_batch_workspace_bytes")) return 0;
+  MhBatchArgs a;
+  int grid, nseg;
+  mh_batch_plan(offsets, B, Q, &a, &grid, &nseg);
+  MhBatchLayout l;
+  return mh_batch_carve(nullptr, 0, B, Q, nseg, backward, &l).off;
+}
+
+extern "C" size_t gf_mask_head_batch_workspace_bytes(const int *offsets, int B, int Q) {
+  return mh_batch_workspace_bytes(offsets, B, Q, false);
+}
+
+extern "C" size_t gf_mask_head_batch_backward_workspace_bytes(const int *offsets, int B, int Q) {
+  return mh_batch_workspace_bytes(offsets, B, Q, true);
+}
+
+// arguments common to both batched entries
+static int mh_batch_check(const float *const *geo, const int *offsets, int B, int Q, int m, const float *feats,
+                          const float *w0, const float *b0, const float *w1, const float *b1, const float *coords,
+                          const float *seed_xyz, const char *who) {
+  int rc = mh_batch_sizes(offsets, B, Q, who);
+  if (rc) return rc;
+  GF_CHECK_ARG(m == MH_M, "%s: m=%d (only m = 16 is supported)", who, m);
+  GF_CHECK_ARG(geo && feats && w0 && b0 && w1 && b1 && coords && seed_xyz, "%s: null pointer", who);
+  for (int b = 0; b < B; ++b) GF_CHECK_ARG(geo[b], "%s: null pointer (geo[%d])", who, b);
+  return GF_OK;
+}
+
+// the plan, the carved workspace and the row maxima, once every argument has been checked
+static int mh_batch_prepare(MhBatchArgs &a, int *grid, MhBatchLayout *l, const float *const *geo, const int *offsets,
+                            int B, int Q, const float *feats, const float *w0, const float *b0, const float *w1,
+                            const float *b1, const float *coords, const float *seed_xyz, const float *row_max,
+                            void *workspace, size_t workspace_bytes, bool backward, cudaStream_t st, const char *who) {
+  int nseg;
+  mh_batch_plan(offsets, B, Q, &a, grid, &nseg);
+  const Arena ar = mh_batch_carve(workspace, workspace_bytes, B, Q, nseg, backward, l);
+  if (!ar.ok) return ar.fail(who);
+  int rc = mh_set_smem();
+  if (rc) return rc;
+  MaskMaps maps;
+  maps.B = B, maps.Q = Q;
+  for (int b = 0; b < B; ++b) maps.geo[b] = geo[b], maps.N[b] = offsets[b + 1] - offsets[b], a.geo[b] = geo[b];
+  if ((rc = bias_mask_rowmax_batch(maps, row_max, l->rowmax, l->gmax, st))) return rc;
+  a.feats = feats, a.coords = coords, a.w0 = w0, a.b0 = b0, a.w1 = w1, a.b1 = b1, a.seed_xyz = seed_xyz;
+  a.rowmax = l->rowmax, a.gmax = l->gmax;
+  a.out = nullptr, a.dlogit = nullptr, a.dfeats = nullptr, a.part = l->part;
+  return GF_OK;
+}
+
+extern "C" int gf_mask_head_logits_batch(const float *const *geo, const int *offsets, int B, int Q, int m,
+                                         const float *feats, const float *w0, const float *b0, const float *w1,
+                                         const float *b1, const float *coords, const float *seed_xyz,
+                                         const float *row_max, float *out, void *workspace, size_t workspace_bytes,
+                                         void *stream) {
+  const char *who = "mask_head_batch";
+  int rc = mh_batch_check(geo, offsets, B, Q, m, feats, w0, b0, w1, b1, coords, seed_xyz, who);
+  if (rc) return rc;
+  GF_CHECK_ARG(out, "%s: null pointer (out)", who);
+  cudaStream_t st = (cudaStream_t)stream;
+  MhBatchArgs a;
+  MhBatchLayout l;
+  int grid;
+  if ((rc = mh_batch_prepare(a, &grid, &l, geo, offsets, B, Q, feats, w0, b0, w1, b1, coords, seed_xyz, row_max,
+                             workspace, workspace_bytes, false, st, who)))
+    return rc;
+  a.out = out;
+  mask_head_batch_kernel<false><<<grid, MH_THREADS, MH_SMEM, st>>>(a);
+  GF_LAUNCHED();
+  return GF_OK;
+}
+
+extern "C" int gf_mask_head_logits_batch_backward(const float *const *geo, const int *offsets, int B, int Q, int m,
+                                                  const float *feats, const float *w0, const float *b0,
+                                                  const float *w1, const float *b1, const float *coords,
+                                                  const float *seed_xyz, const float *row_max, const float *dlogit,
+                                                  float *dfeats, float *dw0, float *db0, float *dw1, float *db1,
+                                                  void *workspace, size_t workspace_bytes, void *stream) {
+  const char *who = "mask_head_batch_backward";
+  int rc = mh_batch_check(geo, offsets, B, Q, m, feats, w0, b0, w1, b1, coords, seed_xyz, who);
+  if (rc) return rc;
+  GF_CHECK_ARG(dlogit && dfeats && dw0 && db0 && dw1 && db1, "%s: null pointer", who);
+  cudaStream_t st = (cudaStream_t)stream;
+  MhBatchArgs a;
+  MhBatchLayout l;
+  int grid;
+  if ((rc = mh_batch_prepare(a, &grid, &l, geo, offsets, B, Q, feats, w0, b0, w1, b1, coords, seed_xyz, row_max,
+                             workspace, workspace_bytes, true, st, who)))
+    return rc;
+  a.dlogit = dlogit, a.dfeats = dfeats;
+  mask_head_batch_kernel<true><<<grid, MH_THREADS, MH_BWD_SMEM, st>>>(a);
+  GF_LAUNCHED();
+  MhSegments sg;
+  for (int b = 0; b <= B; ++b) sg.seg0[b] = a.seg0[b];
+  mask_head_batch_bwd_finish_kernel<<<(B * Q * MH_NPART + 255) / 256, 256, 0, st>>>(l.part, sg, B, Q, dw0, db0, dw1,
+                                                                                    db1);
   GF_LAUNCHED();
   return GF_OK;
 }

@@ -174,11 +174,22 @@ class FewShotForward(nn.Module):
 
     # ---- :302-360, :263-300 -----------------------------------------------------------------------------------
     def mask_logits(self, geo_dists, dec_out, mask_features, locs, query_locs, row_max, impl):
-        """dec_out (Q,B,d) -> list of (Q, N_b) logits"""
+        """dec_out (Q,B,d) -> list of (Q, N_b) logits; "b200" computes a batch of two or more scenes in one call of
+        mask_head.mask_heads_forward_batch, a single scene with mask_head.mask_heads_forward"""
         Qn, B, _ = dec_out.shape
         pk = dec_out.transpose(0, 1).flatten(0, 1)
         controllers = self.controller(self.before_embedding_tower(pk.unsqueeze(2))).squeeze(2).reshape(B, Qn, -1)
         m = self.m
+        if impl == "b200" and B >= 2:  # every scene's logits in one launch, the weights stacked scene after scene
+            w0, w1, b0, b1 = torch.split_with_sizes(controllers, self.weight_nums + self.bias_nums, dim=2)
+            offsets = [0]
+            for b in range(B):
+                offsets.append(offsets[-1] + geo_dists[b].shape[1])
+            return mh.mask_heads_forward_batch(
+                [geo_dists[b] for b in range(B)], torch.cat([mask_features[b] for b in range(B)]), offsets,
+                [w0.reshape(B * Qn * m, -1, 1), w1.reshape(B * Qn, -1, 1)], [b0.reshape(B * Qn * m), b1.reshape(B * Qn)],
+                torch.cat([locs[b] for b in range(B)]), query_locs.contiguous(),
+                row_max=torch.stack([row_max[b] for b in range(B)]) if row_max is not None else None)
         out = []
         for b in range(B):
             w0, w1, b0, b1 = torch.split_with_sizes(controllers[b], self.weight_nums + self.bias_nums, dim=1)

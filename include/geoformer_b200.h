@@ -246,6 +246,28 @@ int gf_mask_head_logits_backward(const float *geo, const float *feats, const flo
                                  float *dw0, float *db0, float *dw1, float *db1, void *workspace,
                                  size_t workspace_bytes, void *stream);
 
+/* A ragged batch of B <= 32 scenes in one launch (forward) or two (backward), plus the row maxima's one or two.
+ * geo: HOST array of B device pointers to contiguous (Q, N_b) maps; offsets: HOST array of B+1 ints from 0, rising
+ * strictly (no empty scene), N_b = offsets[b+1] - offsets[b]; feats (sum N, m) and coords (sum N, 3) flat; the
+ * weights stacked, scene b's queries being rows b*Q..: w0 (B*Q*m, m+3), b0 (B*Q*m), w1 (B*Q, m), b1 (B*Q);
+ * seed_xyz (B, Q, 3); row_max (B, Q) or NULL.  out (and dlogit) hold scene b's (Q, N_b) block at Q * offsets[b].
+ * Every logit and dfeats are bitwise those of gf_mask_head_logits(_backward) on the scene alone; row maxima that
+ * are negative take their own scene's maximum.  The weight gradients sum each CTA's tiles of a scene and then those
+ * partial sums in CTA order: deterministic, though grouped differently from the single-scene call.  Every argument
+ * is checked before any work is enqueued; the _workspace_bytes functions return 0 for arguments the entries refuse. */
+size_t gf_mask_head_batch_workspace_bytes(const int *offsets, int B, int Q);
+int gf_mask_head_logits_batch(const float *const *geo, const int *offsets, int B, int Q, int m, const float *feats,
+                              const float *w0, const float *b0, const float *w1, const float *b1, const float *coords,
+                              const float *seed_xyz, const float *row_max, float *out, void *workspace,
+                              size_t workspace_bytes, void *stream);
+size_t gf_mask_head_batch_backward_workspace_bytes(const int *offsets, int B, int Q);
+int gf_mask_head_logits_batch_backward(const float *const *geo, const int *offsets, int B, int Q, int m,
+                                       const float *feats, const float *w0, const float *b0, const float *w1,
+                                       const float *b1, const float *coords, const float *seed_xyz,
+                                       const float *row_max, const float *dlogit, float *dfeats, float *dw0,
+                                       float *db0, float *dw1, float *db1, void *workspace, size_t workspace_bytes,
+                                       void *stream);
+
 /* ---- set_aggregator.mlp fused with its grouping (SURVEY 8(f) rank 3) --------------------------------------------
  * lib/pointnet2/pointnet2_modules.py:200-249 + QueryAndGroup.forward (pointnet2_utils.py:303-356) + SharedMLP
  * (pytorch_utils.py:9-32): per centre j and ball-query neighbour s the input [(xyz[idx] - new_xyz[j]) / radius |
