@@ -49,6 +49,9 @@ SIGNATURES = {
     "gf_knn_batch": (c_int, [_P, _P, c_int, c_int, c_int, _P, _P, _P, c_size_t, _P]),
     "gf_geodesic_workspace_bytes": (c_size_t, [c_int, c_int, c_int]),
     "gf_geodesic": (c_int, [_P, _P, c_int, c_int, c_int, _P, c_int, c_float, c_int, _P, _P, _P, _P, c_size_t, _P]),
+    "gf_geodesic_batch_workspace_bytes": (c_size_t, [_P, c_int, c_int, c_int]),
+    "gf_geodesic_batch": (c_int, [_P, _P, _P, c_int, _P, c_int, c_int, _P, c_int, c_float, c_int, _P, _P, _P, _P,
+                                  c_size_t, _P]),
     "gf_bias_workspace_bytes": (c_size_t, [c_int, c_int]),
     "gf_bias_decoder": (c_int, [_P, _P, _P, _P, _P, c_int, c_int, c_int, _P, _P, c_size_t, _P]),
     "gf_bias_decoder_fourier": (c_int, [_P, _P, _P, _P, _P, c_int, c_int, c_int, _P, c_int, c_int, _P, _P, _P, _P,

@@ -37,6 +37,7 @@
 #include <string.h>
 
 #include "gf_geodesic.cuh"
+#include "gf_knn.cuh"
 
 namespace gf {
 
@@ -76,8 +77,19 @@ __device__ __forceinline__ uint32_t ld_cg_u32(const uint32_t *p) {
 }
 
 // ---- edge packing ---------------------------------------------------------------------------------
-// tgt[p][j], len[p][j] = I[p][1+j], D[p][1+j] if the edge may ever be used (D <= radius, 0 <= I < N;
-// geodesic_utils.py:123,151), else N, 0; column 0 of the kNN result is dropped (:110-111).
+// Edge j < k - 1 of point p is neighbour 1 + j of the kNN result if it may ever be used (D <= radius, 0 <= I < N;
+// geodesic_utils.py:123,151); column 0 is dropped (:110-111).  Returns whether it is, with its target and length.
+template <bool IS64>
+__device__ __forceinline__ bool geo_edge_usable(const float *__restrict__ D, const void *__restrict__ I, int N, int k,
+                                                float radius, int p, int j, int *t, float *w) {
+  const size_t at = (size_t)p * k + 1 + j;
+  const long long ti = IS64 ? ((const long long *)I)[at] : (long long)((const int *)I)[at];
+  const float wi = __ldg(D + at);
+  *t = (int)ti, *w = wi;
+  return wi <= radius && ti >= 0 && ti < N;
+}
+
+// The table of one scene in the original numbering: tgt[p][j], len[p][j] = the usable edge, else N, 0.
 // Row N (the sentinel point used to pad frontier queues) has only edges to N.  KP >= 4 so that a
 // lane can fetch four targets with one 16-byte load.
 template <bool IS64>
@@ -89,16 +101,46 @@ __global__ void geo_pack_edges_kernel(const float *__restrict__ D, const void *_
   for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < total;
        e += (long long)gridDim.x * blockDim.x) {
     const int p = (int)(e >> slot_bits), j = (int)(e & (KP - 1));
-    int to = N;
-    float wo = 0.f;
-    if (j < K && p < N) {
-      const size_t at = (size_t)p * k + 1 + j;
-      const long long t = IS64 ? ((const long long *)I)[at] : (long long)((const int *)I)[at];
-      const float w = __ldg(D + at);
-      if (w <= radius && t >= 0 && t < N) to = (int)t, wo = w;
-    }
+    int to = N, t;
+    float wo = 0.f, w;
+    if (j < K && p < N && geo_edge_usable<IS64>(D, I, N, k, radius, p, j, &t, &w)) to = t, wo = w;
     tgt[e] = enc ? geo_edge_code((unsigned)to) : to;
     len[e] = wo;
+  }
+}
+
+// The tables of a batch of scenes in one launch (blockIdx.y = scene), each in the CELL ORDER of its kNN grid with
+// encoded targets (the format of the batched kernel): row r holds the edges of point order[r], an edge to t is stored
+// as geo_edge_code(rank[t]).  rank / order null: the original numbering (development builds, GF_GEO_ORIGINAL_ORDER).
+struct GeoPackScene {
+  const float *D;
+  const void *I;
+  const int *rank, *order;
+  int *tgt;
+  float *len;
+  int N;
+};
+struct GeoPackArgs {
+  GeoPackScene sc[GEO_BATCH_MAX];
+  int k, slot_bits;
+  float radius;
+};
+template <bool IS64>
+__global__ void __launch_bounds__(256) geo_pack_edges_batch_kernel(const __grid_constant__ GeoPackArgs a) {
+  const GeoPackScene &S = a.sc[blockIdx.y];
+  const int N = S.N, sb = a.slot_bits, KP = 1 << sb, K = a.k - 1;
+  const long long total = ((long long)N + 1) << sb;
+  for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < total;
+       e += (long long)gridDim.x * blockDim.x) {
+    const int r = (int)(e >> sb), j = (int)(e & (KP - 1));
+    int to = N, t;
+    float wo = 0.f, w;
+    if (j < K && r < N) {
+      const int p = S.order ? __ldg(S.order + r) : r;
+      if (geo_edge_usable<IS64>(S.D, S.I, N, a.k, a.radius, p, j, &t, &w)) to = S.rank ? __ldg(S.rank + t) : t, wo = w;
+    }
+    S.tgt[e] = geo_edge_code((unsigned)to);
+    S.len[e] = wo;
   }
 }
 
@@ -1183,4 +1225,105 @@ extern "C" int gf_geodesic_scatter(const float *knn_dist, const void *knn_idx, i
   GF_CHECK_ARG(knn_dist && knn_idx && seeds && geo, "geodesic: null pointer");
   return geodesic_run(knn_dist, knn_idx, idx_is_i64, N, k, seeds, Q, radius, max_step, geo, stats, workspace,
                       workspace_bytes, (cudaStream_t)stream, peer_geo, n_peers);
+}
+
+// ---- a batch of scenes over the caller's kNN graphs -----------------------------------------------------------------
+namespace gf {
+static_assert(KNN_BATCH_MAX == GEO_BATCH_MAX, "one batched call builds the grids of all its scenes at once");
+// The workspace of a batch over given graphs: per scene the workspace of its kNN grid (only its cell-order numbering is
+// used) and its edge table; then the control blocks of the batched build, the scratch of the batched propagation and
+// the statistics of every scene
+struct GraphBatchLayout {
+  Span knn[GEO_BATCH_MAX];
+  GeoEdges edges[GEO_BATCH_MAX];
+  void *knn_ctl;
+  Span scratch;
+  int64_t *stats;
+};
+static Arena graph_batch_carve(void *workspace, size_t workspace_bytes, const int *Ns, int B, int Q, int k,
+                               GraphBatchLayout *l) {
+  Arena a(workspace, workspace_bytes);
+  int maxN = 1;
+  for (int b = 0; b < B; ++b) {
+    l->knn[b] = a.span(knn_grid_workspace_bytes(Ns[b]));
+    geo_edges_carve(a, Ns[b], k, &l->edges[b]);
+    maxN = Ns[b] > maxN ? Ns[b] : maxN;
+  }
+  l->knn_ctl = a.take<char>(knn_ctl_block_bytes(B));
+  l->scratch = a.span(geodesic_batch_scratch_bytes(maxN, (long long)Q * B));
+  l->stats = a.take<int64_t>(2 * (size_t)B);
+  return a;
+}
+}  // namespace gf
+
+extern "C" size_t gf_geodesic_batch_workspace_bytes(const int *Ns, int B, int Q, int k) {
+  if (!Ns || B <= 0 || B > GEO_BATCH_MAX || Q <= 0 || k <= 0 || k > 256) return 0;
+  for (int b = 0; b < B; ++b)
+    if (Ns[b] <= 0) return 0;
+  GraphBatchLayout l;
+  return graph_batch_carve(nullptr, 0, Ns, B, Q, k, &l).off;
+}
+
+extern "C" int gf_geodesic_batch(const float *const *xyz, const float *const *knn_dist, const void *const *knn_idx,
+                                 int idx_is_i64, const int *Ns, int B, int k, const int *const *seeds, int Q,
+                                 float radius, int max_step, float *const *geo, float *const *row_max, int64_t *stats,
+                                 void *workspace, size_t workspace_bytes, void *stream) {
+  GF_CHECK_ARG(xyz && knn_dist && knn_idx && Ns && seeds && geo, "geodesic_batch: null pointer array");
+  GF_CHECK_ARG(B >= 1 && B <= GEO_BATCH_MAX, "geodesic_batch: B=%d outside [1,%d]", B, GEO_BATCH_MAX);
+  GF_CHECK_ARG(Q >= 1 && (long long)Q * B <= 0x7fffffffll, "geodesic_batch: Q=%d outside [1, 2^31 / B]", Q);
+  GF_CHECK_ARG(k >= 1 && k <= 256, "geodesic_batch: k=%d outside [1,256]", k);
+  GF_CHECK_ARG(idx_is_i64 == 0 || idx_is_i64 == 1, "geodesic_batch: idx_is_i64=%d is not 0 or 1", idx_is_i64);
+  for (int b = 0; b < B; ++b) {
+    GF_CHECK_ARG(Ns[b] >= 1 && xyz[b] && knn_dist[b] && knn_idx[b] && seeds[b] && geo[b],
+                 "geodesic_batch: scene %d: empty or null", b);
+    GF_CHECK_ARG(geodesic_edge_format(Ns[b]) == 1,
+                 "geodesic_batch: scene %d has %d points, beyond the on-chip bitmaps of the batched kernel "
+                 "(use gf_geodesic per scene)", b, Ns[b]);
+  }
+  GraphBatchLayout w;
+  const Arena ar = graph_batch_carve(workspace, workspace_bytes, Ns, B, Q, k, &w);
+  if (!ar.ok) return ar.fail("geodesic_batch");
+  cudaStream_t st = (cudaStream_t)stream;
+  int64_t *d_stats = stats ? w.stats : nullptr;
+  if (d_stats) GF_CUDA(cudaMemsetAsync(d_stats, 0, 16 * (size_t)B, st));
+  // The cell-order numbering of every scene: the five build kernels, each launched once over all scenes.  The grid's
+  // cell size depends on k only for the speed of a kNN query, which is not run here (it is tuned up to KNN_MAX_K).
+  KnnBuildScene ks[GEO_BATCH_MAX];
+  KnnGridBuffers gb[GEO_BATCH_MAX];
+  for (int b = 0; b < B; ++b) ks[b] = {xyz[b], Ns[b], w.knn[b].ptr, w.knn[b].bytes};
+#ifndef GF_GEO_ORIGINAL_ORDER
+  int rc = knn_grid_build_batch(ks, B, k < KNN_MAX_K ? k : KNN_MAX_K, w.knn_ctl, st, gb);
+  if (rc) return rc;
+#else
+  int rc = GF_OK;
+  for (int b = 0; b < B; ++b) gb[b].rank = gb[b].order = nullptr;
+#endif
+  // every scene's edge table in its cell order: one launch
+  GeoPackArgs pa;
+  memset(&pa, 0, sizeof(pa));
+  pa.k = k, pa.slot_bits = w.edges[0].slot_bits, pa.radius = radius;
+  long long maxE = 0;
+  GeoSceneDesc desc[GEO_BATCH_MAX];
+  for (int b = 0; b < B; ++b) {
+    pa.sc[b] = {knn_dist[b], knn_idx[b], gb[b].rank, gb[b].order, w.edges[b].tgt, w.edges[b].len, Ns[b]};
+    const long long E = ((long long)Ns[b] + 1) << pa.slot_bits;
+    maxE = E > maxE ? E : maxE;
+    desc[b].tgt = w.edges[b].tgt, desc[b].len = w.edges[b].len, desc[b].seeds = seeds[b], desc[b].geo = geo[b];
+    desc[b].rank = gb[b].rank, desc[b].order = gb[b].order;
+    desc[b].row_max = row_max ? row_max[b] : nullptr;
+    desc[b].stats = d_stats ? d_stats + 2 * b : nullptr;
+    desc[b].N = Ns[b], desc[b].Q = Q;
+  }
+  const long long per_scene = (long long)num_sms() * 16 / B > 1 ? (long long)num_sms() * 16 / B : 1;
+  const long long need = (maxE + 255) / 256;
+  const dim3 grid((unsigned)(need < per_scene ? need : per_scene), (unsigned)B);
+  if (idx_is_i64)
+    geo_pack_edges_batch_kernel<true><<<grid, 256, 0, st>>>(pa);
+  else
+    geo_pack_edges_batch_kernel<false><<<grid, 256, 0, st>>>(pa);
+  GF_LAUNCHED();
+  rc = geodesic_batch_launch(desc, B, k, max_step, w.scratch.ptr, w.scratch.bytes, st);
+  if (rc) return rc;
+  if (stats) GF_CUDA(cudaMemcpyAsync(stats, d_stats, 16 * (size_t)B, cudaMemcpyDeviceToDevice, st));
+  return GF_OK;
 }

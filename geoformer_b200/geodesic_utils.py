@@ -8,7 +8,7 @@ import ctypes
 import torch
 
 from . import _capi as C
-from .guidance import BATCH_MAX_POINTS, geodesic_guidance_batch
+from .guidance import BATCH_MAX, BATCH_MAX_POINTS, _ptr_array, geodesic_guidance_batch
 
 
 class FlatL2Index:
@@ -130,6 +130,72 @@ def geodesic_from_graph(D, I, seeds, radius, max_step, return_stats=False, row_m
     return (geo, stats) if return_stats else geo
 
 
+def geodesic_from_graph_batch(locs, graphs, seeds, radius, max_step, row_max=False, return_stats=False):
+    """geodesic_from_graph for a BATCH of scenes: one library call per <= 32 scenes (gf_geodesic_batch, seven kernels
+    whatever the number of scenes), every map bitwise the one geodesic_from_graph gives for its scene alone.
+    locs: list of (N_b, 3) f32 CUDA tensors.  They only choose the numbering the propagation runs in (the cell order
+    of a kNN grid over them): the maps do not depend on them, the scene's own points make the call fastest.
+    graphs: list of (D (N_b,k) sqrt'ed f32, I (N_b,k) int64 or int32), one k and one index dtype for all.
+    seeds: list of (Q,) int tensors, one Q for all.
+    Returns the list of (Q, N_b) f32 maps, or (maps[, stats (B,2) i64][, row_max list of (Q,) f32]) when asked.
+    Scenes too large for the batched kernel run through geodesic_from_graph one at a time; a scene without points
+    gets a (Q, 0) map (row maxima -1), a call without seeds (0, N_b) maps."""
+    B = len(graphs)
+    C.require(B > 0 and len(locs) == B and len(seeds) == B, "one point set and one seed tensor per graph")
+    dev = graphs[0][0].device
+    k, idt = graphs[0][0].shape[-1], graphs[0][1].dtype
+    C.require(idt in (torch.int64, torch.int32), "I must be int64/int32 CUDA")
+    for x, (D, I) in zip(locs, graphs):
+        C.check_cuda_f32(D, "D")
+        C.check_cuda_f32(x, "locs")
+        C.require(I.is_cuda and I.is_contiguous() and I.dtype == idt, "I must be contiguous CUDA, one dtype for all")
+        C.require(D.dim() == 2 and D.size(1) == k and tuple(I.shape) == tuple(D.shape), "graphs must be (N_b, k), one k")
+        C.require(tuple(x.shape) == (D.size(0), 3) and x.device == dev and D.device == dev and I.device == dev,
+                  "locs must be (N_b, 3), on the graphs' device")
+    seeds = [s.to(device=dev, dtype=torch.int32).contiguous() for s in seeds]
+    Q = seeds[0].numel()
+    C.require(all(s.numel() == Q for s in seeds), "one (Q,) seed tensor per scene, one Q for all")
+    Ns = [D.size(0) for D, _ in graphs]
+    geo = [torch.empty((Q, n), dtype=torch.float32, device=dev) for n in Ns]
+    rmax = [torch.full((Q,), -1.0, dtype=torch.float32, device=dev) for _ in Ns] if row_max else None
+    stats = torch.zeros((B, 2), dtype=torch.int64, device=dev) if return_stats else None
+    batch = [b for b in range(B) if Q > 0 and 0 < Ns[b] <= BATCH_MAX_POINTS]
+    for b in range(B):
+        if Q > 0 and Ns[b] > BATCH_MAX_POINTS:
+            out = geodesic_from_graph(*graphs[b], seeds[b], radius, max_step, return_stats=return_stats,
+                                      row_max=rmax[b] if rmax else None)
+            geo[b] = out[0] if return_stats else out
+            if return_stats:
+                stats[b] = out[1]
+    L = C.lib()
+    with torch.cuda.device(dev):
+        st = C.stream_of(dev)
+        for b0 in range(0, len(batch), BATCH_MAX):
+            sub = batch[b0:b0 + BATCH_MAX]
+            n = len(sub)
+            Nc = (ctypes.c_int * n)(*[Ns[b] for b in sub])
+            nbytes = L.gf_geodesic_batch_workspace_bytes(Nc, n, Q, k)
+            C.require(nbytes > 0, "geodesic_batch: bad sizes")
+            ws = C.workspace.get(dev, "geodesic_batch", nbytes)
+            st_call = torch.empty((n, 2), dtype=torch.int64, device=dev) if return_stats else None
+            C.check(L.gf_geodesic_batch(_ptr_array([locs[b] for b in sub]), _ptr_array([graphs[b][0] for b in sub]),
+                                        _ptr_array([graphs[b][1] for b in sub]), 1 if idt == torch.int64 else 0, Nc,
+                                        n, k, _ptr_array([seeds[b] for b in sub]), Q, ctypes.c_float(float(radius)),
+                                        int(max_step), _ptr_array([geo[b] for b in sub]),
+                                        _ptr_array([rmax[b] for b in sub]) if rmax else None, C.ptr(st_call),
+                                        C.ptr(ws), nbytes, st), "geodesic_batch")
+            if return_stats:
+                stats.index_copy_(0, torch.tensor(sub, device=dev), st_call)
+    if not (return_stats or row_max):
+        return geo
+    out = [geo]
+    if return_stats:
+        out.append(stats)
+    if row_max:
+        out.append(rmax)
+    return tuple(out)
+
+
 def geodesic_from_points(locs, seeds, neighbor, radius, max_step, return_graph=False, return_stats=False,
                          row_max=None, ws_tag="guidance"):
     """kNN graph + propagation of one scene in one library call (the body of the reference loop,
@@ -173,6 +239,7 @@ def cal_geodesic_vectorize(gpu_index, pre_enc_inds, locs_float_, batch_offset_, 
     dev = locs_float_.device
     geo_dists = [None] * batch_size
     batch = []  # (b, points, seeds) of the scenes that go through the batched library call
+    graphs = []  # (b, points, (D, I), seeds) of the scenes whose graph comes from the caller's index
     for b in range(batch_size):
         start, end = int(offsets[b]), int(offsets[b + 1])
         seeds = pre_enc_inds[b][:n_queries]
@@ -185,11 +252,12 @@ def cal_geodesic_vectorize(gpu_index, pre_enc_inds, locs_float_, batch_offset_, 
         elif fused:
             geo_dists[b] = geodesic_from_points(locs_b, seeds, neighbor, radius, max_step)
         else:
-            D, I = find_knn(gpu_index, locs_b, neighbor=neighbor)
-            geo_dists[b] = geodesic_from_graph(D, I, seeds, radius, max_step)
+            # the index protocol answers one scene per call (:18-21); the graphs are propagated together below
+            graphs.append((b, locs_b, find_knn(gpu_index, locs_b, neighbor=neighbor), seeds))
     # The scenes of a batch are independent (the reference loops over them, :98): their graphs are built side by
     # side and ALL their (scene, seed) pairs are propagated by one launch (gf_guidance_batch) -- the per-seed runs
-    # are chains of dependent latencies, so the GPU is only filled by many of them at once.
+    # are chains of dependent latencies, so the GPU is only filled by many of them at once.  Graphs from the caller's
+    # index take the same launch after one pass that packs them all (gf_geodesic_batch).
     # Scenes with the same number of seeds share a call (pre_enc_inds is one (B, >= n_queries) tensor: all of them).
     groups = {}
     for b, locs_b, seeds in batch:
@@ -198,6 +266,19 @@ def cal_geodesic_vectorize(gpu_index, pre_enc_inds, locs_float_, batch_offset_, 
         _, geos = geodesic_guidance_batch([x for _, x, _ in items], q_n, neighbor, radius, max_step,
                                           seeds=[s for _, _, s in items])
         for (b, _, _), g in zip(items, geos):
+            geo_dists[b] = g
+    groups = {}
+    for item in graphs:
+        groups.setdefault(item[3].numel(), []).append(item)
+    for items in groups.values():
+        if len(items) == 1:
+            # one scene: the grid build of the batched call costs more than its cell order saves (DESIGN 4.3)
+            b, _, (D, I), seeds = items[0]
+            geo_dists[b] = geodesic_from_graph(D, I, seeds, radius, max_step)
+            continue
+        geos = geodesic_from_graph_batch([x for _, x, _, _ in items], [g for _, _, g, _ in items],
+                                         [s for _, _, _, s in items], radius, max_step)
+        for (b, _, _, _), g in zip(items, geos):
             geo_dists[b] = g
     return geo_dists
 

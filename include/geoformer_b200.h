@@ -137,6 +137,22 @@ int gf_geodesic(const float *knn_dist, const void *knn_idx, int idx_is_i64, int 
                 float radius, int max_step, float *geo, int64_t *stats, float *row_max, void *workspace,
                 size_t workspace_bytes, void *stream);
 
+/* A BATCH of B <= 32 scenes over the caller's own kNN graphs (e.g. a faiss index's): scene b's geo[b] (Q,Ns[b]),
+ * row_max[b] and stats row b are bit-identical to what gf_geodesic gives for knn_dist[b] (Ns[b],k),
+ * knn_idx[b] (Ns[b],k) and seeds[b] (Q) alone.  The pointer ARRAYS live in host memory, what they point to in device
+ * memory; row_max (the array) and stats (device (B,2) i64) are optional, as in gf_guidance_batch.  Seven kernels
+ * whatever B: the kNN grids of all scenes are built (no query), every edge table is packed in its grid's cell order
+ * by one launch, and one propagation launch runs all (scene, seed) pairs.
+ * xyz[b] (Ns[b],3) only chooses that numbering: the maps do not depend on it.  Any finite (Ns[b],3) array gives the
+ * same maps, the scene's own points give them fastest (a frontier then touches a few dense runs of the table).
+ * 1 <= k <= 256; every scene needs Ns[b] >= 1 and must fit the on-chip bitmaps of the batched kernel (N <~ 900k):
+ * otherwise the call returns GF_ERR_INVALID having enqueued nothing, and such scenes go through gf_geodesic.     */
+size_t gf_geodesic_batch_workspace_bytes(const int *Ns, int B, int Q, int k);
+int gf_geodesic_batch(const float *const *xyz, const float *const *knn_dist, const void *const *knn_idx,
+                      int idx_is_i64, const int *Ns, int B, int k, const int *const *seeds, int Q, float radius,
+                      int max_step, float *const *geo, float *const *row_max, int64_t *stats,
+                      void *workspace, size_t workspace_bytes, void *stream);
+
 /* ---- distance -> bias epilogues ------------------------------------------------------------- */
 
 /* decoder relative-position bias (geoformer_fs.py:680-702):
