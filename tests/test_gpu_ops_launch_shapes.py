@@ -133,6 +133,7 @@ REGIMES = {
     ("bias_mask_write_kernel<true>", "past two passes"),
     ("bias_mask_write_kernel<false>", "past two passes"),
     ("group_mlp_pool_kernel<1>", "past two passes"),
+    ("group_mlp_pool_kernel<2>", "past two passes"),
     ("group_mlp_pool_kernel<3>", "past two passes"),
     ("group_mlp_pool_kernel<4>", "past two passes"),
     ("knn_brute_kernel<64>", "k in 33..64"),
@@ -143,9 +144,9 @@ _KERNELS = sorted({k.split("<")[0] for k, _ in REGIMES} | {"bias_init_kernel", "
                                                            "bias_rowmax_import_kernel"}, key=len, reverse=True)
 
 
-def _kernel_id(name):
-    """trace name (demangled or not) -> "base<args>" for the kernels above, else None"""
-    for base in _KERNELS:
+def _kernel_id(name, kernels=_KERNELS):
+    """trace name (demangled or not) -> "base<args>" for the kernels named in `kernels` (longest first), else None"""
+    for base in kernels:
         m = re.search(r"(?<![A-Za-z_])" + base + r"(?:<([^<>]*)>|I((?:L[a-z]-?\d+E)+)E)?", name)
         if m:
             if m.group(1) is not None:
@@ -157,9 +158,9 @@ def _kernel_id(name):
     return None
 
 
-def _launched(fn):
-    """fn() under the profiler -> its result and [(kernel id, grid)] of the kernels above it launched, in order; the
-    grid is read from the exported trace"""
+def _launched(fn, kernels=_KERNELS):
+    """fn() under the profiler -> its result and [(kernel id, grid)] of the kernels named in `kernels` it launched, in
+    order; the grid is read from the exported trace"""
     with torch.profiler.profile(activities=[torch.profiler.ProfilerActivity.CUDA]) as prof:
         out = fn()
         torch.cuda.synchronize()
@@ -170,7 +171,7 @@ def _launched(fn):
             events = json.load(f)["traceEvents"]
     found = []
     for e in sorted((e for e in events if str(e.get("cat", "")).lower() == "kernel"), key=lambda e: e["ts"]):
-        k = _kernel_id(e["name"])
+        k = _kernel_id(e["name"], kernels)
         if k is not None:
             found.append((k, tuple(int(v) for v in e["args"]["grid"])))
     return out, found
@@ -778,7 +779,7 @@ def test_mask_head_every_row_unreachable(dev, sms):
 # ------------------------------------------------------------------------------------------ inference aggregator
 @pytest.mark.gpu
 @pytest.mark.parametrize("work", ["one more than a pass", "past two passes"])
-@pytest.mark.parametrize("L", [1, 3, 4])
+@pytest.mark.parametrize("L", [1, 2, 3, 4])
 def test_aggregator_grid_stride(oracle_lib, dev, sms, L, work):
     """against the float64 oracle; every scene of the batch equals a call on that scene alone, bit for bit (a warp's
     arithmetic does not depend on the grid)"""
@@ -800,7 +801,7 @@ def test_aggregator_grid_stride(oracle_lib, dev, sms, L, work):
     else:
         assert launch[1] == launch[2] + 1
     N, Cf, ns, radius = 20000, 16, 16, 0.2
-    widths = {1: [19, 32], 3: [19, 32, 32, 32], 4: [19, 32, 24, 32, 17]}[L]
+    widths = {1: [19, 32], 2: [19, 32, 32], 3: [19, 32, 32, 32], 4: [19, 32, 24, 32, 17]}[L]
     xyz = torch.stack([scene(N, 40 + b) for b in range(B)]).to(dev)
     pick = torch.stack([torch.randperm(N, generator=torch.Generator().manual_seed(b))[:m] for b in range(B)])
     new_xyz = torch.stack([xyz[b, pick[b].to(dev)] for b in range(B)]).contiguous()
